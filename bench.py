@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- smooth Cooper-Frye spectra throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg3|cfg2|cfg4ce]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg3|cfg2|cfg4ce] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A "step" is one pass of the hot path (prepare + spectra kernel + chunk reduction [+ all-reduce]) over the whole synthetic
@@ -63,7 +63,29 @@ def parse():
     ap.add_argument("--single-process", action="store_true",
                     help="--gpus N > 1 without torchrun: ONE process drives N GPUs through is3d_b200_smooth_spectra_multi "
                          "(cells sharded and all-reduced inside the C ABI, host arrays in and out)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float64), so that two "
+                         "builds can be compared output for output on the same seeded inputs")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; the reference arm only times a CPU sample")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory, arrays):
+    """arrays: {name: array} as the timed call returned them (the spectra are flat [y][phi][pT][species], 39 MB for 305 species)."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(directory, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(directory, k + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -285,6 +307,8 @@ def run_single_process(args):
         sts.append(step())
     dt = time.perf_counter() - t0
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"dN": out})
     # the same surface on one device of the same process: bin-by-bin parity of the sharded result
     single = np.zeros(n_bins)
     api.smooth_spectra(fl, {k: v[:min(n_cells, 100_000)] for k, v in host.items()}, sp, g, tab, gla, out=single)
@@ -407,7 +431,16 @@ def main():
             dist.all_reduce(t, op=dist.ReduceOp.SUM)
             flat = t.cpu().numpy()
         last["flat"] = flat; last["dN_dy"] = flat[-len(sp["mass"]):]
+        last["shapes"] = [res[k].shape for k in st_keys]
         return st
+
+    def step_outputs():
+        """what a caller of the timed call receives from the last step: the spectra, or the (all-reduced) histograms"""
+        if not spacetime:
+            return {"dN": out.cpu().numpy()}
+        sizes = [int(np.prod(s)) for s in last["shapes"]]
+        parts = np.split(last["flat"], np.cumsum(sizes)[:-1])
+        return {k: p.reshape(s) for k, p, s in zip(st_keys, parts, last["shapes"])}
 
     def step_device():
         if spacetime:
@@ -442,6 +475,8 @@ def main():
     sync_all()
     clocks = sampler.stop() if sampler else None
     ms_total = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:                # before the untimed repetitions and the e2e leg below recompute them
+        dump_outputs(args.dump_outputs, step_outputs())
     if sampler and world == 1 and clocks.get("sm_mhz") is None:
         # the timed region is shorter than nvidia-smi's sampling period (cfg2: 57 ms per step): sample the clocks while the same
         # steps repeat, untimed, for 1.5 s

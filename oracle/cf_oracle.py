@@ -266,7 +266,7 @@ def run_reference(workdir, what="kernel", omp=False, threads=None, timeout=3600)
     """Run oracle/_ref/is3d_ref inside `workdir`; returns (dN flat, info dict incl. seconds, mcid, breakdown)."""
     exe = ref_binary(omp)
     if exe is None:
-        raise FileNotFoundError("oracle/_ref not built (run `make -C oracle ref` where /root/reference exists)")
+        raise FileNotFoundError("oracle/_ref not built (run `make -C oracle ref` with REF or IS3D_REFERENCE naming an iS3D checkout)")
     env = dict(os.environ)
     if threads:
         env["OMP_NUM_THREADS"] = str(threads)
@@ -295,7 +295,7 @@ def run_vah_reference(aL, Lambda_GeV, fixture=None):
     from is3d_b200 import workdir
     exe = os.path.join(_HERE, "_ref", "vah_ref")
     if not os.path.exists(exe):
-        raise FileNotFoundError("oracle/_ref/vah_ref not built (run `make -C oracle ref` where /root/reference exists)")
+        raise FileNotFoundError("oracle/_ref/vah_ref not built (run `make -C oracle ref` with REF or IS3D_REFERENCE naming an iS3D checkout)")
     aL = np.ascontiguousarray(aL, dtype=np.float64); Lam = np.ascontiguousarray(Lambda_GeV, dtype=np.float64)
     with tempfile.TemporaryDirectory() as wd:
         workdir.materialize(wd, fixture=fixture, vah=True, operation=1, mode=2, hrg_eos=1, dimension=3, df_mode=1)
@@ -345,7 +345,7 @@ def run_reference_decays(workdir_path, dN_in, timeout=3600):
     materialised working directory; returns (amended spectra, info)."""
     exe = os.path.join(_HERE, "_ref", "is3d_ref_decays")
     if not os.path.exists(exe):
-        raise FileNotFoundError("oracle/_ref/is3d_ref_decays not built (run `make -C oracle ref` where /root/reference exists)")
+        raise FileNotFoundError("oracle/_ref/is3d_ref_decays not built (run `make -C oracle ref` with REF or IS3D_REFERENCE naming an iS3D checkout)")
     np.ascontiguousarray(dN_in, dtype=np.float64).tofile(os.path.join(workdir_path, "input", "spectra_in.bin"))
     out = os.path.join(workdir_path, "results", "dN_decays.bin")
     r = subprocess.run([exe, "decays", out], cwd=workdir_path, capture_output=True, text=True, timeout=timeout)

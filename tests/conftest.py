@@ -24,7 +24,7 @@ _LIB_PROBLEM = None
 
 @pytest.fixture(scope="session", autouse=True)
 def _built():
-    """Build the checkers (C oracle; the reference binaries where /root/reference exists are built by __graft_entry__.build) and,
+    """Build the checkers (C oracle; the reference binaries, where IS3D_REFERENCE names an iS3D checkout, are built by __graft_entry__.build) and,
     when nvcc is available, the product library.  Without a CUDA toolkit the oracle / sharding tests still run; the tests that load
     libis3d_b200.so are skipped with a message instead of failing (ADVICE r1)."""
     global _LIB_PROBLEM

@@ -38,8 +38,6 @@ def _full(arr, g, ns):
 @pytest.mark.parametrize("name", ["2d", "3d", "3d_full"])
 def test_oracle_matches_reference_vectors(fx, name):
     rec, dN_in, dN_out, _, mcid = _load(name)
-    if name == "3d_full" and not os.environ.get("IS3D_SLOW_TESTS"):
-        pytest.skip("20 s of oracle time; covered on the GPU tier (set IS3D_SLOW_TESTS=1 to run here)")
     g, tabs, cols, dN, pdg, chosen_idx = mdv.case_inputs(fx, rec)
     assert list(mcid) == rec["chosen"]
     plane = dN_in.size

@@ -40,7 +40,7 @@ def test_histograms_are_consistent(fx):
     np.testing.assert_allclose(yields, out["dN_dy"], rtol=1e-12)
 
 
-@pytest.mark.skipif(cfo.ref_binary() is None, reason="oracle/_ref not built (needs /root/reference)")
+@pytest.mark.skipif(cfo.ref_binary() is None, reason="oracle/_ref not built (needs IS3D_REFERENCE, see oracle/Makefile)")
 @pytest.mark.parametrize("dimension,df_mode,n_cells,stress", [(3, 2, 30, False), (3, 3, 30, True), (2, 4, 8, False)])
 def test_reference_binary_agrees(fx, dimension, df_mode, n_cells, stress):
     bins = dict(tau_min=1.0, tau_max=10.0, tau_bins=9, r_min=2.0, r_max=11.0, r_bins=3)      # cells fall outside on both sides

@@ -8,7 +8,7 @@ from common import jonah_tables
 from is3d_b200 import synthetic, tables, workdir
 from oracle import cf_oracle as cfo
 
-pytestmark = pytest.mark.skipif(cfo.ref_binary() is None, reason="oracle/_ref not built (needs /root/reference)")
+pytestmark = pytest.mark.skipif(cfo.ref_binary() is None, reason="oracle/_ref not built (needs IS3D_REFERENCE, see oracle/Makefile)")
 
 
 @pytest.mark.parametrize("dimension,df_mode,n_cells,stress", [(3, 1, 24, False), (3, 3, 24, True), (3, 4, 24, False), (2, 2, 6, False)])
