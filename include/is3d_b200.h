@@ -190,6 +190,31 @@ typedef struct {
 int is3d_b200_resonance_decays(const is3d_particle_list *particles, int32_t n_chosen, const int32_t *chosen_pdg_index,
                                const is3d_grid *grid, int32_t dimension, const is3d_options *options, double *dN, is3d_stats *stats);
 
+/* ---- spin polarization of hadrons from thermal vorticity (mode 5 surfaces) -------------------------------------------
+ * Mean spin vector of the emitted hadrons at freeze-out (Becattini et al. 2013; Karpenko & Becattini 2017), f_eq only (no delta-f):
+ *    Snorm(p) = g/(2 pi hbar c)^3 sum_cells sum_slots w p.dsigma f,                      f = 1 / (exp(p.u/T) + sign)
+ *    N^mu(p)  = g/(2 pi hbar c)^3 sum_cells sum_slots w p.dsigma f (1 - sign f) (-1/(8m)) eps^{mu rho sigma tau} varpi_{rho sigma} p_tau
+ *    S^mu(p)  = N^mu / Snorm (mean spin vector; rest frame S*_i = S^i - S^t p^i / (E + m), for spin 1/2 P* = 2 S*)
+ * Cells, slots and weights w are those of the ideal-f spectra (u.dsigma <= 0 skipped, Theta(p.dsigma) with outflow = 1, 3+1D: y table at
+ * the cell's eta, 2+1D: y = 0 and the eta quadrature), so Snorm is bin for bin the ideal spectrum.  Components are Cartesian lab
+ * components (t, x, y, z), p^mu = (mT cosh y, pT cos phi, pT sin phi, mT sinh y), eps^{txyz} = +1.
+ * Input: the six vorticity columns of a mode-5 surface, in file order the covariant Milne components varpi_{tau x}, varpi_{tau y},
+ * varpi_{tau eta}, varpi_{xy}, varpi_{x eta}, varpi_{y eta} of varpi_{mu nu} = -(1/2)(d_mu beta_nu - d_nu beta_mu), beta = u/T
+ * (dimensionless); they are converted to Cartesian components at the cell's eta (2+1D: the slot's eta) in cf_polzn.cu, cart_vorticity().
+ * The five result arrays have the spectra layout ipart + n_species*(ipT + n_pT*(iphi + n_phi*iy)), hold the RAW sums N^mu and Snorm
+ * (they add across cell shards and devices; the ratio S^mu does not) and are ADDED into; host or device memory per options->memory.
+ * Errors: IS3D_ERR_UNSUPPORTED for mode = 2 and include_baryon = 1; IS3D_ERR_ARGUMENT for a NULL vorticity or a species with m <= 0.
+ * Only the surface arrays tau, eta, dat, dax, day, dan, ux, uy, un, T are read; df_mode and the delta-f switches do not enter. */
+typedef struct { const double *wtx, *wty, *wtn, *wxy, *wxn, *wyn; } is3d_vorticity;
+typedef struct { double *St, *Sx, *Sy, *Sz, *Snorm; } is3d_polarization_result;
+int is3d_b200_spin_polarization(const is3d_flags *flags, const is3d_surface *surface, const is3d_vorticity *vorticity,
+                                const is3d_species *species, const is3d_grid *grid, const is3d_options *options,
+                                is3d_polarization_result *result, is3d_stats *stats);
+/* Same over the devices of is3d_b200_init_devices(): HOST arrays, contiguous cell shards, the five arrays summed on the host. */
+int is3d_b200_spin_polarization_multi(const is3d_flags *flags, const is3d_surface *surface, const is3d_vorticity *vorticity,
+                                      const is3d_species *species, const is3d_grid *grid, const is3d_options *options,
+                                      is3d_polarization_result *result, is3d_stats *stats);
+
 /* FP64 FMA peak of the current device measured with a dependency-free DFMA chain (the roofline denominator;
  * MEASURED_PEAKS.json carries no FP64 figure).  Returns TFLOP/s in *tflops, SM clock not touched. */
 int is3d_b200_measure_fp64_peak(double *tflops, double *ms);

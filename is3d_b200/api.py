@@ -439,3 +439,77 @@ def resonance_decays(pdg, chosen_pdg_index, grid, dimension, dN, memory="host", 
     f.argtypes = [C.POINTER(ParticleList), C.c_int32, C.POINTER(C.c_int32), C.POINTER(Grid), C.c_int32, C.POINTER(Options), C.c_void_p, C.POINTER(Stats)]
     _check(f(C.byref(p), len(chosen_pdg_index), ia(chosen_pdg_index), C.byref(g), int(dimension), C.byref(opt), ptr, C.byref(st)))
     return out, st.as_dict()
+
+
+VORTICITY_FIELDS = ("wtx", "wty", "wtn", "wxy", "wxn", "wyn")
+POLARIZATION_FIELDS = ("St", "Sx", "Sy", "Sz", "Snorm")
+
+
+class Vorticity(C.Structure):
+    _fields_ = [(k, _D) for k in VORTICITY_FIELDS]
+
+
+class PolarizationResult(C.Structure):
+    _fields_ = [(k, _D) for k in POLARIZATION_FIELDS]
+
+
+def spin_polarization(flags, cells, vorticity, species, grid, memory="host", stream=None, multi=False):
+    """Call is3d_b200_spin_polarization (or the _multi entry point over the devices of init_devices(), host arrays only).
+
+    vorticity: dict wtx, wty, wtn, wxy, wxn, wyn -- the six thermal-vorticity columns of a mode-5 surface (covariant Milne components,
+    dimensionless), numpy for memory='host', float64 CUDA tensors for memory='device'.  Returns (dict St, Sx, Sy, Sz, Snorm of RAW sums,
+    flat [y][phi][pT][species], numpy or CUDA tensors; stats dict).  mean_spin() turns them into the mean spin vector."""
+    device = (memory == "device")
+    m = _Marshal(device)
+    sf, sp, g, _, _ = _marshal_problem(m, cells, species, grid, None, None)
+    vo = None
+    if vorticity is not None:
+        vo = Vorticity()
+        for k in VORTICITY_FIELDS:
+            setattr(vo, k, m.cells(vorticity[k]))
+    n = sp.n * g.n_pT * g.n_phi * g.n_y
+    res = PolarizationResult()
+    if device:
+        import torch
+        out = {k: torch.zeros(n, dtype=torch.float64, device=cells["tau"].device) for k in POLARIZATION_FIELDS}
+        for k in POLARIZATION_FIELDS:
+            setattr(res, k, C.cast(C.c_void_p(out[k].data_ptr()), _D))
+        if stream is None:
+            stream = torch.cuda.current_stream().cuda_stream
+    else:
+        out = {k: np.zeros(n) for k in POLARIZATION_FIELDS}
+        for k in POLARIZATION_FIELDS:
+            setattr(res, k, out[k].ctypes.data_as(_D))
+    opt = Options(); opt.memory = 1 if device else 0; opt.stream = C.c_void_p(stream or 0)
+    st = Stats()
+    fl = make_flags(flags)
+    f = lib().is3d_b200_spin_polarization_multi if multi else lib().is3d_b200_spin_polarization
+    f.restype = C.c_int
+    f.argtypes = [C.POINTER(Flags), C.POINTER(Surface), C.POINTER(Vorticity), C.POINTER(Species), C.POINTER(Grid), C.POINTER(Options),
+                  C.POINTER(PolarizationResult), C.POINTER(Stats)]
+    _check(f(C.byref(fl), C.byref(sf), C.byref(vo) if vo is not None else None, C.byref(sp), C.byref(g), C.byref(opt), C.byref(res),
+             C.byref(st)))
+    return out, st.as_dict()
+
+
+def mean_spin(result, species, grid, dimension):
+    """Mean spin vector from the raw sums of spin_polarization(): returns (S [4][n_bins] = N^mu / Snorm in lab components t, x, y, z,
+    0 where Snorm = 0; S* [3][n_bins] = S^i - S^t p^i / (E + m), the rest-frame spin, P* = 2 S* for spin 1/2).  The same numbers
+    results/polarization/S_<mcid>.dat holds."""
+    r = {k: np.asarray(result[k].cpu() if _is_torch(result[k]) else result[k], dtype=np.float64) for k in POLARIZATION_FIELDS}
+    m = np.asarray(species["mass"], dtype=np.float64)
+    pT = np.asarray(grid["pT"], dtype=np.float64); phi = np.asarray(grid["phi"], dtype=np.float64)
+    y = np.asarray(grid["y"], dtype=np.float64)
+    if dimension == 2:
+        y = np.zeros_like(y)
+    yy, ff, pp, mm = np.meshgrid(y, phi, pT, m, indexing="ij")          # [y][phi][pT][species] = the flat bin order
+    mT = np.sqrt(mm * mm + pp * pp)
+    E = (mT * np.cosh(yy)).ravel()
+    p = np.stack([(pp * np.cos(ff)).ravel(), (pp * np.sin(ff)).ravel(), (mT * np.sinh(yy)).ravel()])
+    sn = r["Snorm"]
+    nz = sn != 0
+    S = np.zeros((4, sn.size))
+    for i, k in enumerate(("St", "Sx", "Sy", "Sz")):
+        S[i, nz] = r[k][nz] / sn[nz]
+    rest = S[1:] - S[0] * p / (E + mm.ravel())
+    return S, rest

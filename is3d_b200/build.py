@@ -25,6 +25,7 @@ SOURCES = [
     ("cf_decays.cu", ["-fmad=false"]),
     ("cf_strict.cu", ["-fmad=false"]),
     ("cf_shift.cu", []),
+    ("cf_polzn.cu", []),
     ("cf_api.cu", []),
     ("host_math.cpp", []),
     ("host_io.cpp", []),

@@ -1158,3 +1158,218 @@ extern "C" int is3d_b200_spacetime_distributions_multi(const is3d_flags *fl, con
   }
   return IS3D_OK;
 }
+
+// =====================================================================================================================
+// Spin polarization from thermal vorticity (cf_polzn.cu): raw sums N^mu and Snorm, added into the caller's five arrays
+// =====================================================================================================================
+namespace is3d {
+
+static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_vorticity *vo, const is3d_species *sp, const is3d_grid *gr,
+                      const is3d_options *opt_in, is3d_polarization_result *res, is3d_stats *stats)
+{
+  if (!fl || !sf || !sp || !gr || !res) return fail(IS3D_ERR_ARGUMENT, "NULL argument");
+  if (!vo) return fail(IS3D_ERR_ARGUMENT, "NULL vorticity");
+  if (!res->St || !res->Sx || !res->Sy || !res->Sz || !res->Snorm) return fail(IS3D_ERR_ARGUMENT, "NULL result array");
+  if (fl->mode == 2) return fail(IS3D_ERR_UNSUPPORTED, "spin polarization needs a viscous-hydro surface with thermal vorticity (mode 5), not mode 2");
+  if (fl->include_baryon) return fail(IS3D_ERR_UNSUPPORTED, "include_baryon = 1 (the reference's (T, muB) lookup reads out of bounds, SURVEY R8)");
+  if (fl->dimension != 2 && fl->dimension != 3) return fail(IS3D_ERR_ARGUMENT, "dimension must be 2 or 3");
+  if (sp->n <= 0 || gr->n_pT <= 0 || gr->n_phi <= 0 || gr->n_y <= 0) return fail(IS3D_ERR_ARGUMENT, "empty species list or momentum table");
+  if (!sp->mass || !sp->sign || !sp->degeneracy || !gr->pT || !gr->phi || !gr->y) return fail(IS3D_ERR_ARGUMENT, "NULL species or momentum table");
+  for (int s = 0; s < sp->n; s++) if (!(sp->mass[s] > 0.0)) return fail(IS3D_ERR_ARGUMENT, "spin polarization needs species with mass > 0");
+  const bool dim2 = (fl->dimension == 2);
+  if (dim2 && (gr->n_eta <= 0 || !gr->eta || !gr->eta_weight)) return fail(IS3D_ERR_ARGUMENT, "dimension = 2 needs the eta table");
+  const int64_t n_cells = sf->n_cells;
+  if (n_cells < 0) return fail(IS3D_ERR_ARGUMENT, "negative cell count");
+  const double *raw_src[15] = {sf->tau, sf->eta, sf->dat, sf->dax, sf->day, sf->dan, sf->ux, sf->uy, sf->un, sf->T,
+                               vo->wtx, vo->wty, vo->wtn, vo->wxy, vo->wxn};
+  for (const double *p : raw_src) if (!p && n_cells > 0) return fail(IS3D_ERR_ARGUMENT, "a required surface or vorticity array is NULL");
+  if (!vo->wyn && n_cells > 0) return fail(IS3D_ERR_ARGUMENT, "a required surface or vorticity array is NULL");
+  Device *Dp = nullptr;
+  { int rc = current_device(&Dp); if (rc) return rc; }
+  Workspace &ws = Dp->ws;
+  std::lock_guard<std::mutex> lk(Dp->mu);
+  is3d_options opt; memset(&opt, 0, sizeof(opt));
+  if (opt_in) opt = *opt_in;
+  cudaStream_t st = (cudaStream_t)opt.stream;
+  const int64_t n_bins = (int64_t)sp->n * gr->n_pT * gr->n_phi * gr->n_y;
+  const int64_t n_active = dim2 ? n_bins / gr->n_y : n_bins;        // 2+1D fills the y = 0 plane (index iy = 0)
+
+  // ---- layout: the cf_kernel decomposition with the register tile of cf_polzn_kernel
+  Layout L; memset(&L, 0, sizeof(L));
+  L.n_species = sp->n; L.n_pT = gr->n_pT; L.n_phi = gr->n_phi; L.n_y_out = gr->n_y;
+  L.dim2 = dim2 ? 1 : 0;
+  L.n_slots = dim2 ? gr->n_eta : gr->n_y;
+  L.rec_y = kPolRecY;
+  int nyt, npt, ct;
+  polzn_shape(L.dim2, &nyt, &npt, &ct);
+  L.nst = dim2 ? L.n_slots : nyt;
+  L.n_ytiles = dim2 ? 1 : (L.n_slots + nyt - 1) / nyt;
+  L.npt = npt; L.n_ptiles = (L.n_phi + npt - 1) / npt;
+  L.ct = ct; L.n_cells = n_cells;
+  L.n_tiles = (n_cells + ct - 1) / ct;
+  L.n_cells_pad = L.n_tiles * ct;
+  const int n_groups = (sp->n * gr->n_pT + 31) / 32;
+  const int n_warps = std::min(kPolWarps, n_groups);
+  const int n_groupblocks = (n_groups + n_warps - 1) / n_warps;
+  const int64_t n_bintiles = (int64_t)n_groupblocks * L.n_ytiles * L.n_ptiles;
+  // chunks: the rule of smooth_core (>= 192 blocks per SM, a chunk's records within a third of L2, partial sums <= 4 GiB)
+  int64_t n_chunks = ((int64_t)Dp->sm_count * 192 + n_bintiles - 1) / n_bintiles;
+  const int64_t rec_per_cell = ((int64_t)L.n_ytiles * L.nst * kPolRecY + (int64_t)L.n_ptiles * L.npt * kPolRecP) * 8;
+  const int64_t l2_target = std::max<int64_t>((int64_t)Dp->l2_bytes / 3, (int64_t)8 << 20);
+  n_chunks = std::max<int64_t>(n_chunks, (n_cells * rec_per_cell + l2_target - 1) / l2_target);
+  const int64_t n_chunks_wanted = n_chunks;
+  n_chunks = std::min<int64_t>(n_chunks, std::max<int64_t>(1, ((int64_t)4 << 30) / (5 * n_bins * 8)));
+  if (opt.n_chunks > 0) n_chunks = opt.n_chunks;
+  n_chunks = std::max<int64_t>(1, std::min<int64_t>(n_chunks, std::max<int64_t>(L.n_tiles, 1)));
+  if (n_bintiles * n_chunks > 2147483647LL) return fail(IS3D_ERR_ARGUMENT, "grid too large");
+
+  // ---- tables and surface to the device
+  SmallArena ar;
+  std::vector<double> cosphi(gr->n_phi), sinphi(gr->n_phi);
+  for (int k = 0; k < gr->n_phi; k++) { cosphi[k] = cos(gr->phi[k]); sinphi[k] = sin(gr->phi[k]); }
+  const size_t o_mass = ar.put(sp->mass, sp->n), o_sign = ar.put(sp->sign, sp->n), o_deg = ar.put(sp->degeneracy, sp->n);
+  const size_t o_pT = ar.put(gr->pT, gr->n_pT), o_cos = ar.put(cosphi.data(), gr->n_phi), o_sin = ar.put(sinphi.data(), gr->n_phi);
+  const size_t o_sloty = dim2 ? ar.put(gr->eta, gr->n_eta) : ar.put(gr->y, gr->n_y);
+  const size_t o_slotw = dim2 ? ar.put(gr->eta_weight, gr->n_eta) : 0;
+  const double *srcs[16] = {sf->tau, sf->eta, sf->dat, sf->dax, sf->day, sf->dan, sf->ux, sf->uy, sf->un, sf->T,
+                            vo->wtx, vo->wty, vo->wtn, vo->wxy, vo->wxn, vo->wyn};
+  const size_t cell_stride = ((size_t)n_cells * 8 + 255) & ~(size_t)255;
+  CU_CHECK(ws.small.reserve(ar.host.size() + 256));
+  CU_CHECK(ws.Y.reserve((size_t)L.n_ytiles * L.n_cells_pad * L.nst * kPolRecY * 8 + 256));
+  CU_CHECK(ws.P.reserve((size_t)L.n_ptiles * L.n_cells_pad * L.npt * kPolRecP * 8 + 256));
+  CU_CHECK(ws.partial.reserve((size_t)5 * n_chunks * n_bins * 8 + 256));
+  CU_CHECK(ws.dN.reserve((size_t)5 * n_bins * 8 + 256));
+  CU_CHECK(ws.counters.reserve(256));
+  if (opt.memory == 0) CU_CHECK(ws.raw.reserve(cell_stride * 16 + 256));
+
+  cudaEvent_t *ev = ws.ev;
+  CU_CHECK(cudaEventRecord(ev[0], st));
+  unsigned char *small_d = ws.small.as<unsigned char>();
+  CU_CHECK(cudaMemcpyAsync(small_d, ar.host.data(), ar.host.size(), cudaMemcpyHostToDevice, st));
+  const double *dev[16];
+  for (int a = 0; a < 16; a++) {
+    dev[a] = srcs[a];
+    if (opt.memory == 0) {
+      double *d = reinterpret_cast<double *>(ws.raw.as<unsigned char>() + cell_stride * a);
+      if (n_cells > 0) CU_CHECK(cudaMemcpyAsync(d, srcs[a], (size_t)n_cells * 8, cudaMemcpyHostToDevice, st));
+      dev[a] = d;
+    }
+  }
+  RawCells rc; memset(&rc, 0, sizeof(rc));
+  rc.n = n_cells; rc.tau = dev[0]; rc.eta = dev[1]; rc.dat = dev[2]; rc.dax = dev[3]; rc.day = dev[4]; rc.dan = dev[5];
+  rc.ux = dev[6]; rc.uy = dev[7]; rc.un = dev[8]; rc.T = dev[9];
+  const VortCells vc{dev[10], dev[11], dev[12], dev[13], dev[14], dev[15]};
+  double *sums_d = ws.dN.as<double>();                         // [5][n_bins]: Snorm, N^t, N^x, N^y, N^z
+  CU_CHECK(cudaMemsetAsync(sums_d, 0, (size_t)5 * n_bins * 8, st));
+  CU_CHECK(cudaMemsetAsync(ws.counters.p, 0, sizeof(PrepCounters), st));
+  CU_CHECK(cudaEventRecord(ev[1], st));
+
+  auto dptr = [&](size_t off) { return reinterpret_cast<const double *>(small_d + off); };
+  PrepTables tab; memset(&tab, 0, sizeof(tab));
+  tab.cosphi = dptr(o_cos); tab.sinphi = dptr(o_sin); tab.slot_y = dptr(o_sloty); tab.slot_w = dim2 ? dptr(o_slotw) : nullptr;
+  PrepCounters *cnt_d = ws.counters.as<PrepCounters>();
+  CU_CHECK(launch_prepare_polzn(rc, vc, tab, L, ws.Y.as<double>(), ws.P.as<double>(), cnt_d, st));
+  CU_CHECK(cudaEventRecord(ev[2], st));
+
+  HotParams hp; memset(&hp, 0, sizeof(hp));
+  hp.L = L; hp.Y = ws.Y.as<double>(); hp.P = ws.P.as<double>();
+  hp.mass = dptr(o_mass); hp.sign = dptr(o_sign); hp.degeneracy = dptr(o_deg); hp.pT = dptr(o_pT);
+  hp.partial = ws.partial.as<double>();
+  hp.n_chunks = (int)n_chunks; hp.n_groupblocks = n_groupblocks; hp.n_warps = n_warps;
+  hp.outflow_thr = fl->outflow ? 0LL : (long long)0x8000000000000000ULL;
+  hp.prefactor = pow(2.0 * M_PI * 0.197327053, -3);
+  CU_CHECK(launch_polzn(hp, st));
+  CU_CHECK(cudaEventRecord(ev[3], st));
+  for (int q = 0; q < 5; q++)
+    CU_CHECK(launch_reduce(hp.partial + (size_t)q * n_chunks * n_bins, (int)n_chunks, n_bins, n_active, sums_d + (size_t)q * n_bins, st));
+  CU_CHECK(cudaEventRecord(ev[4], st));
+
+  double *out[5] = {res->Snorm, res->St, res->Sx, res->Sy, res->Sz};
+  std::vector<double> host;
+  if (opt.memory == 0) {
+    host.resize((size_t)5 * n_bins);
+    CU_CHECK(cudaMemcpyAsync(host.data(), sums_d, (size_t)5 * n_bins * 8, cudaMemcpyDeviceToHost, st));
+  } else {
+    for (int q = 0; q < 5; q++) CU_CHECK(launch_axpy(sums_d + (size_t)q * n_bins, out[q], n_active, st));
+  }
+  PrepCounters cnt; memset(&cnt, 0, sizeof(cnt));
+  CU_CHECK(cudaMemcpyAsync(&cnt, cnt_d, sizeof(cnt), cudaMemcpyDeviceToHost, st));
+  CU_CHECK(cudaEventRecord(ev[5], st));
+  CU_CHECK(cudaEventSynchronize(ev[5]));
+  if (opt.memory == 0)
+    for (int q = 0; q < 5; q++)
+      for (int64_t i = 0; i < n_bins; i++) out[q][i] += host[(size_t)q * n_bins + i];
+
+  is3d_stats stt; memset(&stt, 0, sizeof(stt));
+  float ms;
+  cudaEventElapsedTime(&ms, ev[0], ev[1]); stt.h2d_ms = ms;
+  cudaEventElapsedTime(&ms, ev[1], ev[2]); stt.prepare_ms = ms;
+  cudaEventElapsedTime(&ms, ev[2], ev[3]); stt.kernel_ms = ms;
+  cudaEventElapsedTime(&ms, ev[3], ev[4]); stt.reduce_ms = ms;
+  cudaEventElapsedTime(&ms, ev[4], ev[5]); stt.d2h_ms = ms;
+  cudaEventElapsedTime(&ms, ev[0], ev[5]); stt.total_ms = ms;
+  stt.cells_skipped_udsigma = (int64_t)cnt.skipped;
+  stt.evaluations = n_cells * (int64_t)sp->n * gr->n_pT * gr->n_phi * (int64_t)L.n_slots;
+  stt.gpu_launches = (n_cells > 0 ? 1 : 0) + 1 + 5 + (opt.memory == 0 ? 0 : 5);
+  stt.n_chunks = (int)n_chunks; stt.n_chunks_wanted = (int)n_chunks_wanted;
+  stt.n_gpus = 1;
+  if (stats) *stats = stt;
+  return IS3D_OK;
+}
+
+}  // namespace is3d
+
+extern "C" int is3d_b200_spin_polarization(const is3d_flags *fl, const is3d_surface *sf, const is3d_vorticity *vo, const is3d_species *sp,
+                                           const is3d_grid *gr, const is3d_options *opt, is3d_polarization_result *res, is3d_stats *stats)
+{
+  return polzn_core(fl, sf, vo, sp, gr, opt, res, stats);
+}
+
+// Several devices: HOST arrays, contiguous cell shards, one thread per device; the five raw sums are added on the host in device order
+extern "C" int is3d_b200_spin_polarization_multi(const is3d_flags *fl, const is3d_surface *sf, const is3d_vorticity *vo, const is3d_species *sp,
+                                                 const is3d_grid *gr, const is3d_options *opt_in, is3d_polarization_result *res, is3d_stats *stats)
+{
+  const int G = g_ngpus;
+  if (G <= 1) return is3d_b200_spin_polarization(fl, sf, vo, sp, gr, opt_in, res, stats);
+  if (!fl || !sf || !vo || !sp || !gr || !res) return fail(IS3D_ERR_ARGUMENT, vo ? "NULL argument" : "NULL vorticity");
+  if (opt_in && opt_in->memory != 0) return fail(IS3D_ERR_ARGUMENT, "the multi-GPU entry point takes host arrays");
+  std::lock_guard<std::mutex> lk(g_multi_mutex);
+  const size_t n_bins = (size_t)std::max(sp->n, 0) * std::max(gr->n_pT, 0) * std::max(gr->n_phi, 0) * std::max(gr->n_y, 0);
+  int prev = 0; cudaGetDevice(&prev);
+  std::vector<int> rcs(G, IS3D_OK);
+  std::vector<std::string> errs(G);
+  std::vector<is3d_stats> sts(G);
+  std::vector<std::vector<double>> bufs(G, std::vector<double>(5 * n_bins, 0.0));
+  std::vector<std::thread> workers;
+  for (int d = 0; d < G; d++) {
+    workers.emplace_back([&, d]() {
+      memset(&sts[d], 0, sizeof(is3d_stats));
+      if (cudaSetDevice(d) != cudaSuccess) { rcs[d] = IS3D_ERR_CUDA; errs[d] = "cudaSetDevice failed"; return; }
+      int64_t lo, hi;
+      shard_bounds(sf->n_cells, d, G, &lo, &hi);
+      const is3d_surface shard = shard_surface(*sf, lo, hi);
+      auto off = [&](const double *p) { return p ? p + lo : p; };
+      const is3d_vorticity vs{off(vo->wtx), off(vo->wty), off(vo->wtn), off(vo->wxy), off(vo->wxn), off(vo->wyn)};
+      is3d_options opt; memset(&opt, 0, sizeof(opt));
+      if (opt_in) opt = *opt_in;
+      opt.memory = 0; opt.stream = g_streams[d];
+      double *b = bufs[d].data();
+      is3d_polarization_result r{b, b + n_bins, b + 2 * n_bins, b + 3 * n_bins, b + 4 * n_bins};
+      rcs[d] = polzn_core(fl, &shard, &vs, sp, gr, &opt, &r, &sts[d]);
+      if (rcs[d]) errs[d] = g_last_error;
+    });
+  }
+  for (auto &w : workers) w.join();
+  cudaSetDevice(prev);
+  for (int d = 0; d < G; d++) if (rcs[d]) return fail(rcs[d], errs[d].c_str());
+  double *out[5] = {res->St, res->Sx, res->Sy, res->Sz, res->Snorm};
+  for (int q = 0; q < 5; q++)
+    for (size_t i = 0; i < n_bins; i++) { double v = 0.0; for (int d = 0; d < G; d++) v += bufs[d][q * n_bins + i]; out[q][i] += v; }
+  if (stats) {
+    is3d_stats tot; memset(&tot, 0, sizeof(tot));
+    for (int d = 0; d < G; d++) merge_stats(&tot, sts[d]);
+    tot.n_gpus = G;
+    *stats = tot;
+  }
+  return IS3D_OK;
+}

@@ -134,5 +134,16 @@ void shift_variant_shape(int v, int *nyt, int *npt, int *ct, int *max_warps);
 cudaError_t launch_shift(int model, const HotParams &hp, int v, cudaStream_t st, size_t *smem_out);
 // slot records of padding / skipped cells carry this A = u.p / (mT T): every evaluation is dead (exp overflows, f = 0 exactly)
 constexpr double kDeadSlotA = 1.0e6;
+// spin polarization from thermal vorticity (cf_polzn.cu): ideal-f cells and slots, 5 sums per bin (Snorm, N^t, N^x, N^y, N^z)
+struct VortCells { const double *wtx, *wty, *wtn, *wxy, *wxn, *wyn; };    // device pointers, covariant Milne components
+constexpr int kPolRecY = 12;     // doubles per slot record
+constexpr int kPolRecP = 4;      // doubles per phi record
+constexpr int kPolWarps = 4;     // warps per block (at most)
+constexpr int kPolNyt3D = 7, kPolNpt3D = 1, kPolNpt2D = 4;
+void polzn_shape(int dim2, int *nyt, int *npt, int *ct);
+cudaError_t launch_prepare_polzn(const RawCells &cells, const VortCells &vort, const PrepTables &tab, const Layout &L, double *Y, double *P,
+                                 PrepCounters *counters, cudaStream_t st);
+// partial: [5][n_chunks][n_bins]
+cudaError_t launch_polzn(const HotParams &hp, cudaStream_t st);
 
 }  // namespace is3d

@@ -229,6 +229,7 @@ bool read_surface(const std::string &workdir, const SurfaceFlags &fl, SurfaceDat
   const bool full_pi = (mode == 0 || mode == 2 || mode == 4 || mode == 6);     // formats that store all ten pi components
   if (full_pi) { rs(s->pitt); rs(s->pitx); rs(s->pity); rs(s->pitn); rs(s->pinn); }
   if (mode == 2) { rs(s->PL); rs(s->Wx); rs(s->Wy); rs(s->Lambda); rs(s->aL); rs(s->c0); rs(s->c1); rs(s->c2); rs(s->c3); rs(s->c4); }
+  if (mode == 5) { rs(s->wtx); rs(s->wty); rs(s->wtn); rs(s->wxy); rs(s->wxn); rs(s->wyn); }
 
   Tokens tk{text.data(), text.data() + text.size()};
   double Tavg = 0, Eavg = 0, Pavg = 0, muBavg = 0, nBavg = 0, volume = 0;
@@ -294,7 +295,7 @@ bool read_surface(const std::string &workdir, const SurfaceFlags &fl, SurfaceDat
           if (mode == 0 || mode == 5) rd(&skip);                                  // V^tau column
           rd(&s->Vx[i]); rd(&s->Vy[i]); rd(&s->Vn[i]);
         }
-        if (mode == 5) for (int k = 0; k < 6; k++) rd(&skip);                    // thermal vorticity, unused by this path
+        if (mode == 5) { rd(&s->wtx[i]); rd(&s->wty[i]); rd(&s->wtn[i]); rd(&s->wxy[i]); rd(&s->wxn[i]); rd(&s->wyn[i]); }   // thermal vorticity
       }
     }
     if (writes_averages) {

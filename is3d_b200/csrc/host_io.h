@@ -47,6 +47,7 @@ struct SurfaceData {
   std::vector<double> pitt, pitx, pity, pitn, pixx, pixy, pixn, piyy, piyn, pinn, bulkPi;
   std::vector<double> muB, nB, Vx, Vy, Vn;
   std::vector<double> PL, Wx, Wy, Lambda, aL, c0, c1, c2, c3, c4;     // anisotropic hydro (mode 2)
+  std::vector<double> wtx, wty, wtn, wxy, wxn, wyn;                    // thermal vorticity, covariant Milne components (mode 5)
   bool averages_written = false;
   double avg[5] = {0, 0, 0, 0, 0};   // T, E, P, muB, nB after the 15-digit text round trip of the side file
 };

@@ -176,11 +176,51 @@ static bool write_spacetime_files(const std::string &wd, const std::vector<int> 
   return true;
 }
 
+// results/polarization/S_<mcid>.dat: mean spin vector S^mu = N^mu / Snorm (lab frame, Cartesian t, x, y, z; 0 where Snorm = 0) and its
+// rest-frame spatial part S*_i = S^i - S^t p^i / (E + m), one row per (y, phi, pT) in the loop order, number format and blank line per
+// phi block of write_spectra_files; truncating opens, results/polarization/ must exist
+static bool write_polarization_files(const std::string &wd, const std::vector<double> &sums, const std::vector<int> &mcid,
+                                     const std::vector<double> &mass, const Grids &g, int dimension, std::string *err)
+{
+  const int npart = (int)mcid.size(), npT = (int)g.pT.rows, nphi = (int)g.phi.rows, ny = (int)g.y.rows;
+  const int y_pts = (dimension == 2) ? 1 : ny;
+  const size_t n_bins = (size_t)npart * npT * nphi * ny;
+  const double *St = &sums[0], *Sx = St + n_bins, *Sy = Sx + n_bins, *Sz = Sy + n_bins, *Sn = Sz + n_bins;
+  for (int ipart = 0; ipart < npart; ipart++) {
+    char name[255];
+    std::snprintf(name, sizeof(name), "%s/results/polarization/S_%d.dat", wd.c_str(), mcid[ipart]);
+    std::ofstream f(name, std::ios_base::out);
+    if (!f) { *err = std::string("cannot open ") + name + " (the directory results/polarization/ must exist)"; return false; }
+    f << "y\tphip\tpT\tSnorm\tSt\tSx\tSy\tSz\tSx_rest\tSy_rest\tSz_rest\n";
+    const double m = mass[ipart];
+    for (int iy = 0; iy < y_pts; iy++) {
+      const double y = (dimension == 2) ? 0.0 : g.y.at(1, iy + 1);
+      for (int iphi = 0; iphi < nphi; iphi++) {
+        const double phi = g.phi.at(1, iphi + 1);
+        for (int ipT = 0; ipT < npT; ipT++) {
+          const double pT = g.pT.at(1, ipT + 1), mT = std::sqrt(m * m + pT * pT);
+          const double E = mT * std::cosh(y), p[3] = {pT * std::cos(phi), pT * std::sin(phi), mT * std::sinh(y)};
+          const size_t b = (size_t)bin_index(ipart, npart, ipT, npT, iphi, nphi, iy);
+          double S[4] = {0.0, 0.0, 0.0, 0.0};
+          if (Sn[b] != 0.0) { S[0] = St[b] / Sn[b]; S[1] = Sx[b] / Sn[b]; S[2] = Sy[b] / Sn[b]; S[3] = Sz[b] / Sn[b]; }
+          f << std::scientific << std::setw(5) << std::setprecision(8) << y << "\t" << phi << "\t" << pT << "\t" << Sn[b];
+          for (int k = 0; k < 4; k++) f << "\t" << S[k];
+          for (int k = 0; k < 3; k++) f << "\t" << S[k + 1] - S[0] * p[k] / (E + m);
+          f << "\n";
+        }
+        f << "\n";
+      }
+    }
+  }
+  return true;
+}
+
 // everything the host layer derives from the input files
 struct Problem {
   Params par;
   is3d_flags fl;
   int operation = 0, hrg_eos = 0, group_particles = 0, do_resonance_decays = 0;
+  int spin_polarization = 0;               // optional key (absent: 0): mode-5 spin polarization after the spectra
   std::vector<int> pick;                   // particle-list index of every chosen species (chosen_particles_sampling_table)
   SurfaceData sf;
   std::vector<Particle> pdg;
@@ -220,6 +260,8 @@ static int load_problem(const std::string &wd, bool need_surface, Problem *p, st
   if (p->operation == 0 && fl.mode == 2) { err = "operation = 0 has no anisotropic-hydro routine in the reference (emissionfunction.cpp:1644-1673)"; return IS3D_ERR_UNSUPPORTED; }
   p->do_resonance_decays = (int)par.get("do_resonance_decays", &err);
   if (p->do_resonance_decays && p->operation != 1) { err = "do_resonance_decays = 1 applies to operation = 1 (the reference runs it after the spectra, emissionfunction.cpp:1689)"; return IS3D_ERR_UNSUPPORTED; }
+  p->spin_polarization = par.has("spin_polarization") ? (int)par.get("spin_polarization", &err) : 0;
+  if (p->spin_polarization && (p->operation != 1 || fl.mode != 5)) { err = "spin_polarization = 1 needs operation = 1 and a mode 5 surface (the thermal vorticity columns)"; return IS3D_ERR_UNSUPPORTED; }
   if (p->do_resonance_decays && p->hrg_eos == 3) { err = "do_resonance_decays = 1 needs a particle list with decay tables (hrg_eos = 1, 2); pdg_box.dat has none"; return IS3D_ERR_UNSUPPORTED; }
 
   // ---- surface (+ averages side file)
@@ -268,7 +310,7 @@ static int load_problem(const std::string &wd, bool need_surface, Problem *p, st
   return IS3D_OK;
 }
 
-static int run_problem(const std::string &wd, Problem &P, const is3d_surface &s, double *dN_raw, int64_t n_raw, int32_t *mcid_out,
+static int run_problem(const std::string &wd, Problem &P, const is3d_surface &s, const is3d_vorticity *vort, double *dN_raw, int64_t n_raw, int32_t *mcid_out,
                        int32_t n_mcid_max, is3d_stats *stats, std::string *err_out)
 {
   std::string &err = *err_out;
@@ -330,6 +372,15 @@ static int run_problem(const std::string &wd, Problem &P, const is3d_surface &s,
     std::cout << std::setw(5) << std::setprecision(4) << "\nfeqmod breaks down for " << st.cells_feqmod_breakdown << " cells\n" << std::endl;
   if (mcid_out) for (int i = 0; i < npart && i < n_mcid_max; i++) mcid_out[i] = P.mcid[i];
   if (!write_spectra_files(wd, dN, P.mcid, g, P.fl.dimension, &err)) return IS3D_ERR_IO;
+  if (P.spin_polarization) {
+    std::vector<double> sums(5 * n_bins, 0.0);                   // St | Sx | Sy | Sz | Snorm
+    is3d_polarization_result r{&sums[0], &sums[n_bins], &sums[2 * n_bins], &sums[3 * n_bins], &sums[4 * n_bins]};
+    is3d_stats sp_st; std::memset(&sp_st, 0, sizeof(sp_st));
+    const int rcp = is3d_b200_spin_polarization_multi(&P.fl, &s, vort, &sp, &gr, nullptr, &r, &sp_st);
+    if (rcp != IS3D_OK) { err = std::string("spin polarization failed: ") + is3d_b200_last_error(); return rcp; }
+    if (stats) { stats->gpu_launches += sp_st.gpu_launches; stats->total_ms += sp_st.total_ms; }
+    if (!write_polarization_files(wd, sums, P.mcid, P.mass, g, P.fl.dimension, &err)) return IS3D_ERR_IO;
+  }
   if (P.do_resonance_decays) {
     // feed-down on the GPU, then the two amended-spectra files (emissionfunction.cpp:1689-1698)
     std::printf("Starting resonance decays: \n\n");
@@ -382,7 +433,8 @@ extern "C" int is3d_b200_run_workdir(const char *workdir, double *dN_raw, int64_
     s.Wx = sf.Wx.data(); s.Wy = sf.Wy.data(); s.Lambda = sf.Lambda.data(); s.aL = sf.aL.data();
     s.c0 = sf.c0.data(); s.c1 = sf.c1.data(); s.c2 = sf.c2.data(); s.c3 = sf.c3.data(); s.c4 = sf.c4.data();
   }
-  rc = run_problem(wd, P, s, dN_raw, n_raw, mcid_out, n_mcid_max, stats, &err);
+  const is3d_vorticity vort{sf.wtx.data(), sf.wty.data(), sf.wtn.data(), sf.wxy.data(), sf.wxn.data(), sf.wyn.data()};
+  rc = run_problem(wd, P, s, P.fl.mode == 5 ? &vort : nullptr, dN_raw, n_raw, mcid_out, n_mcid_max, stats, &err);
   return rc == IS3D_OK ? rc : fail(rc);
 }
 
@@ -406,7 +458,7 @@ extern "C" int is3d_b200_run_surface(const char *workdir, const is3d_surface *su
     if (rc != IS3D_OK) { err = "cannot average an empty surface"; return fail(rc); }
     compute_jonah_tables(P.pdg, avg[0], P.gla, &P.dft);
   }
-  rc = run_problem(wd, P, *surface, dN_raw, n_raw, mcid_out, n_mcid_max, stats, &err);
+  rc = run_problem(wd, P, *surface, nullptr, dN_raw, n_raw, mcid_out, n_mcid_max, stats, &err);
   return rc == IS3D_OK ? rc : fail(rc);
 }
 
@@ -462,6 +514,7 @@ extern "C" int is3d_b200_host_dump(const char *workdir, const char *out_path)
   put("pitt", s.pitt); put("pitx", s.pitx); put("pity", s.pity); put("pitn", s.pitn); put("pinn", s.pinn);
   put("Wx", s.Wx); put("Wy", s.Wy); put("Lambda", s.Lambda); put("aL", s.aL);
   put("c0", s.c0); put("c1", s.c1); put("c2", s.c2); put("c3", s.c3); put("c4", s.c4);
+  put("wtx", s.wtx); put("wty", s.wty); put("wtn", s.wtn); put("wxy", s.wxy); put("wxn", s.wxn); put("wyn", s.wyn);
   tmp.assign(s.avg, s.avg + 5); put("avg", tmp);
   put("df_T", P.dft.T); put("df_c0", P.dft.c0); put("df_c2", P.dft.c2); put("df_F", P.dft.F); put("df_betabulk", P.dft.betabulk);
   put("df_betapi", P.dft.betapi); put("jonah_x", P.dft.jonah_x); put("jonah_lambda2", P.dft.jonah_lambda2); put("jonah_z", P.dft.jonah_z);

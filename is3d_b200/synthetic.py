@@ -111,3 +111,15 @@ def columns_to_cells(columns, mode=1):
         col = np.ascontiguousarray(a[:, j])
         out[nm] = col * HBARC if nm in _GEV_FIELDS else col
     return out
+
+
+VORTICITY_COLUMNS = ("wtx", "wty", "wtn", "wxy", "wxn", "wyn")
+
+
+def vorticity(n_cells, seed):
+    """Thermal vorticity of a mode-5 surface: the six extra columns (covariant Milne components varpi_{tau x}, varpi_{tau y},
+    varpi_{tau eta}, varpi_{xy}, varpi_{x eta}, varpi_{y eta}, dimensionless) as a dict of arrays.  The eta components carry a factor
+    tau ~ 5 fm relative to the others, as covariant components do."""
+    rng = np.random.default_rng(seed)
+    s = np.array([0.02, 0.02, 0.1, 0.02, 0.1, 0.1])
+    return {k: rng.normal(0.0, s[j], n_cells) for j, k in enumerate(VORTICITY_COLUMNS)}

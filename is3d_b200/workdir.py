@@ -29,6 +29,9 @@ DEFAULT_PARAMETERS = [
     ("r_max", 12.0), ("r_bins", 60),
 ]
 
+# keys of this drop-in that the reference does not read: written only when a caller sets them (absent means 0)
+OPTIONAL_PARAMETERS = ("spin_polarization",)
+
 _EOS_DIR = {1: "urqmd", 2: "smash", 3: "smash_box"}
 _EOS_PDG = {1: ("pdg_urqmd", "pdg-urqmd_v3.3+.dat"), 2: ("pdg_smash", "pdg_smash.dat"), 3: ("pdg_box", "pdg_box.dat")}
 _DF_NAMES = ("c0", "c1", "c2", "c3", "c4", "F", "G", "betabulk", "betaV", "betapi")
@@ -45,12 +48,12 @@ def _r(x):
 def write_parameters(path, **overrides):
     """Write iS3D_parameters.dat (`name = value # comment`, ParameterReader.cpp:38-98)."""
     low = {k.lower(): v for k, v in overrides.items()}
-    known = {k.lower() for k, _ in DEFAULT_PARAMETERS}
+    known = {k.lower() for k, _ in DEFAULT_PARAMETERS} | set(OPTIONAL_PARAMETERS)
     unknown = set(low) - known
     if unknown:
         raise KeyError("unknown iS3D parameter(s): %s" % sorted(unknown))
     with open(path, "w") as f:
-        for k, v in DEFAULT_PARAMETERS:
+        for k, v in DEFAULT_PARAMETERS + [(k, low[k]) for k in OPTIONAL_PARAMETERS if k in low]:
             v = low.get(k.lower(), v)
             f.write("%-28s = %s\t# written by is3d_b200.workdir\n" % (k, repr(v) if isinstance(v, float) else v))
 
@@ -133,7 +136,7 @@ def materialize(root, surface_columns=None, chosen=None, fixture=None, tables=No
     fx = fixture if fixture is not None else load_fixture()
     p = {k.lower(): v for k, v in params.items()}
     hrg_eos = int(p.get("hrg_eos", dict(DEFAULT_PARAMETERS)["hrg_eos"]))
-    for d in ("input", "PDG", "tables/eta", "results/vn_continuous", "results/continuous", "results/sampled", "results/spacetime_distribution",
+    for d in ("input", "PDG", "tables/eta", "results/vn_continuous", "results/continuous", "results/sampled", "results/spacetime_distribution", "results/polarization",
               "deltaf_coefficients/vh", "deltaf_coefficients/vah"):
         os.makedirs(os.path.join(root, d), exist_ok=True)
     write_parameters(os.path.join(root, "iS3D_parameters.dat"), **params)
