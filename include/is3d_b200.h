@@ -45,7 +45,7 @@ typedef struct {
   const double *muB, *nB, *Vx, *Vy, *Vn;
   /* anisotropic hydro (mode 2) only: all ten pi_perp components, W_perp, Lambda, alpha_L and per-cell c0..c4 */
   const double *pitt, *pitx, *pity, *pitn, *pinn, *Wx, *Wy, *Lambda, *aL, *c0, *c1, *c2, *c3, *c4;
-  /* transverse cell positions: read by operation = 0 (spacetime distributions) only, NULL otherwise */
+  /* transverse cell positions: read by operation = 0 (spacetime distributions) and the HBT moments only, NULL otherwise */
   const double *x, *y;
 } is3d_surface;
 
@@ -214,6 +214,33 @@ int is3d_b200_spin_polarization(const is3d_flags *flags, const is3d_surface *sur
 int is3d_b200_spin_polarization_multi(const is3d_flags *flags, const is3d_surface *surface, const is3d_vorticity *vorticity,
                                       const is3d_species *species, const is3d_grid *grid, const is3d_options *options,
                                       is3d_polarization_result *result, is3d_stats *stats);
+
+/* ---- HBT radii: space-time variances of the Cooper-Frye emission function ---------------------------------------------
+ * Gaussian (moment) approximation with pair momentum K = p (Wiedemann & Heinz, Phys. Rept. 319 (1999) 145).  For every spectra bin
+ * (species, pT, phi, y; 2+1D: y = 0) the frame is the bin's longitudinally co-moving frame (LCMS): a longitudinal boost by the bin's
+ * y, out = (cos phi, sin phi, 0), side = (-sin phi, cos phi, 0), long = beam axis, beta_perp = pT / mT.  Each evaluation (cell, slot)
+ * of the spectra contributes at the LCMS coordinates, with (x_c, y_c) = is3d_surface.x, .y [fm] and eta the cell's eta (3+1D) or the
+ * slot's eta (2+1D):
+ *    t* = tau cosh(eta - y)          z* = tau sinh(eta - y)
+ *    o  = x_c cos phi + y_c sin phi - beta_perp t*        s = -x_c sin phi + y_c cos phi        l = z*
+ * and the weight w = g/(2 pi hbar c)^3 (slot weight) p.dsigma f_eq (1 + df), exactly the summand of is3d_b200_smooth_spectra with the
+ * same flags (cells with u.dsigma <= 0 skipped, Theta(p.dsigma) with outflow = 1, regulate_deltaf as there), so S0 is bin for bin the
+ * spectrum.  The ten result arrays hold the RAW sums (they add across cell shards and devices):
+ *    S0 = sum w, So = sum w o, Ss = sum w s, Sl = sum w l, Soo = sum w o^2, Sss, Sll, Sos = sum w o s, Sol, Ssl
+ * The radii are R^2_ij = S_ij / S0 - (S_i / S0)(S_j / S0), i, j in {o, s, l} [fm^2]; a bin with S0 = 0 has radii 0.  Negative
+ * weights (outflow = 0, delta-f without regulate_deltaf) are summed as they are, never clamped, so such radii may be unphysical.
+ * Arrays have the spectra layout ipart + n_species*(ipT + n_pT*(iphi + n_phi*iy)) and are ADDED into; host or device memory per
+ * options->memory.  Weights: df_mode 1 (14-moment) and 2 (Chapman-Enskog), ideal f_eq when both delta-f switches are off; 3+1D and
+ * 2+1D; every viscous-hydro surface mode.
+ * Errors: IS3D_ERR_UNSUPPORTED for df_mode 3 / 4, mode = 2 and include_baryon = 1; IS3D_ERR_ARGUMENT for NULL x or y;
+ * IS3D_ERR_TABLE_RANGE as is3d_b200_smooth_spectra. */
+typedef struct { double *S0, *So, *Ss, *Sl, *Soo, *Sss, *Sll, *Sos, *Sol, *Ssl; } is3d_hbt_result;
+int is3d_b200_hbt_moments(const is3d_flags *flags, const is3d_surface *surface, const is3d_species *species, const is3d_grid *grid,
+                          const is3d_df_tables *df, const is3d_options *options, is3d_hbt_result *result, is3d_stats *stats);
+/* Same over the devices of is3d_b200_init_devices(): HOST arrays, contiguous cell shards, the ten arrays summed on the host in device
+ * order. */
+int is3d_b200_hbt_moments_multi(const is3d_flags *flags, const is3d_surface *surface, const is3d_species *species, const is3d_grid *grid,
+                                const is3d_df_tables *df, const is3d_options *options, is3d_hbt_result *result, is3d_stats *stats);
 
 /* FP64 FMA peak of the current device measured with a dependency-free DFMA chain (the roofline denominator;
  * MEASURED_PEAKS.json carries no FP64 figure).  Returns TFLOP/s in *tflops, SM clock not touched. */

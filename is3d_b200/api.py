@@ -513,3 +513,58 @@ def mean_spin(result, species, grid, dimension):
         S[i, nz] = r[k][nz] / sn[nz]
     rest = S[1:] - S[0] * p / (E + mm.ravel())
     return S, rest
+
+
+HBT_FIELDS = ("S0", "So", "Ss", "Sl", "Soo", "Sss", "Sll", "Sos", "Sol", "Ssl")
+HBT_RADII = ("out", "side", "long", "outside", "outlong", "sidelong")
+
+
+class HbtResult(C.Structure):
+    _fields_ = [(k, _D) for k in HBT_FIELDS]
+
+
+def hbt_moments(flags, cells, species, grid, df_tables, memory="host", stream=None, multi=False):
+    """Call is3d_b200_hbt_moments (or the _multi entry point over the devices of init_devices(), host arrays only).
+
+    cells must carry the transverse positions "x" and "y" [fm] besides the spectra's arrays (numpy for memory='host', float64 CUDA
+    tensors for memory='device').  Returns (dict S0, So, Ss, Sl, Soo, Sss, Sll, Sos, Sol, Ssl of RAW sums, flat [y][phi][pT][species],
+    numpy or CUDA tensors; stats dict).  S0 is the spectrum; hbt_radii() turns the sums into the radii."""
+    device = (memory == "device")
+    m = _Marshal(device)
+    sf, sp, g, dft, _ = _marshal_problem(m, cells, species, grid, df_tables, None)
+    n = sp.n * g.n_pT * g.n_phi * g.n_y
+    res = HbtResult()
+    if device:
+        import torch
+        out = {k: torch.zeros(n, dtype=torch.float64, device=cells["tau"].device) for k in HBT_FIELDS}
+        for k in HBT_FIELDS:
+            setattr(res, k, C.cast(C.c_void_p(out[k].data_ptr()), _D))
+        if stream is None:
+            stream = torch.cuda.current_stream().cuda_stream
+    else:
+        out = {k: np.zeros(n) for k in HBT_FIELDS}
+        for k in HBT_FIELDS:
+            setattr(res, k, out[k].ctypes.data_as(_D))
+    opt = Options(); opt.memory = 1 if device else 0; opt.stream = C.c_void_p(stream or 0)
+    st = Stats()
+    fl = make_flags(flags)
+    f = lib().is3d_b200_hbt_moments_multi if multi else lib().is3d_b200_hbt_moments
+    f.restype = C.c_int
+    f.argtypes = [C.POINTER(Flags), C.POINTER(Surface), C.POINTER(Species), C.POINTER(Grid), C.POINTER(DfTables), C.POINTER(Options),
+                  C.POINTER(HbtResult), C.POINTER(Stats)]
+    _check(f(C.byref(fl), C.byref(sf), C.byref(sp), C.byref(g), C.byref(dft), C.byref(opt), C.byref(res), C.byref(st)))
+    return out, st.as_dict()
+
+
+def hbt_radii(sums):
+    """HBT radii [fm^2] from the raw sums of hbt_moments(): dict out, side, long, outside, outlong, sidelong of
+    R^2_ij = S_ij / S0 - (S_i / S0)(S_j / S0), 0 where S0 = 0 -- the numbers results/hbt/R2_<mcid>.dat holds."""
+    r = {k: np.asarray(sums[k].cpu() if _is_torch(sums[k]) else sums[k], dtype=np.float64) for k in HBT_FIELDS}
+    s0 = r["S0"]
+    nz = s0 != 0
+    first = {i: np.where(nz, r["S" + i], 0.0) / np.where(nz, s0, 1.0) for i in "osl"}
+    out = {}
+    for name, (i, j) in zip(HBT_RADII, (("o", "o"), ("s", "s"), ("l", "l"), ("o", "s"), ("o", "l"), ("s", "l"))):
+        v = np.where(nz, r["S" + i + j], 0.0) / np.where(nz, s0, 1.0) - first[i] * first[j]
+        out[name] = np.where(nz, v, 0.0)
+    return out

@@ -1373,3 +1373,250 @@ extern "C" int is3d_b200_spin_polarization_multi(const is3d_flags *fl, const is3
   }
   return IS3D_OK;
 }
+
+// =====================================================================================================================
+// HBT moments (cf_hbt.cu): the ten raw space-time sums of the linear-delta-f emission function, added into the caller's arrays
+// =====================================================================================================================
+namespace is3d {
+
+static int hbt_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_species *sp, const is3d_grid *gr, const is3d_df_tables *df,
+                    const is3d_options *opt_in, is3d_hbt_result *res, is3d_stats *stats)
+{
+  if (!fl || !sf || !sp || !gr || !res) return fail(IS3D_ERR_ARGUMENT, "NULL argument");
+  double *out[kHbtSums] = {res->S0, res->So, res->Ss, res->Sl, res->Soo, res->Sss, res->Sll, res->Sos, res->Sol, res->Ssl};
+  for (double *p : out) if (!p) return fail(IS3D_ERR_ARGUMENT, "NULL result array");
+  if (fl->mode == 2) return fail(IS3D_ERR_UNSUPPORTED, "HBT moments need a viscous-hydro surface, not mode 2 (anisotropic hydro)");
+  if (fl->include_baryon) return fail(IS3D_ERR_UNSUPPORTED, "include_baryon = 1 (the reference's (T, muB) lookup reads out of bounds, SURVEY R8)");
+  if (fl->df_mode == 3 || fl->df_mode == 4) return fail(IS3D_ERR_UNSUPPORTED, "HBT moments cover the linear delta-f models (df_mode 1, 2), not the modified equilibrium");
+  if (fl->df_mode != 1 && fl->df_mode != 2) return fail(IS3D_ERR_ARGUMENT, "df_mode must be 1..4");
+  if (!sf->x || !sf->y) return fail(IS3D_ERR_ARGUMENT, "HBT moments need the transverse cell positions (surface x, y)");
+  if (fl->dimension != 2 && fl->dimension != 3) return fail(IS3D_ERR_ARGUMENT, "dimension must be 2 or 3");
+  if (sp->n <= 0 || gr->n_pT <= 0 || gr->n_phi <= 0 || gr->n_y <= 0) return fail(IS3D_ERR_ARGUMENT, "empty species list or momentum table");
+  if (!sp->mass || !sp->sign || !sp->degeneracy || !gr->pT || !gr->phi || !gr->y) return fail(IS3D_ERR_ARGUMENT, "NULL species or momentum table");
+  const bool dim2 = (fl->dimension == 2);
+  if (dim2 && (gr->n_eta <= 0 || !gr->eta || !gr->eta_weight)) return fail(IS3D_ERR_ARGUMENT, "dimension = 2 needs the eta table");
+  if (!df || df->n_T < 3 || !df->T) return fail(IS3D_ERR_ARGUMENT, "delta-f coefficient tables missing");
+  if (fl->df_mode == 1 && (!df->c0 || !df->c2)) return fail(IS3D_ERR_ARGUMENT, "df_mode 1 needs the c0 and c2 tables");
+  if (fl->df_mode == 2 && (!df->F || !df->betabulk || !df->betapi)) return fail(IS3D_ERR_ARGUMENT, "df_mode 2 needs the F, betabulk and betapi tables");
+  const int64_t n_cells = sf->n_cells;
+  if (n_cells < 0) return fail(IS3D_ERR_ARGUMENT, "negative cell count");
+  const bool sh = fl->include_shear_deltaf != 0, bk = fl->include_bulk_deltaf != 0;
+  const int model = (!sh && !bk) ? M_IDEAL : (fl->df_mode == 1 ? M_LIN14 : M_LINCE);
+  // the surface arrays prepare_vh_kernel reads, then the positions
+  constexpr int kRaw = 20;
+  const double *srcs[kRaw] = {sf->tau, sf->eta, sf->dat, sf->dax, sf->day, sf->dan, sf->ux, sf->uy, sf->un, sf->T, sf->P, sf->E,
+                              sf->pixx, sf->pixy, sf->pixn, sf->piyy, sf->piyn, sf->bulkPi, sf->x, sf->y};
+  const bool need[kRaw] = {true, true, true, true, true, true, true, true, true, true, true, true, sh, sh, sh, sh, sh, bk, true, true};
+  for (int a = 0; a < kRaw; a++) if (need[a] && !srcs[a] && n_cells > 0) return fail(IS3D_ERR_ARGUMENT, "a required surface array is NULL");
+  Device *Dp = nullptr;
+  { int rc = current_device(&Dp); if (rc) return rc; }
+  Workspace &ws = Dp->ws;
+  std::lock_guard<std::mutex> lk(Dp->mu);
+  is3d_options opt; memset(&opt, 0, sizeof(opt));
+  if (opt_in) opt = *opt_in;
+  cudaStream_t st = (cudaStream_t)opt.stream;
+  const int64_t n_bins = (int64_t)sp->n * gr->n_pT * gr->n_phi * gr->n_y;
+  const int64_t n_active = dim2 ? n_bins / gr->n_y : n_bins;        // 2+1D fills the y = 0 plane (index iy = 0)
+
+  // ---- layout: the cf_kernel decomposition with the register tile of cf_hbt_kernel; records of prepare_vh_kernel
+  Layout L; memset(&L, 0, sizeof(L));
+  L.n_species = sp->n; L.n_pT = gr->n_pT; L.n_phi = gr->n_phi; L.n_y_out = gr->n_y;
+  L.dim2 = dim2 ? 1 : 0;
+  L.n_slots = dim2 ? gr->n_eta : gr->n_y;
+  L.rec_y = kRec;
+  int nyt, npt, ct;
+  hbt_shape(L.dim2, &nyt, &npt, &ct);
+  L.nst = dim2 ? L.n_slots : nyt;
+  L.n_ytiles = dim2 ? 1 : (L.n_slots + nyt - 1) / nyt;
+  L.npt = npt; L.n_ptiles = (L.n_phi + npt - 1) / npt;
+  L.ct = ct; L.n_cells = n_cells;
+  L.n_tiles = (n_cells + ct - 1) / ct;
+  L.n_cells_pad = L.n_tiles * ct;
+  const int n_groups = (sp->n * gr->n_pT + 31) / 32;
+  const int n_warps = std::min(kHbtWarps, n_groups);
+  const int n_groupblocks = (n_groups + n_warps - 1) / n_warps;
+  const int64_t n_bintiles = (int64_t)n_groupblocks * L.n_ytiles * L.n_ptiles;
+  // chunks: the rule of smooth_core (>= 192 blocks per SM, a chunk's records within a third of L2, partial sums <= 4 GiB)
+  int64_t n_chunks = ((int64_t)Dp->sm_count * 192 + n_bintiles - 1) / n_bintiles;
+  const int64_t rec_per_cell = ((int64_t)L.n_ytiles * L.nst * kRec + (int64_t)L.n_ptiles * L.npt * kRec + kScal + kHbtRecC) * 8;
+  const int64_t l2_target = std::max<int64_t>((int64_t)Dp->l2_bytes / 3, (int64_t)8 << 20);
+  n_chunks = std::max<int64_t>(n_chunks, (n_cells * rec_per_cell + l2_target - 1) / l2_target);
+  const int64_t n_chunks_wanted = n_chunks;
+  n_chunks = std::min<int64_t>(n_chunks, std::max<int64_t>(1, ((int64_t)4 << 30) / (kHbtSums * n_bins * 8)));
+  if (opt.n_chunks > 0) n_chunks = opt.n_chunks;
+  n_chunks = std::max<int64_t>(1, std::min<int64_t>(n_chunks, std::max<int64_t>(L.n_tiles, 1)));
+  if (n_bintiles * n_chunks > 2147483647LL) return fail(IS3D_ERR_ARGUMENT, "grid too large");
+
+  // ---- tables and surface to the device
+  SmallArena ar;
+  std::vector<double> cosphi(gr->n_phi), sinphi(gr->n_phi);
+  for (int k = 0; k < gr->n_phi; k++) { cosphi[k] = cos(gr->phi[k]); sinphi[k] = sin(gr->phi[k]); }
+  const size_t o_mass = ar.put(sp->mass, sp->n), o_sign = ar.put(sp->sign, sp->n), o_deg = ar.put(sp->degeneracy, sp->n);
+  const size_t o_pT = ar.put(gr->pT, gr->n_pT), o_cos = ar.put(cosphi.data(), gr->n_phi), o_sin = ar.put(sinphi.data(), gr->n_phi);
+  const size_t o_sloty = dim2 ? ar.put(gr->eta, gr->n_eta) : ar.put(gr->y, gr->n_y);
+  const size_t o_slotw = dim2 ? ar.put(gr->eta_weight, gr->n_eta) : 0;
+  struct SplineOff { size_t x, y, c; int n; };
+  auto put_spline = [&](const double *x, const double *y, int n) {
+    SplineOff o{0, 0, 0, 0};
+    if (!x || !y || n < 3) return o;
+    std::vector<double> c(n);
+    host_spline_init(x, y, n, c.data());
+    o.x = ar.put(x, n); o.y = ar.put(y, n); o.c = ar.put(c.data(), n); o.n = n;
+    return o;
+  };
+  const SplineOff s_c0 = put_spline(df->T, df->c0, df->n_T), s_c2 = put_spline(df->T, df->c2, df->n_T), s_F = put_spline(df->T, df->F, df->n_T);
+  const SplineOff s_bb = put_spline(df->T, df->betabulk, df->n_T), s_bp = put_spline(df->T, df->betapi, df->n_T);
+  const size_t cell_stride = ((size_t)n_cells * 8 + 255) & ~(size_t)255;
+  CU_CHECK(ws.small.reserve(ar.host.size() + 256));
+  CU_CHECK(ws.Y.reserve((size_t)L.n_ytiles * L.n_cells_pad * L.nst * kRec * 8 + 256));
+  CU_CHECK(ws.P.reserve((size_t)L.n_ptiles * L.n_cells_pad * L.npt * kRec * 8 + 256));
+  CU_CHECK(ws.S.reserve((size_t)L.n_cells_pad * kScal * 8 + 256));
+  CU_CHECK(ws.extra.reserve((size_t)L.n_cells_pad * kHbtRecC * 8 + 256));          // per-cell [tau, x, y, 0]
+  CU_CHECK(ws.partial.reserve((size_t)kHbtSums * n_chunks * n_bins * 8 + 256));
+  CU_CHECK(ws.dN.reserve((size_t)kHbtSums * n_bins * 8 + 256));
+  CU_CHECK(ws.counters.reserve(256));
+  if (opt.memory == 0) CU_CHECK(ws.raw.reserve(cell_stride * kRaw + 256));
+
+  cudaEvent_t *ev = ws.ev;
+  CU_CHECK(cudaEventRecord(ev[0], st));
+  unsigned char *small_d = ws.small.as<unsigned char>();
+  CU_CHECK(cudaMemcpyAsync(small_d, ar.host.data(), ar.host.size(), cudaMemcpyHostToDevice, st));
+  const double *dev[kRaw];
+  for (int a = 0; a < kRaw; a++) {
+    dev[a] = need[a] ? srcs[a] : nullptr;
+    if (opt.memory == 0 && need[a]) {
+      double *d = reinterpret_cast<double *>(ws.raw.as<unsigned char>() + cell_stride * a);
+      if (n_cells > 0) CU_CHECK(cudaMemcpyAsync(d, srcs[a], (size_t)n_cells * 8, cudaMemcpyHostToDevice, st));
+      dev[a] = d;
+    }
+  }
+  RawCells rc; memset(&rc, 0, sizeof(rc));
+  rc.n = n_cells; rc.tau = dev[0]; rc.eta = dev[1]; rc.dat = dev[2]; rc.dax = dev[3]; rc.day = dev[4]; rc.dan = dev[5];
+  rc.ux = dev[6]; rc.uy = dev[7]; rc.un = dev[8]; rc.T = dev[9]; rc.P = dev[10]; rc.E = dev[11];
+  rc.pixx = dev[12]; rc.pixy = dev[13]; rc.pixn = dev[14]; rc.piyy = dev[15]; rc.piyn = dev[16]; rc.bulkPi = dev[17];
+  double *sums_d = ws.dN.as<double>();                         // [10][n_bins] in the order of is3d_hbt_result
+  CU_CHECK(cudaMemsetAsync(sums_d, 0, (size_t)kHbtSums * n_bins * 8, st));
+  CU_CHECK(cudaMemsetAsync(ws.counters.p, 0, sizeof(PrepCounters), st));
+  CU_CHECK(cudaEventRecord(ev[1], st));
+
+  // ---- prepare: the spectra's records, then the positions
+  auto dptr = [&](size_t off) { return reinterpret_cast<const double *>(small_d + off); };
+  PrepTables tab; memset(&tab, 0, sizeof(tab));
+  auto mk = [&](const SplineOff &o) { Spline s; s.x = dptr(o.x); s.y = dptr(o.y); s.c = dptr(o.c); s.n = o.n; return s; };
+  tab.c0 = mk(s_c0); tab.c2 = mk(s_c2); tab.F = mk(s_F); tab.betabulk = mk(s_bb); tab.betapi = mk(s_bp);
+  tab.bulkPi_over_Peq_max = df->bulkPi_over_Peq_max;
+  tab.cosphi = dptr(o_cos); tab.sinphi = dptr(o_sin); tab.slot_y = dptr(o_sloty); tab.slot_w = dim2 ? dptr(o_slotw) : nullptr;
+  tab.deta_min = fl->deta_min; tab.mass_pion0 = fl->mass_pion0;
+  PrepCounters *cnt_d = ws.counters.as<PrepCounters>();
+  CU_CHECK(launch_prepare_vh(*fl, rc, tab, L, ws.Y.as<double>(), ws.P.as<double>(), ws.S.as<double>(), cnt_d, st));
+  CU_CHECK(launch_prepare_hbt_cells(dev[0], dev[18], dev[19], n_cells, L.n_cells_pad, ws.extra.as<double>(), st));
+  CU_CHECK(cudaEventRecord(ev[2], st));
+  // a cell outside the coefficient tables: stop before anything is added to the result, as the spectra do
+  PrepCounters cnt; memset(&cnt, 0, sizeof(cnt));
+  CU_CHECK(cudaMemcpyAsync(&cnt, cnt_d, sizeof(cnt), cudaMemcpyDeviceToHost, st));
+  CU_CHECK(cudaStreamSynchronize(st));
+  if (cnt.range_error) return fail(IS3D_ERR_TABLE_RANGE, "a cell's T lies outside the delta-f coefficient table");
+
+  HbtParams prm; memset(&prm, 0, sizeof(prm));
+  HotParams &hp = prm.hp;
+  hp.L = L; hp.Y = ws.Y.as<double>(); hp.P = ws.P.as<double>(); hp.S = ws.S.as<double>();
+  hp.mass = dptr(o_mass); hp.sign = dptr(o_sign); hp.degeneracy = dptr(o_deg); hp.pT = dptr(o_pT);
+  hp.partial = ws.partial.as<double>();
+  hp.n_chunks = (int)n_chunks; hp.n_groupblocks = n_groupblocks; hp.n_warps = n_warps;
+  hp.regulate_thr = fl->regulate_deltaf ? 0x3ff00000 : 0x7ff80000;        // as smooth_core
+  hp.one_hi = 0x3ff00000;
+  hp.outflow_thr = fl->outflow ? 0LL : (long long)0x8000000000000000ULL;
+  hp.prefactor = pow(2.0 * M_PI * 0.197327053, -3);
+  prm.C = ws.extra.as<double>(); prm.cosphi = dptr(o_cos); prm.sinphi = dptr(o_sin);
+  CU_CHECK(launch_hbt(model, prm, st));
+  CU_CHECK(cudaEventRecord(ev[3], st));
+  for (int q = 0; q < kHbtSums; q++)
+    CU_CHECK(launch_reduce(hp.partial + (size_t)q * n_chunks * n_bins, (int)n_chunks, n_bins, n_active, sums_d + (size_t)q * n_bins, st));
+  CU_CHECK(cudaEventRecord(ev[4], st));
+
+  std::vector<double> host;
+  if (opt.memory == 0) {
+    host.resize((size_t)kHbtSums * n_bins);
+    CU_CHECK(cudaMemcpyAsync(host.data(), sums_d, (size_t)kHbtSums * n_bins * 8, cudaMemcpyDeviceToHost, st));
+  } else {
+    for (int q = 0; q < kHbtSums; q++) CU_CHECK(launch_axpy(sums_d + (size_t)q * n_bins, out[q], n_active, st));
+  }
+  CU_CHECK(cudaEventRecord(ev[5], st));
+  CU_CHECK(cudaEventSynchronize(ev[5]));
+  if (opt.memory == 0)
+    for (int q = 0; q < kHbtSums; q++)
+      for (int64_t i = 0; i < n_bins; i++) out[q][i] += host[(size_t)q * n_bins + i];
+
+  is3d_stats stt; memset(&stt, 0, sizeof(stt));
+  float ms;
+  cudaEventElapsedTime(&ms, ev[0], ev[1]); stt.h2d_ms = ms;
+  cudaEventElapsedTime(&ms, ev[1], ev[2]); stt.prepare_ms = ms;
+  cudaEventElapsedTime(&ms, ev[2], ev[3]); stt.kernel_ms = ms;
+  cudaEventElapsedTime(&ms, ev[3], ev[4]); stt.reduce_ms = ms;
+  cudaEventElapsedTime(&ms, ev[4], ev[5]); stt.d2h_ms = ms;
+  cudaEventElapsedTime(&ms, ev[0], ev[5]); stt.total_ms = ms;
+  stt.cells_skipped_udsigma = (int64_t)cnt.skipped;
+  stt.evaluations = n_cells * (int64_t)sp->n * gr->n_pT * gr->n_phi * (int64_t)L.n_slots;
+  stt.gpu_launches = (n_cells > 0 ? 2 : 0) + 1 + kHbtSums + (opt.memory == 0 ? 0 : kHbtSums);
+  stt.n_chunks = (int)n_chunks; stt.n_chunks_wanted = (int)n_chunks_wanted;
+  stt.n_gpus = 1;
+  if (stats) *stats = stt;
+  return IS3D_OK;
+}
+
+}  // namespace is3d
+
+extern "C" int is3d_b200_hbt_moments(const is3d_flags *fl, const is3d_surface *sf, const is3d_species *sp, const is3d_grid *gr,
+                                     const is3d_df_tables *df, const is3d_options *opt, is3d_hbt_result *res, is3d_stats *stats)
+{
+  return hbt_core(fl, sf, sp, gr, df, opt, res, stats);
+}
+
+// Several devices: HOST arrays, contiguous cell shards, one thread per device; the ten raw sums are added on the host in device order
+extern "C" int is3d_b200_hbt_moments_multi(const is3d_flags *fl, const is3d_surface *sf, const is3d_species *sp, const is3d_grid *gr,
+                                           const is3d_df_tables *df, const is3d_options *opt_in, is3d_hbt_result *res, is3d_stats *stats)
+{
+  const int G = g_ngpus;
+  if (G <= 1) return is3d_b200_hbt_moments(fl, sf, sp, gr, df, opt_in, res, stats);
+  if (!fl || !sf || !sp || !gr || !res) return fail(IS3D_ERR_ARGUMENT, "NULL argument");
+  if (opt_in && opt_in->memory != 0) return fail(IS3D_ERR_ARGUMENT, "the multi-GPU entry point takes host arrays");
+  double *out[kHbtSums] = {res->S0, res->So, res->Ss, res->Sl, res->Soo, res->Sss, res->Sll, res->Sos, res->Sol, res->Ssl};
+  for (double *p : out) if (!p) return fail(IS3D_ERR_ARGUMENT, "NULL result array");
+  std::lock_guard<std::mutex> lk(g_multi_mutex);
+  const size_t n_bins = (size_t)std::max(sp->n, 0) * std::max(gr->n_pT, 0) * std::max(gr->n_phi, 0) * std::max(gr->n_y, 0);
+  int prev = 0; cudaGetDevice(&prev);
+  std::vector<int> rcs(G, IS3D_OK);
+  std::vector<std::string> errs(G);
+  std::vector<is3d_stats> sts(G);
+  std::vector<std::vector<double>> bufs(G, std::vector<double>(kHbtSums * n_bins, 0.0));
+  std::vector<std::thread> workers;
+  for (int d = 0; d < G; d++) {
+    workers.emplace_back([&, d]() {
+      memset(&sts[d], 0, sizeof(is3d_stats));
+      if (cudaSetDevice(d) != cudaSuccess) { rcs[d] = IS3D_ERR_CUDA; errs[d] = "cudaSetDevice failed"; return; }
+      int64_t lo, hi;
+      shard_bounds(sf->n_cells, d, G, &lo, &hi);
+      const is3d_surface shard = shard_surface(*sf, lo, hi);
+      is3d_options opt; memset(&opt, 0, sizeof(opt));
+      if (opt_in) opt = *opt_in;
+      opt.memory = 0; opt.stream = g_streams[d];
+      double *b = bufs[d].data();
+      is3d_hbt_result r{b, b + n_bins, b + 2 * n_bins, b + 3 * n_bins, b + 4 * n_bins, b + 5 * n_bins, b + 6 * n_bins, b + 7 * n_bins,
+                        b + 8 * n_bins, b + 9 * n_bins};
+      rcs[d] = hbt_core(fl, &shard, sp, gr, df, &opt, &r, &sts[d]);
+      if (rcs[d]) errs[d] = g_last_error;
+    });
+  }
+  for (auto &w : workers) w.join();
+  cudaSetDevice(prev);
+  for (int d = 0; d < G; d++) if (rcs[d]) return fail(rcs[d], errs[d].c_str());
+  for (int q = 0; q < kHbtSums; q++)
+    for (size_t i = 0; i < n_bins; i++) { double v = 0.0; for (int d = 0; d < G; d++) v += bufs[d][q * n_bins + i]; out[q][i] += v; }
+  if (stats) {
+    is3d_stats tot; memset(&tot, 0, sizeof(tot));
+    for (int d = 0; d < G; d++) merge_stats(&tot, sts[d]);
+    tot.n_gpus = G;
+    *stats = tot;
+  }
+  return IS3D_OK;
+}

@@ -6,7 +6,9 @@
 //    in shared memory, degree-4 polynomial -- 9 FP64-pipe instructions (the table-free degree-11 form needs 15), integer
 //    exponent insertion on the ALU pipe, and the IEEE overflow semantics of the reference's
 //    `1.0 / (exp(x) + sign)` (smooth_kernels.cpp:289): exactly 0 once exp(x) would overflow, gradual underflow below;
-//  * rcp_fast(): MUFU.RCP64H seed + one cubically convergent correction (3 DFMA), relative error < 1e-15.
+//  * rcp_fast(): MUFU.RCP64H seed + one cubically convergent correction (3 DFMA), relative error < 1e-15;
+//  * distribution<MODEL>() / distribution_group<MODEL, N>(): f_eq (1 + df) of the linear-df models per evaluation / per group,
+//    shared by cf_kernel and the kernels built on its records (cf_hbt.cu).
 #pragma once
 #include <cstdint>
 #include <cuda_runtime.h>
@@ -261,6 +263,21 @@ __device__ __forceinline__ double occupation_bar(double a, double sign, double &
 // dilute form, a < 2^-18: 1 / (1 + Theta a) = 1 - Theta a + a^2 - ... truncated after a^2 (|error| < a^3 < 5.2e-17)
 __device__ __forceinline__ double occupation_bar_dilute(double a, double sign, double &feqbar)
 { feqbar = fma(a, a, fma(-sign, a, 1.0)); return a * feqbar; }
+
+// f_eq (1 + df) of the linear-df models; x = u.p/T, s = partial delta-f polynomial (see cf_prepare.cu)
+template <int MODEL>
+__device__ __forceinline__ double distribution(double x, double s, double K2, double K3, double sign, int reg_thr, int one_hi)
+{
+  if (MODEL == M_IDEAL) return occupation(exp_neg(x), sign);      // df = 0: f = f_eq (1 + 0)
+  double dfs;
+  if (MODEL == M_LIN14) dfs = fma(K2 * x, x, s);               // + Pi bulk2 (u.p)^2
+  else dfs = fma(s, rcp_fast(x), K2 * x);                      // [..]/(u.p) + (..)(u.p)
+  const double feq = occupation(exp_neg(x), sign);
+  const double feqbar = fma(-sign, feq, 1.0);
+  double df = (MODEL == M_JONAHLIN) ? fma(feqbar, dfs, K3) : feqbar * dfs;
+  df = clamp_unit(df, reg_thr, one_hi);                                // regulate_deltaf
+  return fma(feq, df, feq);
+}
 
 // f_eq (1 + df) of the linear-df models (x = u.p/T, s = partial delta-f polynomial, see cf_prepare.cu) for a group of N evaluations, staged so that the N dependency chains can be interleaved
 template <int MODEL, int N>

@@ -145,5 +145,19 @@ cudaError_t launch_prepare_polzn(const RawCells &cells, const VortCells &vort, c
                                  PrepCounters *counters, cudaStream_t st);
 // partial: [5][n_chunks][n_bins]
 cudaError_t launch_polzn(const HotParams &hp, cudaStream_t st);
+// HBT moments (cf_hbt.cu): the records of prepare_vh_kernel plus a per-cell record [tau, x, y, 0]; 10 sums per bin
+constexpr int kHbtRecC = 4;      // doubles per per-cell position record
+constexpr int kHbtSums = 10;     // S0, So, Ss, Sl, Soo, Sss, Sll, Sos, Sol, Ssl
+constexpr int kHbtWarps = 4;     // warps per block (at most)
+constexpr int kHbtMinBlocks = 3; // blocks per SM the register budget is sized for (__launch_bounds__)
+constexpr int kHbtNyt3D = 3, kHbtNpt3D = 1, kHbtNpt2D = 2;
+struct HbtParams {
+  HotParams hp;                  // layout, records Y / P / S, species and pT tables, partial [10][n_chunks][n_bins], flags
+  const double *C;               // [n_cells_pad][kHbtRecC]
+  const double *cosphi, *sinphi; // [n_phi]
+};
+void hbt_shape(int dim2, int *nyt, int *npt, int *ct);
+cudaError_t launch_prepare_hbt_cells(const double *tau, const double *x, const double *y, int64_t n, int64_t n_pad, double *C, cudaStream_t st);
+cudaError_t launch_hbt(int model, const HbtParams &prm, cudaStream_t st);
 
 }  // namespace is3d

@@ -22,21 +22,6 @@
 
 namespace is3d {
 
-// f_eq (1 + df) of the linear-df models; x = u.p/T, s = partial delta-f polynomial (see cf_prepare.cu)
-template <int MODEL>
-__device__ __forceinline__ double distribution(double x, double s, double K2, double K3, double sign, int reg_thr, int one_hi)
-{
-  if (MODEL == M_IDEAL) return occupation(exp_neg(x), sign);      // df = 0: f = f_eq (1 + 0)
-  double dfs;
-  if (MODEL == M_LIN14) dfs = fma(K2 * x, x, s);               // + Pi bulk2 (u.p)^2
-  else dfs = fma(s, rcp_fast(x), K2 * x);                      // [..]/(u.p) + (..)(u.p)
-  const double feq = occupation(exp_neg(x), sign);
-  const double feqbar = fma(-sign, feq, 1.0);
-  double df = (MODEL == M_JONAHLIN) ? fma(feqbar, dfs, K3) : feqbar * dfs;
-  df = clamp_unit(df, reg_thr, one_hi);                                // regulate_deltaf
-  return fma(feq, df, feq);
-}
-
 // SB selects how the NPT evaluations of a (cell, slot) are scheduled:
 //   0  one divergent region per evaluation (distribution());
 //   1  the NPT evaluations form one staged group (distribution_group()): their exp / reciprocal chains interleave (ILP); the

@@ -215,12 +215,47 @@ static bool write_polarization_files(const std::string &wd, const std::vector<do
   return true;
 }
 
+// results/hbt/R2_<mcid>.dat: S0 and the HBT radii R^2_ij = S_ij / S0 - (S_i / S0)(S_j / S0) [fm^2] (all 0 where S0 = 0) of the raw sums of
+// is3d_b200_hbt_moments, one row per (y, phi, pT) in the loop order, number format and blank line per phi block of write_spectra_files;
+// truncating opens, results/hbt/ must exist
+static bool write_hbt_files(const std::string &wd, const std::vector<double> &sums, const std::vector<int> &mcid, const Grids &g,
+                            int dimension, std::string *err)
+{
+  const int npart = (int)mcid.size(), npT = (int)g.pT.rows, nphi = (int)g.phi.rows, ny = (int)g.y.rows;
+  const int y_pts = (dimension == 2) ? 1 : ny;
+  const size_t n_bins = (size_t)npart * npT * nphi * ny;
+  auto S = [&](int q, size_t b) { return sums[(size_t)q * n_bins + b]; };     // S0 So Ss Sl Soo Sss Sll Sos Sol Ssl
+  static const int pairs[6][3] = {{4, 1, 1}, {5, 2, 2}, {6, 3, 3}, {7, 1, 2}, {8, 1, 3}, {9, 2, 3}};   // (S_ij, i, j): out side long os ol sl
+  for (int ipart = 0; ipart < npart; ipart++) {
+    char name[255];
+    std::snprintf(name, sizeof(name), "%s/results/hbt/R2_%d.dat", wd.c_str(), mcid[ipart]);
+    std::ofstream f(name, std::ios_base::out);
+    if (!f) { *err = std::string("cannot open ") + name + " (the directory results/hbt/ must exist)"; return false; }
+    f << "y\tphip\tpT\tS0\tR2_out\tR2_side\tR2_long\tR2_outside\tR2_outlong\tR2_sidelong\n";
+    for (int iy = 0; iy < y_pts; iy++) {
+      const double y = (dimension == 2) ? 0.0 : g.y.at(1, iy + 1);
+      for (int iphi = 0; iphi < nphi; iphi++) {
+        for (int ipT = 0; ipT < npT; ipT++) {
+          const size_t b = (size_t)bin_index(ipart, npart, ipT, npT, iphi, nphi, iy);
+          const double s0 = S(0, b);
+          f << std::scientific << std::setw(5) << std::setprecision(8) << y << "\t" << g.phi.at(1, iphi + 1) << "\t" << g.pT.at(1, ipT + 1) << "\t" << s0;
+          for (const int *pr : pairs) f << "\t" << (s0 != 0.0 ? S(pr[0], b) / s0 - (S(pr[1], b) / s0) * (S(pr[2], b) / s0) : 0.0);
+          f << "\n";
+        }
+        f << "\n";
+      }
+    }
+  }
+  return true;
+}
+
 // everything the host layer derives from the input files
 struct Problem {
   Params par;
   is3d_flags fl;
   int operation = 0, hrg_eos = 0, group_particles = 0, do_resonance_decays = 0;
   int spin_polarization = 0;               // optional key (absent: 0): mode-5 spin polarization after the spectra
+  int hbt_radii = 0;                       // optional key (absent: 0): HBT radii of the linear-delta-f spectra after the spectra
   std::vector<int> pick;                   // particle-list index of every chosen species (chosen_particles_sampling_table)
   SurfaceData sf;
   std::vector<Particle> pdg;
@@ -262,6 +297,10 @@ static int load_problem(const std::string &wd, bool need_surface, Problem *p, st
   if (p->do_resonance_decays && p->operation != 1) { err = "do_resonance_decays = 1 applies to operation = 1 (the reference runs it after the spectra, emissionfunction.cpp:1689)"; return IS3D_ERR_UNSUPPORTED; }
   p->spin_polarization = par.has("spin_polarization") ? (int)par.get("spin_polarization", &err) : 0;
   if (p->spin_polarization && (p->operation != 1 || fl.mode != 5)) { err = "spin_polarization = 1 needs operation = 1 and a mode 5 surface (the thermal vorticity columns)"; return IS3D_ERR_UNSUPPORTED; }
+  p->hbt_radii = par.has("hbt_radii") ? (int)par.get("hbt_radii", &err) : 0;
+  if (p->hbt_radii && (p->operation != 1 || fl.mode == 2 || (fl.df_mode != 1 && fl.df_mode != 2) || fl.include_baryon)) {
+    err = "hbt_radii = 1 needs operation = 1, a viscous-hydro surface (mode != 2), df_mode 1 or 2 and include_baryon = 0"; return IS3D_ERR_UNSUPPORTED;
+  }
   if (p->do_resonance_decays && p->hrg_eos == 3) { err = "do_resonance_decays = 1 needs a particle list with decay tables (hrg_eos = 1, 2); pdg_box.dat has none"; return IS3D_ERR_UNSUPPORTED; }
 
   // ---- surface (+ averages side file)
@@ -380,6 +419,17 @@ static int run_problem(const std::string &wd, Problem &P, const is3d_surface &s,
     if (rcp != IS3D_OK) { err = std::string("spin polarization failed: ") + is3d_b200_last_error(); return rcp; }
     if (stats) { stats->gpu_launches += sp_st.gpu_launches; stats->total_ms += sp_st.total_ms; }
     if (!write_polarization_files(wd, sums, P.mcid, P.mass, g, P.fl.dimension, &err)) return IS3D_ERR_IO;
+  }
+  if (P.hbt_radii) {
+    std::vector<double> sums(10 * n_bins, 0.0);                  // S0 | So | Ss | Sl | Soo | Sss | Sll | Sos | Sol | Ssl
+    double *b = sums.data();
+    is3d_hbt_result r{b, b + n_bins, b + 2 * n_bins, b + 3 * n_bins, b + 4 * n_bins, b + 5 * n_bins, b + 6 * n_bins, b + 7 * n_bins,
+                      b + 8 * n_bins, b + 9 * n_bins};
+    is3d_stats hb_st; std::memset(&hb_st, 0, sizeof(hb_st));
+    const int rch = is3d_b200_hbt_moments_multi(&P.fl, &s, &sp, &gr, &dt, nullptr, &r, &hb_st);
+    if (rch != IS3D_OK) { err = std::string("HBT moments failed: ") + is3d_b200_last_error(); return rch; }
+    if (stats) { stats->gpu_launches += hb_st.gpu_launches; stats->total_ms += hb_st.total_ms; }
+    if (!write_hbt_files(wd, sums, P.mcid, g, P.fl.dimension, &err)) return IS3D_ERR_IO;
   }
   if (P.do_resonance_decays) {
     // feed-down on the GPU, then the two amended-spectra files (emissionfunction.cpp:1689-1698)

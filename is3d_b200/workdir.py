@@ -30,7 +30,7 @@ DEFAULT_PARAMETERS = [
 ]
 
 # keys of this drop-in that the reference does not read: written only when a caller sets them (absent means 0)
-OPTIONAL_PARAMETERS = ("spin_polarization",)
+OPTIONAL_PARAMETERS = ("spin_polarization", "hbt_radii")
 
 _EOS_DIR = {1: "urqmd", 2: "smash", 3: "smash_box"}
 _EOS_PDG = {1: ("pdg_urqmd", "pdg-urqmd_v3.3+.dat"), 2: ("pdg_smash", "pdg_smash.dat"), 3: ("pdg_box", "pdg_box.dat")}
@@ -137,6 +137,7 @@ def materialize(root, surface_columns=None, chosen=None, fixture=None, tables=No
     p = {k.lower(): v for k, v in params.items()}
     hrg_eos = int(p.get("hrg_eos", dict(DEFAULT_PARAMETERS)["hrg_eos"]))
     for d in ("input", "PDG", "tables/eta", "results/vn_continuous", "results/continuous", "results/sampled", "results/spacetime_distribution", "results/polarization",
+              "results/hbt",
               "deltaf_coefficients/vh", "deltaf_coefficients/vah"):
         os.makedirs(os.path.join(root, d), exist_ok=True)
     write_parameters(os.path.join(root, "iS3D_parameters.dat"), **params)
