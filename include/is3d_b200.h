@@ -45,7 +45,7 @@ typedef struct {
   const double *muB, *nB, *Vx, *Vy, *Vn;
   /* anisotropic hydro (mode 2) only: all ten pi_perp components, W_perp, Lambda, alpha_L and per-cell c0..c4 */
   const double *pitt, *pitx, *pity, *pitn, *pinn, *Wx, *Wy, *Lambda, *aL, *c0, *c1, *c2, *c3, *c4;
-  /* transverse cell positions: read by operation = 0 (spacetime distributions) and the HBT moments only, NULL otherwise */
+  /* transverse cell positions: read by operation = 0 (spacetime distributions) and the HBT paths only, NULL otherwise */
   const double *x, *y;
 } is3d_surface;
 
@@ -241,6 +241,34 @@ int is3d_b200_hbt_moments(const is3d_flags *flags, const is3d_surface *surface, 
  * order. */
 int is3d_b200_hbt_moments_multi(const is3d_flags *flags, const is3d_surface *surface, const is3d_species *species, const is3d_grid *grid,
                                 const is3d_df_tables *df, const is3d_options *options, is3d_hbt_result *result, is3d_stats *stats);
+
+/* ---- HBT correlation functions: Fourier transform of the Cooper-Frye emission function --------------------------------------
+ * Smoothness and on-shell approximation with pair momentum K = p (Wiedemann & Heinz, Phys. Rept. 319 (1999) 145), the frame, the
+ * coordinates (o, s, l) and the weight w of is3d_b200_hbt_moments (same flags, skip rules and errors).  q is given in each bin's LCMS,
+ * q = (q_o, q_s, q_l) [GeV], with q^0 = beta_perp q_o from q.K = 0, so that q.x = -(q_o o + q_s s + q_l l) exactly.  q is sampled on
+ * rays: the caller's n_dir direction vectors d = (d_o, d_s, d_l) (host memory, not normalised by the library) and the points
+ * q_k = k dq d, k = 0 .. n_q - 1.  The result arrays hold the RAW sums (they add across cell shards and devices)
+ *    Re[d][k][bin] = sum w cos(theta),   Im[d][k][bin] = sum w sin(theta),   theta = k dq (d_o o + d_s s + d_l l) / hbar c
+ * with hbar c = 0.197327053 GeV fm; Re[d][0] is S0 (the spectrum) for every d and Im[d][0] = 0, exactly.  The correlation function of
+ * identical particles of an unpolarised source is C = 1 - sign (Re^2 + Im^2) / (g Re[d][0]^2) (sign = -1 bosons, +1 fermions,
+ * g = degeneracy; C = 1 where S0 = 0).  Negative weights are summed as they are.  Not included: final-state interactions, resonance-
+ * decay halos, K != p, non-identical pairs, the modified-equilibrium, anisotropic and baryon weights.
+ * Arrays are [n_dir][n_q][n_bins] with the spectra bin layout inside, ADDED into; host or device memory per options->memory.
+ * Errors: as is3d_b200_hbt_moments; IS3D_ERR_ARGUMENT also for NULL Re, Im, q rays or dir, n_dir < 1, n_q < 1, dq <= 0 or not finite,
+ * a direction component that is not finite, and 2 n_dir n_q n_bins partial sums beyond 4 GiB (one cell chunk). */
+typedef struct {
+  int32_t n_dir, n_q;   /* rays and q points per ray */
+  double dq;            /* step along every ray [GeV] */
+  const double *dir;    /* [n_dir][3] (o, s, l), host memory */
+} is3d_hbt_qrays;
+typedef struct { double *Re, *Im; /* [n_dir][n_q][n_bins] */ } is3d_hbt_fourier_result;
+int is3d_b200_hbt_fourier(const is3d_flags *flags, const is3d_surface *surface, const is3d_species *species, const is3d_grid *grid,
+                          const is3d_df_tables *df, const is3d_hbt_qrays *qrays, const is3d_options *options,
+                          is3d_hbt_fourier_result *result, is3d_stats *stats);
+/* Same over the devices of is3d_b200_init_devices(): HOST arrays, contiguous cell shards, Re and Im summed on the host in device order. */
+int is3d_b200_hbt_fourier_multi(const is3d_flags *flags, const is3d_surface *surface, const is3d_species *species, const is3d_grid *grid,
+                                const is3d_df_tables *df, const is3d_hbt_qrays *qrays, const is3d_options *options,
+                                is3d_hbt_fourier_result *result, is3d_stats *stats);
 
 /* FP64 FMA peak of the current device measured with a dependency-free DFMA chain (the roofline denominator;
  * MEASURED_PEAKS.json carries no FP64 figure).  Returns TFLOP/s in *tflops, SM clock not touched. */

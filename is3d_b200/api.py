@@ -568,3 +568,66 @@ def hbt_radii(sums):
         v = np.where(nz, r["S" + i + j], 0.0) / np.where(nz, s0, 1.0) - first[i] * first[j]
         out[name] = np.where(nz, v, 0.0)
     return out
+
+
+HBARC = 0.197327053          # GeV fm
+
+
+class HbtQrays(C.Structure):
+    _fields_ = [("n_dir", C.c_int32), ("n_q", C.c_int32), ("dq", C.c_double), ("dir", _D)]
+
+
+class HbtFourierResult(C.Structure):
+    _fields_ = [("Re", _D), ("Im", _D)]
+
+
+def hbt_fourier(flags, cells, species, grid, df_tables, qrays, memory="host", stream=None, multi=False):
+    """Call is3d_b200_hbt_fourier (or the _multi entry point over the devices of init_devices(), host arrays only).
+
+    qrays: dict dir (n_dir x 3 directions (o, s, l), not normalised), dq [GeV] and n_q; the q points are q_k = k dq dir, k < n_q.
+    cells must carry "x" and "y" [fm] as for hbt_moments().  Returns (dict Re, Im of RAW sums sum w cos(q.r / hbar c), sum w sin(...),
+    shape (n_dir, n_q, n_bins) with the spectra bin layout inside, numpy or CUDA tensors; stats dict).  Re[d, 0] is the spectrum;
+    hbt_correlation() turns the sums into C."""
+    device = (memory == "device")
+    m = _Marshal(device)
+    sf, sp, g, dft, _ = _marshal_problem(m, cells, species, grid, df_tables, None)
+    d = np.ascontiguousarray(np.asarray(qrays["dir"], dtype=np.float64).reshape(-1, 3))
+    n_dir, n_q = d.shape[0], int(qrays["n_q"])
+    qr = HbtQrays(n_dir, n_q, float(qrays["dq"]), d.ctypes.data_as(_D))
+    shape = (n_dir, max(n_q, 0), sp.n * g.n_pT * g.n_phi * g.n_y)
+    res = HbtFourierResult()
+    if device:
+        import torch
+        out = {k: torch.zeros(shape, dtype=torch.float64, device=cells["tau"].device) for k in ("Re", "Im")}
+        for k in out:
+            setattr(res, k, C.cast(C.c_void_p(out[k].data_ptr()), _D))
+        if stream is None:
+            stream = torch.cuda.current_stream().cuda_stream
+    else:
+        out = {k: np.zeros(shape) for k in ("Re", "Im")}
+        for k in out:
+            setattr(res, k, out[k].ctypes.data_as(_D))
+    opt = Options(); opt.memory = 1 if device else 0; opt.stream = C.c_void_p(stream or 0)
+    st = Stats()
+    fl = make_flags(flags)
+    f = lib().is3d_b200_hbt_fourier_multi if multi else lib().is3d_b200_hbt_fourier
+    f.restype = C.c_int
+    f.argtypes = [C.POINTER(Flags), C.POINTER(Surface), C.POINTER(Species), C.POINTER(Grid), C.POINTER(DfTables), C.POINTER(HbtQrays),
+                  C.POINTER(Options), C.POINTER(HbtFourierResult), C.POINTER(Stats)]
+    _check(f(C.byref(fl), C.byref(sf), C.byref(sp), C.byref(g), C.byref(dft), C.byref(qr), C.byref(opt), C.byref(res), C.byref(st)))
+    return out, st.as_dict()
+
+
+def hbt_correlation(sums, species):
+    """Correlation functions of identical particles from the raw sums of hbt_fourier(): C = 1 - sign (Re^2 + Im^2) / (g S0^2) with
+    S0 = Re[d, 0], sign = -1 (bosons) / +1 (fermions) and g the degeneracy of each bin's species; 1 where S0 = 0.  Shape (n_dir, n_q,
+    n_bins) -- the numbers results/hbt/C_<mcid>.dat holds."""
+    re, im = (np.asarray(sums[k].cpu() if _is_torch(sums[k]) else sums[k], dtype=np.float64) for k in ("Re", "Im"))
+    ns = len(species["sign"])
+    sign = np.resize(np.asarray(species["sign"], dtype=np.float64), re.shape[-1])        # bin = species + n_species * (...)
+    g = np.resize(np.asarray(species["degeneracy"], dtype=np.float64), re.shape[-1])
+    assert re.shape[-1] % ns == 0
+    s0 = re[:, :1, :]
+    nz = s0 != 0
+    r, m = re / np.where(nz, s0, 1.0), im / np.where(nz, s0, 1.0)          # ratios first: S0^2 underflows in the far tails
+    return np.where(nz, 1.0 - sign * (r * r + m * m) / g, 1.0)

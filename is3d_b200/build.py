@@ -27,6 +27,7 @@ SOURCES = [
     ("cf_shift.cu", []),
     ("cf_polzn.cu", []),
     ("cf_hbt.cu", []),
+    ("cf_hbtq.cu", []),
     ("cf_api.cu", []),
     ("host_math.cpp", []),
     ("host_io.cpp", []),

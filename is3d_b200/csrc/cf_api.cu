@@ -1379,17 +1379,40 @@ extern "C" int is3d_b200_spin_polarization_multi(const is3d_flags *fl, const is3
 // =====================================================================================================================
 namespace is3d {
 
-static int hbt_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_species *sp, const is3d_grid *gr, const is3d_df_tables *df,
-                    const is3d_options *opt_in, is3d_hbt_result *res, is3d_stats *stats)
+// What hbt_setup leaves for the kernel of an HBT entry point: the records of prepare_vh_kernel and prepare_hbt_cells_kernel on the
+// device, the HotParams both HBT kernels read, a zeroed sums buffer [n_arrays][n_bins], and the device's call lock, held until the
+// caller returns.  Events ev[0..2] are recorded (H2D, prepare); the caller launches its kernel and calls hbt_finish.
+struct HbtSetup {
+  std::unique_lock<std::mutex> lk;
+  Workspace *ws = nullptr;
+  is3d_options opt;
+  cudaStream_t st = nullptr;
+  int model = 0;
+  int64_t n_cells = 0, n_bins = 0, n_active = 0, n_chunks_wanted = 0, n_arrays = 0;
+  HotParams hp;
+  const double *C = nullptr, *cosphi = nullptr, *sinphi = nullptr;
+  const double *table = nullptr;         // the caller's extra table on the device
+  double *sums = nullptr;                // [n_arrays][n_bins]
+  PrepCounters cnt;
+};
+
+// Validation, layout, chunking, tables and surface to the device, prepare kernels and the table-range stop of every HBT entry point.
+//   what:               the path's name in error messages
+//   nyt, npt, ct:       register tile and TMA tile of the caller's kernel
+//   n_arrays:           partial rows per chunk and bin (the 4 GiB cap on the partial sums divides by it)
+//   blocks_per_bintile: blocks of the caller's grid per (group block, y tile, phi tile) and chunk
+//   table:              doubles the caller's kernel reads beside the species and momentum tables (may be empty)
+// The result arrays and any argument of the caller's own are checked by the caller first.
+static int hbt_setup(const is3d_flags *fl, const is3d_surface *sf, const is3d_species *sp, const is3d_grid *gr, const is3d_df_tables *df,
+                     const is3d_options *opt_in, const char *what, int nyt, int npt, int ct, int64_t n_arrays, int64_t blocks_per_bintile,
+                     const std::vector<double> &table, HbtSetup *S)
 {
-  if (!fl || !sf || !sp || !gr || !res) return fail(IS3D_ERR_ARGUMENT, "NULL argument");
-  double *out[kHbtSums] = {res->S0, res->So, res->Ss, res->Sl, res->Soo, res->Sss, res->Sll, res->Sos, res->Sol, res->Ssl};
-  for (double *p : out) if (!p) return fail(IS3D_ERR_ARGUMENT, "NULL result array");
-  if (fl->mode == 2) return fail(IS3D_ERR_UNSUPPORTED, "HBT moments need a viscous-hydro surface, not mode 2 (anisotropic hydro)");
+  const std::string name(what);
+  if (fl->mode == 2) return fail(IS3D_ERR_UNSUPPORTED, (name + " need a viscous-hydro surface, not mode 2 (anisotropic hydro)").c_str());
   if (fl->include_baryon) return fail(IS3D_ERR_UNSUPPORTED, "include_baryon = 1 (the reference's (T, muB) lookup reads out of bounds, SURVEY R8)");
-  if (fl->df_mode == 3 || fl->df_mode == 4) return fail(IS3D_ERR_UNSUPPORTED, "HBT moments cover the linear delta-f models (df_mode 1, 2), not the modified equilibrium");
+  if (fl->df_mode == 3 || fl->df_mode == 4) return fail(IS3D_ERR_UNSUPPORTED, (name + " cover the linear delta-f models (df_mode 1, 2), not the modified equilibrium").c_str());
   if (fl->df_mode != 1 && fl->df_mode != 2) return fail(IS3D_ERR_ARGUMENT, "df_mode must be 1..4");
-  if (!sf->x || !sf->y) return fail(IS3D_ERR_ARGUMENT, "HBT moments need the transverse cell positions (surface x, y)");
+  if (!sf->x || !sf->y) return fail(IS3D_ERR_ARGUMENT, (name + " need the transverse cell positions (surface x, y)").c_str());
   if (fl->dimension != 2 && fl->dimension != 3) return fail(IS3D_ERR_ARGUMENT, "dimension must be 2 or 3");
   if (sp->n <= 0 || gr->n_pT <= 0 || gr->n_phi <= 0 || gr->n_y <= 0) return fail(IS3D_ERR_ARGUMENT, "empty species list or momentum table");
   if (!sp->mass || !sp->sign || !sp->degeneracy || !gr->pT || !gr->phi || !gr->y) return fail(IS3D_ERR_ARGUMENT, "NULL species or momentum table");
@@ -1411,21 +1434,19 @@ static int hbt_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_spe
   Device *Dp = nullptr;
   { int rc = current_device(&Dp); if (rc) return rc; }
   Workspace &ws = Dp->ws;
-  std::lock_guard<std::mutex> lk(Dp->mu);
+  S->lk = std::unique_lock<std::mutex>(Dp->mu);
   is3d_options opt; memset(&opt, 0, sizeof(opt));
   if (opt_in) opt = *opt_in;
   cudaStream_t st = (cudaStream_t)opt.stream;
   const int64_t n_bins = (int64_t)sp->n * gr->n_pT * gr->n_phi * gr->n_y;
   const int64_t n_active = dim2 ? n_bins / gr->n_y : n_bins;        // 2+1D fills the y = 0 plane (index iy = 0)
 
-  // ---- layout: the cf_kernel decomposition with the register tile of cf_hbt_kernel; records of prepare_vh_kernel
+  // ---- layout: the cf_kernel decomposition with the caller's register tile; records of prepare_vh_kernel
   Layout L; memset(&L, 0, sizeof(L));
   L.n_species = sp->n; L.n_pT = gr->n_pT; L.n_phi = gr->n_phi; L.n_y_out = gr->n_y;
   L.dim2 = dim2 ? 1 : 0;
   L.n_slots = dim2 ? gr->n_eta : gr->n_y;
   L.rec_y = kRec;
-  int nyt, npt, ct;
-  hbt_shape(L.dim2, &nyt, &npt, &ct);
   L.nst = dim2 ? L.n_slots : nyt;
   L.n_ytiles = dim2 ? 1 : (L.n_slots + nyt - 1) / nyt;
   L.npt = npt; L.n_ptiles = (L.n_phi + npt - 1) / npt;
@@ -1435,14 +1456,14 @@ static int hbt_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_spe
   const int n_groups = (sp->n * gr->n_pT + 31) / 32;
   const int n_warps = std::min(kHbtWarps, n_groups);
   const int n_groupblocks = (n_groups + n_warps - 1) / n_warps;
-  const int64_t n_bintiles = (int64_t)n_groupblocks * L.n_ytiles * L.n_ptiles;
+  const int64_t n_bintiles = (int64_t)n_groupblocks * L.n_ytiles * L.n_ptiles * blocks_per_bintile;
   // chunks: the rule of smooth_core (>= 192 blocks per SM, a chunk's records within a third of L2, partial sums <= 4 GiB)
   int64_t n_chunks = ((int64_t)Dp->sm_count * 192 + n_bintiles - 1) / n_bintiles;
   const int64_t rec_per_cell = ((int64_t)L.n_ytiles * L.nst * kRec + (int64_t)L.n_ptiles * L.npt * kRec + kScal + kHbtRecC) * 8;
   const int64_t l2_target = std::max<int64_t>((int64_t)Dp->l2_bytes / 3, (int64_t)8 << 20);
   n_chunks = std::max<int64_t>(n_chunks, (n_cells * rec_per_cell + l2_target - 1) / l2_target);
   const int64_t n_chunks_wanted = n_chunks;
-  n_chunks = std::min<int64_t>(n_chunks, std::max<int64_t>(1, ((int64_t)4 << 30) / (kHbtSums * n_bins * 8)));
+  n_chunks = std::min<int64_t>(n_chunks, std::max<int64_t>(1, ((int64_t)4 << 30) / (n_arrays * n_bins * 8)));
   if (opt.n_chunks > 0) n_chunks = opt.n_chunks;
   n_chunks = std::max<int64_t>(1, std::min<int64_t>(n_chunks, std::max<int64_t>(L.n_tiles, 1)));
   if (n_bintiles * n_chunks > 2147483647LL) return fail(IS3D_ERR_ARGUMENT, "grid too large");
@@ -1455,6 +1476,7 @@ static int hbt_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_spe
   const size_t o_pT = ar.put(gr->pT, gr->n_pT), o_cos = ar.put(cosphi.data(), gr->n_phi), o_sin = ar.put(sinphi.data(), gr->n_phi);
   const size_t o_sloty = dim2 ? ar.put(gr->eta, gr->n_eta) : ar.put(gr->y, gr->n_y);
   const size_t o_slotw = dim2 ? ar.put(gr->eta_weight, gr->n_eta) : 0;
+  const size_t o_table = ar.put(table.data(), table.size());
   struct SplineOff { size_t x, y, c; int n; };
   auto put_spline = [&](const double *x, const double *y, int n) {
     SplineOff o{0, 0, 0, 0};
@@ -1472,8 +1494,8 @@ static int hbt_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_spe
   CU_CHECK(ws.P.reserve((size_t)L.n_ptiles * L.n_cells_pad * L.npt * kRec * 8 + 256));
   CU_CHECK(ws.S.reserve((size_t)L.n_cells_pad * kScal * 8 + 256));
   CU_CHECK(ws.extra.reserve((size_t)L.n_cells_pad * kHbtRecC * 8 + 256));          // per-cell [tau, x, y, 0]
-  CU_CHECK(ws.partial.reserve((size_t)kHbtSums * n_chunks * n_bins * 8 + 256));
-  CU_CHECK(ws.dN.reserve((size_t)kHbtSums * n_bins * 8 + 256));
+  CU_CHECK(ws.partial.reserve((size_t)n_arrays * n_chunks * n_bins * 8 + 256));
+  CU_CHECK(ws.dN.reserve((size_t)n_arrays * n_bins * 8 + 256));
   CU_CHECK(ws.counters.reserve(256));
   if (opt.memory == 0) CU_CHECK(ws.raw.reserve(cell_stride * kRaw + 256));
 
@@ -1494,8 +1516,8 @@ static int hbt_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_spe
   rc.n = n_cells; rc.tau = dev[0]; rc.eta = dev[1]; rc.dat = dev[2]; rc.dax = dev[3]; rc.day = dev[4]; rc.dan = dev[5];
   rc.ux = dev[6]; rc.uy = dev[7]; rc.un = dev[8]; rc.T = dev[9]; rc.P = dev[10]; rc.E = dev[11];
   rc.pixx = dev[12]; rc.pixy = dev[13]; rc.pixn = dev[14]; rc.piyy = dev[15]; rc.piyn = dev[16]; rc.bulkPi = dev[17];
-  double *sums_d = ws.dN.as<double>();                         // [10][n_bins] in the order of is3d_hbt_result
-  CU_CHECK(cudaMemsetAsync(sums_d, 0, (size_t)kHbtSums * n_bins * 8, st));
+  double *sums_d = ws.dN.as<double>();                         // [n_arrays][n_bins]
+  CU_CHECK(cudaMemsetAsync(sums_d, 0, (size_t)n_arrays * n_bins * 8, st));
   CU_CHECK(cudaMemsetAsync(ws.counters.p, 0, sizeof(PrepCounters), st));
   CU_CHECK(cudaEventRecord(ev[1], st));
 
@@ -1517,8 +1539,8 @@ static int hbt_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_spe
   CU_CHECK(cudaStreamSynchronize(st));
   if (cnt.range_error) return fail(IS3D_ERR_TABLE_RANGE, "a cell's T lies outside the delta-f coefficient table");
 
-  HbtParams prm; memset(&prm, 0, sizeof(prm));
-  HotParams &hp = prm.hp;
+  HotParams &hp = S->hp;
+  memset(&hp, 0, sizeof(hp));
   hp.L = L; hp.Y = ws.Y.as<double>(); hp.P = ws.P.as<double>(); hp.S = ws.S.as<double>();
   hp.mass = dptr(o_mass); hp.sign = dptr(o_sign); hp.degeneracy = dptr(o_deg); hp.pT = dptr(o_pT);
   hp.partial = ws.partial.as<double>();
@@ -1527,26 +1549,40 @@ static int hbt_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_spe
   hp.one_hi = 0x3ff00000;
   hp.outflow_thr = fl->outflow ? 0LL : (long long)0x8000000000000000ULL;
   hp.prefactor = pow(2.0 * M_PI * 0.197327053, -3);
-  prm.C = ws.extra.as<double>(); prm.cosphi = dptr(o_cos); prm.sinphi = dptr(o_sin);
-  CU_CHECK(launch_hbt(model, prm, st));
+  S->ws = &ws; S->opt = opt; S->st = st; S->model = model;
+  S->n_cells = n_cells; S->n_bins = n_bins; S->n_active = n_active; S->n_chunks_wanted = n_chunks_wanted; S->n_arrays = n_arrays;
+  S->C = ws.extra.as<double>(); S->cosphi = dptr(o_cos); S->sinphi = dptr(o_sin); S->table = dptr(o_table);
+  S->sums = sums_d; S->cnt = cnt;
+  return IS3D_OK;
+}
+
+// After the caller's kernel: fold the partial rows [n_arrays][n_chunks][n_bins] in a fixed order, add array q into out[q] (host or
+// device per options->memory), fill the stats.
+static int hbt_finish(HbtSetup &S, double *const *out, is3d_stats *stats)
+{
+  const HotParams &hp = S.hp;
+  const int64_t n_arrays = S.n_arrays, n_bins = S.n_bins, n_chunks = hp.n_chunks;
+  cudaStream_t st = S.st;
+  cudaEvent_t *ev = S.ws->ev;
   CU_CHECK(cudaEventRecord(ev[3], st));
-  for (int q = 0; q < kHbtSums; q++)
-    CU_CHECK(launch_reduce(hp.partial + (size_t)q * n_chunks * n_bins, (int)n_chunks, n_bins, n_active, sums_d + (size_t)q * n_bins, st));
+  for (int64_t q = 0; q < n_arrays; q++)
+    CU_CHECK(launch_reduce(hp.partial + (size_t)q * n_chunks * n_bins, (int)n_chunks, n_bins, S.n_active, S.sums + (size_t)q * n_bins, st));
   CU_CHECK(cudaEventRecord(ev[4], st));
 
   std::vector<double> host;
-  if (opt.memory == 0) {
-    host.resize((size_t)kHbtSums * n_bins);
-    CU_CHECK(cudaMemcpyAsync(host.data(), sums_d, (size_t)kHbtSums * n_bins * 8, cudaMemcpyDeviceToHost, st));
+  if (S.opt.memory == 0) {
+    host.resize((size_t)n_arrays * n_bins);
+    CU_CHECK(cudaMemcpyAsync(host.data(), S.sums, (size_t)n_arrays * n_bins * 8, cudaMemcpyDeviceToHost, st));
   } else {
-    for (int q = 0; q < kHbtSums; q++) CU_CHECK(launch_axpy(sums_d + (size_t)q * n_bins, out[q], n_active, st));
+    for (int64_t q = 0; q < n_arrays; q++) CU_CHECK(launch_axpy(S.sums + (size_t)q * n_bins, out[q], S.n_active, st));
   }
   CU_CHECK(cudaEventRecord(ev[5], st));
   CU_CHECK(cudaEventSynchronize(ev[5]));
-  if (opt.memory == 0)
-    for (int q = 0; q < kHbtSums; q++)
+  if (S.opt.memory == 0)
+    for (int64_t q = 0; q < n_arrays; q++)
       for (int64_t i = 0; i < n_bins; i++) out[q][i] += host[(size_t)q * n_bins + i];
 
+  const Layout &L = hp.L;
   is3d_stats stt; memset(&stt, 0, sizeof(stt));
   float ms;
   cudaEventElapsedTime(&ms, ev[0], ev[1]); stt.h2d_ms = ms;
@@ -1555,13 +1591,72 @@ static int hbt_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_spe
   cudaEventElapsedTime(&ms, ev[3], ev[4]); stt.reduce_ms = ms;
   cudaEventElapsedTime(&ms, ev[4], ev[5]); stt.d2h_ms = ms;
   cudaEventElapsedTime(&ms, ev[0], ev[5]); stt.total_ms = ms;
-  stt.cells_skipped_udsigma = (int64_t)cnt.skipped;
-  stt.evaluations = n_cells * (int64_t)sp->n * gr->n_pT * gr->n_phi * (int64_t)L.n_slots;
-  stt.gpu_launches = (n_cells > 0 ? 2 : 0) + 1 + kHbtSums + (opt.memory == 0 ? 0 : kHbtSums);
-  stt.n_chunks = (int)n_chunks; stt.n_chunks_wanted = (int)n_chunks_wanted;
+  stt.cells_skipped_udsigma = (int64_t)S.cnt.skipped;
+  stt.evaluations = S.n_cells * (int64_t)L.n_species * L.n_pT * L.n_phi * (int64_t)L.n_slots;
+  stt.gpu_launches = (int)((S.n_cells > 0 ? 2 : 0) + 1 + n_arrays + (S.opt.memory == 0 ? 0 : n_arrays));
+  stt.n_chunks = (int)n_chunks; stt.n_chunks_wanted = (int)S.n_chunks_wanted;
   stt.n_gpus = 1;
   if (stats) *stats = stt;
   return IS3D_OK;
+}
+
+static int hbt_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_species *sp, const is3d_grid *gr, const is3d_df_tables *df,
+                    const is3d_options *opt_in, is3d_hbt_result *res, is3d_stats *stats)
+{
+  if (!fl || !sf || !sp || !gr || !res) return fail(IS3D_ERR_ARGUMENT, "NULL argument");
+  double *out[kHbtSums] = {res->S0, res->So, res->Ss, res->Sl, res->Soo, res->Sss, res->Sll, res->Sos, res->Sol, res->Ssl};
+  for (double *p : out) if (!p) return fail(IS3D_ERR_ARGUMENT, "NULL result array");
+  int nyt, npt, ct;
+  hbt_shape(fl->dimension == 2, &nyt, &npt, &ct);
+  HbtSetup S;
+  { int rc = hbt_setup(fl, sf, sp, gr, df, opt_in, "HBT moments", nyt, npt, ct, kHbtSums, 1, std::vector<double>(), &S); if (rc) return rc; }
+  HbtParams prm; memset(&prm, 0, sizeof(prm));
+  prm.hp = S.hp; prm.C = S.C; prm.cosphi = S.cosphi; prm.sinphi = S.sinphi;
+  CU_CHECK(launch_hbt(S.model, prm, S.st));
+  return hbt_finish(S, out, stats);
+}
+
+// HBT Fourier sums (cf_hbtq.cu): the arguments of their own, checked before any set-up (the _multi entry point sizes its buffers by them)
+static int hbtq_check(const is3d_flags *fl, const is3d_surface *sf, const is3d_species *sp, const is3d_grid *gr, const is3d_hbt_qrays *qr,
+                      const is3d_hbt_fourier_result *res)
+{
+  if (!fl || !sf || !sp || !gr || !res || !qr) return fail(IS3D_ERR_ARGUMENT, "NULL argument");
+  if (!res->Re || !res->Im) return fail(IS3D_ERR_ARGUMENT, "NULL result array");
+  if (qr->n_dir < 1 || qr->n_q < 1) return fail(IS3D_ERR_ARGUMENT, "the q rays need n_dir >= 1 and n_q >= 1");
+  if (!qr->dir) return fail(IS3D_ERR_ARGUMENT, "NULL q-ray directions");
+  if (!std::isfinite(qr->dq) || qr->dq <= 0.0) return fail(IS3D_ERR_ARGUMENT, "the q step dq must be finite and > 0");
+  for (int64_t i = 0; i < 3 * (int64_t)qr->n_dir; i++)
+    if (!std::isfinite(qr->dir[i])) return fail(IS3D_ERR_ARGUMENT, "a q-ray direction component is not finite");
+  // the partial sums of one chunk: 2 n_dir n_q rows of n_bins doubles within the 4 GiB cap
+  const double n_arrays = 2.0 * qr->n_dir * (double)qr->n_q;
+  const double n_bins = (double)std::max(sp->n, 0) * std::max(gr->n_pT, 0) * std::max(gr->n_phi, 0) * std::max(gr->n_y, 0);
+  if (n_arrays * n_bins * 8.0 > (double)((int64_t)4 << 30))
+    return fail(IS3D_ERR_ARGUMENT, "2 n_dir n_q x n_bins sums exceed the 4 GiB partial-sum buffer even in one chunk: fewer q points, rays or bins per call");
+  return IS3D_OK;
+}
+
+// HBT Fourier sums (cf_hbtq.cu): Re / Im [n_dir][n_q][n_bins] of sum w e^{i theta}, added into the caller's arrays
+static int hbt_fourier_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_species *sp, const is3d_grid *gr, const is3d_df_tables *df,
+                            const is3d_hbt_qrays *qr, const is3d_options *opt_in, is3d_hbt_fourier_result *res, is3d_stats *stats)
+{
+  { int rc = hbtq_check(fl, sf, sp, gr, qr, res); if (rc) return rc; }
+  const int64_t n_arrays = 2 * (int64_t)qr->n_dir * qr->n_q;
+  const int n_qtiles = (qr->n_q + kHbtqKQ - 1) / kHbtqKQ;
+  const double step = qr->dq / 0.197327053;                      // [1/fm per GeV of q]
+  std::vector<double> dir(3 * (size_t)qr->n_dir);
+  for (size_t i = 0; i < dir.size(); i++) dir[i] = qr->dir[i] * step;
+  int nyt, npt, ct;
+  hbtq_shape(fl->dimension == 2, &nyt, &npt, &ct);
+  HbtSetup S;
+  { int rc = hbt_setup(fl, sf, sp, gr, df, opt_in, "HBT Fourier sums", nyt, npt, ct, n_arrays, (int64_t)qr->n_dir * n_qtiles, dir, &S); if (rc) return rc; }
+  HbtqParams prm; memset(&prm, 0, sizeof(prm));
+  prm.hp = S.hp; prm.C = S.C; prm.cosphi = S.cosphi; prm.sinphi = S.sinphi;
+  prm.dir = S.table; prm.n_dir = qr->n_dir; prm.n_q = qr->n_q; prm.n_qtiles = n_qtiles;
+  CU_CHECK(launch_hbt_fourier(S.model, prm, S.st));
+  const int64_t half = (int64_t)qr->n_dir * qr->n_q;
+  std::vector<double *> out((size_t)n_arrays);
+  for (int64_t a = 0; a < half; a++) { out[a] = res->Re + a * S.n_bins; out[half + a] = res->Im + a * S.n_bins; }
+  return hbt_finish(S, out.data(), stats);
 }
 
 }  // namespace is3d
@@ -1612,6 +1707,61 @@ extern "C" int is3d_b200_hbt_moments_multi(const is3d_flags *fl, const is3d_surf
   for (int d = 0; d < G; d++) if (rcs[d]) return fail(rcs[d], errs[d].c_str());
   for (int q = 0; q < kHbtSums; q++)
     for (size_t i = 0; i < n_bins; i++) { double v = 0.0; for (int d = 0; d < G; d++) v += bufs[d][q * n_bins + i]; out[q][i] += v; }
+  if (stats) {
+    is3d_stats tot; memset(&tot, 0, sizeof(tot));
+    for (int d = 0; d < G; d++) merge_stats(&tot, sts[d]);
+    tot.n_gpus = G;
+    *stats = tot;
+  }
+  return IS3D_OK;
+}
+
+extern "C" int is3d_b200_hbt_fourier(const is3d_flags *fl, const is3d_surface *sf, const is3d_species *sp, const is3d_grid *gr,
+                                     const is3d_df_tables *df, const is3d_hbt_qrays *qr, const is3d_options *opt, is3d_hbt_fourier_result *res,
+                                     is3d_stats *stats)
+{
+  return hbt_fourier_core(fl, sf, sp, gr, df, qr, opt, res, stats);
+}
+
+// Several devices: HOST arrays, contiguous cell shards, one thread per device; Re and Im are added on the host in device order
+extern "C" int is3d_b200_hbt_fourier_multi(const is3d_flags *fl, const is3d_surface *sf, const is3d_species *sp, const is3d_grid *gr,
+                                           const is3d_df_tables *df, const is3d_hbt_qrays *qr, const is3d_options *opt_in,
+                                           is3d_hbt_fourier_result *res, is3d_stats *stats)
+{
+  const int G = g_ngpus;
+  if (G <= 1) return is3d_b200_hbt_fourier(fl, sf, sp, gr, df, qr, opt_in, res, stats);
+  { int rc = hbtq_check(fl, sf, sp, gr, qr, res); if (rc) return rc; }
+  if (opt_in && opt_in->memory != 0) return fail(IS3D_ERR_ARGUMENT, "the multi-GPU entry point takes host arrays");
+  std::lock_guard<std::mutex> lk(g_multi_mutex);
+  const size_t n_bins = (size_t)std::max(sp->n, 0) * std::max(gr->n_pT, 0) * std::max(gr->n_phi, 0) * std::max(gr->n_y, 0);
+  const size_t n = (size_t)qr->n_dir * qr->n_q * n_bins;          // doubles per array (Re or Im)
+  int prev = 0; cudaGetDevice(&prev);
+  std::vector<int> rcs(G, IS3D_OK);
+  std::vector<std::string> errs(G);
+  std::vector<is3d_stats> sts(G);
+  std::vector<std::vector<double>> bufs(G, std::vector<double>(2 * n, 0.0));
+  std::vector<std::thread> workers;
+  for (int d = 0; d < G; d++) {
+    workers.emplace_back([&, d]() {
+      memset(&sts[d], 0, sizeof(is3d_stats));
+      if (cudaSetDevice(d) != cudaSuccess) { rcs[d] = IS3D_ERR_CUDA; errs[d] = "cudaSetDevice failed"; return; }
+      int64_t lo, hi;
+      shard_bounds(sf->n_cells, d, G, &lo, &hi);
+      const is3d_surface shard = shard_surface(*sf, lo, hi);
+      is3d_options opt; memset(&opt, 0, sizeof(opt));
+      if (opt_in) opt = *opt_in;
+      opt.memory = 0; opt.stream = g_streams[d];
+      is3d_hbt_fourier_result r{bufs[d].data(), bufs[d].data() + n};
+      rcs[d] = hbt_fourier_core(fl, &shard, sp, gr, df, qr, &opt, &r, &sts[d]);
+      if (rcs[d]) errs[d] = g_last_error;
+    });
+  }
+  for (auto &w : workers) w.join();
+  cudaSetDevice(prev);
+  for (int d = 0; d < G; d++) if (rcs[d]) return fail(rcs[d], errs[d].c_str());
+  double *out[2] = {res->Re, res->Im};
+  for (int q = 0; q < 2; q++)
+    for (size_t i = 0; i < n; i++) { double v = 0.0; for (int d = 0; d < G; d++) v += bufs[d][q * n + i]; out[q][i] += v; }
   if (stats) {
     is3d_stats tot; memset(&tot, 0, sizeof(tot));
     for (int d = 0; d < G; d++) merge_stats(&tot, sts[d]);

@@ -159,5 +159,18 @@ struct HbtParams {
 void hbt_shape(int dim2, int *nyt, int *npt, int *ct);
 cudaError_t launch_prepare_hbt_cells(const double *tau, const double *x, const double *y, int64_t n, int64_t n_pad, double *C, cudaStream_t st);
 cudaError_t launch_hbt(int model, const HbtParams &prm, cudaStream_t st);
+// HBT Fourier sums (cf_hbtq.cu): the records of cf_hbt_kernel; per bin and q point q_k = k dq d of every ray, sum w cos and sum w sin
+constexpr int kHbtqKQ = 21;       // q points per block (register tile of 2 KQ sums per bin); the phase recurrence restarts every KQ
+constexpr int kHbtqMinBlocks = 3; // blocks per SM of kHbtWarps warps the register budget is sized for (__launch_bounds__)
+constexpr int kHbtqNyt3D = 1, kHbtqNpt3D = 1, kHbtqNpt2D = 1;
+struct HbtqParams {
+  HotParams hp;                  // layout, records Y / P / S, species and pT tables, partial [2 n_dir n_q][n_chunks][n_bins], flags
+  const double *C;               // [n_cells_pad][kHbtRecC]
+  const double *cosphi, *sinphi; // [n_phi]
+  const double *dir;             // [n_dir][3]: d dq / hbar c [1/fm], (o, s, l)
+  int n_dir, n_q, n_qtiles;      // n_qtiles = ceil(n_q / kHbtqKQ)
+};
+void hbtq_shape(int dim2, int *nyt, int *npt, int *ct);
+cudaError_t launch_hbt_fourier(int model, const HbtqParams &prm, cudaStream_t st);
 
 }  // namespace is3d

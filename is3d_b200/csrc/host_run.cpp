@@ -249,6 +249,43 @@ static bool write_hbt_files(const std::string &wd, const std::vector<double> &su
   return true;
 }
 
+// results/hbt/C_<mcid>.dat: the correlation functions C = 1 - sign (Re^2 + Im^2) / (g S0^2) (C = 1 where S0 = 0) along the out, side and long
+// rays of is3d_b200_hbt_fourier for one species (re, im: [3][n_q][n_bins] of the one-species call), one row per (y, phi, pT, q) in that loop
+// order, the number format and blank line per phi block of write_hbt_files; truncating open, results/hbt/ must exist
+static bool write_correlation_file(const std::string &wd, const std::vector<double> &re, const std::vector<double> &im, int mcid, double sign,
+                                   double degeneracy, int n_q, double dq, const Grids &g, int dimension, std::string *err)
+{
+  const int npT = (int)g.pT.rows, nphi = (int)g.phi.rows, ny = (int)g.y.rows;
+  const int y_pts = (dimension == 2) ? 1 : ny;
+  const size_t n_bins = (size_t)npT * nphi * ny;
+  char name[255];
+  std::snprintf(name, sizeof(name), "%s/results/hbt/C_%d.dat", wd.c_str(), mcid);
+  std::ofstream f(name, std::ios_base::out);
+  if (!f) { *err = std::string("cannot open ") + name + " (the directory results/hbt/ must exist)"; return false; }
+  f << "y\tphip\tpT\tq\tS0\tC_out\tC_side\tC_long\n";
+  for (int iy = 0; iy < y_pts; iy++) {
+    const double y = (dimension == 2) ? 0.0 : g.y.at(1, iy + 1);
+    for (int iphi = 0; iphi < nphi; iphi++) {
+      for (int ipT = 0; ipT < npT; ipT++) {
+        const size_t b = (size_t)bin_index(0, 1, ipT, npT, iphi, nphi, iy);
+        const double s0 = re[b];
+        for (int k = 0; k < n_q; k++) {
+          f << std::scientific << std::setw(5) << std::setprecision(8) << y << "\t" << g.phi.at(1, iphi + 1) << "\t" << g.pT.at(1, ipT + 1) << "\t"
+            << k * dq << "\t" << s0;
+          for (int d = 0; d < 3; d++) {
+            const size_t i = ((size_t)d * n_q + k) * n_bins + b;
+            const double r = re[i] / s0, m = im[i] / s0;                 // ratios first: S0^2 underflows in the far tails
+            f << "\t" << (s0 != 0.0 ? 1.0 - sign * (r * r + m * m) / degeneracy : 1.0);
+          }
+          f << "\n";
+        }
+      }
+      f << "\n";
+    }
+  }
+  return true;
+}
+
 // everything the host layer derives from the input files
 struct Problem {
   Params par;
@@ -256,6 +293,10 @@ struct Problem {
   int operation = 0, hrg_eos = 0, group_particles = 0, do_resonance_decays = 0;
   int spin_polarization = 0;               // optional key (absent: 0): mode-5 spin polarization after the spectra
   int hbt_radii = 0;                       // optional key (absent: 0): HBT radii of the linear-delta-f spectra after the spectra
+  int hbt_correlation = 0;                 // optional key (absent: 0): MC id of the species whose HBT correlation functions are written
+  int hbt_species = -1;                    // its index among the chosen species
+  double hbt_dq = 0.005;                   // optional key: q step of the out, side and long rays [GeV]
+  int hbt_q_points = 41;                   // optional key: q points per ray (q = 0 included)
   std::vector<int> pick;                   // particle-list index of every chosen species (chosen_particles_sampling_table)
   SurfaceData sf;
   std::vector<Particle> pdg;
@@ -301,6 +342,15 @@ static int load_problem(const std::string &wd, bool need_surface, Problem *p, st
   if (p->hbt_radii && (p->operation != 1 || fl.mode == 2 || (fl.df_mode != 1 && fl.df_mode != 2) || fl.include_baryon)) {
     err = "hbt_radii = 1 needs operation = 1, a viscous-hydro surface (mode != 2), df_mode 1 or 2 and include_baryon = 0"; return IS3D_ERR_UNSUPPORTED;
   }
+  p->hbt_correlation = par.has("hbt_correlation") ? (int)par.get("hbt_correlation", &err) : 0;
+  if (p->hbt_correlation && (p->operation != 1 || fl.mode == 2 || (fl.df_mode != 1 && fl.df_mode != 2) || fl.include_baryon)) {
+    err = "hbt_correlation needs operation = 1, a viscous-hydro surface (mode != 2), df_mode 1 or 2 and include_baryon = 0"; return IS3D_ERR_UNSUPPORTED;
+  }
+  if (par.has("hbt_dq")) p->hbt_dq = par.get("hbt_dq", &err);
+  if (par.has("hbt_q_points")) p->hbt_q_points = (int)par.get("hbt_q_points", &err);
+  if (p->hbt_correlation && (!std::isfinite(p->hbt_dq) || p->hbt_dq <= 0.0 || p->hbt_q_points < 1)) {
+    err = "hbt_dq must be > 0 and hbt_q_points >= 1"; return IS3D_ERR_ARGUMENT;
+  }
   if (p->do_resonance_decays && p->hrg_eos == 3) { err = "do_resonance_decays = 1 needs a particle list with decay tables (hrg_eos = 1, 2); pdg_box.dat has none"; return IS3D_ERR_UNSUPPORTED; }
 
   // ---- surface (+ averages side file)
@@ -339,6 +389,10 @@ static int load_problem(const std::string &wd, bool need_surface, Problem *p, st
   for (int i = 0; i < npart; i++) {
     const Particle &h = p->pdg[pick[i]];
     p->mass[i] = h.mass; p->sign[i] = h.sign; p->degen[i] = h.gspin; p->baryon[i] = h.baryon; p->mcid[i] = (int)h.mcid;
+  }
+  if (p->hbt_correlation) {
+    for (int i = 0; i < npart && p->hbt_species < 0; i++) if (p->mcid[i] == p->hbt_correlation) p->hbt_species = i;
+    if (p->hbt_species < 0) { err = "hbt_correlation = " + std::to_string(p->hbt_correlation) + " is not among the chosen particles"; return IS3D_ERR_ARGUMENT; }
   }
   // ---- momentum tables (iS3D.cpp:161-167)
   Grids &g = p->g;
@@ -430,6 +484,20 @@ static int run_problem(const std::string &wd, Problem &P, const is3d_surface &s,
     if (rch != IS3D_OK) { err = std::string("HBT moments failed: ") + is3d_b200_last_error(); return rch; }
     if (stats) { stats->gpu_launches += hb_st.gpu_launches; stats->total_ms += hb_st.total_ms; }
     if (!write_hbt_files(wd, sums, P.mcid, g, P.fl.dimension, &err)) return IS3D_ERR_IO;
+  }
+  if (P.hbt_correlation) {
+    const int i = P.hbt_species, n_q = P.hbt_q_points;
+    is3d_species one{1, &P.mass[i], &P.sign[i], &P.degen[i], &P.baryon[i]};
+    static const double rays[9] = {1.0, 0.0, 0.0, 0.0, 1.0, 0.0, 0.0, 0.0, 1.0};        // out, side, long
+    is3d_hbt_qrays qr{3, n_q, P.hbt_dq, rays};
+    const size_t n = (size_t)3 * n_q * (n_bins / npart);
+    std::vector<double> re(n, 0.0), im(n, 0.0);
+    is3d_hbt_fourier_result r{re.data(), im.data()};
+    is3d_stats hq_st; std::memset(&hq_st, 0, sizeof(hq_st));
+    const int rcq = is3d_b200_hbt_fourier_multi(&P.fl, &s, &one, &gr, &dt, &qr, nullptr, &r, &hq_st);
+    if (rcq != IS3D_OK) { err = std::string("HBT correlation failed: ") + is3d_b200_last_error(); return rcq; }
+    if (stats) { stats->gpu_launches += hq_st.gpu_launches; stats->total_ms += hq_st.total_ms; }
+    if (!write_correlation_file(wd, re, im, P.mcid[i], P.sign[i], P.degen[i], n_q, P.hbt_dq, g, P.fl.dimension, &err)) return IS3D_ERR_IO;
   }
   if (P.do_resonance_decays) {
     // feed-down on the GPU, then the two amended-spectra files (emissionfunction.cpp:1689-1698)

@@ -29,8 +29,8 @@ DEFAULT_PARAMETERS = [
     ("r_max", 12.0), ("r_bins", 60),
 ]
 
-# keys of this drop-in that the reference does not read: written only when a caller sets them (absent means 0)
-OPTIONAL_PARAMETERS = ("spin_polarization", "hbt_radii")
+# keys of this drop-in that the reference does not read: written only when a caller sets them (absent: 0, or the default of the host layer)
+OPTIONAL_PARAMETERS = ("spin_polarization", "hbt_radii", "hbt_correlation", "hbt_dq", "hbt_q_points")
 
 _EOS_DIR = {1: "urqmd", 2: "smash", 3: "smash_box"}
 _EOS_PDG = {1: ("pdg_urqmd", "pdg-urqmd_v3.3+.dat"), 2: ("pdg_smash", "pdg_smash.dat"), 3: ("pdg_box", "pdg_box.dat")}
