@@ -200,7 +200,7 @@ int is3d_b200_resonance_decays(const is3d_particle_list *particles, int32_t n_ch
  * components (t, x, y, z), p^mu = (mT cosh y, pT cos phi, pT sin phi, mT sinh y), eps^{txyz} = +1.
  * Input: the six vorticity columns of a mode-5 surface, in file order the covariant Milne components varpi_{tau x}, varpi_{tau y},
  * varpi_{tau eta}, varpi_{xy}, varpi_{x eta}, varpi_{y eta} of varpi_{mu nu} = -(1/2)(d_mu beta_nu - d_nu beta_mu), beta = u/T
- * (dimensionless); they are converted to Cartesian components at the cell's eta (2+1D: the slot's eta) in cf_polzn.cu, cart_vorticity().
+ * (dimensionless); they are converted to Cartesian components at the cell's eta (2+1D: the slot's eta) in cf_polzn.cuh, cart_vorticity().
  * The five result arrays have the spectra layout ipart + n_species*(ipT + n_pT*(iphi + n_phi*iy)), hold the RAW sums N^mu and Snorm
  * (they add across cell shards and devices; the ratio S^mu does not) and are ADDED into; host or device memory per options->memory.
  * Errors: IS3D_ERR_UNSUPPORTED for mode = 2 and include_baryon = 1; IS3D_ERR_ARGUMENT for a NULL vorticity or a species with m <= 0.
@@ -214,6 +214,29 @@ int is3d_b200_spin_polarization(const is3d_flags *flags, const is3d_surface *sur
 int is3d_b200_spin_polarization_multi(const is3d_flags *flags, const is3d_surface *surface, const is3d_vorticity *vorticity,
                                       const is3d_species *species, const is3d_grid *grid, const is3d_options *options,
                                       is3d_polarization_result *result, is3d_stats *stats);
+
+/* ---- spin polarization of hadrons from thermal shear (shear-induced polarization) --------------------------------------------
+ * The second first-order term of the local-equilibrium mean spin vector (Becattini, Buzzegoli, Palermo 2021; Becattini, Buzzegoli,
+ * Inghirami, Karpenko, Palermo 2021), over the cells, slots, weights, species and bins of is3d_b200_spin_polarization:
+ *    N_xi^mu(p) = g/(2 pi hbar c)^3 sum_cells sum_slots w p.dsigma f (1 - sign f) (-1/(8m)) eps^{mu rho sigma tau} p_tau 2 that_rho xi_{sigma lambda} p^lambda / E
+ * with the thermal shear xi_{mu nu} = (1/2)(d_mu beta_nu + d_nu beta_mu), beta = u/T, that = (1, 0, 0, 0) the lab time direction,
+ * E = p^t = mT cosh y, and the prefactor and eps^{txyz} = +1 of the vorticity term, so that S^mu = (N^mu + N_xi^mu) / Snorm.
+ * In Cartesian lab components N_xi^t = 0 exactly and N_xi = -(1/(4 m E)) sum W (v x p), v_j = xi_jt E + xi_jl p^l (p.N_xi = 0).
+ * Input: the ten covariant Milne components xi_{tau tau}, xi_{tau x}, xi_{tau y}, xi_{tau eta}, xi_{xx}, xi_{xy}, xi_{x eta}, xi_{yy},
+ * xi_{y eta}, xi_{eta eta} (dimensionless, the convention of the mode-5 vorticity columns), converted to Cartesian components at the
+ * cell's eta (2+1D: the slot's eta) in cf_polzn.cuh, cart_shear().
+ * Results go into an is3d_polarization_result: St receives exact zeros, Sx, Sy, Sz the RAW sums N_xi, Snorm the ideal spectrum (bit for
+ * bit what is3d_b200_spin_polarization returns on the same device with the same options).  All are ADDED into; host or device memory
+ * per options->memory.  Errors: IS3D_ERR_UNSUPPORTED for mode = 2 and include_baryon = 1; IS3D_ERR_ARGUMENT for a NULL shear or shear
+ * array or a species with m <= 0. */
+typedef struct { const double *xtt, *xtx, *xty, *xtn, *xxx, *xxy, *xxn, *xyy, *xyn, *xnn; } is3d_thermal_shear;
+int is3d_b200_spin_polarization_shear(const is3d_flags *flags, const is3d_surface *surface, const is3d_thermal_shear *shear,
+                                      const is3d_species *species, const is3d_grid *grid, const is3d_options *options,
+                                      is3d_polarization_result *result, is3d_stats *stats);
+/* Same over the devices of is3d_b200_init_devices(): HOST arrays, contiguous cell shards, the five arrays summed on the host. */
+int is3d_b200_spin_polarization_shear_multi(const is3d_flags *flags, const is3d_surface *surface, const is3d_thermal_shear *shear,
+                                            const is3d_species *species, const is3d_grid *grid, const is3d_options *options,
+                                            is3d_polarization_result *result, is3d_stats *stats);
 
 /* ---- HBT radii: space-time variances of the Cooper-Frye emission function ---------------------------------------------
  * Gaussian (moment) approximation with pair momentum K = p (Wiedemann & Heinz, Phys. Rept. 319 (1999) 145).  For every spectra bin

@@ -492,11 +492,63 @@ def spin_polarization(flags, cells, vorticity, species, grid, memory="host", str
     return out, st.as_dict()
 
 
-def mean_spin(result, species, grid, dimension):
+THERMAL_SHEAR_FIELDS = ("xtt", "xtx", "xty", "xtn", "xxx", "xxy", "xxn", "xyy", "xyn", "xnn")
+
+
+class ThermalShear(C.Structure):
+    _fields_ = [(k, _D) for k in THERMAL_SHEAR_FIELDS]
+
+
+def spin_polarization_shear(flags, cells, shear, species, grid, memory="host", stream=None, multi=False):
+    """Call is3d_b200_spin_polarization_shear (or the _multi entry point over the devices of init_devices(), host arrays only).
+
+    shear: dict xtt, xtx, xty, xtn, xxx, xxy, xxn, xyy, xyn, xnn -- the ten covariant Milne components of the thermal shear
+    (dimensionless), numpy for memory='host', float64 CUDA tensors for memory='device'.  Returns (dict St, Sx, Sy, Sz, Snorm of RAW sums,
+    flat [y][phi][pT][species]: St = 0, Sx, Sy, Sz = N_xi, Snorm the ideal spectrum; stats dict).  mean_spin(vorticity_sums, ...,
+    shear=these) forms the total mean spin vector."""
+    device = (memory == "device")
+    m = _Marshal(device)
+    sf, sp, g, _, _ = _marshal_problem(m, cells, species, grid, None, None)
+    xi = None
+    if shear is not None:
+        xi = ThermalShear()
+        for k in THERMAL_SHEAR_FIELDS:
+            if shear.get(k) is not None:                      # a missing column stays NULL (the library rejects it)
+                setattr(xi, k, m.cells(shear[k]))
+    n = sp.n * g.n_pT * g.n_phi * g.n_y
+    res = PolarizationResult()
+    if device:
+        import torch
+        out = {k: torch.zeros(n, dtype=torch.float64, device=cells["tau"].device) for k in POLARIZATION_FIELDS}
+        for k in POLARIZATION_FIELDS:
+            setattr(res, k, C.cast(C.c_void_p(out[k].data_ptr()), _D))
+        if stream is None:
+            stream = torch.cuda.current_stream().cuda_stream
+    else:
+        out = {k: np.zeros(n) for k in POLARIZATION_FIELDS}
+        for k in POLARIZATION_FIELDS:
+            setattr(res, k, out[k].ctypes.data_as(_D))
+    opt = Options(); opt.memory = 1 if device else 0; opt.stream = C.c_void_p(stream or 0)
+    st = Stats()
+    fl = make_flags(flags)
+    f = lib().is3d_b200_spin_polarization_shear_multi if multi else lib().is3d_b200_spin_polarization_shear
+    f.restype = C.c_int
+    f.argtypes = [C.POINTER(Flags), C.POINTER(Surface), C.POINTER(ThermalShear), C.POINTER(Species), C.POINTER(Grid), C.POINTER(Options),
+                  C.POINTER(PolarizationResult), C.POINTER(Stats)]
+    _check(f(C.byref(fl), C.byref(sf), C.byref(xi) if xi is not None else None, C.byref(sp), C.byref(g), C.byref(opt), C.byref(res),
+             C.byref(st)))
+    return out, st.as_dict()
+
+
+def mean_spin(result, species, grid, dimension, shear=None):
     """Mean spin vector from the raw sums of spin_polarization(): returns (S [4][n_bins] = N^mu / Snorm in lab components t, x, y, z,
     0 where Snorm = 0; S* [3][n_bins] = S^i - S^t p^i / (E + m), the rest-frame spin, P* = 2 S* for spin 1/2).  The same numbers
-    results/polarization/S_<mcid>.dat holds."""
+    results/polarization/S_<mcid>.dat holds.  shear (optional): the raw sums of spin_polarization_shear() on the same problem; S is then
+    the total (N^mu + N_xi^mu) / Snorm and S* its rest-frame part, the totals of results/polarization/S_xi_<mcid>.dat."""
     r = {k: np.asarray(result[k].cpu() if _is_torch(result[k]) else result[k], dtype=np.float64) for k in POLARIZATION_FIELDS}
+    if shear is not None:
+        for k in ("St", "Sx", "Sy", "Sz"):
+            r[k] = r[k] + np.asarray(shear[k].cpu() if _is_torch(shear[k]) else shear[k], dtype=np.float64)
     m = np.asarray(species["mass"], dtype=np.float64)
     pT = np.asarray(grid["pT"], dtype=np.float64); phi = np.asarray(grid["phi"], dtype=np.float64)
     y = np.asarray(grid["y"], dtype=np.float64)

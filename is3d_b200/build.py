@@ -26,6 +26,7 @@ SOURCES = [
     ("cf_strict.cu", ["-fmad=false"]),
     ("cf_shift.cu", []),
     ("cf_polzn.cu", []),
+    ("cf_polzn_xi.cu", []),
     ("cf_hbt.cu", []),
     ("cf_hbtq.cu", []),
     ("cf_api.cu", []),

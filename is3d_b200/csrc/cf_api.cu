@@ -1160,15 +1160,19 @@ extern "C" int is3d_b200_spacetime_distributions_multi(const is3d_flags *fl, con
 }
 
 // =====================================================================================================================
-// Spin polarization from thermal vorticity (cf_polzn.cu): raw sums N^mu and Snorm, added into the caller's five arrays
+// Spin polarization from thermal vorticity (cf_polzn.cu) and thermal shear (cf_polzn_xi.cu): raw sums N^mu and Snorm, added into the
+// caller's five arrays
 // =====================================================================================================================
 namespace is3d {
 
-static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_vorticity *vo, const is3d_species *sp, const is3d_grid *gr,
-                      const is3d_options *opt_in, is3d_polarization_result *res, is3d_stats *stats)
+// tensor: the 6 vorticity columns (shear = false) or the 10 thermal-shear columns (shear = true), NULL for a NULL struct.  Both terms
+// run on the same layout and chunk split, so their Snorm is bit-identical; the shear kernel leaves St alone (N_xi^t = 0 exactly).
+static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const double *const *tensor, bool shear, const is3d_species *sp,
+                      const is3d_grid *gr, const is3d_options *opt_in, is3d_polarization_result *res, is3d_stats *stats)
 {
+  const int n_tensor = shear ? 10 : 6;
   if (!fl || !sf || !sp || !gr || !res) return fail(IS3D_ERR_ARGUMENT, "NULL argument");
-  if (!vo) return fail(IS3D_ERR_ARGUMENT, "NULL vorticity");
+  if (!tensor) return fail(IS3D_ERR_ARGUMENT, shear ? "NULL thermal shear" : "NULL vorticity");
   if (!res->St || !res->Sx || !res->Sy || !res->Sz || !res->Snorm) return fail(IS3D_ERR_ARGUMENT, "NULL result array");
   if (fl->mode == 2) return fail(IS3D_ERR_UNSUPPORTED, "spin polarization needs a viscous-hydro surface with thermal vorticity (mode 5), not mode 2");
   if (fl->include_baryon) return fail(IS3D_ERR_UNSUPPORTED, "include_baryon = 1 (the reference's (T, muB) lookup reads out of bounds, SURVEY R8)");
@@ -1180,10 +1184,12 @@ static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_v
   if (dim2 && (gr->n_eta <= 0 || !gr->eta || !gr->eta_weight)) return fail(IS3D_ERR_ARGUMENT, "dimension = 2 needs the eta table");
   const int64_t n_cells = sf->n_cells;
   if (n_cells < 0) return fail(IS3D_ERR_ARGUMENT, "negative cell count");
-  const double *raw_src[15] = {sf->tau, sf->eta, sf->dat, sf->dax, sf->day, sf->dan, sf->ux, sf->uy, sf->un, sf->T,
-                               vo->wtx, vo->wty, vo->wtn, vo->wxy, vo->wxn};
-  for (const double *p : raw_src) if (!p && n_cells > 0) return fail(IS3D_ERR_ARGUMENT, "a required surface or vorticity array is NULL");
-  if (!vo->wyn && n_cells > 0) return fail(IS3D_ERR_ARGUMENT, "a required surface or vorticity array is NULL");
+  const double *srcs[20] = {sf->tau, sf->eta, sf->dat, sf->dax, sf->day, sf->dan, sf->ux, sf->uy, sf->un, sf->T};
+  for (int a = 0; a < n_tensor; a++) srcs[10 + a] = tensor[a];
+  const int n_src = 10 + n_tensor;
+  for (int a = 0; a < n_src; a++)
+    if (!srcs[a] && n_cells > 0)
+      return fail(IS3D_ERR_ARGUMENT, shear ? "a required surface or thermal-shear array is NULL" : "a required surface or vorticity array is NULL");
   Device *Dp = nullptr;
   { int rc = current_device(&Dp); if (rc) return rc; }
   Workspace &ws = Dp->ws;
@@ -1231,8 +1237,6 @@ static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_v
   const size_t o_pT = ar.put(gr->pT, gr->n_pT), o_cos = ar.put(cosphi.data(), gr->n_phi), o_sin = ar.put(sinphi.data(), gr->n_phi);
   const size_t o_sloty = dim2 ? ar.put(gr->eta, gr->n_eta) : ar.put(gr->y, gr->n_y);
   const size_t o_slotw = dim2 ? ar.put(gr->eta_weight, gr->n_eta) : 0;
-  const double *srcs[16] = {sf->tau, sf->eta, sf->dat, sf->dax, sf->day, sf->dan, sf->ux, sf->uy, sf->un, sf->T,
-                            vo->wtx, vo->wty, vo->wtn, vo->wxy, vo->wxn, vo->wyn};
   const size_t cell_stride = ((size_t)n_cells * 8 + 255) & ~(size_t)255;
   CU_CHECK(ws.small.reserve(ar.host.size() + 256));
   CU_CHECK(ws.Y.reserve((size_t)L.n_ytiles * L.n_cells_pad * L.nst * kPolRecY * 8 + 256));
@@ -1240,14 +1244,14 @@ static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_v
   CU_CHECK(ws.partial.reserve((size_t)5 * n_chunks * n_bins * 8 + 256));
   CU_CHECK(ws.dN.reserve((size_t)5 * n_bins * 8 + 256));
   CU_CHECK(ws.counters.reserve(256));
-  if (opt.memory == 0) CU_CHECK(ws.raw.reserve(cell_stride * 16 + 256));
+  if (opt.memory == 0) CU_CHECK(ws.raw.reserve(cell_stride * n_src + 256));
 
   cudaEvent_t *ev = ws.ev;
   CU_CHECK(cudaEventRecord(ev[0], st));
   unsigned char *small_d = ws.small.as<unsigned char>();
   CU_CHECK(cudaMemcpyAsync(small_d, ar.host.data(), ar.host.size(), cudaMemcpyHostToDevice, st));
-  const double *dev[16];
-  for (int a = 0; a < 16; a++) {
+  const double *dev[20];
+  for (int a = 0; a < n_src; a++) {
     dev[a] = srcs[a];
     if (opt.memory == 0) {
       double *d = reinterpret_cast<double *>(ws.raw.as<unsigned char>() + cell_stride * a);
@@ -1258,9 +1262,9 @@ static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_v
   RawCells rc; memset(&rc, 0, sizeof(rc));
   rc.n = n_cells; rc.tau = dev[0]; rc.eta = dev[1]; rc.dat = dev[2]; rc.dax = dev[3]; rc.day = dev[4]; rc.dan = dev[5];
   rc.ux = dev[6]; rc.uy = dev[7]; rc.un = dev[8]; rc.T = dev[9];
-  const VortCells vc{dev[10], dev[11], dev[12], dev[13], dev[14], dev[15]};
-  double *sums_d = ws.dN.as<double>();                         // [5][n_bins]: Snorm, N^t, N^x, N^y, N^z
-  CU_CHECK(cudaMemsetAsync(sums_d, 0, (size_t)5 * n_bins * 8, st));
+  const int n_arr = shear ? 4 : 5;
+  double *sums_d = ws.dN.as<double>();                         // [n_arr][n_bins]: Snorm, (N^t,) N^x, N^y, N^z
+  CU_CHECK(cudaMemsetAsync(sums_d, 0, (size_t)n_arr * n_bins * 8, st));
   CU_CHECK(cudaMemsetAsync(ws.counters.p, 0, sizeof(PrepCounters), st));
   CU_CHECK(cudaEventRecord(ev[1], st));
 
@@ -1268,7 +1272,14 @@ static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_v
   PrepTables tab; memset(&tab, 0, sizeof(tab));
   tab.cosphi = dptr(o_cos); tab.sinphi = dptr(o_sin); tab.slot_y = dptr(o_sloty); tab.slot_w = dim2 ? dptr(o_slotw) : nullptr;
   PrepCounters *cnt_d = ws.counters.as<PrepCounters>();
-  CU_CHECK(launch_prepare_polzn(rc, vc, tab, L, ws.Y.as<double>(), ws.P.as<double>(), cnt_d, st));
+  if (shear) {
+    ShearCells xc;
+    for (int a = 0; a < 10; a++) xc.x[a] = dev[10 + a];
+    CU_CHECK(launch_prepare_polzn_xi(rc, xc, tab, L, ws.Y.as<double>(), ws.P.as<double>(), cnt_d, st));
+  } else {
+    const VortCells vc{dev[10], dev[11], dev[12], dev[13], dev[14], dev[15]};
+    CU_CHECK(launch_prepare_polzn(rc, vc, tab, L, ws.Y.as<double>(), ws.P.as<double>(), cnt_d, st));
+  }
   CU_CHECK(cudaEventRecord(ev[2], st));
 
   HotParams hp; memset(&hp, 0, sizeof(hp));
@@ -1278,26 +1289,32 @@ static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_v
   hp.n_chunks = (int)n_chunks; hp.n_groupblocks = n_groupblocks; hp.n_warps = n_warps;
   hp.outflow_thr = fl->outflow ? 0LL : (long long)0x8000000000000000ULL;
   hp.prefactor = pow(2.0 * M_PI * 0.197327053, -3);
-  CU_CHECK(launch_polzn(hp, st));
+  if (shear) {
+    const PolXiParams prm{hp, dptr(o_cos), dptr(o_sin), dim2 ? nullptr : dptr(o_sloty)};
+    CU_CHECK(launch_polzn_xi(prm, st));
+  } else {
+    CU_CHECK(launch_polzn(hp, st));
+  }
   CU_CHECK(cudaEventRecord(ev[3], st));
-  for (int q = 0; q < 5; q++)
+  for (int q = 0; q < n_arr; q++)
     CU_CHECK(launch_reduce(hp.partial + (size_t)q * n_chunks * n_bins, (int)n_chunks, n_bins, n_active, sums_d + (size_t)q * n_bins, st));
   CU_CHECK(cudaEventRecord(ev[4], st));
 
-  double *out[5] = {res->Snorm, res->St, res->Sx, res->Sy, res->Sz};
+  double *out_vort[5] = {res->Snorm, res->St, res->Sx, res->Sy, res->Sz}, *out_xi[4] = {res->Snorm, res->Sx, res->Sy, res->Sz};
+  double *const *out = shear ? out_xi : out_vort;
   std::vector<double> host;
   if (opt.memory == 0) {
-    host.resize((size_t)5 * n_bins);
-    CU_CHECK(cudaMemcpyAsync(host.data(), sums_d, (size_t)5 * n_bins * 8, cudaMemcpyDeviceToHost, st));
+    host.resize((size_t)n_arr * n_bins);
+    CU_CHECK(cudaMemcpyAsync(host.data(), sums_d, (size_t)n_arr * n_bins * 8, cudaMemcpyDeviceToHost, st));
   } else {
-    for (int q = 0; q < 5; q++) CU_CHECK(launch_axpy(sums_d + (size_t)q * n_bins, out[q], n_active, st));
+    for (int q = 0; q < n_arr; q++) CU_CHECK(launch_axpy(sums_d + (size_t)q * n_bins, out[q], n_active, st));
   }
   PrepCounters cnt; memset(&cnt, 0, sizeof(cnt));
   CU_CHECK(cudaMemcpyAsync(&cnt, cnt_d, sizeof(cnt), cudaMemcpyDeviceToHost, st));
   CU_CHECK(cudaEventRecord(ev[5], st));
   CU_CHECK(cudaEventSynchronize(ev[5]));
   if (opt.memory == 0)
-    for (int q = 0; q < 5; q++)
+    for (int q = 0; q < n_arr; q++)
       for (int64_t i = 0; i < n_bins; i++) out[q][i] += host[(size_t)q * n_bins + i];
 
   is3d_stats stt; memset(&stt, 0, sizeof(stt));
@@ -1310,7 +1327,7 @@ static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_v
   cudaEventElapsedTime(&ms, ev[0], ev[5]); stt.total_ms = ms;
   stt.cells_skipped_udsigma = (int64_t)cnt.skipped;
   stt.evaluations = n_cells * (int64_t)sp->n * gr->n_pT * gr->n_phi * (int64_t)L.n_slots;
-  stt.gpu_launches = (n_cells > 0 ? 1 : 0) + 1 + 5 + (opt.memory == 0 ? 0 : 5);
+  stt.gpu_launches = (n_cells > 0 ? 1 : 0) + 1 + n_arr + (opt.memory == 0 ? 0 : n_arr);
   stt.n_chunks = (int)n_chunks; stt.n_chunks_wanted = (int)n_chunks_wanted;
   stt.n_gpus = 1;
   if (stats) *stats = stt;
@@ -1319,21 +1336,18 @@ static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_v
 
 }  // namespace is3d
 
-extern "C" int is3d_b200_spin_polarization(const is3d_flags *fl, const is3d_surface *sf, const is3d_vorticity *vo, const is3d_species *sp,
-                                           const is3d_grid *gr, const is3d_options *opt, is3d_polarization_result *res, is3d_stats *stats)
-{
-  return polzn_core(fl, sf, vo, sp, gr, opt, res, stats);
-}
+namespace is3d {
 
 // Several devices: HOST arrays, contiguous cell shards, one thread per device; the five raw sums are added on the host in device order
-extern "C" int is3d_b200_spin_polarization_multi(const is3d_flags *fl, const is3d_surface *sf, const is3d_vorticity *vo, const is3d_species *sp,
-                                                 const is3d_grid *gr, const is3d_options *opt_in, is3d_polarization_result *res, is3d_stats *stats)
+static int polzn_multi(const is3d_flags *fl, const is3d_surface *sf, const double *const *tensor, bool shear, const is3d_species *sp,
+                       const is3d_grid *gr, const is3d_options *opt_in, is3d_polarization_result *res, is3d_stats *stats)
 {
   const int G = g_ngpus;
-  if (G <= 1) return is3d_b200_spin_polarization(fl, sf, vo, sp, gr, opt_in, res, stats);
-  if (!fl || !sf || !vo || !sp || !gr || !res) return fail(IS3D_ERR_ARGUMENT, vo ? "NULL argument" : "NULL vorticity");
+  if (G <= 1) return polzn_core(fl, sf, tensor, shear, sp, gr, opt_in, res, stats);
+  if (!fl || !sf || !tensor || !sp || !gr || !res) return fail(IS3D_ERR_ARGUMENT, tensor ? "NULL argument" : shear ? "NULL thermal shear" : "NULL vorticity");
   if (opt_in && opt_in->memory != 0) return fail(IS3D_ERR_ARGUMENT, "the multi-GPU entry point takes host arrays");
   std::lock_guard<std::mutex> lk(g_multi_mutex);
+  const int n_tensor = shear ? 10 : 6;
   const size_t n_bins = (size_t)std::max(sp->n, 0) * std::max(gr->n_pT, 0) * std::max(gr->n_phi, 0) * std::max(gr->n_y, 0);
   int prev = 0; cudaGetDevice(&prev);
   std::vector<int> rcs(G, IS3D_OK);
@@ -1348,14 +1362,14 @@ extern "C" int is3d_b200_spin_polarization_multi(const is3d_flags *fl, const is3
       int64_t lo, hi;
       shard_bounds(sf->n_cells, d, G, &lo, &hi);
       const is3d_surface shard = shard_surface(*sf, lo, hi);
-      auto off = [&](const double *p) { return p ? p + lo : p; };
-      const is3d_vorticity vs{off(vo->wtx), off(vo->wty), off(vo->wtn), off(vo->wxy), off(vo->wxn), off(vo->wyn)};
+      const double *ts[10];
+      for (int a = 0; a < n_tensor; a++) ts[a] = tensor[a] ? tensor[a] + lo : tensor[a];
       is3d_options opt; memset(&opt, 0, sizeof(opt));
       if (opt_in) opt = *opt_in;
       opt.memory = 0; opt.stream = g_streams[d];
       double *b = bufs[d].data();
       is3d_polarization_result r{b, b + n_bins, b + 2 * n_bins, b + 3 * n_bins, b + 4 * n_bins};
-      rcs[d] = polzn_core(fl, &shard, &vs, sp, gr, &opt, &r, &sts[d]);
+      rcs[d] = polzn_core(fl, &shard, ts, shear, sp, gr, &opt, &r, &sts[d]);
       if (rcs[d]) errs[d] = g_last_error;
     });
   }
@@ -1372,6 +1386,54 @@ extern "C" int is3d_b200_spin_polarization_multi(const is3d_flags *fl, const is3
     *stats = tot;
   }
   return IS3D_OK;
+}
+
+// the columns of the two input structs in the order of the prepare kernels, or NULL for a NULL struct
+static const double *const *vort_columns(const is3d_vorticity *vo, const double **c)
+{
+  if (!vo) return nullptr;
+  const double *v[6] = {vo->wtx, vo->wty, vo->wtn, vo->wxy, vo->wxn, vo->wyn};
+  for (int a = 0; a < 6; a++) c[a] = v[a];
+  return c;
+}
+static const double *const *shear_columns(const is3d_thermal_shear *xi, const double **c)
+{
+  if (!xi) return nullptr;
+  const double *v[10] = {xi->xtt, xi->xtx, xi->xty, xi->xtn, xi->xxx, xi->xxy, xi->xxn, xi->xyy, xi->xyn, xi->xnn};
+  for (int a = 0; a < 10; a++) c[a] = v[a];
+  return c;
+}
+
+}  // namespace is3d
+
+extern "C" int is3d_b200_spin_polarization(const is3d_flags *fl, const is3d_surface *sf, const is3d_vorticity *vo, const is3d_species *sp,
+                                           const is3d_grid *gr, const is3d_options *opt, is3d_polarization_result *res, is3d_stats *stats)
+{
+  const double *c[6];
+  return polzn_core(fl, sf, vort_columns(vo, c), false, sp, gr, opt, res, stats);
+}
+
+extern "C" int is3d_b200_spin_polarization_multi(const is3d_flags *fl, const is3d_surface *sf, const is3d_vorticity *vo, const is3d_species *sp,
+                                                 const is3d_grid *gr, const is3d_options *opt, is3d_polarization_result *res, is3d_stats *stats)
+{
+  const double *c[6];
+  return polzn_multi(fl, sf, vort_columns(vo, c), false, sp, gr, opt, res, stats);
+}
+
+extern "C" int is3d_b200_spin_polarization_shear(const is3d_flags *fl, const is3d_surface *sf, const is3d_thermal_shear *xi,
+                                                 const is3d_species *sp, const is3d_grid *gr, const is3d_options *opt,
+                                                 is3d_polarization_result *res, is3d_stats *stats)
+{
+  const double *c[10];
+  return polzn_core(fl, sf, shear_columns(xi, c), true, sp, gr, opt, res, stats);
+}
+
+extern "C" int is3d_b200_spin_polarization_shear_multi(const is3d_flags *fl, const is3d_surface *sf, const is3d_thermal_shear *xi,
+                                                       const is3d_species *sp, const is3d_grid *gr, const is3d_options *opt,
+                                                       is3d_polarization_result *res, is3d_stats *stats)
+{
+  const double *c[10];
+  return polzn_multi(fl, sf, shear_columns(xi, c), true, sp, gr, opt, res, stats);
 }
 
 // =====================================================================================================================

@@ -145,6 +145,16 @@ cudaError_t launch_prepare_polzn(const RawCells &cells, const VortCells &vort, c
                                  PrepCounters *counters, cudaStream_t st);
 // partial: [5][n_chunks][n_bins]
 cudaError_t launch_polzn(const HotParams &hp, cudaStream_t st);
+// thermal-shear part of the spin polarization (cf_polzn_xi.cu): the layout, records sizes and chunks of cf_polzn.cu, 4 sums per bin
+struct ShearCells { const double *x[10]; };    // device pointers, covariant Milne components tautau taux tauy taueta xx xy xeta yy yeta etaeta
+struct PolXiParams {
+  HotParams hp;                  // layout, records Y / P, species and pT tables, partial [4][n_chunks][n_bins] (Snorm, N^x, N^y, N^z)
+  const double *cosphi, *sinphi; // [n_phi]
+  const double *y;               // 3+1D: the y table [n_y]; 2+1D: unused (y = 0)
+};
+cudaError_t launch_prepare_polzn_xi(const RawCells &cells, const ShearCells &shear, const PrepTables &tab, const Layout &L, double *Y,
+                                    double *P, PrepCounters *counters, cudaStream_t st);
+cudaError_t launch_polzn_xi(const PolXiParams &prm, cudaStream_t st);
 // HBT moments (cf_hbt.cu): the records of prepare_vh_kernel plus a per-cell record [tau, x, y, 0]; 10 sums per bin
 constexpr int kHbtRecC = 4;      // doubles per per-cell position record
 constexpr int kHbtSums = 10;     // S0, So, Ss, Sl, Soo, Sss, Sll, Sos, Sol, Ssl

@@ -208,6 +208,33 @@ struct Tokens {
   }
 };
 
+bool read_thermal_shear(const std::string &workdir, SurfaceData *s, std::string *err)
+{
+  const std::string path = workdir + "/input/thermal_shear.dat";
+  std::string text;
+  if (!slurp(path, &text)) { if (err) *err = "cannot open " + path + " (thermal_shear_polarization = 1 reads it)"; return false; }
+  int64_t lines = 0;
+  for (char c : text) if (c == '\n') lines++;
+  if (lines != s->n) {
+    if (err) *err = path + " has " + std::to_string(lines) + " lines, the surface has " + std::to_string(s->n) + " cells";
+    return false;
+  }
+  std::vector<double> *col[10] = {&s->xtt, &s->xtx, &s->xty, &s->xtn, &s->xxx, &s->xxy, &s->xxn, &s->xyy, &s->xyn, &s->xnn};
+  for (std::vector<double> *v : col) v->assign((size_t)s->n, 0.0);
+  const char *p = text.data(), *end = text.data() + text.size();
+  for (int64_t i = 0; i < s->n; i++) {
+    const char *eol = static_cast<const char *>(std::memchr(p, '\n', (size_t)(end - p)));
+    Tokens tk{p, eol};
+    for (std::vector<double> *v : col)
+      if (!tk.next(&(*v)[i])) {
+        if (err) *err = path + ": line " + std::to_string(i + 1) + " has fewer than ten numbers";
+        return false;
+      }
+    p = eol + 1;
+  }
+  return true;
+}
+
 bool read_surface(const std::string &workdir, const SurfaceFlags &fl, SurfaceData *s, std::string *err)
 {
   const std::string path = workdir + "/input/surface.dat";

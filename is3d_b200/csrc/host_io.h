@@ -48,6 +48,7 @@ struct SurfaceData {
   std::vector<double> muB, nB, Vx, Vy, Vn;
   std::vector<double> PL, Wx, Wy, Lambda, aL, c0, c1, c2, c3, c4;     // anisotropic hydro (mode 2)
   std::vector<double> wtx, wty, wtn, wxy, wxn, wyn;                    // thermal vorticity, covariant Milne components (mode 5)
+  std::vector<double> xtt, xtx, xty, xtn, xxx, xxy, xxn, xyy, xyn, xnn;   // thermal shear, covariant Milne components (input/thermal_shear.dat)
   bool averages_written = false;
   double avg[5] = {0, 0, 0, 0, 0};   // T, E, P, muB, nB after the 15-digit text round trip of the side file
 };
@@ -55,6 +56,10 @@ struct SurfaceFlags { int mode, dimension, df_mode, include_baryon, include_bary
 // input/surface.dat, formats of FO_data_reader::read_surf_VH_old / read_surf_VH / read_surf_VAH_PLMatch
 // (readindata.cpp:148-468, 813-928); also writes and re-reads average_thermodynamic_quantities.dat like the reference.
 bool read_surface(const std::string &workdir, const SurfaceFlags &fl, SurfaceData *out, std::string *err);
+// input/thermal_shear.dat (this project's own format): one newline-terminated line per surface cell, in surface order, with the ten
+// covariant Milne components xi_{tau tau} xi_{tau x} xi_{tau y} xi_{tau eta} xi_{xx} xi_{xy} xi_{x eta} xi_{yy} xi_{y eta} xi_{eta eta}
+// (dimensionless).  A missing file, a line count other than out->n or a line with fewer than ten numbers is an error.
+bool read_thermal_shear(const std::string &workdir, SurfaceData *out, std::string *err);
 
 struct DfTables {
   int n_T = 0, n_muB_file = 0;

@@ -178,20 +178,25 @@ static bool write_spacetime_files(const std::string &wd, const std::vector<int> 
 
 // results/polarization/S_<mcid>.dat: mean spin vector S^mu = N^mu / Snorm (lab frame, Cartesian t, x, y, z; 0 where Snorm = 0) and its
 // rest-frame spatial part S*_i = S^i - S^t p^i / (E + m), one row per (y, phi, pT) in the loop order, number format and blank line per
-// phi block of write_spectra_files; truncating opens, results/polarization/ must exist
-static bool write_polarization_files(const std::string &wd, const std::vector<double> &sums, const std::vector<int> &mcid,
-                                     const std::vector<double> &mass, const Grids &g, int dimension, std::string *err)
+// phi block of write_spectra_files; truncating opens, results/polarization/ must exist.
+// With the thermal-shear sums xi (St | Sx | Sy | Sz | Snorm of is3d_b200_spin_polarization_shear, non-NULL) it writes S_xi_<mcid>.dat
+// instead: Snorm, the shear part N_xi / Snorm, the total S = (N + N_xi) / Snorm and the rest-frame part of the total.
+static bool write_polarization_files(const std::string &wd, const std::vector<double> &sums, const std::vector<double> *xi,
+                                     const std::vector<int> &mcid, const std::vector<double> &mass, const Grids &g, int dimension,
+                                     std::string *err)
 {
   const int npart = (int)mcid.size(), npT = (int)g.pT.rows, nphi = (int)g.phi.rows, ny = (int)g.y.rows;
   const int y_pts = (dimension == 2) ? 1 : ny;
   const size_t n_bins = (size_t)npart * npT * nphi * ny;
   const double *St = &sums[0], *Sx = St + n_bins, *Sy = Sx + n_bins, *Sz = Sy + n_bins, *Sn = Sz + n_bins;
+  const double *Xx = xi ? &(*xi)[n_bins] : nullptr, *Xy = xi ? Xx + n_bins : nullptr, *Xz = xi ? Xy + n_bins : nullptr;
   for (int ipart = 0; ipart < npart; ipart++) {
     char name[255];
-    std::snprintf(name, sizeof(name), "%s/results/polarization/S_%d.dat", wd.c_str(), mcid[ipart]);
+    std::snprintf(name, sizeof(name), xi ? "%s/results/polarization/S_xi_%d.dat" : "%s/results/polarization/S_%d.dat", wd.c_str(), mcid[ipart]);
     std::ofstream f(name, std::ios_base::out);
     if (!f) { *err = std::string("cannot open ") + name + " (the directory results/polarization/ must exist)"; return false; }
-    f << "y\tphip\tpT\tSnorm\tSt\tSx\tSy\tSz\tSx_rest\tSy_rest\tSz_rest\n";
+    f << (xi ? "y\tphip\tpT\tSnorm\tSx_xi\tSy_xi\tSz_xi\tSx\tSy\tSz\tSx_rest\tSy_rest\tSz_rest\n"
+             : "y\tphip\tpT\tSnorm\tSt\tSx\tSy\tSz\tSx_rest\tSy_rest\tSz_rest\n");
     const double m = mass[ipart];
     for (int iy = 0; iy < y_pts; iy++) {
       const double y = (dimension == 2) ? 0.0 : g.y.at(1, iy + 1);
@@ -201,10 +206,15 @@ static bool write_polarization_files(const std::string &wd, const std::vector<do
           const double pT = g.pT.at(1, ipT + 1), mT = std::sqrt(m * m + pT * pT);
           const double E = mT * std::cosh(y), p[3] = {pT * std::cos(phi), pT * std::sin(phi), mT * std::sinh(y)};
           const size_t b = (size_t)bin_index(ipart, npart, ipT, npT, iphi, nphi, iy);
-          double S[4] = {0.0, 0.0, 0.0, 0.0};
+          double S[4] = {0.0, 0.0, 0.0, 0.0}, X[3] = {0.0, 0.0, 0.0};
           if (Sn[b] != 0.0) { S[0] = St[b] / Sn[b]; S[1] = Sx[b] / Sn[b]; S[2] = Sy[b] / Sn[b]; S[3] = Sz[b] / Sn[b]; }
+          if (xi && Sn[b] != 0.0) {
+            X[0] = Xx[b] / Sn[b]; X[1] = Xy[b] / Sn[b]; X[2] = Xz[b] / Sn[b];
+            S[1] = (Sx[b] + Xx[b]) / Sn[b]; S[2] = (Sy[b] + Xy[b]) / Sn[b]; S[3] = (Sz[b] + Xz[b]) / Sn[b];
+          }
           f << std::scientific << std::setw(5) << std::setprecision(8) << y << "\t" << phi << "\t" << pT << "\t" << Sn[b];
-          for (int k = 0; k < 4; k++) f << "\t" << S[k];
+          if (xi) for (int k = 0; k < 3; k++) f << "\t" << X[k];
+          for (int k = xi ? 1 : 0; k < 4; k++) f << "\t" << S[k];
           for (int k = 0; k < 3; k++) f << "\t" << S[k + 1] - S[0] * p[k] / (E + m);
           f << "\n";
         }
@@ -292,6 +302,7 @@ struct Problem {
   is3d_flags fl;
   int operation = 0, hrg_eos = 0, group_particles = 0, do_resonance_decays = 0;
   int spin_polarization = 0;               // optional key (absent: 0): mode-5 spin polarization after the spectra
+  int thermal_shear_polarization = 0;      // optional key (absent: 0): add the thermal-shear term (input/thermal_shear.dat)
   int hbt_radii = 0;                       // optional key (absent: 0): HBT radii of the linear-delta-f spectra after the spectra
   int hbt_correlation = 0;                 // optional key (absent: 0): MC id of the species whose HBT correlation functions are written
   int hbt_species = -1;                    // its index among the chosen species
@@ -338,6 +349,10 @@ static int load_problem(const std::string &wd, bool need_surface, Problem *p, st
   if (p->do_resonance_decays && p->operation != 1) { err = "do_resonance_decays = 1 applies to operation = 1 (the reference runs it after the spectra, emissionfunction.cpp:1689)"; return IS3D_ERR_UNSUPPORTED; }
   p->spin_polarization = par.has("spin_polarization") ? (int)par.get("spin_polarization", &err) : 0;
   if (p->spin_polarization && (p->operation != 1 || fl.mode != 5)) { err = "spin_polarization = 1 needs operation = 1 and a mode 5 surface (the thermal vorticity columns)"; return IS3D_ERR_UNSUPPORTED; }
+  p->thermal_shear_polarization = par.has("thermal_shear_polarization") ? (int)par.get("thermal_shear_polarization", &err) : 0;
+  if (p->thermal_shear_polarization && (p->operation != 1 || fl.mode != 5 || !p->spin_polarization)) {
+    err = "thermal_shear_polarization = 1 needs operation = 1, a mode 5 surface and spin_polarization = 1"; return IS3D_ERR_UNSUPPORTED;
+  }
   p->hbt_radii = par.has("hbt_radii") ? (int)par.get("hbt_radii", &err) : 0;
   if (p->hbt_radii && (p->operation != 1 || fl.mode == 2 || (fl.df_mode != 1 && fl.df_mode != 2) || fl.include_baryon)) {
     err = "hbt_radii = 1 needs operation = 1, a viscous-hydro surface (mode != 2), df_mode 1 or 2 and include_baryon = 0"; return IS3D_ERR_UNSUPPORTED;
@@ -357,6 +372,7 @@ static int load_problem(const std::string &wd, bool need_surface, Problem *p, st
   if (need_surface) {
     SurfaceFlags sfl{fl.mode, fl.dimension, fl.df_mode, fl.include_baryon, fl.include_baryondiff_deltaf};
     if (!read_surface(wd, sfl, &p->sf, &err)) return IS3D_ERR_IO;
+    if (p->thermal_shear_polarization && !read_thermal_shear(wd, &p->sf, &err)) return IS3D_ERR_IO;
   }
   // ---- particle list, delta-f tables
   if (!read_pdg(wd, p->hrg_eos, &p->pdg, &err)) return IS3D_ERR_IO;
@@ -403,8 +419,8 @@ static int load_problem(const std::string &wd, bool need_surface, Problem *p, st
   return IS3D_OK;
 }
 
-static int run_problem(const std::string &wd, Problem &P, const is3d_surface &s, const is3d_vorticity *vort, double *dN_raw, int64_t n_raw, int32_t *mcid_out,
-                       int32_t n_mcid_max, is3d_stats *stats, std::string *err_out)
+static int run_problem(const std::string &wd, Problem &P, const is3d_surface &s, const is3d_vorticity *vort, const is3d_thermal_shear *shear,
+                       double *dN_raw, int64_t n_raw, int32_t *mcid_out, int32_t n_mcid_max, is3d_stats *stats, std::string *err_out)
 {
   std::string &err = *err_out;
   const Grids &g = P.g; const DfTables &dft = P.dft; const Laguerre &gla = P.gla;
@@ -472,7 +488,16 @@ static int run_problem(const std::string &wd, Problem &P, const is3d_surface &s,
     const int rcp = is3d_b200_spin_polarization_multi(&P.fl, &s, vort, &sp, &gr, nullptr, &r, &sp_st);
     if (rcp != IS3D_OK) { err = std::string("spin polarization failed: ") + is3d_b200_last_error(); return rcp; }
     if (stats) { stats->gpu_launches += sp_st.gpu_launches; stats->total_ms += sp_st.total_ms; }
-    if (!write_polarization_files(wd, sums, P.mcid, P.mass, g, P.fl.dimension, &err)) return IS3D_ERR_IO;
+    if (!write_polarization_files(wd, sums, nullptr, P.mcid, P.mass, g, P.fl.dimension, &err)) return IS3D_ERR_IO;
+    if (P.thermal_shear_polarization) {
+      std::vector<double> xi(5 * n_bins, 0.0);                   // St (zeros) | Sx | Sy | Sz | Snorm
+      is3d_polarization_result rx{&xi[0], &xi[n_bins], &xi[2 * n_bins], &xi[3 * n_bins], &xi[4 * n_bins]};
+      std::memset(&sp_st, 0, sizeof(sp_st));
+      const int rcx = is3d_b200_spin_polarization_shear_multi(&P.fl, &s, shear, &sp, &gr, nullptr, &rx, &sp_st);
+      if (rcx != IS3D_OK) { err = std::string("thermal-shear polarization failed: ") + is3d_b200_last_error(); return rcx; }
+      if (stats) { stats->gpu_launches += sp_st.gpu_launches; stats->total_ms += sp_st.total_ms; }
+      if (!write_polarization_files(wd, sums, &xi, P.mcid, P.mass, g, P.fl.dimension, &err)) return IS3D_ERR_IO;
+    }
   }
   if (P.hbt_radii) {
     std::vector<double> sums(10 * n_bins, 0.0);                  // S0 | So | Ss | Sl | Soo | Sss | Sll | Sos | Sol | Ssl
@@ -552,7 +577,10 @@ extern "C" int is3d_b200_run_workdir(const char *workdir, double *dN_raw, int64_
     s.c0 = sf.c0.data(); s.c1 = sf.c1.data(); s.c2 = sf.c2.data(); s.c3 = sf.c3.data(); s.c4 = sf.c4.data();
   }
   const is3d_vorticity vort{sf.wtx.data(), sf.wty.data(), sf.wtn.data(), sf.wxy.data(), sf.wxn.data(), sf.wyn.data()};
-  rc = run_problem(wd, P, s, P.fl.mode == 5 ? &vort : nullptr, dN_raw, n_raw, mcid_out, n_mcid_max, stats, &err);
+  const is3d_thermal_shear shear{sf.xtt.data(), sf.xtx.data(), sf.xty.data(), sf.xtn.data(), sf.xxx.data(), sf.xxy.data(), sf.xxn.data(),
+                                 sf.xyy.data(), sf.xyn.data(), sf.xnn.data()};
+  rc = run_problem(wd, P, s, P.fl.mode == 5 ? &vort : nullptr, P.thermal_shear_polarization ? &shear : nullptr, dN_raw, n_raw, mcid_out,
+                   n_mcid_max, stats, &err);
   return rc == IS3D_OK ? rc : fail(rc);
 }
 
@@ -576,7 +604,7 @@ extern "C" int is3d_b200_run_surface(const char *workdir, const is3d_surface *su
     if (rc != IS3D_OK) { err = "cannot average an empty surface"; return fail(rc); }
     compute_jonah_tables(P.pdg, avg[0], P.gla, &P.dft);
   }
-  rc = run_problem(wd, P, *surface, nullptr, dN_raw, n_raw, mcid_out, n_mcid_max, stats, &err);
+  rc = run_problem(wd, P, *surface, nullptr, nullptr, dN_raw, n_raw, mcid_out, n_mcid_max, stats, &err);
   return rc == IS3D_OK ? rc : fail(rc);
 }
 
@@ -633,6 +661,10 @@ extern "C" int is3d_b200_host_dump(const char *workdir, const char *out_path)
   put("Wx", s.Wx); put("Wy", s.Wy); put("Lambda", s.Lambda); put("aL", s.aL);
   put("c0", s.c0); put("c1", s.c1); put("c2", s.c2); put("c3", s.c3); put("c4", s.c4);
   put("wtx", s.wtx); put("wty", s.wty); put("wtn", s.wtn); put("wxy", s.wxy); put("wxn", s.wxn); put("wyn", s.wyn);
+  if (P.thermal_shear_polarization) {
+    put("xtt", s.xtt); put("xtx", s.xtx); put("xty", s.xty); put("xtn", s.xtn); put("xxx", s.xxx);
+    put("xxy", s.xxy); put("xxn", s.xxn); put("xyy", s.xyy); put("xyn", s.xyn); put("xnn", s.xnn);
+  }
   tmp.assign(s.avg, s.avg + 5); put("avg", tmp);
   put("df_T", P.dft.T); put("df_c0", P.dft.c0); put("df_c2", P.dft.c2); put("df_F", P.dft.F); put("df_betabulk", P.dft.betabulk);
   put("df_betapi", P.dft.betapi); put("jonah_x", P.dft.jonah_x); put("jonah_lambda2", P.dft.jonah_lambda2); put("jonah_z", P.dft.jonah_z);

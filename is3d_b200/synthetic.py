@@ -123,3 +123,15 @@ def vorticity(n_cells, seed):
     rng = np.random.default_rng(seed)
     s = np.array([0.02, 0.02, 0.1, 0.02, 0.1, 0.1])
     return {k: rng.normal(0.0, s[j], n_cells) for j, k in enumerate(VORTICITY_COLUMNS)}
+
+
+THERMAL_SHEAR_COLUMNS = ("xtt", "xtx", "xty", "xtn", "xxx", "xxy", "xxn", "xyy", "xyn", "xnn")
+
+
+def thermal_shear(n_cells, seed):
+    """Thermal shear xi_{mu nu} = (1/2)(d_mu beta_nu + d_nu beta_mu) for input/thermal_shear.dat: the ten covariant Milne components
+    xi_{tau tau}, xi_{tau x}, xi_{tau y}, xi_{tau eta}, xi_{xx}, xi_{xy}, xi_{x eta}, xi_{yy}, xi_{y eta}, xi_{eta eta} (dimensionless)
+    as a dict of arrays.  Each eta index carries a factor tau ~ 5 fm relative to the others, as covariant components do."""
+    rng = np.random.default_rng(seed)
+    s = np.array([0.02, 0.02, 0.02, 0.1, 0.02, 0.02, 0.1, 0.02, 0.1, 0.5])
+    return {k: rng.normal(0.0, s[j], n_cells) for j, k in enumerate(THERMAL_SHEAR_COLUMNS)}

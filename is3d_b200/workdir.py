@@ -13,6 +13,8 @@ import os
 
 import numpy as np
 
+from is3d_b200.synthetic import THERMAL_SHEAR_COLUMNS
+
 _FIXTURE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "data", "is3d_tables.npz")
 
 # every key the reference constructor getVal()s (emissionfunction.cpp:170-222, readindata.cpp:111-118,
@@ -30,7 +32,7 @@ DEFAULT_PARAMETERS = [
 ]
 
 # keys of this drop-in that the reference does not read: written only when a caller sets them (absent: 0, or the default of the host layer)
-OPTIONAL_PARAMETERS = ("spin_polarization", "hbt_radii", "hbt_correlation", "hbt_dq", "hbt_q_points")
+OPTIONAL_PARAMETERS = ("spin_polarization", "thermal_shear_polarization", "hbt_radii", "hbt_correlation", "hbt_dq", "hbt_q_points")
 
 _EOS_DIR = {1: "urqmd", 2: "smash", 3: "smash_box"}
 _EOS_PDG = {1: ("pdg_urqmd", "pdg-urqmd_v3.3+.dat"), 2: ("pdg_smash", "pdg_smash.dat"), 3: ("pdg_box", "pdg_box.dat")}
@@ -125,12 +127,14 @@ def _write_df_vah(dirname, fx):
                 f.write("%s\t\t%s\t\t%s\n" % (_r(a), _r(b), _r(c)))
 
 
-def materialize(root, surface_columns=None, chosen=None, fixture=None, tables=None, vah=False, **params):
+def materialize(root, surface_columns=None, chosen=None, fixture=None, tables=None, vah=False, thermal_shear=None, **params):
     """Create `root` as an iS3D working directory.
 
     surface_columns : (n_cells, n_cols) array in file units, or None for the shipped one-cell toy surface.
     chosen          : iterable of MC ids, or the name of a fixture list ("chosen_pikp", "chosen_urqmd", ...).
     tables          : optional dict overriding quadrature tables: keys pT, phi, y, eta -> (n, 2) arrays.
+    thermal_shear   : optional (n_cells, 10) array or dict of the ten columns of synthetic.THERMAL_SHEAR_COLUMNS, written to
+                      input/thermal_shear.dat (read when thermal_shear_polarization = 1).
     params          : iS3D_parameters.dat overrides (operation, mode, df_mode, dimension, ...).
     """
     fx = fixture if fixture is not None else load_fixture()
@@ -144,6 +148,10 @@ def materialize(root, surface_columns=None, chosen=None, fixture=None, tables=No
     if surface_columns is None:
         surface_columns = fx["toy_surface"]
     write_surface(os.path.join(root, "input", "surface.dat"), surface_columns)
+    if thermal_shear is not None:
+        if isinstance(thermal_shear, dict):
+            thermal_shear = np.column_stack([thermal_shear[k] for k in THERMAL_SHEAR_COLUMNS])
+        write_surface(os.path.join(root, "input", "thermal_shear.dat"), thermal_shear)
     key, fname = _EOS_PDG[hrg_eos]
     if hrg_eos == 3:
         _write_pdg_box(os.path.join(root, "PDG", fname), fx)
