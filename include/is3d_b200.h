@@ -238,6 +238,34 @@ int is3d_b200_spin_polarization_shear_multi(const is3d_flags *flags, const is3d_
                                             const is3d_species *species, const is3d_grid *grid, const is3d_options *options,
                                             is3d_polarization_result *result, is3d_stats *stats);
 
+/* ---- feed-down of the spin polarization through resonance decays ------------------------------------------------------------
+ * Amends, in place, the five raw-sum arrays of is3d_b200_spin_polarization (or vorticity + shear sums added component by component) so
+ * that they describe all hadrons of a species, primary and from decays.  Parents, order, channels, daughter groups, kernels and
+ * arithmetic are those of is3d_b200_resonance_decays, and:
+ *  - Snorm receives exactly the spectra feed-down: bit for bit is3d_b200_resonance_decays applied to the input Snorm;
+ *  - St, Sx, Sy, Sz of a daughter gain, at every point of the 2-body integral (12 x 12 (v, zeta) nodes, both parent azimuths), the
+ *    point's weight times the daughter's spin four-vector S_D there.  The parent's rest-frame spin S*_P = (N^i - N^t p^i/(E + m))/Snorm
+ *    (its physical mass; 0 where log Snorm is not finite) is interpolated linearly in (M_T, Phi[, Y]) at the cell and with the weights
+ *    of the log spectrum, held at the last M_T point beyond the table.  With p* = L(P)^-1 p (L(P) the pure boost to the parent's rest
+ *    frame) and n = p* / |p*|, the daughter's rest-frame spin is s* = a' S*_P + b' (S*_P.n) n; its four-vector is carried back by L(P).
+ *    2+1D: the parent's spin four-vector at rapidity Y is the longitudinal boost by Y of the one at (M_T, Phi, 0).
+ *  - 3-body channels and 2-body channels without a transfer law feed Snorm only: their daughters are diluted, not polarized.
+ * Normalisation: the arrays carry the spin-1/2 prefactor -1/(8m) for every species; a spin-J parent's true mean spin is 4J(J+1)/3 times
+ * S*_P (Becattini et al. 2013), and that factor is folded into (a', b').  Laws, for a daughter with J_D = 1/2 (C = <S*_D>/S*_P of the true
+ * spins):
+ *    J_P = 1/2 -> 1/2 + photon (partner MC id 22)                     a' = 0                 b' = -1       C = -1/3
+ *    J_P -> 1/2 + spin-0 meson, the three parities known             a' = -eta (2J_P+1)/2   b' = 1 - a'   C = (1 - eta (2J_P+1)) / (4J_P(J_P+1))
+ *    with eta = -(-1)^(J_P - 1/2) P_P P_D P_meson.  Any other 2-body channel has no law.
+ * is3d_spin_parity has one entry per particle-list entry: spin2 = 2J >= 0, parity = +1 / -1, or 0 when unknown.
+ * Arrays: spectra layout ipart + n_species*(ipT + n_pT*(iphi + n_phi*iy)); host or device memory per options->memory.
+ * Errors: those of is3d_b200_resonance_decays (a parent whose tail fit has fewer than 2 points is IS3D_ERR_ARGUMENT, and all five arrays
+ * stay untouched); IS3D_ERR_ARGUMENT also for a NULL spin / parity table or array, a NULL result array, spin2 < 0 or a parity outside
+ * {-1, 0, 1}. */
+typedef struct { const int32_t *spin2, *parity; } is3d_spin_parity;
+int is3d_b200_polarization_decays(const is3d_particle_list *particles, const is3d_spin_parity *spin_parity, int32_t n_chosen,
+                                  const int32_t *chosen_pdg_index, const is3d_grid *grid, int32_t dimension, const is3d_options *options,
+                                  is3d_polarization_result *sums, is3d_stats *stats);
+
 /* ---- HBT radii: space-time variances of the Cooper-Frye emission function ---------------------------------------------
  * Gaussian (moment) approximation with pair momentum K = p (Wiedemann & Heinz, Phys. Rept. 319 (1999) 145).  For every spectra bin
  * (species, pT, phi, y; 2+1D: y = 0) the frame is the bin's longitudinally co-moving frame (LCMS): a longitudinal boost by the bin's

@@ -401,18 +401,14 @@ class ParticleList(C.Structure):
                 ("dec_npart", _I), ("dec_br", _D), ("dec_part", _I)]
 
 
-def resonance_decays(pdg, chosen_pdg_index, grid, dimension, dN, memory="host", stream=None):
-    """Call is3d_b200_resonance_decays (SURVEY 8f, row N3): feed-down of the unstable chosen species into their chosen daughters.
-
-    pdg: dict of arrays mcid, mass, width, stable, decays, dec_first, dec_npart, dec_br, dec_part[rows, 5] (tables.pdg_decay_table);
-    dN: numpy array (memory='host'; a copy is amended and returned) or float64 CUDA tensor (memory='device'; amended in place)."""
-    keep = []
-
+def _decay_problem(pdg, grid, keep):
+    """ParticleList and Grid structures for the decay entry points; the arrays they point to are appended to keep."""
     def ia(x):
         a = np.ascontiguousarray(x, dtype=np.int32); keep.append(a)
         return a.ctypes.data_as(C.POINTER(C.c_int32))
 
     m = _Marshal(False)
+    keep.append(m)
     p = ParticleList()
     p.n_particles = len(pdg["mcid"])
     p.mcid = ia(pdg["mcid"]); p.mass = m.host(pdg["mass"]); p.width = m.host(pdg["width"]); p.stable = ia(pdg["stable"])
@@ -422,6 +418,16 @@ def resonance_decays(pdg, chosen_pdg_index, grid, dimension, dN, memory="host", 
     g.n_pT, g.n_phi, g.n_y, g.n_eta = len(grid["pT"]), len(grid["phi"]), len(grid["y"]), len(grid["eta"])
     for k in ("pT", "phi", "y", "eta", "eta_weight"):
         setattr(g, k, m.host(grid[k]))
+    return p, g, ia
+
+
+def resonance_decays(pdg, chosen_pdg_index, grid, dimension, dN, memory="host", stream=None):
+    """Call is3d_b200_resonance_decays (SURVEY 8f, row N3): feed-down of the unstable chosen species into their chosen daughters.
+
+    pdg: dict of arrays mcid, mass, width, stable, decays, dec_first, dec_npart, dec_br, dec_part[rows, 5] (tables.pdg_decay_table);
+    dN: numpy array (memory='host'; a copy is amended and returned) or float64 CUDA tensor (memory='device'; amended in place)."""
+    keep = []
+    p, g, ia = _decay_problem(pdg, grid, keep)
     device = (memory == "device")
     if device:
         import torch
@@ -438,6 +444,47 @@ def resonance_decays(pdg, chosen_pdg_index, grid, dimension, dN, memory="host", 
     f.restype = C.c_int
     f.argtypes = [C.POINTER(ParticleList), C.c_int32, C.POINTER(C.c_int32), C.POINTER(Grid), C.c_int32, C.POINTER(Options), C.c_void_p, C.POINTER(Stats)]
     _check(f(C.byref(p), len(chosen_pdg_index), ia(chosen_pdg_index), C.byref(g), int(dimension), C.byref(opt), ptr, C.byref(st)))
+    return out, st.as_dict()
+
+
+class SpinParity(C.Structure):
+    _fields_ = [("spin2", C.POINTER(C.c_int32)), ("parity", C.POINTER(C.c_int32))]
+
+
+def polarization_decays(pdg, spin_parity, chosen_pdg_index, grid, dimension, sums, memory="host", stream=None):
+    """Call is3d_b200_polarization_decays: feed-down of the spin-polarization raw sums through the decay tables.
+
+    pdg as for resonance_decays; spin_parity: dict spin2 (2J), parity (+1 / -1, 0 unknown) per particle-list entry
+    (tables.spin_parity); sums: dict St, Sx, Sy, Sz, Snorm as spin_polarization returns them (or vorticity + shear sums added).
+    memory='host': numpy arrays, an amended copy is returned; memory='device': float64 CUDA tensors, amended in place.  Returns
+    (sums, stats dict); mean_spin() forms S and S* from the result.  spin_parity=None passes a NULL table (the library rejects it)."""
+    keep = []
+    p, g, ia = _decay_problem(pdg, grid, keep)
+    sp = None
+    if spin_parity is not None:
+        sp = SpinParity()
+        sp.spin2 = ia(spin_parity["spin2"]); sp.parity = ia(spin_parity["parity"])
+    device = (memory == "device")
+    res = PolarizationResult()
+    if device:
+        import torch
+        out = sums
+        for k in POLARIZATION_FIELDS:
+            setattr(res, k, C.cast(C.c_void_p(out[k].data_ptr()), _D))
+        if stream is None:
+            stream = torch.cuda.current_stream().cuda_stream
+    else:
+        out = {k: np.array(sums[k], dtype=np.float64, copy=True) for k in POLARIZATION_FIELDS}
+        for k in POLARIZATION_FIELDS:
+            setattr(res, k, out[k].ctypes.data_as(_D))
+    opt = Options(); opt.memory = 1 if device else 0; opt.stream = C.c_void_p(stream or 0)
+    st = Stats()
+    f = lib().is3d_b200_polarization_decays
+    f.restype = C.c_int
+    f.argtypes = [C.POINTER(ParticleList), C.POINTER(SpinParity), C.c_int32, C.POINTER(C.c_int32), C.POINTER(Grid), C.c_int32,
+                  C.POINTER(Options), C.POINTER(PolarizationResult), C.POINTER(Stats)]
+    _check(f(C.byref(p), C.byref(sp) if sp is not None else None, len(chosen_pdg_index), ia(chosen_pdg_index), C.byref(g), int(dimension),
+             C.byref(opt), C.byref(res), C.byref(st)))
     return out, st.as_dict()
 
 

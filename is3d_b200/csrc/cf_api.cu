@@ -866,15 +866,22 @@ extern "C" int is3d_b200_mean_yield(const is3d_flags *fl, const is3d_surface *sf
 
 
 // Resonance-decay feed-down (SURVEY 8f, row N3): see cf_decays.cu
-extern "C" int is3d_b200_resonance_decays(const is3d_particle_list *pdg, int32_t n_chosen, const int32_t *chosen, const is3d_grid *gr,
-                                          int32_t dimension, const is3d_options *opt_in, double *dN, is3d_stats *stats)
+static int check_decay_args(const is3d_particle_list *pdg, int32_t n_chosen, const int32_t *chosen, const is3d_grid *gr, int32_t dimension)
 {
-  if (!pdg || !chosen || !gr || !dN || n_chosen <= 0) return fail(IS3D_ERR_ARGUMENT, "NULL argument");
+  if (!pdg || !chosen || !gr || n_chosen <= 0) return fail(IS3D_ERR_ARGUMENT, "NULL argument");
   if (dimension != 2 && dimension != 3) return fail(IS3D_ERR_ARGUMENT, "dimension must be 2 or 3");
   if (!pdg->mcid || !pdg->mass || !pdg->width || !pdg->stable || !pdg->decays || !pdg->dec_first || !pdg->dec_npart || !pdg->dec_br || !pdg->dec_part)
     return fail(IS3D_ERR_ARGUMENT, "incomplete particle list");
   if (!gr->pT || !gr->phi || !gr->y || gr->n_pT <= 0 || gr->n_phi <= 0 || gr->n_y <= 0) return fail(IS3D_ERR_ARGUMENT, "momentum tables missing");
   for (int i = 0; i < n_chosen; i++) if (chosen[i] < 0 || chosen[i] >= pdg->n_particles) return fail(IS3D_ERR_ARGUMENT, "chosen particle index out of range");
+  return IS3D_OK;
+}
+
+extern "C" int is3d_b200_resonance_decays(const is3d_particle_list *pdg, int32_t n_chosen, const int32_t *chosen, const is3d_grid *gr,
+                                          int32_t dimension, const is3d_options *opt_in, double *dN, is3d_stats *stats)
+{
+  if (!dN) return fail(IS3D_ERR_ARGUMENT, "NULL argument");
+  { const int rc = check_decay_args(pdg, n_chosen, chosen, gr, dimension); if (rc) return rc; }
   Device *Dp = nullptr;
   { int rc = current_device(&Dp); if (rc) return rc; }
   Workspace &ws = Dp->ws;
@@ -895,6 +902,57 @@ extern "C" int is3d_b200_resonance_decays(const is3d_particle_list *pdg, int32_t
   if (rc != IS3D_OK) { cudaStreamSynchronize(st); return fail(rc, err.c_str()); }
   CU_CHECK(cudaEventRecord(ev[2], st));
   CU_CHECK(cudaMemcpyAsync(dN, dev, (size_t)n_bins * 8, opt.memory == 0 ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, st));
+  CU_CHECK(cudaEventRecord(ev[3], st));
+  CU_CHECK(cudaEventSynchronize(ev[3]));
+  if (stats) {
+    is3d_stats stt; memset(&stt, 0, sizeof(stt));
+    float ms;
+    cudaEventElapsedTime(&ms, ev[0], ev[1]); stt.h2d_ms = ms;
+    cudaEventElapsedTime(&ms, ev[1], ev[2]); stt.kernel_ms = ms;
+    cudaEventElapsedTime(&ms, ev[2], ev[3]); stt.d2h_ms = ms;
+    cudaEventElapsedTime(&ms, ev[0], ev[3]); stt.total_ms = ms;
+    stt.gpu_launches = launches; stt.n_gpus = 1;
+    *stats = stt;
+  }
+  return IS3D_OK;
+}
+
+// Feed-down of the spin-polarization sums through 2-body decays (cf_decays.cu).  Like is3d_b200_resonance_decays it works on a device
+// copy of all five arrays, so an error leaves the caller's arrays untouched.
+extern "C" int is3d_b200_polarization_decays(const is3d_particle_list *pdg, const is3d_spin_parity *spin_parity, int32_t n_chosen,
+                                             const int32_t *chosen, const is3d_grid *gr, int32_t dimension, const is3d_options *opt_in,
+                                             is3d_polarization_result *sums, is3d_stats *stats)
+{
+  if (!sums || !sums->St || !sums->Sx || !sums->Sy || !sums->Sz || !sums->Snorm) return fail(IS3D_ERR_ARGUMENT, "NULL result array");
+  { const int rc = check_decay_args(pdg, n_chosen, chosen, gr, dimension); if (rc) return rc; }
+  if (!spin_parity || !spin_parity->spin2 || !spin_parity->parity) return fail(IS3D_ERR_ARGUMENT, "NULL spin / parity table");
+  for (int i = 0; i < pdg->n_particles; i++) {
+    if (spin_parity->spin2[i] < 0) return fail(IS3D_ERR_ARGUMENT, "negative 2J in the spin / parity table");
+    if (spin_parity->parity[i] < -1 || spin_parity->parity[i] > 1) return fail(IS3D_ERR_ARGUMENT, "parity must be -1, 0 (unknown) or +1");
+  }
+  Device *Dp = nullptr;
+  { int rc = current_device(&Dp); if (rc) return rc; }
+  Workspace &ws = Dp->ws;
+  std::lock_guard<std::mutex> lk(Dp->mu);
+  is3d_options opt; memset(&opt, 0, sizeof(opt));
+  if (opt_in) opt = *opt_in;
+  cudaStream_t st = (cudaStream_t)opt.stream;
+  const int64_t n_bins = (int64_t)n_chosen * gr->n_pT * gr->n_phi * gr->n_y;
+  double *const arr[5] = {sums->St, sums->Sx, sums->Sy, sums->Sz, sums->Snorm};
+  const cudaMemcpyKind in = opt.memory == 0 ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
+  const cudaMemcpyKind out = opt.memory == 0 ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
+  cudaEvent_t *ev = ws.ev;
+  CU_CHECK(cudaEventRecord(ev[0], st));
+  CU_CHECK(ws.dN.reserve((size_t)n_bins * 8 * 5 + 256));
+  double *dev = ws.dN.as<double>();
+  for (int k = 0; k < 5; k++) CU_CHECK(cudaMemcpyAsync(dev + k * n_bins, arr[k], (size_t)n_bins * 8, in, st));
+  CU_CHECK(cudaEventRecord(ev[1], st));
+  int launches = 0; std::string err;
+  const int rc = polarization_decays_device(pdg, spin_parity->spin2, spin_parity->parity, n_chosen, chosen, gr, dimension, dev, n_bins, st,
+                                            &launches, &err);
+  if (rc != IS3D_OK) { cudaStreamSynchronize(st); return fail(rc, err.c_str()); }
+  CU_CHECK(cudaEventRecord(ev[2], st));
+  for (int k = 0; k < 5; k++) CU_CHECK(cudaMemcpyAsync(arr[k], dev + k * n_bins, (size_t)n_bins * 8, out, st));
   CU_CHECK(cudaEventRecord(ev[3], st));
   CU_CHECK(cudaEventSynchronize(ev[3]));
   if (stats) {

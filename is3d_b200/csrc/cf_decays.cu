@@ -14,6 +14,8 @@
 // and a second kernel adds them to the daughters in (channel, group) order, so the result does not depend on the launch geometry
 // and follows the reference's accumulation order.  The parent's log table (129 KB) is read through L1/L2.  Parents are inherently
 // sequential (a parent's spectrum must have received its own feed-down first).
+// The same driver feeds the spin-polarization sums down (is3d_b200_polarization_decays, DESIGN §17): Snorm through exactly these
+// launches, and N^mu through decay2_spin_kernel, which shares the 2-body points and interpolation with decay2_kernel.
 // Compiled with -fmad=false: products and sums round one by one like the reference's scalar C++.
 #include "cf_internal.h"
 #include <algorithm>
@@ -151,7 +153,13 @@ __device__ __forceinline__ void phi_points(const ParentView &P, double &Phip, in
   }
 }
 
-__device__ double parent_2d(const ParentView &P, double MT, double Phip1, double Phip2)                     // :1413-1676
+// Polarization feed-down (is3d_b200_polarization_decays): the parent's rest-frame mean spin S*_P, tabulated like logdN ([3][bins]),
+// is interpolated LINEARLY at the cell and with the weights of the log spectrum; above MTmax it is held at the last M_T point.
+// SpinOut receives, per parent azimuth, exp(log dN) and S*_P there.  The plain feed-down instantiates everything with SPIN = false.
+struct SpinOut { double e1, e2, S1[3], S2[3]; };
+
+template <bool SPIN>
+__device__ double parent_2d(const ParentView &P, double MT, double Phip1, double Phip2, const double *Sstar = nullptr, SpinOut *so = nullptr)   // :1413-1676
 {
   double logdN1, logdN2;
   int i1L, i1R, i2L, i2R; double P1L, P1R, P2L, P2R;
@@ -167,17 +175,37 @@ __device__ double parent_2d(const ParentView &P, double MT, double Phip1, double
     const double b_LL = P.logdN[iMTL + npT * i2L], b_RL = P.logdN[iMTL + npT * i2R], b_LR = P.logdN[iMTR + npT * i2L], b_RR = P.logdN[iMTR + npT * i2R];
     logdN1 = ((a_LL * (P1R - Phip1) + a_RL * (Phip1 - P1L)) * (MTR - MT) + (a_LR * (P1R - Phip1) + a_RR * (Phip1 - P1L)) * (MT - MTL)) / (dPhip1 * dMT);
     logdN2 = ((b_LL * (P2R - Phip2) + b_RL * (Phip2 - P2L)) * (MTR - MT) + (b_LR * (P2R - Phip2) + b_RR * (Phip2 - P2L)) * (MT - MTL)) / (dPhip2 * dMT);
+    if constexpr (SPIN) {
+      for (int c = 0; c < 3; c++) {
+#define SG(im, ip) Sstar[3 * ((im) + npT * (ip)) + c]
+        so->S1[c] = ((SG(iMTL, i1L) * (P1R - Phip1) + SG(iMTL, i1R) * (Phip1 - P1L)) * (MTR - MT)
+                   + (SG(iMTR, i1L) * (P1R - Phip1) + SG(iMTR, i1R) * (Phip1 - P1L)) * (MT - MTL)) / (dPhip1 * dMT);
+        so->S2[c] = ((SG(iMTL, i2L) * (P2R - Phip2) + SG(iMTL, i2R) * (Phip2 - P2L)) * (MTR - MT)
+                   + (SG(iMTR, i2L) * (P2R - Phip2) + SG(iMTR, i2R) * (Phip2 - P2L)) * (MT - MTL)) / (dPhip2 * dMT);
+#undef SG
+      }
+    }
   } else {
     const Fit f1L = P.fit[i1L], f1R = P.fit[i1R], f2L = P.fit[i2L], f2R = P.fit[i2R];
     const double a_L = f1L.constant + f1L.slope * MT, a_R = f1R.constant + f1R.slope * MT;
     const double b_L = f2L.constant + f2L.slope * MT, b_R = f2R.constant + f2R.slope * MT;
     logdN1 = (a_L * (P1R - Phip1) + a_R * (Phip1 - P1L)) / dPhip1;
     logdN2 = (b_L * (P2R - Phip2) + b_R * (Phip2 - P2L)) / dPhip2;
+    if constexpr (SPIN) {
+      const int im = P.n_pT - 1, npT = P.n_pT;
+      for (int c = 0; c < 3; c++) {
+        so->S1[c] = (Sstar[3 * (im + npT * i1L) + c] * (P1R - Phip1) + Sstar[3 * (im + npT * i1R) + c] * (Phip1 - P1L)) / dPhip1;
+        so->S2[c] = (Sstar[3 * (im + npT * i2L) + c] * (P2R - Phip2) + Sstar[3 * (im + npT * i2R) + c] * (Phip2 - P2L)) / dPhip2;
+      }
+    }
   }
+  if constexpr (SPIN) { so->e1 = exp(logdN1); so->e2 = exp(logdN2); return 0.0; }
   return (exp(logdN1) + exp(logdN2));
 }
 
-__device__ double parent_3d(const ParentView &P, int iYL, int iYR, double YL, double YR, double MT, double Phip1, double Phip2, double Y)   // :1680-2028
+template <bool SPIN>
+__device__ double parent_3d(const ParentView &P, int iYL, int iYR, double YL, double YR, double MT, double Phip1, double Phip2, double Y,   // :1680-2028
+                            const double *Sstar = nullptr, SpinOut *so = nullptr)
 {
   double logdN1, logdN2;
   int i1L, i1R, i2L, i2R; double P1L, P1R, P2L, P2R;
@@ -202,6 +230,18 @@ __device__ double parent_3d(const ParentView &P, int iYL, int iYR, double YL, do
     logdN2 = (MTR - MT) * ((b_LLL * (YR - Y) + b_RLL * (Y - YL)) * (P2R - Phip2) + (b_LRL * (YR - Y) + b_RRL * (Y - YL)) * (Phip2 - P2L))
            + (MT - MTL) * ((b_LLR * (YR - Y) + b_RLR * (Y - YL)) * (P2R - Phip2) + (b_LRR * (YR - Y) + b_RRR * (Y - YL)) * (Phip2 - P2L));
     logdN2 /= (dY * dPhip2 * dMT);
+    if constexpr (SPIN) {
+      for (int c = 0; c < 3; c++) {
+#define SG(im, ip, iy) Sstar[3 * ((im) + npT * ((ip) + nphi * (iy))) + c]
+        so->S1[c] = ((MTR - MT) * ((SG(iMTL, i1L, iYL) * (YR - Y) + SG(iMTL, i1L, iYR) * (Y - YL)) * (P1R - Phip1) + (SG(iMTL, i1R, iYL) * (YR - Y) + SG(iMTL, i1R, iYR) * (Y - YL)) * (Phip1 - P1L))
+                   + (MT - MTL) * ((SG(iMTR, i1L, iYL) * (YR - Y) + SG(iMTR, i1L, iYR) * (Y - YL)) * (P1R - Phip1) + (SG(iMTR, i1R, iYL) * (YR - Y) + SG(iMTR, i1R, iYR) * (Y - YL)) * (Phip1 - P1L)))
+                   / (dY * dPhip1 * dMT);
+        so->S2[c] = ((MTR - MT) * ((SG(iMTL, i2L, iYL) * (YR - Y) + SG(iMTL, i2L, iYR) * (Y - YL)) * (P2R - Phip2) + (SG(iMTL, i2R, iYL) * (YR - Y) + SG(iMTL, i2R, iYR) * (Y - YL)) * (Phip2 - P2L))
+                   + (MT - MTL) * ((SG(iMTR, i2L, iYL) * (YR - Y) + SG(iMTR, i2L, iYR) * (Y - YL)) * (P2R - Phip2) + (SG(iMTR, i2R, iYL) * (YR - Y) + SG(iMTR, i2R, iYR) * (Y - YL)) * (Phip2 - P2L)))
+                   / (dY * dPhip2 * dMT);
+#undef SG
+      }
+    }
   } else {
     const Fit f1LL = P.fit[iYL * nphi + i1L], f1RL = P.fit[iYR * nphi + i1L], f1LR = P.fit[iYL * nphi + i1R], f1RR = P.fit[iYR * nphi + i1R];
     const Fit f2LL = P.fit[iYL * nphi + i2L], f2RL = P.fit[iYR * nphi + i2L], f2LR = P.fit[iYL * nphi + i2R], f2RR = P.fit[iYR * nphi + i2R];
@@ -211,13 +251,67 @@ __device__ double parent_3d(const ParentView &P, int iYL, int iYR, double YL, do
     logdN1 /= (dY * dPhip1);
     logdN2 = (b_LL * (YR - Y) + b_RL * (Y - YL)) * (P2R - Phip2) + (b_LR * (YR - Y) + b_RR * (Y - YL)) * (Phip2 - P2L);
     logdN2 /= (dY * dPhip2);
+    if constexpr (SPIN) {
+      const int im = npT - 1;
+      for (int c = 0; c < 3; c++) {
+#define SG(ip, iy) Sstar[3 * (im + npT * ((ip) + nphi * (iy))) + c]
+        so->S1[c] = ((SG(i1L, iYL) * (YR - Y) + SG(i1L, iYR) * (Y - YL)) * (P1R - Phip1) + (SG(i1R, iYL) * (YR - Y) + SG(i1R, iYR) * (Y - YL)) * (Phip1 - P1L)) / (dY * dPhip1);
+        so->S2[c] = ((SG(i2L, iYL) * (YR - Y) + SG(i2L, iYR) * (Y - YL)) * (P2R - Phip2) + (SG(i2R, iYL) * (YR - Y) + SG(i2R, iYR) * (Y - YL)) * (Phip2 - P2L)) / (dY * dPhip2);
+#undef SG
+      }
+    }
   }
+  if constexpr (SPIN) { so->e1 = exp(logdN1); so->e2 = exp(logdN2); return 0.0; }
   return (exp(logdN1) + exp(logdN2));
 }
 
-// zeta integral at fixed (v [, s]): the innermost loop of the four integration routines (:588-628, 753-784, 1183-1213, 1352-1380)
+// Polarization feed-down: per-thread context of the daughter spin at a point of the 2-body integral (see daughter_spin)
+struct SpinCtx {
+  const double *Sstar;           // parent rest-frame spin table [bins][3]
+  double M, mD, a, b;            // mass_parent of the term, daughter mass, transfer law s* = a S*_P + b (S*_P.n) n
+  double E, px, py, pz;          // the bin's four-momentum (daughter)
+  double Y;                      // parent rapidity at the current v node (y + v DeltaY; 2+1D: v DeltaY)
+  int dim;
+};
+
+// Spin four-vector S_D (lab) of the daughter at one integrand point: parent P = (MT cosh Y, PT cos Phi, PT sin Phi, MT sinh Y) with
+// rest-frame spin Sp (2+1D: Sp is the y = 0 table value, its four-vector is boosted longitudinally by Y first), p* = L(P)^-1 p,
+// n = p*/|p*|, s* = a Sp + b (Sp.n) n in the daughter's rest frame, then back through L(P).  All boosts are pure boosts.
+__device__ __forceinline__ void daughter_spin(const SpinCtx &c, double MT, double PT, double Phi, const double Sp[3], double out[4])
+{
+  const double M = c.M, chY = cosh(c.Y), shY = sinh(c.Y);
+  const double Px = PT * cos(Phi), Py = PT * sin(Phi), Pz = MT * shY, EP = MT * chY;
+  double S[3] = {Sp[0], Sp[1], Sp[2]};
+  if (c.dim == 2) {                                  // four-vector at (MT, Px, Py, 0), boost by Y, rest-frame part w.r.t. L(P)
+    const double P0S = Px * Sp[0] + Py * Sp[1];
+    const double s0t = P0S / M, k = P0S / (M * (MT + M));
+    const double sx = Sp[0] + k * Px, sy = Sp[1] + k * Py;
+    const double st = s0t * chY + Sp[2] * shY, sz = s0t * shY + Sp[2] * chY;
+    const double r = st / (EP + M);
+    S[0] = sx - r * Px; S[1] = sy - r * Py; S[2] = sz - r * Pz;
+  }
+  const double Pp = Px * c.px + Py * c.py + Pz * c.pz;
+  const double pst = (EP * c.E - Pp) / M, kp = Pp / (M * (EP + M)) - c.E / M;
+  const double ps[3] = {c.px + kp * Px, c.py + kp * Py, c.pz + kp * Pz};
+  const double ip = 1.0 / sqrt(ps[0] * ps[0] + ps[1] * ps[1] + ps[2] * ps[2]);
+  const double n[3] = {ps[0] * ip, ps[1] * ip, ps[2] * ip};
+  const double Sn = S[0] * n[0] + S[1] * n[1] + S[2] * n[2];
+  const double s[3] = {c.a * S[0] + c.b * Sn * n[0], c.a * S[1] + c.b * Sn * n[1], c.a * S[2] + c.b * Sn * n[2]};
+  const double pss = ps[0] * s[0] + ps[1] * s[1] + ps[2] * s[2];
+  const double q0 = pss / c.mD, kq = pss / (c.mD * (pst + c.mD));
+  const double q[3] = {s[0] + kq * ps[0], s[1] + kq * ps[1], s[2] + kq * ps[2]};
+  const double Pq = Px * q[0] + Py * q[1] + Pz * q[2];
+  const double kk = Pq / (M * (EP + M)) + q0 / M;
+  out[0] = (EP * q0 + Pq) / M;
+  out[1] = q[0] + kk * Px; out[2] = q[1] + kk * Py; out[3] = q[2] + kk * Pz;
+}
+
+// zeta integral at fixed (v [, s]): the innermost loop of the four integration routines (:588-628, 753-784, 1183-1213, 1352-1380).
+// SPIN: instead, zs[mu] += w_zeta MT (exp(log dN_1) S_D^mu(Phi_1) + exp(log dN_2) S_D^mu(Phi_2)) at the same points.
+template <bool SPIN>
 __device__ double zeta_integral_at(const ParentView &P, double MTbar, double DeltaMT, double mTc_over_pT, double Estar_M_over_pT, double parent_mass2,
-                                   double phip, int dim, bool cutoff_Y, int iYL, int iYR, double YL, double YR, double Y)
+                                   double phip, int dim, bool cutoff_Y, int iYL, int iYR, double YL, double YR, double Y,
+                                   const SpinCtx *sc = nullptr, double *zs = nullptr)
 {
   const double two_Pi = 2.0 * M_PI;
   double zeta_integral = 0.0;
@@ -231,8 +325,19 @@ __device__ double zeta_integral_at(const ParentView &P, double MTbar, double Del
     double Phip_1 = fmod(Phip_tilde + phip, two_Pi), Phip_2 = fmod(-Phip_tilde + phip, two_Pi);
     if (Phip_1 < 0.0) Phip_1 += two_Pi;
     if (Phip_2 < 0.0) Phip_2 += two_Pi;
-    const double integrand = MT * (dim == 2 ? parent_2d(P, MT, Phip_1, Phip_2) : parent_3d(P, iYL, iYR, YL, YR, MT, Phip_1, Phip_2, Y));
-    zeta_integral += (kGLWeight[izeta] * integrand);
+    if constexpr (SPIN) {
+      SpinOut so;
+      if (dim == 2) parent_2d<true>(P, MT, Phip_1, Phip_2, sc->Sstar, &so);
+      else parent_3d<true>(P, iYL, iYR, YL, YR, MT, Phip_1, Phip_2, Y, sc->Sstar, &so);
+      double S1[4], S2[4];
+      daughter_spin(*sc, MT, PT, Phip_1, so.S1, S1);
+      daughter_spin(*sc, MT, PT, Phip_2, so.S2, S2);
+      const double w1 = MT * so.e1, w2 = MT * so.e2;
+      for (int mu = 0; mu < 4; mu++) zs[mu] += (kGLWeight[izeta] * (w1 * S1[mu] + w2 * S2[mu]));
+    } else {
+      const double integrand = MT * (dim == 2 ? parent_2d<false>(P, MT, Phip_1, Phip_2) : parent_3d<false>(P, iYL, iYR, YL, YR, MT, Phip_1, Phip_2, Y));
+      zeta_integral += (kGLWeight[izeta] * integrand);
+    }
   }
   return zeta_integral;
 }
@@ -256,6 +361,28 @@ __device__ __forceinline__ ParentView parent_view(const DecayGrid &G, const doub
   return P;
 }
 
+// The per-bin set-up and the kinematics of one v node of the 2-body integral (:521-806), shared by decay2_kernel and
+// decay2_spin_kernel.  Macros rather than functions: the statements then compile in decay2_kernel exactly as they always have.
+#define TWO_BODY_BIN_SETUP                                                                                                             \
+  const double mass_parent = T.mass_parent, parent_mass2 = mass_parent * mass_parent;                                                 \
+  const double Estar = T.Estar, Estar2 = Estar * Estar, pstar = T.pstar, Estar_M = Estar * mass_parent;                              \
+  const double pT = G.pT[ipT], pT2 = pT * pT, mT2 = pT2 + T.mass2, mT = sqrt(mT2);                                                    \
+  const double M_pT = mass_parent * pT, Estar_M_mT = Estar_M * mT, Estar_M_over_pT = Estar_M / pT, Estar2_plus_pT2 = Estar2 + pT2;  \
+  const double DeltaY = log((pstar + sqrt(Estar2_plus_pT2)) / mT);                                                                    \
+  const double phip = G.phi[iphip], y = (G.dim == 2) ? 0.0 : G.y[iy];                                                                 \
+  const double Ymax = (G.dim == 2) ? 0.0 : fabs(G.y[G.y_pts - 1]);
+#define TWO_BODY_V_NODE                                                                                                                \
+    const double v = kGLRoot[iv];                                                                                                      \
+    int iYL = 0, iYR = 0; double YL = 0.0, YR = 0.0, Y = 0.0; bool cutoff_Y = false;                                                  \
+    if (G.dim == 3) { Y = y + v * DeltaY; cutoff_Y = y_points(G, Y, Ymax, iYL, iYR, YL, YR); }                                         \
+    const double coshvDeltaY = cosh(v * DeltaY);                                                                                       \
+    const double mT2_coshvDeltaY2 = mT2 * coshvDeltaY * coshvDeltaY;                                                                   \
+    const double den = mT2_coshvDeltaY2 - pT2;                                                                                         \
+    const double MTbar = Estar_M_mT * coshvDeltaY / den;                                                                               \
+    const double DeltaMT = M_pT * sqrt(fabs(Estar2_plus_pT2 - mT2_coshvDeltaY2)) / den;                                                \
+    const double mTc = mT * coshvDeltaY / pT;                                                                                          \
+    const double vw = DeltaY * kGLWeight[iv] / sqrt(fabs(den));
+
 // EmissionFunctionArray::two_body_decay, integration part (:521-806): one thread per (term, bin)
 __global__ void __launch_bounds__(128) decay2_kernel(DecayGrid G, const DecayTerm *__restrict__ terms, const int *__restrict__ term_ids, int n_terms2,
                                                     const double *__restrict__ logdN, const double *__restrict__ MT_all, const Fit *__restrict__ fit_all,
@@ -269,29 +396,81 @@ __global__ void __launch_bounds__(128) decay2_kernel(DecayGrid G, const DecayTer
   const DecayTerm T = terms[term];
   const int ipT = bin % G.n_pT, iphip = (bin / G.n_pT) % G.n_phi, iy = bin / (G.n_pT * G.n_phi);
   const ParentView P = parent_view(G, logdN, MT_all, fit_all, term);
-  const double mass_parent = T.mass_parent, parent_mass2 = mass_parent * mass_parent;
-  const double Estar = T.Estar, Estar2 = Estar * Estar, pstar = T.pstar, Estar_M = Estar * mass_parent;
-  const double pT = G.pT[ipT], pT2 = pT * pT, mT2 = pT2 + T.mass2, mT = sqrt(mT2);
-  const double M_pT = mass_parent * pT, Estar_M_mT = Estar_M * mT, Estar_M_over_pT = Estar_M / pT, Estar2_plus_pT2 = Estar2 + pT2;
-  const double DeltaY = log((pstar + sqrt(Estar2_plus_pT2)) / mT);
-  const double phip = G.phi[iphip], y = (G.dim == 2) ? 0.0 : G.y[iy];
-  const double Ymax = (G.dim == 2) ? 0.0 : fabs(G.y[G.y_pts - 1]);
+  TWO_BODY_BIN_SETUP
   double decay2D_integral = 0.0;
   for (int iv = 0; iv < GP; iv++) {
-    const double v = kGLRoot[iv];
-    int iYL = 0, iYR = 0; double YL = 0.0, YR = 0.0, Y = 0.0; bool cutoff_Y = false;
-    if (G.dim == 3) { Y = y + v * DeltaY; cutoff_Y = y_points(G, Y, Ymax, iYL, iYR, YL, YR); }
-    const double coshvDeltaY = cosh(v * DeltaY);
-    const double mT2_coshvDeltaY2 = mT2 * coshvDeltaY * coshvDeltaY;
-    const double den = mT2_coshvDeltaY2 - pT2;
-    const double MTbar = Estar_M_mT * coshvDeltaY / den;
-    const double DeltaMT = M_pT * sqrt(fabs(Estar2_plus_pT2 - mT2_coshvDeltaY2)) / den;
-    const double mTc = mT * coshvDeltaY / pT;
-    const double vw = DeltaY * kGLWeight[iv] / sqrt(fabs(den));
-    const double zi = zeta_integral_at(P, MTbar, DeltaMT, mTc, Estar_M_over_pT, parent_mass2, phip, G.dim, cutoff_Y, iYL, iYR, YL, YR, Y);
+    TWO_BODY_V_NODE
+    const double zi = zeta_integral_at<false>(P, MTbar, DeltaMT, mTc, Estar_M_over_pT, parent_mass2, phip, G.dim, cutoff_Y, iYL, iYR, YL, YR, Y);
     decay2D_integral += (vw * zi);
   }
   scratch[(size_t)term * n_bins + bin] = T.prefactor * decay2D_integral;
+}
+
+// ---- polarization feed-down (is3d_b200_polarization_decays)
+struct SpinLaw { double a, b; };       // per term; only 2-body terms listed in spin_ids have one
+
+// the parent's rest-frame mean spin S*_P = (N^i - N^t p^i / (E + m)) / Snorm on its own bins, physical mass m; 0 where log Snorm is not
+// finite.  S: the five arrays [St | Sx | Sy | Sz | Snorm], each n_total long.  Sstar[3 * i + c], i = ipT + n_pT (iphi + n_phi iy).
+__global__ void spin_table_kernel(DecayGrid G, const double *__restrict__ S, int64_t n_total, int parent, double mass, double *__restrict__ Sstar)
+{
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  const int n = G.n_pT * G.n_phi * G.y_pts;
+  if (i >= n) return;
+  const int ipT = i % G.n_pT, iphi = (i / G.n_pT) % G.n_phi, iy = i / (G.n_pT * G.n_phi);
+  const int64_t k = (int64_t)parent + (int64_t)G.n_species * i;
+  const double sn = S[4 * n_total + k];
+  double out[3] = {0.0, 0.0, 0.0};
+  if (isfinite(log(sn))) {
+    const double pT = G.pT[ipT], phi = G.phi[iphi], y = (G.dim == 2) ? 0.0 : G.y[iy];
+    const double mT = sqrt(pT * pT + mass * mass), E = mT * cosh(y);
+    const double p[3] = {pT * cos(phi), pT * sin(phi), mT * sinh(y)};
+    const double r = S[k] / (E + mass);
+    for (int c = 0; c < 3; c++) out[c] = (S[(c + 1) * n_total + k] - r * p[c]) / sn;
+  }
+  for (int c = 0; c < 3; c++) Sstar[3 * i + c] = out[c];
+}
+
+// one thread per (term with a transfer law, bin): spin_scratch[term][mu][bin] = prefactor x integral of spectrum x S_D^mu
+__global__ void __launch_bounds__(128) decay2_spin_kernel(DecayGrid G, const DecayTerm *__restrict__ terms, const SpinLaw *__restrict__ laws,
+                                                         const int *__restrict__ spin_ids, int n_spin, const double *__restrict__ logdN,
+                                                         const double *__restrict__ MT_all, const Fit *__restrict__ fit_all,
+                                                         const double *__restrict__ Sstar, double *__restrict__ spin_scratch)
+{
+  const int n_bins = G.n_pT * G.n_phi * G.y_pts;
+  const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (gid >= (int64_t)n_spin * n_bins) return;
+  const int it = (int)(gid / n_bins), bin = (int)(gid - (int64_t)it * n_bins);
+  const int term = spin_ids[it];
+  const DecayTerm T = terms[term];
+  const int ipT = bin % G.n_pT, iphip = (bin / G.n_pT) % G.n_phi, iy = bin / (G.n_pT * G.n_phi);
+  const ParentView P = parent_view(G, logdN, MT_all, fit_all, term);
+  TWO_BODY_BIN_SETUP
+  SpinCtx sc;
+  sc.Sstar = Sstar; sc.a = laws[term].a; sc.b = laws[term].b; sc.M = mass_parent; sc.mD = sqrt(T.mass2); sc.dim = G.dim;
+  sc.E = mT * cosh(y); sc.px = pT * cos(phip); sc.py = pT * sin(phip); sc.pz = mT * sinh(y);
+  double acc[4] = {0.0, 0.0, 0.0, 0.0};
+  for (int iv = 0; iv < GP; iv++) {
+    TWO_BODY_V_NODE
+    sc.Y = y + v * DeltaY;
+    double zs[4] = {0.0, 0.0, 0.0, 0.0};
+    zeta_integral_at<true>(P, MTbar, DeltaMT, mTc, Estar_M_over_pT, parent_mass2, phip, G.dim, cutoff_Y, iYL, iYR, YL, YR, Y, &sc, zs);
+    for (int mu = 0; mu < 4; mu++) acc[mu] += (vw * zs[mu]);
+  }
+  for (int mu = 0; mu < 4; mu++) spin_scratch[((size_t)term * 4 + mu) * n_bins + bin] = T.prefactor * acc[mu];
+}
+
+// N^mu[daughter] += spin_scratch[term][mu], terms with a law in (channel, group) order
+__global__ void spin_add_kernel(DecayGrid G, const DecayTerm *__restrict__ terms, const int *__restrict__ has_law, int n_terms,
+                                const double *__restrict__ spin_scratch, double *__restrict__ S, int64_t n_total)
+{
+  const int n_bins = G.n_pT * G.n_phi * G.y_pts;
+  const int bin = blockIdx.x * blockDim.x + threadIdx.x;
+  if (bin >= n_bins) return;
+  for (int t = 0; t < n_terms; t++) {
+    if (!has_law[t]) continue;
+    const int64_t k = (int64_t)terms[t].daughter + (int64_t)G.n_species * bin;
+    for (int mu = 0; mu < 4; mu++) S[mu * n_total + k] += spin_scratch[((size_t)t * 4 + mu) * n_bins + bin];
+  }
 }
 
 // EmissionFunctionArray::three_body_decay, integration part (:1048-1398): 12 threads per (term, bin), one per s node
@@ -339,7 +518,7 @@ __global__ void __launch_bounds__(GP * kBins3) decay3_kernel(DecayGrid G, const 
       const double MTbar = Estar_M_mT * coshvDeltaY / den;
       const double DeltaMT = M_pT * sqrt(fabs(Estar2_plus_pT2 - mT2_coshvDeltaY2)) / den;
       const double vw = DeltaY * kGLWeight[iv] / sqrt(fabs(den));
-      const double zi = zeta_integral_at(P, MTbar, DeltaMT, mTc, Estar_M_over_pT, parent_mass2, phip, G.dim, cutoff_Y, iYL, iYR, YL, YR, Y);
+      const double zi = zeta_integral_at<false>(P, MTbar, DeltaMT, mTc, Estar_M_over_pT, parent_mass2, phip, G.dim, cutoff_Y, iYL, iYR, YL, YR, Y);
       v_integral += vw * zi;
     }
     contrib = s_integrand_weight * v_integral;
@@ -410,11 +589,37 @@ struct Host {                       // bookkeeping helpers, all on the host and 
   }
 };
 
+// Transfer law (a', b') of a 2-body channel parent -> daughter + partner for the spin-1/2-normalised arrays (include/is3d_b200.h):
+// s*_D = a' S*_P + b' (S*_P.n) n.  false: no law (the channel only dilutes).
+bool transfer_law(const is3d_particle_list *pdg, const int32_t *spin2, const int32_t *parity, int parent, int daughter, int partner,
+                  double *a, double *b)
+{
+  if (spin2[daughter] != 1) return false;
+  const int jp2 = spin2[parent];
+  if (std::abs(pdg->mcid[partner]) == 22) {                  // 1/2 -> 1/2 + photon: only the longitudinal part survives
+    if (jp2 != 1) return false;
+    *a = 0.0; *b = -1.0; return true;
+  }
+  if (spin2[partner] != 0 || jp2 % 2 != 1) return false;
+  const int pp = parity[parent], pd = parity[daughter], pm = parity[partner];
+  if (pp == 0 || pd == 0 || pm == 0) return false;
+  const int sign_j = (((jp2 - 1) / 2) % 2 == 0) ? 1 : -1;     // (-1)^(J_P - 1/2)
+  const double eta = (double)(-sign_j * pp * pd * pm);
+  *a = -eta * (double)(jp2 + 1) / 2.0;
+  *b = 1.0 - *a;
+  return true;
+}
+
 }  // namespace
 
-// Host driver.  dN_dev: device pointer to the spectra [y][phi][pT][species], amended in place.
-int resonance_decays_device(const is3d_particle_list *pdg, int n_chosen, const int32_t *chosen, const is3d_grid *gr, int dimension,
-                            double *dN_dev, cudaStream_t st, int *launches, std::string *err)
+// Polarization feed-down inputs of decays_core: 2J and parity per particle-list entry, and the length of each of the five arrays.
+struct SpinFeedDown { const int32_t *spin2, *parity; int64_t n_total; };
+
+// Host driver.  Without spin, dN_dev is the spectra [y][phi][pT][species], amended in place.  With spin, dN_dev holds the five arrays
+// [St | Sx | Sy | Sz | Snorm] (n_total each); Snorm goes through exactly the launches of the spectra feed-down, and the 2-body terms with
+// a transfer law add their spin integrals to St..Sz.
+static int decays_core(const is3d_particle_list *pdg, int n_chosen, const int32_t *chosen, const is3d_grid *gr, int dimension,
+                       double *dN_dev, const SpinFeedDown *spin, cudaStream_t st, int *launches, std::string *err)
 {
   if (n_chosen - 1 <= 0) { *err = "need at least two chosen particles for the resonance decay routine"; return IS3D_ERR_ARGUMENT; }
   DecayGrid G; memset(&G, 0, sizeof(G));
@@ -427,7 +632,9 @@ int resonance_decays_device(const is3d_particle_list *pdg, int n_chosen, const i
   // device buffers (freed on every path out of this function)
   struct Buffers {
     double *tables = nullptr, *logdN = nullptr, *MT = nullptr, *scratch = nullptr; Fit *fit = nullptr; DecayTerm *terms = nullptr; int *ids = nullptr, *error = nullptr;
-    ~Buffers() { cudaFree(tables); cudaFree(logdN); cudaFree(MT); cudaFree(scratch); cudaFree(fit); cudaFree(terms); cudaFree(ids); cudaFree(error); }
+    double *Sstar = nullptr, *spin_scratch = nullptr; SpinLaw *laws = nullptr; int *spin_ids = nullptr;
+    ~Buffers() { cudaFree(tables); cudaFree(logdN); cudaFree(MT); cudaFree(scratch); cudaFree(fit); cudaFree(terms); cudaFree(ids); cudaFree(error);
+                 cudaFree(Sstar); cudaFree(spin_scratch); cudaFree(laws); cudaFree(spin_ids); }
   } B;
   const int max_terms = 50 * 3;                       // <= 50 channels per particle (readindata.h Maxdecaychannel) x 3 daughter groups
   auto ck = [&](cudaError_t e, const char *what) { if (e != cudaSuccess) { *err = std::string(what) + ": " + cudaGetErrorString(e); return false; } return true; };
@@ -439,6 +646,11 @@ int resonance_decays_device(const is3d_particle_list *pdg, int n_chosen, const i
       !ck(cudaMalloc(&B.terms, sizeof(DecayTerm) * (size_t)max_terms), "cudaMalloc") ||
       !ck(cudaMalloc(&B.ids, sizeof(int) * (size_t)max_terms * 2), "cudaMalloc") ||
       !ck(cudaMalloc(&B.error, sizeof(int)), "cudaMalloc")) return IS3D_ERR_CUDA;
+  if (spin && (!ck(cudaMalloc(&B.Sstar, sizeof(double) * 3 * (size_t)n_bins), "cudaMalloc") ||
+               !ck(cudaMalloc(&B.spin_scratch, sizeof(double) * 4 * (size_t)max_terms * n_bins), "cudaMalloc") ||
+               !ck(cudaMalloc(&B.laws, sizeof(SpinLaw) * (size_t)max_terms), "cudaMalloc") ||
+               !ck(cudaMalloc(&B.spin_ids, sizeof(int) * (size_t)max_terms * 2), "cudaMalloc"))) return IS3D_ERR_CUDA;
+  double *const dN_spec = spin ? dN_dev + 4 * spin->n_total : dN_dev;       // the array the spectra feed-down amends
   if (!ck(cudaMemcpyAsync(B.tables, gr->pT, sizeof(double) * G.n_pT, cudaMemcpyHostToDevice, st), "H2D") ||
       !ck(cudaMemcpyAsync(B.tables + G.n_pT, gr->phi, sizeof(double) * G.n_phi, cudaMemcpyHostToDevice, st), "H2D") ||
       !ck(cudaMemcpyAsync(B.tables + G.n_pT + G.n_phi, gr->y, sizeof(double) * G.n_y_tab, cudaMemcpyHostToDevice, st), "H2D") ||
@@ -450,6 +662,8 @@ int resonance_decays_device(const is3d_particle_list *pdg, int n_chosen, const i
     if (pdg->stable[ipart]) continue;
     // ---- the parent's channels -> terms (host; resonance_decay_channel + the set-up halves of two_/three_body_decay)
     std::vector<DecayTerm> terms;
+    std::vector<SpinLaw> laws;
+    std::vector<int> has_law;
     for (int ich = 0; ich < pdg->decays[ipart]; ich++) {
       const int row = pdg->dec_first[ipart] + ich;
       const int decay_products = std::abs(pdg->dec_npart[row]);
@@ -480,6 +694,9 @@ int resonance_decays_device(const is3d_particle_list *pdg, int n_chosen, const i
           T.mass_parent = mass_parent; T.mass2 = mass * mass; T.Estar = Estar; T.pstar = std::sqrt(Estar * Estar - mass * mass);
           T.prefactor = (double)members[gi] * mass_parent * branch_ratio / (8.0 * T.pstar);
           terms.push_back(T);
+          SpinLaw L{0.0, 0.0};
+          has_law.push_back(spin && transfer_law(pdg, spin->spin2, spin->parity, ipart, groups[gi], idx[0] == groups[gi] ? idx[1] : idx[0], &L.a, &L.b));
+          laws.push_back(L);
         }
       } else {
         const double mass_parent = pdg->mass[ipart];
@@ -497,6 +714,7 @@ int resonance_decays_device(const is3d_particle_list *pdg, int n_chosen, const i
           T.d = (mass_2 - mass_3) * (mass_2 - mass_3);
           T.prefactor = (double)members[gi] * (mass_parent * mass_parent) * (T.s_plus - T.s_minus) * branch_ratio / (8.0 * Q_norm);
           terms.push_back(T);
+          laws.push_back(SpinLaw{0.0, 0.0}); has_law.push_back(0);                // 3-body channels only dilute
         }
       }
     }
@@ -505,12 +723,22 @@ int resonance_decays_device(const is3d_particle_list *pdg, int n_chosen, const i
     std::vector<int> ids2, ids3;
     for (int t = 0; t < (int)terms.size(); t++) (terms[t].body == 2 ? ids2 : ids3).push_back(t);
     std::vector<int> ids(ids2); ids.insert(ids.end(), ids3.begin(), ids3.end());
+    std::vector<int> spin_ids;                                                // 2-body terms with a law, then the has_law flags
+    for (int t : ids2) if (has_law[t]) spin_ids.push_back(t);
+    const int n_spin = (int)spin_ids.size();
+    spin_ids.insert(spin_ids.end(), has_law.begin(), has_law.end());
     // pageable host memory: these copies complete before cudaMemcpyAsync returns, so the vectors may go out of scope
     if (!ck(cudaMemcpyAsync(B.terms, terms.data(), sizeof(DecayTerm) * terms.size(), cudaMemcpyHostToDevice, st), "H2D") ||
         !ck(cudaMemcpyAsync(B.ids, ids.data(), sizeof(int) * ids.size(), cudaMemcpyHostToDevice, st), "H2D")) return IS3D_ERR_CUDA;
-    log_parent_kernel<<<(n_bins + 255) / 256, 256, 0, st>>>(G, dN_dev, ichosen, B.logdN);
+    if (spin && (!ck(cudaMemcpyAsync(B.laws, laws.data(), sizeof(SpinLaw) * laws.size(), cudaMemcpyHostToDevice, st), "H2D") ||
+                 !ck(cudaMemcpyAsync(B.spin_ids, spin_ids.data(), sizeof(int) * spin_ids.size(), cudaMemcpyHostToDevice, st), "H2D"))) return IS3D_ERR_CUDA;
+    log_parent_kernel<<<(n_bins + 255) / 256, 256, 0, st>>>(G, dN_spec, ichosen, B.logdN);
     decay_setup_kernel<<<(unsigned)terms.size(), 128, 0, st>>>(G, B.terms, B.logdN, B.MT, B.fit, B.error);
     *launches += 2;
+    if (n_spin > 0) {                                 // the parent's arrays are final here: its own feed-down came from heavier parents
+      spin_table_kernel<<<(n_bins + 255) / 256, 256, 0, st>>>(G, dN_dev, spin->n_total, ichosen, pdg->mass[ipart], B.Sstar);
+      (*launches)++;
+    }
     if (!ids2.empty()) {
       const int64_t n = (int64_t)ids2.size() * n_bins;
       decay2_kernel<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(G, B.terms, B.ids, (int)ids2.size(), B.logdN, B.MT, B.fit, B.scratch);
@@ -521,8 +749,17 @@ int resonance_decays_device(const is3d_particle_list *pdg, int n_chosen, const i
       decay3_kernel<<<(unsigned)((n + kBins3 - 1) / kBins3), dim3(GP, kBins3), 0, st>>>(G, B.terms, B.ids + ids2.size(), (int)ids3.size(), B.logdN, B.MT, B.fit, B.scratch);
       (*launches)++;
     }
-    decay_add_kernel<<<(n_bins + 255) / 256, 256, 0, st>>>(G, B.terms, (int)terms.size(), B.scratch, dN_dev);
+    if (n_spin > 0) {
+      const int64_t n = (int64_t)n_spin * n_bins;
+      decay2_spin_kernel<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(G, B.terms, B.laws, B.spin_ids, n_spin, B.logdN, B.MT, B.fit, B.Sstar, B.spin_scratch);
+      (*launches)++;
+    }
+    decay_add_kernel<<<(n_bins + 255) / 256, 256, 0, st>>>(G, B.terms, (int)terms.size(), B.scratch, dN_spec);
     (*launches)++;
+    if (n_spin > 0) {
+      spin_add_kernel<<<(n_bins + 255) / 256, 256, 0, st>>>(G, B.terms, B.spin_ids + n_spin, (int)terms.size(), B.spin_scratch, dN_dev, spin->n_total);
+      (*launches)++;
+    }
     if (!ck(cudaGetLastError(), "decay kernels")) return IS3D_ERR_CUDA;
     // the term list of the next parent reuses B.terms: the stream must be done with it (also surfaces kernel faults per parent)
     if (!ck(cudaStreamSynchronize(st), "decay kernels")) return IS3D_ERR_CUDA;
@@ -531,6 +768,20 @@ int resonance_decays_device(const is3d_particle_list *pdg, int n_chosen, const i
   if (!ck(cudaMemcpyAsync(&flag, B.error, sizeof(int), cudaMemcpyDeviceToHost, st), "D2H") || !ck(cudaStreamSynchronize(st), "sync")) return IS3D_ERR_CUDA;
   if (flag) { *err = "not enough positive points of a parent spectrum beyond mT = 1.65 M to fit its large-mT tail (the reference exits here)"; return IS3D_ERR_ARGUMENT; }
   return IS3D_OK;
+}
+
+int resonance_decays_device(const is3d_particle_list *pdg, int n_chosen, const int32_t *chosen, const is3d_grid *gr, int dimension,
+                            double *dN_dev, cudaStream_t st, int *launches, std::string *err)
+{
+  return decays_core(pdg, n_chosen, chosen, gr, dimension, dN_dev, nullptr, st, launches, err);
+}
+
+// S_dev: the five arrays [St | Sx | Sy | Sz | Snorm] on the device, n_total doubles each, amended in place
+int polarization_decays_device(const is3d_particle_list *pdg, const int32_t *spin2, const int32_t *parity, int n_chosen, const int32_t *chosen,
+                               const is3d_grid *gr, int dimension, double *S_dev, int64_t n_total, cudaStream_t st, int *launches, std::string *err)
+{
+  const SpinFeedDown spin{spin2, parity, n_total};
+  return decays_core(pdg, n_chosen, chosen, gr, dimension, S_dev, &spin, st, launches, err);
 }
 
 }  // namespace is3d

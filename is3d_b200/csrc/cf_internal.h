@@ -110,6 +110,10 @@ cudaError_t launch_fp64_peak(double *sink, int iters, cudaStream_t st, int *bloc
 // resonance-decay feed-down on device-resident spectra (cf_decays.cu)
 int resonance_decays_device(const is3d_particle_list *pdg, int n_chosen, const int32_t *chosen, const is3d_grid *gr, int dimension,
                             double *dN_dev, cudaStream_t st, int *launches, std::string *err);
+// polarization feed-down (cf_decays.cu): S_dev = [St | Sx | Sy | Sz | Snorm], n_total doubles each, amended in place; spin2 / parity
+// (host) per particle-list entry
+int polarization_decays_device(const is3d_particle_list *pdg, const int32_t *spin2, const int32_t *parity, int n_chosen, const int32_t *chosen,
+                               const is3d_grid *gr, int dimension, double *S_dev, int64_t n_total, cudaStream_t st, int *launches, std::string *err);
 // strict (reference-order) diagnostic variant, df_mode 1 / 2 (cf_strict.cu); cell_scratch: n_cells * strict_cell_bytes()
 size_t strict_cell_bytes();
 cudaError_t launch_strict(const is3d_flags &fl, const RawCells &cells, const PrepTables &tab, const Layout &L, const double *mass, const double *sign,

@@ -170,6 +170,7 @@ static bool read_pdg_smash_box(const std::string &path, std::vector<Particle> *o
       const bool hadron = !deuteron && nq3 != 0 && nq2 != 0;
       const bool meson = hadron && nq1 == 0, bary = hadron && nq1 != 0;
       Particle p; p.name = name; p.mass = mass; p.width = width; p.mcid = ids[k];
+      p.parity = (parity == '+') ? 1 : (parity == '-') ? -1 : 0;
       if (hadron) { p.gspin = (nJ > 0) ? nJ : 1; p.baryon = bary ? 1 : 0; p.sign = meson ? -1 : 1; }
       else if (deuteron) { p.gspin = 3; p.baryon = 2; p.sign = -1; }
       else { p.gspin = nq3 + 1; p.baryon = 0; p.sign = nq3 % 2; }
@@ -179,6 +180,18 @@ static bool read_pdg_smash_box(const std::string &path, std::vector<Particle> *o
     }
   }
   *out = v;
+  return true;
+}
+
+bool read_box_parities(const std::string &workdir, std::map<long, int> *out, std::string *err)
+{
+  std::vector<Particle> box;
+  if (!read_pdg_smash_box(workdir + "/PDG/pdg_box.dat", &box, err)) {
+    if (err) *err += " (polarization_feed_down = 1 reads the parities there)";
+    return false;
+  }
+  out->clear();
+  for (const Particle &p : box) if (p.parity != 0) out->emplace(std::labs(p.mcid), p.parity);       // first entry of an id wins
   return true;
 }
 

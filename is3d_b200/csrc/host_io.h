@@ -36,10 +36,14 @@ struct Particle {
   double mass = 0, width = 0;
   int gspin = 0, baryon = 0, strange = 0, charm = 0, bottom = 0, gisospin = 0, charge = 0, decays = 0, sign = 0;
   int stable = 0;                          // first channel has a single product (readindata.cpp:1487-1488)
+  int parity = 0;                          // pdg_box.dat only: intrinsic parity +1 / -1 (0 for the conventional lists)
   std::vector<DecayChannel> channels;      // conventional lists only (pdg_box.dat carries no decay table)
 };
 // PDG/pdg-urqmd_v3.3+.dat, PDG/pdg_smash.dat (readindata.cpp:1440-1568) and PDG/pdg_box.dat (:1571-1684)
 bool read_pdg(const std::string &workdir, int hrg_eos, std::vector<Particle> *out, std::string *err);
+// intrinsic parities by |MC id| from the PARITY column of PDG/pdg_box.dat (the polarization feed-down reads them next to a conventional
+// list); a missing file is an error, an id the file lacks is simply absent from the map
+bool read_box_parities(const std::string &workdir, std::map<long, int> *out, std::string *err);
 
 struct SurfaceData {
   int64_t n = 0;

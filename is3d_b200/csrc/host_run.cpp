@@ -181,9 +181,10 @@ static bool write_spacetime_files(const std::string &wd, const std::vector<int> 
 // phi block of write_spectra_files; truncating opens, results/polarization/ must exist.
 // With the thermal-shear sums xi (St | Sx | Sy | Sz | Snorm of is3d_b200_spin_polarization_shear, non-NULL) it writes S_xi_<mcid>.dat
 // instead: Snorm, the shear part N_xi / Snorm, the total S = (N + N_xi) / Snorm and the rest-frame part of the total.
+// stem: the file name stem of the plain form ("S"; "S_fd" for the sums after the feed-down through decays).
 static bool write_polarization_files(const std::string &wd, const std::vector<double> &sums, const std::vector<double> *xi,
                                      const std::vector<int> &mcid, const std::vector<double> &mass, const Grids &g, int dimension,
-                                     std::string *err)
+                                     std::string *err, const char *stem = "S")
 {
   const int npart = (int)mcid.size(), npT = (int)g.pT.rows, nphi = (int)g.phi.rows, ny = (int)g.y.rows;
   const int y_pts = (dimension == 2) ? 1 : ny;
@@ -192,7 +193,8 @@ static bool write_polarization_files(const std::string &wd, const std::vector<do
   const double *Xx = xi ? &(*xi)[n_bins] : nullptr, *Xy = xi ? Xx + n_bins : nullptr, *Xz = xi ? Xy + n_bins : nullptr;
   for (int ipart = 0; ipart < npart; ipart++) {
     char name[255];
-    std::snprintf(name, sizeof(name), xi ? "%s/results/polarization/S_xi_%d.dat" : "%s/results/polarization/S_%d.dat", wd.c_str(), mcid[ipart]);
+    if (xi) std::snprintf(name, sizeof(name), "%s/results/polarization/S_xi_%d.dat", wd.c_str(), mcid[ipart]);
+    else std::snprintf(name, sizeof(name), "%s/results/polarization/%s_%d.dat", wd.c_str(), stem, mcid[ipart]);
     std::ofstream f(name, std::ios_base::out);
     if (!f) { *err = std::string("cannot open ") + name + " (the directory results/polarization/ must exist)"; return false; }
     f << (xi ? "y\tphip\tpT\tSnorm\tSx_xi\tSy_xi\tSz_xi\tSx\tSy\tSz\tSx_rest\tSy_rest\tSz_rest\n"
@@ -303,6 +305,8 @@ struct Problem {
   int operation = 0, hrg_eos = 0, group_particles = 0, do_resonance_decays = 0;
   int spin_polarization = 0;               // optional key (absent: 0): mode-5 spin polarization after the spectra
   int thermal_shear_polarization = 0;      // optional key (absent: 0): add the thermal-shear term (input/thermal_shear.dat)
+  int polarization_feed_down = 0;          // optional key (absent: 0): feed the polarization sums down through the decay tables
+  std::map<long, int> box_parity;          // its parities by |MC id| (PDG/pdg_box.dat)
   int hbt_radii = 0;                       // optional key (absent: 0): HBT radii of the linear-delta-f spectra after the spectra
   int hbt_correlation = 0;                 // optional key (absent: 0): MC id of the species whose HBT correlation functions are written
   int hbt_species = -1;                    // its index among the chosen species
@@ -353,6 +357,12 @@ static int load_problem(const std::string &wd, bool need_surface, Problem *p, st
   if (p->thermal_shear_polarization && (p->operation != 1 || fl.mode != 5 || !p->spin_polarization)) {
     err = "thermal_shear_polarization = 1 needs operation = 1, a mode 5 surface and spin_polarization = 1"; return IS3D_ERR_UNSUPPORTED;
   }
+  p->polarization_feed_down = par.has("polarization_feed_down") ? (int)par.get("polarization_feed_down", &err) : 0;
+  if (p->polarization_feed_down && (p->operation != 1 || fl.mode != 5 || !p->spin_polarization || (p->hrg_eos != 1 && p->hrg_eos != 2))) {
+    err = "polarization_feed_down = 1 needs operation = 1, a mode 5 surface, spin_polarization = 1 and a particle list with decay tables "
+          "(hrg_eos = 1, 2)";
+    return IS3D_ERR_UNSUPPORTED;
+  }
   p->hbt_radii = par.has("hbt_radii") ? (int)par.get("hbt_radii", &err) : 0;
   if (p->hbt_radii && (p->operation != 1 || fl.mode == 2 || (fl.df_mode != 1 && fl.df_mode != 2) || fl.include_baryon)) {
     err = "hbt_radii = 1 needs operation = 1, a viscous-hydro surface (mode != 2), df_mode 1 or 2 and include_baryon = 0"; return IS3D_ERR_UNSUPPORTED;
@@ -376,6 +386,7 @@ static int load_problem(const std::string &wd, bool need_surface, Problem *p, st
   }
   // ---- particle list, delta-f tables
   if (!read_pdg(wd, p->hrg_eos, &p->pdg, &err)) return IS3D_ERR_IO;
+  if (p->polarization_feed_down && !read_box_parities(wd, &p->box_parity, &err)) return IS3D_ERR_IO;
   if ((int)p->pdg.size() > 600) { err = "number of particles exceeds Maxparticle = 600"; return IS3D_ERR_IO; }
   if (!read_df_tables(wd, p->hrg_eos, &p->dft, &err)) return IS3D_ERR_IO;
   if (!read_laguerre(wd + "/tables/gla_roots_weights_32_points.txt", &p->gla, &err)) return IS3D_ERR_IO;
@@ -418,6 +429,28 @@ static int load_problem(const std::string &wd, bool need_surface, Problem *p, st
   if (g.pT.cols.size() < 2 || g.phi.cols.size() < 2 || g.eta.cols.size() < 2) { err = "momentum tables need a weight column"; return IS3D_ERR_IO; }
   return IS3D_OK;
 }
+
+// the particle list with its decay channels flattened for is3d_b200_resonance_decays / is3d_b200_polarization_decays
+struct FlatList {
+  std::vector<int32_t> mcid, stable, decays, first, npart, parts;
+  std::vector<double> mass, width, br;
+  explicit FlatList(const std::vector<Particle> &pdg)
+  {
+    for (const Particle &h : pdg) {
+      mcid.push_back((int32_t)h.mcid); mass.push_back(h.mass); width.push_back(h.width); stable.push_back(h.stable);
+      decays.push_back((int32_t)h.channels.size()); first.push_back((int32_t)npart.size());
+      for (const DecayChannel &ch : h.channels) {
+        npart.push_back(ch.npart); br.push_back(ch.branch_ratio);
+        for (int k = 0; k < 5; k++) parts.push_back((int32_t)ch.part[k]);
+      }
+    }
+  }
+  is3d_particle_list view()
+  {
+    return is3d_particle_list{(int32_t)mcid.size(), mcid.data(), mass.data(), width.data(), stable.data(), decays.data(), first.data(),
+                              npart.data(), br.data(), parts.data()};
+  }
+};
 
 static int run_problem(const std::string &wd, Problem &P, const is3d_surface &s, const is3d_vorticity *vort, const is3d_thermal_shear *shear,
                        double *dN_raw, int64_t n_raw, int32_t *mcid_out, int32_t n_mcid_max, is3d_stats *stats, std::string *err_out)
@@ -497,6 +530,25 @@ static int run_problem(const std::string &wd, Problem &P, const is3d_surface &s,
       if (rcx != IS3D_OK) { err = std::string("thermal-shear polarization failed: ") + is3d_b200_last_error(); return rcx; }
       if (stats) { stats->gpu_launches += sp_st.gpu_launches; stats->total_ms += sp_st.total_ms; }
       if (!write_polarization_files(wd, sums, &xi, P.mcid, P.mass, g, P.fl.dimension, &err)) return IS3D_ERR_IO;
+      for (size_t k = 0; k < 4 * n_bins; k++) sums[k] += xi[k];  // the feed-down below runs on the total (vorticity + shear)
+    }
+    if (P.polarization_feed_down) {
+      // 2J = gspin - 1 of the list, parities by |MC id| from pdg_box.dat (0, unknown: the channel only dilutes)
+      std::vector<int32_t> spin2, parity, chosen(P.pick.begin(), P.pick.end());
+      for (const Particle &h : P.pdg) {
+        spin2.push_back(h.gspin - 1);
+        const auto it = P.box_parity.find(std::labs(h.mcid));
+        parity.push_back(it == P.box_parity.end() ? 0 : it->second);
+      }
+      FlatList flat(P.pdg);
+      const is3d_particle_list pl = flat.view();
+      const is3d_spin_parity spp{spin2.data(), parity.data()};
+      is3d_polarization_result r{&sums[0], &sums[n_bins], &sums[2 * n_bins], &sums[3 * n_bins], &sums[4 * n_bins]};
+      is3d_stats fd_st; std::memset(&fd_st, 0, sizeof(fd_st));
+      const int rcf = is3d_b200_polarization_decays(&pl, &spp, npart, chosen.data(), &gr, P.fl.dimension, nullptr, &r, &fd_st);
+      if (rcf != IS3D_OK) { err = std::string("polarization feed-down failed: ") + is3d_b200_last_error(); return rcf; }
+      if (stats) { stats->gpu_launches += fd_st.gpu_launches; stats->total_ms += fd_st.total_ms; }
+      if (!write_polarization_files(wd, sums, nullptr, P.mcid, P.mass, g, P.fl.dimension, &err, "S_fd")) return IS3D_ERR_IO;
     }
   }
   if (P.hbt_radii) {
@@ -527,18 +579,9 @@ static int run_problem(const std::string &wd, Problem &P, const is3d_surface &s,
   if (P.do_resonance_decays) {
     // feed-down on the GPU, then the two amended-spectra files (emissionfunction.cpp:1689-1698)
     std::printf("Starting resonance decays: \n\n");
-    std::vector<int32_t> mcid, stable, decays, first, npartv, parts, chosen(P.pick.begin(), P.pick.end());
-    std::vector<double> mass, width, br;
-    for (const Particle &h : P.pdg) {
-      mcid.push_back((int32_t)h.mcid); mass.push_back(h.mass); width.push_back(h.width); stable.push_back(h.stable);
-      decays.push_back((int32_t)h.channels.size()); first.push_back((int32_t)npartv.size());
-      for (const DecayChannel &ch : h.channels) {
-        npartv.push_back(ch.npart); br.push_back(ch.branch_ratio);
-        for (int k = 0; k < 5; k++) parts.push_back((int32_t)ch.part[k]);
-      }
-    }
-    is3d_particle_list pl{(int32_t)P.pdg.size(), mcid.data(), mass.data(), width.data(), stable.data(), decays.data(), first.data(),
-                          npartv.data(), br.data(), parts.data()};
+    std::vector<int32_t> chosen(P.pick.begin(), P.pick.end());
+    FlatList flat(P.pdg);
+    const is3d_particle_list pl = flat.view();
     is3d_stats sd; std::memset(&sd, 0, sizeof(sd));
     const int rcd = is3d_b200_resonance_decays(&pl, npart, chosen.data(), &gr, P.fl.dimension, nullptr, dN.data(), &sd);
     if (rcd != IS3D_OK) { err = std::string("resonance decays failed: ") + is3d_b200_last_error(); return rcd; }
@@ -664,6 +707,12 @@ extern "C" int is3d_b200_host_dump(const char *workdir, const char *out_path)
   if (P.thermal_shear_polarization) {
     put("xtt", s.xtt); put("xtx", s.xtx); put("xty", s.xty); put("xtn", s.xtn); put("xxx", s.xxx);
     put("xxy", s.xxy); put("xxn", s.xxn); put("xyy", s.xyy); put("xyn", s.xyn); put("xnn", s.xnn);
+  }
+  if (P.polarization_feed_down) {        // what the feed-down passes as is3d_spin_parity: 2J = gspin - 1, parity by |MC id| (0 unknown)
+    tmp.clear(); for (auto &h : P.pdg) tmp.push_back(h.gspin - 1); put("pdg_spin2", tmp);
+    tmp.clear();
+    for (auto &h : P.pdg) { const auto it = P.box_parity.find(std::labs(h.mcid)); tmp.push_back(it == P.box_parity.end() ? 0 : it->second); }
+    put("pdg_parity", tmp);
   }
   tmp.assign(s.avg, s.avg + 5); put("avg", tmp);
   put("df_T", P.dft.T); put("df_c0", P.dft.c0); put("df_c2", P.dft.c2); put("df_F", P.dft.F); put("df_betabulk", P.dft.betabulk);

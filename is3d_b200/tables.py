@@ -87,6 +87,28 @@ def pdg_decay_table(fx, hrg_eos):
     return {k: np.asarray(v) for k, v in out.items()}
 
 
+def box_parities(fx):
+    """Intrinsic parity by |MC id| from the SMASH box list (PDG/pdg_box.dat, the column read_pdg_smash_box parses): {|mcid|: +1 / -1}."""
+    out = {}
+    for i in range(len(fx["pdg_box/name"])):
+        p = str(fx["pdg_box/parity"][i])
+        for m in fx["pdg_box/mcid"][i]:
+            if int(m) != 0 and p in "+-":
+                out.setdefault(abs(int(m)), 1 if p == "+" else -1)
+    return out
+
+
+def spin_parity(fx, pdg, hrg_eos=1):
+    """The is3d_spin_parity table of a particle list pdg (tables.pdg_decay_table order): spin2 = 2J = gspin - 1 of the list, parity
+    from PDG/pdg_box.dat by |MC id| (charge conjugation keeps the product of parities of a decay), 0 for an id the box list lacks."""
+    key = _PDG_KEY[hrg_eos]
+    gspin = {abs(int(m)): int(g) for m, g in zip(fx[key + "/mcid"], fx[key + "/gspin"])}
+    par = box_parities(fx)
+    spin2 = np.array([gspin[abs(int(m))] - 1 for m in pdg["mcid"]], dtype=np.int32)
+    parity = np.array([par.get(abs(int(m)), 0) for m in pdg["mcid"]], dtype=np.int32)
+    return dict(spin2=spin2, parity=parity)
+
+
 def species(fx, hrg_eos=1, chosen="chosen_urqmd", group_particles=False):
     pdg = pdg_table(fx, hrg_eos)
     ids = fx[chosen] if isinstance(chosen, str) else np.asarray(chosen, dtype=np.int64)

@@ -32,7 +32,8 @@ DEFAULT_PARAMETERS = [
 ]
 
 # keys of this drop-in that the reference does not read: written only when a caller sets them (absent: 0, or the default of the host layer)
-OPTIONAL_PARAMETERS = ("spin_polarization", "thermal_shear_polarization", "hbt_radii", "hbt_correlation", "hbt_dq", "hbt_q_points")
+OPTIONAL_PARAMETERS = ("spin_polarization", "thermal_shear_polarization", "polarization_feed_down", "hbt_radii", "hbt_correlation", "hbt_dq",
+                       "hbt_q_points")
 
 _EOS_DIR = {1: "urqmd", 2: "smash", 3: "smash_box"}
 _EOS_PDG = {1: ("pdg_urqmd", "pdg-urqmd_v3.3+.dat"), 2: ("pdg_smash", "pdg_smash.dat"), 3: ("pdg_box", "pdg_box.dat")}
@@ -157,6 +158,8 @@ def materialize(root, surface_columns=None, chosen=None, fixture=None, tables=No
         _write_pdg_box(os.path.join(root, "PDG", fname), fx)
     else:
         _write_pdg_conventional(os.path.join(root, "PDG", fname), fx, key)
+        if int(p.get("polarization_feed_down", 0)):
+            _write_pdg_box(os.path.join(root, "PDG", "pdg_box.dat"), fx)     # the parities the polarization feed-down reads
     if chosen is None:
         chosen = "chosen_pikp"
     if isinstance(chosen, str):
