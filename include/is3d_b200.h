@@ -238,6 +238,37 @@ int is3d_b200_spin_polarization_shear_multi(const is3d_flags *flags, const is3d_
                                             const is3d_species *species, const is3d_grid *grid, const is3d_options *options,
                                             is3d_polarization_result *result, is3d_stats *stats);
 
+/* ---- spin density matrix of hadrons from thermal vorticity: all-order mean spin, rank-2 spin tensor, vector-meson rho00 ---------
+ * The local-equilibrium distribution with the spin term exponentiated, [exp(beta.p - (1/2) varpi:Sigma) + Theta]^-1 (Becattini, Chandra,
+ * Del Zanna, Grossi, Ann. Phys. 338 (2013) 32), for any spin J = (g - 1)/2, over the cells, slots, weights, u.dsigma <= 0 skip, outflow
+ * rule, species and bins of is3d_b200_spin_polarization (the same vorticity input and conventions).  Per evaluation:
+ *    theta^mu = -(1/(2m)) eps^{mu rho sigma tau} varpi_{rho sigma} p_tau = (1/m)(omega.p, E omega - e x p)   (4 x the vector of the N^mu
+ *               sum, without (1 - Theta f)),  theta*_i = theta^i - theta^t p^i/(E + m) (rest frame of the pure boost along p),
+ *    theta = |theta* |, that = theta* / theta,  f_m = 1/(exp(u.p/T - m theta) + Theta) for the levels m = -J .. J along that.
+ * Nine RAW sums per bin (K = 1/(2 pi hbar c)^3, W = slot weight x p.dsigma), which add across cell shards and devices:
+ *    Snorm = K sum W sum_m f_m
+ *    P_i   = K sum W sum_m m f_m that_i                                          i = x, y, z
+ *    Q_ij  = K sum W sum_m f_m (3m^2 - J(J+1))/2 (that_i that_j - delta_ij/3)    ij = xx, xy, xz, yy, yz  (Q_zz = -Q_xx - Q_yy)
+ * Ratios: <S*_i> = P_i/Snorm; T_ij = <S*_i S*_j> - J(J+1) delta_ij/3 = Q_ij/Snorm; for J = 1, rho00 along a rest-frame unit axis n is
+ * 1/3 - n.T.n.  At theta = 0 (varpi = 0, or J = 0) P and Q are exactly 0 and Snorm is the Snorm of is3d_b200_spin_polarization; at
+ * linear order P_i/Snorm = (J(J+1)/3)(1 - Theta f) theta*_i, i.e. 4J(J+1)/3 times its rest-frame S*.
+ * Only the varpi term is exponentiated: rho00 - 1/3 is the second order of that exponent, not a complete second-order gradient expansion
+ * (shear-induced alignment and other second-order terms are not included).
+ * All nine arrays are ADDED into; host or device memory per options->memory.
+ * Errors: IS3D_ERR_UNSUPPORTED for mode = 2 and include_baryon = 1; IS3D_ERR_ARGUMENT for a NULL vorticity, a NULL result array, a
+ * species with m <= 0 or with a degeneracy that is not an integer in [1, 16], and for a boson (Theta = -1) evaluation with
+ * u.p/T - J theta <= 0, where the top level has no valid occupation (the count is in is3d_b200_last_error()).  On any error every result
+ * array is left untouched. */
+typedef struct { double *Snorm, *Px, *Py, *Pz, *Qxx, *Qxy, *Qxz, *Qyy, *Qyz; } is3d_spin_density_result;
+int is3d_b200_spin_density(const is3d_flags *flags, const is3d_surface *surface, const is3d_vorticity *vorticity,
+                           const is3d_species *species, const is3d_grid *grid, const is3d_options *options,
+                           is3d_spin_density_result *result, is3d_stats *stats);
+/* Same over the devices of is3d_b200_init_devices(): HOST arrays, contiguous cell shards, the nine arrays summed on the host in device
+ * order. */
+int is3d_b200_spin_density_multi(const is3d_flags *flags, const is3d_surface *surface, const is3d_vorticity *vorticity,
+                                 const is3d_species *species, const is3d_grid *grid, const is3d_options *options,
+                                 is3d_spin_density_result *result, is3d_stats *stats);
+
 /* ---- feed-down of the spin polarization through resonance decays ------------------------------------------------------------
  * Amends, in place, the five raw-sum arrays of is3d_b200_spin_polarization (or vorticity + shear sums added component by component) so
  * that they describe all hadrons of a species, primary and from decays.  Parents, order, channels, daughter groups, kernels and

@@ -614,6 +614,97 @@ def mean_spin(result, species, grid, dimension, shear=None):
     return S, rest
 
 
+SPIN_DENSITY_FIELDS = ("Snorm", "Px", "Py", "Pz", "Qxx", "Qxy", "Qxz", "Qyy", "Qyz")
+SPIN_TENSOR_FIELDS = ("xx", "xy", "xz", "yy", "yz", "zz")
+
+
+class SpinDensityResult(C.Structure):
+    _fields_ = [(k, _D) for k in SPIN_DENSITY_FIELDS]
+
+
+def spin_density(flags, cells, vorticity, species, grid, memory="host", stream=None, multi=False):
+    """Call is3d_b200_spin_density (or the _multi entry point over the devices of init_devices(), host arrays only): the spin density
+    matrix of every species (spin J = (degeneracy - 1)/2) with the thermal-vorticity term exponentiated, on a mode-5 surface.
+
+    vorticity: as for spin_polarization().  Returns (dict Snorm, Px, Py, Pz, Qxx, Qxy, Qxz, Qyy, Qyz of RAW sums, flat
+    [y][phi][pT][species], numpy or CUDA tensors; stats dict).  spin_moments() and spin_alignment() form the ratios."""
+    device = (memory == "device")
+    m = _Marshal(device)
+    sf, sp, g, _, _ = _marshal_problem(m, cells, species, grid, None, None)
+    vo = None
+    if vorticity is not None:
+        vo = Vorticity()
+        for k in VORTICITY_FIELDS:
+            setattr(vo, k, m.cells(vorticity[k]))
+    n = sp.n * g.n_pT * g.n_phi * g.n_y
+    res = SpinDensityResult()
+    if device:
+        import torch
+        out = {k: torch.zeros(n, dtype=torch.float64, device=cells["tau"].device) for k in SPIN_DENSITY_FIELDS}
+        for k in SPIN_DENSITY_FIELDS:
+            setattr(res, k, C.cast(C.c_void_p(out[k].data_ptr()), _D))
+        if stream is None:
+            stream = torch.cuda.current_stream().cuda_stream
+    else:
+        out = {k: np.zeros(n) for k in SPIN_DENSITY_FIELDS}
+        for k in SPIN_DENSITY_FIELDS:
+            setattr(res, k, out[k].ctypes.data_as(_D))
+    opt = Options(); opt.memory = 1 if device else 0; opt.stream = C.c_void_p(stream or 0)
+    st = Stats()
+    fl = make_flags(flags)
+    f = lib().is3d_b200_spin_density_multi if multi else lib().is3d_b200_spin_density
+    f.restype = C.c_int
+    f.argtypes = [C.POINTER(Flags), C.POINTER(Surface), C.POINTER(Vorticity), C.POINTER(Species), C.POINTER(Grid), C.POINTER(Options),
+                  C.POINTER(SpinDensityResult), C.POINTER(Stats)]
+    _check(f(C.byref(fl), C.byref(sf), C.byref(vo) if vo is not None else None, C.byref(sp), C.byref(g), C.byref(opt), C.byref(res),
+             C.byref(st)))
+    return out, st.as_dict()
+
+
+def spin_moments(result, species):
+    """Ratios of the raw sums of spin_density(): returns (S* [3][n_bins] = <S*_i> = P_i / Snorm, the all-order rest-frame mean spin;
+    T [6][n_bins] = <S*_i S*_j> - J(J+1) delta_ij / 3 = Q_ij / Snorm in the order xx, xy, xz, yy, yz, zz), 0 where Snorm = 0.  The
+    numbers results/polarization/spin_<mcid>.dat holds.  species is accepted for symmetry with mean_spin(); the ratios need only the sums."""
+    r = {k: np.asarray(result[k].cpu() if _is_torch(result[k]) else result[k], dtype=np.float64) for k in SPIN_DENSITY_FIELDS}
+    sn = r["Snorm"]
+    nz = sn != 0
+    S = np.zeros((3, sn.size)); T = np.zeros((6, sn.size))
+    for i, k in enumerate(("Px", "Py", "Pz")):
+        S[i, nz] = r[k][nz] / sn[nz]
+    for i, k in enumerate(("Qxx", "Qxy", "Qxz", "Qyy", "Qyz")):
+        T[i, nz] = r[k][nz] / sn[nz]
+    T[5, nz] = -(r["Qxx"][nz] + r["Qyy"][nz]) / sn[nz]
+    return S, T
+
+
+def spin_alignment(result, species, grid, dimension, axis):
+    """Vector-meson spin alignment rho00 = 1/3 - n.T.n from the raw sums of spin_density(), [n_bins], for the species with J = 1
+    (degeneracy 3); NaN for every other species.  axis: "x", "y", "z" (a fixed rest-frame axis) or "helicity" (n = p / |p|, the bin's
+    momentum direction; 2+1D bins have y = 0)."""
+    _, T = spin_moments(result, species)
+    m = np.asarray(species["mass"], dtype=np.float64)
+    deg = np.asarray(species["degeneracy"], dtype=np.float64)
+    pT = np.asarray(grid["pT"], dtype=np.float64); phi = np.asarray(grid["phi"], dtype=np.float64)
+    y = np.asarray(grid["y"], dtype=np.float64)
+    if dimension == 2:
+        y = np.zeros_like(y)
+    yy, ff, pp, mm = np.meshgrid(y, phi, pT, m, indexing="ij")          # [y][phi][pT][species] = the flat bin order
+    _, _, _, gg = np.meshgrid(y, phi, pT, deg, indexing="ij")
+    if axis == "helicity":
+        mT = np.sqrt(mm * mm + pp * pp)
+        p = np.stack([(pp * np.cos(ff)).ravel(), (pp * np.sin(ff)).ravel(), (mT * np.sinh(yy)).ravel()])
+        n = p / np.linalg.norm(p, axis=0)
+    elif axis in ("x", "y", "z"):
+        n = np.zeros((3, T.shape[1]))
+        n["xyz".index(axis)] = 1.0
+    else:
+        raise ValueError("axis must be 'x', 'y', 'z' or 'helicity'")
+    Tm = {k: T[i] for i, k in enumerate(SPIN_TENSOR_FIELDS)}
+    nTn = (n[0] * n[0] * Tm["xx"] + n[1] * n[1] * Tm["yy"] + n[2] * n[2] * Tm["zz"]
+           + 2.0 * (n[0] * n[1] * Tm["xy"] + n[0] * n[2] * Tm["xz"] + n[1] * n[2] * Tm["yz"]))
+    return np.where(gg.ravel() == 3, 1.0 / 3.0 - nTn, np.nan)
+
+
 HBT_FIELDS = ("S0", "So", "Ss", "Sl", "Soo", "Sss", "Sll", "Sos", "Sol", "Ssl")
 HBT_RADII = ("out", "side", "long", "outside", "outlong", "sidelong")
 

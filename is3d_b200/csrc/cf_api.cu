@@ -1219,25 +1219,40 @@ extern "C" int is3d_b200_spacetime_distributions_multi(const is3d_flags *fl, con
 
 // =====================================================================================================================
 // Spin polarization from thermal vorticity (cf_polzn.cu) and thermal shear (cf_polzn_xi.cu): raw sums N^mu and Snorm, added into the
-// caller's five arrays
+// caller's five arrays; spin density matrix from thermal vorticity (cf_spin_density.cu): nine raw sums
 // =====================================================================================================================
 namespace is3d {
 
-// tensor: the 6 vorticity columns (shear = false) or the 10 thermal-shear columns (shear = true), NULL for a NULL struct.  Both terms
-// run on the same layout and chunk split, so their Snorm is bit-identical; the shear kernel leaves St alone (N_xi^t = 0 exactly).
-static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const double *const *tensor, bool shear, const is3d_species *sp,
-                      const is3d_grid *gr, const is3d_options *opt_in, is3d_polarization_result *res, is3d_stats *stats)
+enum PolTerm { kPolVorticity, kPolShear, kPolSpinDensity };
+
+// result arrays per term, in the order of the kernel's partial rows; the shear term's fifth array (St) must be non-NULL but is left
+// alone (N_xi^t = 0 exactly)
+static int pol_n_out(PolTerm term) { return term == kPolSpinDensity ? kSdSums : 5; }
+
+// tensor: the 6 vorticity columns (vorticity, spin density) or the 10 thermal-shear columns (shear), NULL for a NULL struct.  out: the
+// pol_n_out(term) result arrays, NULL for a NULL result struct.  The vorticity and shear terms run on the same layout and chunk split, so
+// their Snorm is bit-identical.  The spin-density kernel has its own register tile but the same cell chunks, so at varpi = 0 its Snorm is
+// bit-identical too (unless the 4 GiB cap on its nine partial arrays lowers the chunk count).
+static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const double *const *tensor, PolTerm term, const is3d_species *sp,
+                      const is3d_grid *gr, const is3d_options *opt_in, double *const *out, is3d_stats *stats)
 {
+  const bool shear = (term == kPolShear);
   const int n_tensor = shear ? 10 : 6;
-  if (!fl || !sf || !sp || !gr || !res) return fail(IS3D_ERR_ARGUMENT, "NULL argument");
+  if (!fl || !sf || !sp || !gr || !out) return fail(IS3D_ERR_ARGUMENT, "NULL argument");
   if (!tensor) return fail(IS3D_ERR_ARGUMENT, shear ? "NULL thermal shear" : "NULL vorticity");
-  if (!res->St || !res->Sx || !res->Sy || !res->Sz || !res->Snorm) return fail(IS3D_ERR_ARGUMENT, "NULL result array");
+  for (int q = 0; q < pol_n_out(term); q++) if (!out[q]) return fail(IS3D_ERR_ARGUMENT, "NULL result array");
   if (fl->mode == 2) return fail(IS3D_ERR_UNSUPPORTED, "spin polarization needs a viscous-hydro surface with thermal vorticity (mode 5), not mode 2");
   if (fl->include_baryon) return fail(IS3D_ERR_UNSUPPORTED, "include_baryon = 1 (the reference's (T, muB) lookup reads out of bounds, SURVEY R8)");
   if (fl->dimension != 2 && fl->dimension != 3) return fail(IS3D_ERR_ARGUMENT, "dimension must be 2 or 3");
   if (sp->n <= 0 || gr->n_pT <= 0 || gr->n_phi <= 0 || gr->n_y <= 0) return fail(IS3D_ERR_ARGUMENT, "empty species list or momentum table");
   if (!sp->mass || !sp->sign || !sp->degeneracy || !gr->pT || !gr->phi || !gr->y) return fail(IS3D_ERR_ARGUMENT, "NULL species or momentum table");
   for (int s = 0; s < sp->n; s++) if (!(sp->mass[s] > 0.0)) return fail(IS3D_ERR_ARGUMENT, "spin polarization needs species with mass > 0");
+  if (term == kPolSpinDensity)
+    for (int s = 0; s < sp->n; s++) {
+      const double g = sp->degeneracy[s];
+      if (!(g >= 1.0 && g <= 16.0 && g == std::floor(g)))
+        return fail(IS3D_ERR_ARGUMENT, "the spin density needs species whose degeneracy 2J + 1 is an integer in [1, 16]");
+    }
   const bool dim2 = (fl->dimension == 2);
   if (dim2 && (gr->n_eta <= 0 || !gr->eta || !gr->eta_weight)) return fail(IS3D_ERR_ARGUMENT, "dimension = 2 needs the eta table");
   const int64_t n_cells = sf->n_cells;
@@ -1258,14 +1273,16 @@ static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const double
   const int64_t n_bins = (int64_t)sp->n * gr->n_pT * gr->n_phi * gr->n_y;
   const int64_t n_active = dim2 ? n_bins / gr->n_y : n_bins;        // 2+1D fills the y = 0 plane (index iy = 0)
 
-  // ---- layout: the cf_kernel decomposition with the register tile of cf_polzn_kernel
+  // ---- layout: the cf_kernel decomposition with the register tile of the term's kernel
   Layout L; memset(&L, 0, sizeof(L));
   L.n_species = sp->n; L.n_pT = gr->n_pT; L.n_phi = gr->n_phi; L.n_y_out = gr->n_y;
   L.dim2 = dim2 ? 1 : 0;
   L.n_slots = dim2 ? gr->n_eta : gr->n_y;
   L.rec_y = kPolRecY;
-  int nyt, npt, ct;
-  polzn_shape(L.dim2, &nyt, &npt, &ct);
+  int nyt, npt, ct, vnyt, vnpt, vct;
+  polzn_shape(L.dim2, &vnyt, &vnpt, &vct);
+  if (term == kPolSpinDensity) spin_density_shape(L.dim2, &nyt, &npt, &ct);
+  else { nyt = vnyt; npt = vnpt; ct = vct; }
   L.nst = dim2 ? L.n_slots : nyt;
   L.n_ytiles = dim2 ? 1 : (L.n_slots + nyt - 1) / nyt;
   L.npt = npt; L.n_ptiles = (L.n_phi + npt - 1) / npt;
@@ -1276,13 +1293,17 @@ static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const double
   const int n_warps = std::min(kPolWarps, n_groups);
   const int n_groupblocks = (n_groups + n_warps - 1) / n_warps;
   const int64_t n_bintiles = (int64_t)n_groupblocks * L.n_ytiles * L.n_ptiles;
-  // chunks: the rule of smooth_core (>= 192 blocks per SM, a chunk's records within a third of L2, partial sums <= 4 GiB)
-  int64_t n_chunks = ((int64_t)Dp->sm_count * 192 + n_bintiles - 1) / n_bintiles;
-  const int64_t rec_per_cell = ((int64_t)L.n_ytiles * L.nst * kPolRecY + (int64_t)L.n_ptiles * L.npt * kPolRecP) * 8;
+  // chunks: the rule of smooth_core (>= 192 blocks per SM, a chunk's records within a third of L2, partial sums <= 4 GiB), evaluated
+  // on the tile of cf_polzn_kernel for every term (same cells per TMA tile), so that all terms split the cells alike
+  const int64_t v_ytiles = dim2 ? 1 : (L.n_slots + vnyt - 1) / vnyt, v_ptiles = (L.n_phi + vnpt - 1) / vnpt;
+  const int64_t v_bintiles = (int64_t)n_groupblocks * v_ytiles * v_ptiles;
+  int64_t n_chunks = ((int64_t)Dp->sm_count * 192 + v_bintiles - 1) / v_bintiles;
+  const int64_t rec_per_cell = (v_ytiles * (dim2 ? L.n_slots : vnyt) * kPolRecY + v_ptiles * vnpt * kPolRecP) * 8;
   const int64_t l2_target = std::max<int64_t>((int64_t)Dp->l2_bytes / 3, (int64_t)8 << 20);
   n_chunks = std::max<int64_t>(n_chunks, (n_cells * rec_per_cell + l2_target - 1) / l2_target);
   const int64_t n_chunks_wanted = n_chunks;
-  n_chunks = std::min<int64_t>(n_chunks, std::max<int64_t>(1, ((int64_t)4 << 30) / (5 * n_bins * 8)));
+  const int n_part = (term == kPolSpinDensity) ? kSdSums : 5;       // partial arrays the 4 GiB cap counts (the shear term keeps 5)
+  n_chunks = std::min<int64_t>(n_chunks, std::max<int64_t>(1, ((int64_t)4 << 30) / (n_part * n_bins * 8)));
   if (opt.n_chunks > 0) n_chunks = opt.n_chunks;
   n_chunks = std::max<int64_t>(1, std::min<int64_t>(n_chunks, std::max<int64_t>(L.n_tiles, 1)));
   if (n_bintiles * n_chunks > 2147483647LL) return fail(IS3D_ERR_ARGUMENT, "grid too large");
@@ -1299,8 +1320,8 @@ static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const double
   CU_CHECK(ws.small.reserve(ar.host.size() + 256));
   CU_CHECK(ws.Y.reserve((size_t)L.n_ytiles * L.n_cells_pad * L.nst * kPolRecY * 8 + 256));
   CU_CHECK(ws.P.reserve((size_t)L.n_ptiles * L.n_cells_pad * L.npt * kPolRecP * 8 + 256));
-  CU_CHECK(ws.partial.reserve((size_t)5 * n_chunks * n_bins * 8 + 256));
-  CU_CHECK(ws.dN.reserve((size_t)5 * n_bins * 8 + 256));
+  CU_CHECK(ws.partial.reserve((size_t)n_part * n_chunks * n_bins * 8 + 256));
+  CU_CHECK(ws.dN.reserve((size_t)n_part * n_bins * 8 + 256));
   CU_CHECK(ws.counters.reserve(256));
   if (opt.memory == 0) CU_CHECK(ws.raw.reserve(cell_stride * n_src + 256));
 
@@ -1320,8 +1341,8 @@ static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const double
   RawCells rc; memset(&rc, 0, sizeof(rc));
   rc.n = n_cells; rc.tau = dev[0]; rc.eta = dev[1]; rc.dat = dev[2]; rc.dax = dev[3]; rc.day = dev[4]; rc.dan = dev[5];
   rc.ux = dev[6]; rc.uy = dev[7]; rc.un = dev[8]; rc.T = dev[9];
-  const int n_arr = shear ? 4 : 5;
-  double *sums_d = ws.dN.as<double>();                         // [n_arr][n_bins]: Snorm, (N^t,) N^x, N^y, N^z
+  const int n_arr = shear ? 4 : pol_n_out(term);
+  double *sums_d = ws.dN.as<double>();                         // [n_arr][n_bins] in the order of out
   CU_CHECK(cudaMemsetAsync(sums_d, 0, (size_t)n_arr * n_bins * 8, st));
   CU_CHECK(cudaMemsetAsync(ws.counters.p, 0, sizeof(PrepCounters), st));
   CU_CHECK(cudaEventRecord(ev[1], st));
@@ -1350,6 +1371,10 @@ static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const double
   if (shear) {
     const PolXiParams prm{hp, dptr(o_cos), dptr(o_sin), dim2 ? nullptr : dptr(o_sloty)};
     CU_CHECK(launch_polzn_xi(prm, st));
+  } else if (term == kPolSpinDensity) {
+    // the prepare kernel never touches range_error: here it counts the boson evaluations without a valid occupation
+    const SpinDensityParams prm{hp, dim2 ? nullptr : dptr(o_sloty), &cnt_d->range_error};
+    CU_CHECK(launch_spin_density(prm, st));
   } else {
     CU_CHECK(launch_polzn(hp, st));
   }
@@ -1357,9 +1382,19 @@ static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const double
   for (int q = 0; q < n_arr; q++)
     CU_CHECK(launch_reduce(hp.partial + (size_t)q * n_chunks * n_bins, (int)n_chunks, n_bins, n_active, sums_d + (size_t)q * n_bins, st));
   CU_CHECK(cudaEventRecord(ev[4], st));
+  if (term == kPolSpinDensity) {
+    // decided before anything is added to the caller's arrays, like the table-range errors of smooth_core
+    PrepCounters c0; memset(&c0, 0, sizeof(c0));
+    CU_CHECK(cudaMemcpyAsync(&c0, cnt_d, sizeof(c0), cudaMemcpyDeviceToHost, st));
+    CU_CHECK(cudaStreamSynchronize(st));
+    if (c0.range_error) {
+      char msg[256];
+      snprintf(msg, sizeof(msg), "%llu boson evaluations have u.p/T - J theta <= 0: the spin level m = J has no valid occupation "
+               "(thermal vorticity too large for this surface)", c0.range_error);
+      return fail(IS3D_ERR_ARGUMENT, msg);
+    }
+  }
 
-  double *out_vort[5] = {res->Snorm, res->St, res->Sx, res->Sy, res->Sz}, *out_xi[4] = {res->Snorm, res->Sx, res->Sy, res->Sz};
-  double *const *out = shear ? out_xi : out_vort;
   std::vector<double> host;
   if (opt.memory == 0) {
     host.resize((size_t)n_arr * n_bins);
@@ -1396,22 +1431,23 @@ static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const double
 
 namespace is3d {
 
-// Several devices: HOST arrays, contiguous cell shards, one thread per device; the five raw sums are added on the host in device order
-static int polzn_multi(const is3d_flags *fl, const is3d_surface *sf, const double *const *tensor, bool shear, const is3d_species *sp,
-                       const is3d_grid *gr, const is3d_options *opt_in, is3d_polarization_result *res, is3d_stats *stats)
+// Several devices: HOST arrays, contiguous cell shards, one thread per device; the raw sums are added on the host in device order
+static int polzn_multi(const is3d_flags *fl, const is3d_surface *sf, const double *const *tensor, PolTerm term, const is3d_species *sp,
+                       const is3d_grid *gr, const is3d_options *opt_in, double *const *out, is3d_stats *stats)
 {
   const int G = g_ngpus;
-  if (G <= 1) return polzn_core(fl, sf, tensor, shear, sp, gr, opt_in, res, stats);
-  if (!fl || !sf || !tensor || !sp || !gr || !res) return fail(IS3D_ERR_ARGUMENT, tensor ? "NULL argument" : shear ? "NULL thermal shear" : "NULL vorticity");
+  const bool shear = (term == kPolShear);
+  if (G <= 1) return polzn_core(fl, sf, tensor, term, sp, gr, opt_in, out, stats);
+  if (!fl || !sf || !tensor || !sp || !gr || !out) return fail(IS3D_ERR_ARGUMENT, tensor ? "NULL argument" : shear ? "NULL thermal shear" : "NULL vorticity");
   if (opt_in && opt_in->memory != 0) return fail(IS3D_ERR_ARGUMENT, "the multi-GPU entry point takes host arrays");
   std::lock_guard<std::mutex> lk(g_multi_mutex);
-  const int n_tensor = shear ? 10 : 6;
+  const int n_tensor = shear ? 10 : 6, n_out = pol_n_out(term);
   const size_t n_bins = (size_t)std::max(sp->n, 0) * std::max(gr->n_pT, 0) * std::max(gr->n_phi, 0) * std::max(gr->n_y, 0);
   int prev = 0; cudaGetDevice(&prev);
   std::vector<int> rcs(G, IS3D_OK);
   std::vector<std::string> errs(G);
   std::vector<is3d_stats> sts(G);
-  std::vector<std::vector<double>> bufs(G, std::vector<double>(5 * n_bins, 0.0));
+  std::vector<std::vector<double>> bufs(G, std::vector<double>(n_out * n_bins, 0.0));
   std::vector<std::thread> workers;
   for (int d = 0; d < G; d++) {
     workers.emplace_back([&, d]() {
@@ -1425,17 +1461,16 @@ static int polzn_multi(const is3d_flags *fl, const is3d_surface *sf, const doubl
       is3d_options opt; memset(&opt, 0, sizeof(opt));
       if (opt_in) opt = *opt_in;
       opt.memory = 0; opt.stream = g_streams[d];
-      double *b = bufs[d].data();
-      is3d_polarization_result r{b, b + n_bins, b + 2 * n_bins, b + 3 * n_bins, b + 4 * n_bins};
-      rcs[d] = polzn_core(fl, &shard, ts, shear, sp, gr, &opt, &r, &sts[d]);
+      double *r[kSdSums];
+      for (int q = 0; q < n_out; q++) r[q] = bufs[d].data() + q * n_bins;
+      rcs[d] = polzn_core(fl, &shard, ts, term, sp, gr, &opt, r, &sts[d]);
       if (rcs[d]) errs[d] = g_last_error;
     });
   }
   for (auto &w : workers) w.join();
   cudaSetDevice(prev);
   for (int d = 0; d < G; d++) if (rcs[d]) return fail(rcs[d], errs[d].c_str());
-  double *out[5] = {res->St, res->Sx, res->Sy, res->Sz, res->Snorm};
-  for (int q = 0; q < 5; q++)
+  for (int q = 0; q < n_out; q++)
     for (size_t i = 0; i < n_bins; i++) { double v = 0.0; for (int d = 0; d < G; d++) v += bufs[d][q * n_bins + i]; out[q][i] += v; }
   if (stats) {
     is3d_stats tot; memset(&tot, 0, sizeof(tot));
@@ -1461,37 +1496,71 @@ static const double *const *shear_columns(const is3d_thermal_shear *xi, const do
   for (int a = 0; a < 10; a++) c[a] = v[a];
   return c;
 }
+// the result arrays of the three terms in the order of pol_n_out(), or NULL for a NULL struct
+static double *const *vort_arrays(is3d_polarization_result *r, double **a)
+{
+  if (!r) return nullptr;
+  a[0] = r->Snorm; a[1] = r->St; a[2] = r->Sx; a[3] = r->Sy; a[4] = r->Sz;
+  return a;
+}
+static double *const *shear_arrays(is3d_polarization_result *r, double **a)
+{
+  if (!r) return nullptr;
+  a[0] = r->Snorm; a[1] = r->Sx; a[2] = r->Sy; a[3] = r->Sz; a[4] = r->St;
+  return a;
+}
+static double *const *spin_density_arrays(is3d_spin_density_result *r, double **a)
+{
+  if (!r) return nullptr;
+  double *v[kSdSums] = {r->Snorm, r->Px, r->Py, r->Pz, r->Qxx, r->Qxy, r->Qxz, r->Qyy, r->Qyz};
+  for (int q = 0; q < kSdSums; q++) a[q] = v[q];
+  return a;
+}
 
 }  // namespace is3d
 
 extern "C" int is3d_b200_spin_polarization(const is3d_flags *fl, const is3d_surface *sf, const is3d_vorticity *vo, const is3d_species *sp,
                                            const is3d_grid *gr, const is3d_options *opt, is3d_polarization_result *res, is3d_stats *stats)
 {
-  const double *c[6];
-  return polzn_core(fl, sf, vort_columns(vo, c), false, sp, gr, opt, res, stats);
+  const double *c[6]; double *a[5];
+  return polzn_core(fl, sf, vort_columns(vo, c), kPolVorticity, sp, gr, opt, vort_arrays(res, a), stats);
 }
 
 extern "C" int is3d_b200_spin_polarization_multi(const is3d_flags *fl, const is3d_surface *sf, const is3d_vorticity *vo, const is3d_species *sp,
                                                  const is3d_grid *gr, const is3d_options *opt, is3d_polarization_result *res, is3d_stats *stats)
 {
-  const double *c[6];
-  return polzn_multi(fl, sf, vort_columns(vo, c), false, sp, gr, opt, res, stats);
+  const double *c[6]; double *a[5];
+  return polzn_multi(fl, sf, vort_columns(vo, c), kPolVorticity, sp, gr, opt, vort_arrays(res, a), stats);
 }
 
 extern "C" int is3d_b200_spin_polarization_shear(const is3d_flags *fl, const is3d_surface *sf, const is3d_thermal_shear *xi,
                                                  const is3d_species *sp, const is3d_grid *gr, const is3d_options *opt,
                                                  is3d_polarization_result *res, is3d_stats *stats)
 {
-  const double *c[10];
-  return polzn_core(fl, sf, shear_columns(xi, c), true, sp, gr, opt, res, stats);
+  const double *c[10]; double *a[5];
+  return polzn_core(fl, sf, shear_columns(xi, c), kPolShear, sp, gr, opt, shear_arrays(res, a), stats);
 }
 
 extern "C" int is3d_b200_spin_polarization_shear_multi(const is3d_flags *fl, const is3d_surface *sf, const is3d_thermal_shear *xi,
                                                        const is3d_species *sp, const is3d_grid *gr, const is3d_options *opt,
                                                        is3d_polarization_result *res, is3d_stats *stats)
 {
-  const double *c[10];
-  return polzn_multi(fl, sf, shear_columns(xi, c), true, sp, gr, opt, res, stats);
+  const double *c[10]; double *a[5];
+  return polzn_multi(fl, sf, shear_columns(xi, c), kPolShear, sp, gr, opt, shear_arrays(res, a), stats);
+}
+
+extern "C" int is3d_b200_spin_density(const is3d_flags *fl, const is3d_surface *sf, const is3d_vorticity *vo, const is3d_species *sp,
+                                      const is3d_grid *gr, const is3d_options *opt, is3d_spin_density_result *res, is3d_stats *stats)
+{
+  const double *c[6]; double *a[kSdSums];
+  return polzn_core(fl, sf, vort_columns(vo, c), kPolSpinDensity, sp, gr, opt, spin_density_arrays(res, a), stats);
+}
+
+extern "C" int is3d_b200_spin_density_multi(const is3d_flags *fl, const is3d_surface *sf, const is3d_vorticity *vo, const is3d_species *sp,
+                                            const is3d_grid *gr, const is3d_options *opt, is3d_spin_density_result *res, is3d_stats *stats)
+{
+  const double *c[6]; double *a[kSdSums];
+  return polzn_multi(fl, sf, vort_columns(vo, c), kPolSpinDensity, sp, gr, opt, spin_density_arrays(res, a), stats);
 }
 
 // =====================================================================================================================

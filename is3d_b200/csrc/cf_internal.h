@@ -159,6 +159,18 @@ struct PolXiParams {
 cudaError_t launch_prepare_polzn_xi(const RawCells &cells, const ShearCells &shear, const PrepTables &tab, const Layout &L, double *Y,
                                     double *P, PrepCounters *counters, cudaStream_t st);
 cudaError_t launch_polzn_xi(const PolXiParams &prm, cudaStream_t st);
+// spin density matrix from thermal vorticity (cf_spin_density.cu): the records of prepare_polzn_kernel, its own register tile,
+// 9 sums per bin (Snorm, P_x, P_y, P_z, Q_xx, Q_xy, Q_xz, Q_yy, Q_yz)
+constexpr int kSdSums = 9;
+constexpr int kSdMinBlocks = 3;  // blocks per SM of kPolWarps warps the register budget is sized for (__launch_bounds__)
+constexpr int kSdNyt3D = 3, kSdNpt3D = 1, kSdNpt2D = 2;
+struct SpinDensityParams {
+  HotParams hp;                  // layout, records Y / P, species and pT tables, partial [9][n_chunks][n_bins]
+  const double *y;               // 3+1D: the y table [n_y]; 2+1D: unused (y = 0)
+  unsigned long long *boson_bad; // device counter: boson evaluations with u.p/T - J theta <= 0 (one atomic per block that has any)
+};
+void spin_density_shape(int dim2, int *nyt, int *npt, int *ct);
+cudaError_t launch_spin_density(const SpinDensityParams &prm, cudaStream_t st);
 // HBT moments (cf_hbt.cu): the records of prepare_vh_kernel plus a per-cell record [tau, x, y, 0]; 10 sums per bin
 constexpr int kHbtRecC = 4;      // doubles per per-cell position record
 constexpr int kHbtSums = 10;     // S0, So, Ss, Sl, Soo, Sss, Sll, Sos, Sol, Ssl

@@ -227,6 +227,47 @@ static bool write_polarization_files(const std::string &wd, const std::vector<do
   return true;
 }
 
+// results/polarization/spin_<mcid>.dat, for every chosen species with degeneracy g >= 2: Snorm, the all-order rest-frame mean spin
+// <S*_i> = P_i / Snorm and the rank-2 spin tensor T_ij = Q_ij / Snorm (T_zz = -T_xx - T_yy; all 0 where Snorm = 0) of the nine raw sums
+// of is3d_b200_spin_density (Snorm | Px | Py | Pz | Qxx | Qxy | Qxz | Qyy | Qyz), one row per (y, phi, pT) in the loop order, number
+// format and blank line per phi block of write_spectra_files; truncating opens, results/polarization/ must exist
+static bool write_spin_density_files(const std::string &wd, const std::vector<double> &sums, const std::vector<int> &mcid,
+                                     const std::vector<double> &degen, const Grids &g, int dimension, std::string *err)
+{
+  const int npart = (int)mcid.size(), npT = (int)g.pT.rows, nphi = (int)g.phi.rows, ny = (int)g.y.rows;
+  const int y_pts = (dimension == 2) ? 1 : ny;
+  const size_t n_bins = (size_t)npart * npT * nphi * ny;
+  const double *Sn = &sums[0];
+  for (int ipart = 0; ipart < npart; ipart++) {
+    if (degen[ipart] < 2.0) continue;
+    char name[255];
+    std::snprintf(name, sizeof(name), "%s/results/polarization/spin_%d.dat", wd.c_str(), mcid[ipart]);
+    std::ofstream f(name, std::ios_base::out);
+    if (!f) { *err = std::string("cannot open ") + name + " (the directory results/polarization/ must exist)"; return false; }
+    f << "y\tphip\tpT\tSnorm\tSx\tSy\tSz\tTxx\tTxy\tTxz\tTyy\tTyz\tTzz\n";
+    for (int iy = 0; iy < y_pts; iy++) {
+      const double y = (dimension == 2) ? 0.0 : g.y.at(1, iy + 1);
+      for (int iphi = 0; iphi < nphi; iphi++) {
+        const double phi = g.phi.at(1, iphi + 1);
+        for (int ipT = 0; ipT < npT; ipT++) {
+          const double pT = g.pT.at(1, ipT + 1);
+          const size_t b = (size_t)bin_index(ipart, npart, ipT, npT, iphi, nphi, iy);
+          double v[9] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};    // Sx Sy Sz Txx Txy Txz Tyy Tyz Tzz
+          if (Sn[b] != 0.0) {
+            for (int q = 0; q < 8; q++) v[q] = sums[(q + 1) * n_bins + b] / Sn[b];
+            v[8] = -(sums[4 * n_bins + b] + sums[7 * n_bins + b]) / Sn[b];
+          }
+          f << std::scientific << std::setw(5) << std::setprecision(8) << y << "\t" << phi << "\t" << pT << "\t" << Sn[b];
+          for (int q = 0; q < 9; q++) f << "\t" << v[q];
+          f << "\n";
+        }
+        f << "\n";
+      }
+    }
+  }
+  return true;
+}
+
 // results/hbt/R2_<mcid>.dat: S0 and the HBT radii R^2_ij = S_ij / S0 - (S_i / S0)(S_j / S0) [fm^2] (all 0 where S0 = 0) of the raw sums of
 // is3d_b200_hbt_moments, one row per (y, phi, pT) in the loop order, number format and blank line per phi block of write_spectra_files;
 // truncating opens, results/hbt/ must exist
@@ -306,6 +347,7 @@ struct Problem {
   int spin_polarization = 0;               // optional key (absent: 0): mode-5 spin polarization after the spectra
   int thermal_shear_polarization = 0;      // optional key (absent: 0): add the thermal-shear term (input/thermal_shear.dat)
   int polarization_feed_down = 0;          // optional key (absent: 0): feed the polarization sums down through the decay tables
+  int spin_density = 0;                    // optional key (absent: 0): mode-5 spin density matrix (all-order spin, rank-2 tensor)
   std::map<long, int> box_parity;          // its parities by |MC id| (PDG/pdg_box.dat)
   int hbt_radii = 0;                       // optional key (absent: 0): HBT radii of the linear-delta-f spectra after the spectra
   int hbt_correlation = 0;                 // optional key (absent: 0): MC id of the species whose HBT correlation functions are written
@@ -363,6 +405,8 @@ static int load_problem(const std::string &wd, bool need_surface, Problem *p, st
           "(hrg_eos = 1, 2)";
     return IS3D_ERR_UNSUPPORTED;
   }
+  p->spin_density = par.has("spin_density") ? (int)par.get("spin_density", &err) : 0;
+  if (p->spin_density && (p->operation != 1 || fl.mode != 5)) { err = "spin_density = 1 needs operation = 1 and a mode 5 surface (the thermal vorticity columns)"; return IS3D_ERR_UNSUPPORTED; }
   p->hbt_radii = par.has("hbt_radii") ? (int)par.get("hbt_radii", &err) : 0;
   if (p->hbt_radii && (p->operation != 1 || fl.mode == 2 || (fl.df_mode != 1 && fl.df_mode != 2) || fl.include_baryon)) {
     err = "hbt_radii = 1 needs operation = 1, a viscous-hydro surface (mode != 2), df_mode 1 or 2 and include_baryon = 0"; return IS3D_ERR_UNSUPPORTED;
@@ -550,6 +594,17 @@ static int run_problem(const std::string &wd, Problem &P, const is3d_surface &s,
       if (stats) { stats->gpu_launches += fd_st.gpu_launches; stats->total_ms += fd_st.total_ms; }
       if (!write_polarization_files(wd, sums, nullptr, P.mcid, P.mass, g, P.fl.dimension, &err, "S_fd")) return IS3D_ERR_IO;
     }
+  }
+  if (P.spin_density) {
+    std::vector<double> sums(9 * n_bins, 0.0);                   // Snorm | Px | Py | Pz | Qxx | Qxy | Qxz | Qyy | Qyz
+    double *b = sums.data();
+    is3d_spin_density_result r{b, b + n_bins, b + 2 * n_bins, b + 3 * n_bins, b + 4 * n_bins, b + 5 * n_bins, b + 6 * n_bins,
+                               b + 7 * n_bins, b + 8 * n_bins};
+    is3d_stats sd_st; std::memset(&sd_st, 0, sizeof(sd_st));
+    const int rcs = is3d_b200_spin_density_multi(&P.fl, &s, vort, &sp, &gr, nullptr, &r, &sd_st);
+    if (rcs != IS3D_OK) { err = std::string("spin density failed: ") + is3d_b200_last_error(); return rcs; }
+    if (stats) { stats->gpu_launches += sd_st.gpu_launches; stats->total_ms += sd_st.total_ms; }
+    if (!write_spin_density_files(wd, sums, P.mcid, P.degen, g, P.fl.dimension, &err)) return IS3D_ERR_IO;
   }
   if (P.hbt_radii) {
     std::vector<double> sums(10 * n_bins, 0.0);                  // S0 | So | Ss | Sl | Soo | Sss | Sll | Sos | Sol | Ssl

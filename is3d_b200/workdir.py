@@ -32,7 +32,7 @@ DEFAULT_PARAMETERS = [
 ]
 
 # keys of this drop-in that the reference does not read: written only when a caller sets them (absent: 0, or the default of the host layer)
-OPTIONAL_PARAMETERS = ("spin_polarization", "thermal_shear_polarization", "polarization_feed_down", "hbt_radii", "hbt_correlation", "hbt_dq",
+OPTIONAL_PARAMETERS = ("spin_polarization", "thermal_shear_polarization", "polarization_feed_down", "spin_density", "hbt_radii", "hbt_correlation", "hbt_dq",
                        "hbt_q_points")
 
 _EOS_DIR = {1: "urqmd", 2: "smash", 3: "smash_box"}
