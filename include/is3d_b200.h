@@ -238,6 +238,32 @@ int is3d_b200_spin_polarization_shear_multi(const is3d_flags *flags, const is3d_
                                             const is3d_species *species, const is3d_grid *grid, const is3d_options *options,
                                             is3d_polarization_result *result, is3d_stats *stats);
 
+/* ---- spin polarization of baryons from the spin Hall effect (gradient of alpha_B = muB/T) ------------------------------------
+ * The baryonic spin Hall term of the first-order local-equilibrium mean spin vector (Liu & Yin, JHEP 07 (2021) 188; Ryu, Jupic, Shen,
+ * PRC 104 (2021) 054908), in the lab-frame (that) form of the thermal-shear term, over the cells, slots, weights, species and bins of
+ * is3d_b200_spin_polarization:
+ *    N_she^mu(p) = g/(2 pi hbar c)^3 sum_cells sum_slots w p.dsigma f (1 - sign f) (-1/(8m)) eps^{mu rho sigma tau} p_tau (-2 q_B that_rho d_sigma alpha_B / E)
+ * with q_B = species->baryon, that = (1, 0, 0, 0), E = p^t = mT cosh y, and the prefactor and eps^{txyz} = +1 of the vorticity term, so
+ * that S^mu = (N^mu + N_xi^mu + N_she^mu) / Snorm.  It is the shear term with xi_{sigma lambda} p^lambda -> xi_{sigma lambda} p^lambda -
+ * q_B d_sigma alpha_B, the gradient of the argument beta.p - q_B alpha_B of f.  In Cartesian lab components N_she^t = 0 exactly and
+ * N_she = +(q_B / (4 m E)) sum W (zeta x p), zeta_j = hbar c d_j alpha_B (GeV); mesons (q_B = 0) give exact zeros.
+ * f is the muB-free weight of the other polarization terms (include_baryon = 1 is rejected): the term is exact at first order in
+ * d alpha_B around that weight, and Snorm is the Snorm of the vorticity call, so the three N arrays add.
+ * Input: the covariant Milne components d_tau alpha_B, d_x alpha_B, d_y alpha_B (1/fm) and d_eta alpha_B (dimensionless), converted to
+ * Cartesian components at the cell's eta (2+1D: the slot's eta) in cf_polzn.cuh, cart_gradient().
+ * Results go into an is3d_polarization_result: St receives exact zeros, Sx, Sy, Sz the RAW sums N_she, Snorm the ideal spectrum (bit for
+ * bit what is3d_b200_spin_polarization returns on the same device with the same options).  All are ADDED into; host or device memory
+ * per options->memory.  Errors: IS3D_ERR_UNSUPPORTED for mode = 2 and include_baryon = 1; IS3D_ERR_ARGUMENT for a NULL gradient or
+ * gradient array, a NULL species->baryon or a species with m <= 0. */
+typedef struct { const double *dt, *dx, *dy, *dn; } is3d_baryon_gradient;
+int is3d_b200_spin_polarization_spin_hall(const is3d_flags *flags, const is3d_surface *surface, const is3d_baryon_gradient *gradient,
+                                          const is3d_species *species, const is3d_grid *grid, const is3d_options *options,
+                                          is3d_polarization_result *result, is3d_stats *stats);
+/* Same over the devices of is3d_b200_init_devices(): HOST arrays, contiguous cell shards, the five arrays summed on the host. */
+int is3d_b200_spin_polarization_spin_hall_multi(const is3d_flags *flags, const is3d_surface *surface, const is3d_baryon_gradient *gradient,
+                                                const is3d_species *species, const is3d_grid *grid, const is3d_options *options,
+                                                is3d_polarization_result *result, is3d_stats *stats);
+
 /* ---- spin density matrix of hadrons from thermal vorticity: all-order mean spin, rank-2 spin tensor, vector-meson rho00 ---------
  * The local-equilibrium distribution with the spin term exponentiated, [exp(beta.p - (1/2) varpi:Sigma) + Theta]^-1 (Becattini, Chandra,
  * Del Zanna, Grossi, Ann. Phys. 338 (2013) 32), for any spin J = (g - 1)/2, over the cells, slots, weights, u.dsigma <= 0 skip, outflow

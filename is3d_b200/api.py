@@ -587,15 +587,66 @@ def spin_polarization_shear(flags, cells, shear, species, grid, memory="host", s
     return out, st.as_dict()
 
 
-def mean_spin(result, species, grid, dimension, shear=None):
+BARYON_GRADIENT_FIELDS = ("dt", "dx", "dy", "dn")
+
+
+class BaryonGradient(C.Structure):
+    _fields_ = [(k, _D) for k in BARYON_GRADIENT_FIELDS]
+
+
+def spin_polarization_spin_hall(flags, cells, gradient, species, grid, memory="host", stream=None, multi=False):
+    """Call is3d_b200_spin_polarization_spin_hall (or the _multi entry point over the devices of init_devices(), host arrays only).
+
+    gradient: dict dt, dx, dy, dn -- the covariant Milne components of the gradient of alpha_B = muB/T (d_tau, d_x, d_y in 1/fm, d_eta
+    dimensionless), numpy for memory='host', float64 CUDA tensors for memory='device'.  species needs 'baryon' (q_B).  Returns (dict St,
+    Sx, Sy, Sz, Snorm of RAW sums, flat [y][phi][pT][species]: St = 0, Sx, Sy, Sz = N_she, Snorm the ideal spectrum; stats dict).
+    mean_spin(vorticity_sums, ..., spin_hall=these) forms the total mean spin vector."""
+    device = (memory == "device")
+    m = _Marshal(device)
+    sf, sp, g, _, _ = _marshal_problem(m, cells, species, grid, None, None)
+    gd = None
+    if gradient is not None:
+        gd = BaryonGradient()
+        for k in BARYON_GRADIENT_FIELDS:
+            if gradient.get(k) is not None:                   # a missing column stays NULL (the library rejects it)
+                setattr(gd, k, m.cells(gradient[k]))
+    n = sp.n * g.n_pT * g.n_phi * g.n_y
+    res = PolarizationResult()
+    if device:
+        import torch
+        out = {k: torch.zeros(n, dtype=torch.float64, device=cells["tau"].device) for k in POLARIZATION_FIELDS}
+        for k in POLARIZATION_FIELDS:
+            setattr(res, k, C.cast(C.c_void_p(out[k].data_ptr()), _D))
+        if stream is None:
+            stream = torch.cuda.current_stream().cuda_stream
+    else:
+        out = {k: np.zeros(n) for k in POLARIZATION_FIELDS}
+        for k in POLARIZATION_FIELDS:
+            setattr(res, k, out[k].ctypes.data_as(_D))
+    opt = Options(); opt.memory = 1 if device else 0; opt.stream = C.c_void_p(stream or 0)
+    st = Stats()
+    fl = make_flags(flags)
+    f = lib().is3d_b200_spin_polarization_spin_hall_multi if multi else lib().is3d_b200_spin_polarization_spin_hall
+    f.restype = C.c_int
+    f.argtypes = [C.POINTER(Flags), C.POINTER(Surface), C.POINTER(BaryonGradient), C.POINTER(Species), C.POINTER(Grid), C.POINTER(Options),
+                  C.POINTER(PolarizationResult), C.POINTER(Stats)]
+    _check(f(C.byref(fl), C.byref(sf), C.byref(gd) if gd is not None else None, C.byref(sp), C.byref(g), C.byref(opt), C.byref(res),
+             C.byref(st)))
+    return out, st.as_dict()
+
+
+def mean_spin(result, species, grid, dimension, shear=None, spin_hall=None):
     """Mean spin vector from the raw sums of spin_polarization(): returns (S [4][n_bins] = N^mu / Snorm in lab components t, x, y, z,
     0 where Snorm = 0; S* [3][n_bins] = S^i - S^t p^i / (E + m), the rest-frame spin, P* = 2 S* for spin 1/2).  The same numbers
     results/polarization/S_<mcid>.dat holds.  shear (optional): the raw sums of spin_polarization_shear() on the same problem; S is then
-    the total (N^mu + N_xi^mu) / Snorm and S* its rest-frame part, the totals of results/polarization/S_xi_<mcid>.dat."""
+    the total (N^mu + N_xi^mu) / Snorm and S* its rest-frame part, the totals of results/polarization/S_xi_<mcid>.dat.  spin_hall
+    (optional): the raw sums of spin_polarization_spin_hall() on the same problem, added the same way (after shear), the totals of
+    results/polarization/S_she_<mcid>.dat."""
     r = {k: np.asarray(result[k].cpu() if _is_torch(result[k]) else result[k], dtype=np.float64) for k in POLARIZATION_FIELDS}
-    if shear is not None:
-        for k in ("St", "Sx", "Sy", "Sz"):
-            r[k] = r[k] + np.asarray(shear[k].cpu() if _is_torch(shear[k]) else shear[k], dtype=np.float64)
+    for extra in (shear, spin_hall):
+        if extra is not None:
+            for k in ("St", "Sx", "Sy", "Sz"):
+                r[k] = r[k] + np.asarray(extra[k].cpu() if _is_torch(extra[k]) else extra[k], dtype=np.float64)
     m = np.asarray(species["mass"], dtype=np.float64)
     pT = np.asarray(grid["pT"], dtype=np.float64); phi = np.asarray(grid["phi"], dtype=np.float64)
     y = np.asarray(grid["y"], dtype=np.float64)

@@ -27,6 +27,7 @@ SOURCES = [
     ("cf_shift.cu", []),
     ("cf_polzn.cu", []),
     ("cf_polzn_xi.cu", []),
+    ("cf_polzn_she.cu", []),
     ("cf_spin_density.cu", []),
     ("cf_hbt.cu", []),
     ("cf_hbtq.cu", []),

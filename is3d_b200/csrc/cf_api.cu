@@ -1218,34 +1218,35 @@ extern "C" int is3d_b200_spacetime_distributions_multi(const is3d_flags *fl, con
 }
 
 // =====================================================================================================================
-// Spin polarization from thermal vorticity (cf_polzn.cu) and thermal shear (cf_polzn_xi.cu): raw sums N^mu and Snorm, added into the
-// caller's five arrays; spin density matrix from thermal vorticity (cf_spin_density.cu): nine raw sums
+// Spin polarization from thermal vorticity (cf_polzn.cu), thermal shear (cf_polzn_xi.cu) and the spin Hall effect (cf_polzn_she.cu): raw
+// sums N^mu and Snorm, added into the caller's five arrays; spin density matrix from thermal vorticity (cf_spin_density.cu): nine raw sums
 // =====================================================================================================================
 namespace is3d {
 
-enum PolTerm { kPolVorticity, kPolShear, kPolSpinDensity };
+enum PolTerm { kPolVorticity, kPolShear, kPolSpinDensity, kPolSpinHall };
 
-// result arrays per term, in the order of the kernel's partial rows; the shear term's fifth array (St) must be non-NULL but is left
-// alone (N_xi^t = 0 exactly)
+// result arrays per term, in the order of the kernel's partial rows; the fifth array (St) of the shear and spin Hall terms must be
+// non-NULL but is left alone (N_xi^t = N_she^t = 0 exactly)
 static int pol_n_out(PolTerm term) { return term == kPolSpinDensity ? kSdSums : 5; }
 
-// tensor: the 6 vorticity columns (vorticity, spin density) or the 10 thermal-shear columns (shear), NULL for a NULL struct.  out: the
-// pol_n_out(term) result arrays, NULL for a NULL result struct.  The vorticity and shear terms run on the same layout and chunk split, so
-// their Snorm is bit-identical.  The spin-density kernel has its own register tile but the same cell chunks, so at varpi = 0 its Snorm is
+// tensor: the 6 vorticity columns (vorticity, spin density), the 10 thermal-shear columns (shear) or the 4 columns of d alpha_B (spin
+// Hall), NULL for a NULL struct.  out: the pol_n_out(term) result arrays, NULL for a NULL result struct.  The vorticity, shear and spin
+// Hall terms run on the same layout and chunk split, so their Snorm is bit-identical.  The spin-density kernel has its own register tile but the same cell chunks, so at varpi = 0 its Snorm is
 // bit-identical too (unless the 4 GiB cap on its nine partial arrays lowers the chunk count).
 static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const double *const *tensor, PolTerm term, const is3d_species *sp,
                       const is3d_grid *gr, const is3d_options *opt_in, double *const *out, is3d_stats *stats)
 {
-  const bool shear = (term == kPolShear);
-  const int n_tensor = shear ? 10 : 6;
+  const bool shear = (term == kPolShear), she = (term == kPolSpinHall);
+  const int n_tensor = shear ? 10 : she ? 4 : 6;
   if (!fl || !sf || !sp || !gr || !out) return fail(IS3D_ERR_ARGUMENT, "NULL argument");
-  if (!tensor) return fail(IS3D_ERR_ARGUMENT, shear ? "NULL thermal shear" : "NULL vorticity");
+  if (!tensor) return fail(IS3D_ERR_ARGUMENT, shear ? "NULL thermal shear" : she ? "NULL baryon gradient" : "NULL vorticity");
   for (int q = 0; q < pol_n_out(term); q++) if (!out[q]) return fail(IS3D_ERR_ARGUMENT, "NULL result array");
   if (fl->mode == 2) return fail(IS3D_ERR_UNSUPPORTED, "spin polarization needs a viscous-hydro surface with thermal vorticity (mode 5), not mode 2");
   if (fl->include_baryon) return fail(IS3D_ERR_UNSUPPORTED, "include_baryon = 1 (the reference's (T, muB) lookup reads out of bounds, SURVEY R8)");
   if (fl->dimension != 2 && fl->dimension != 3) return fail(IS3D_ERR_ARGUMENT, "dimension must be 2 or 3");
   if (sp->n <= 0 || gr->n_pT <= 0 || gr->n_phi <= 0 || gr->n_y <= 0) return fail(IS3D_ERR_ARGUMENT, "empty species list or momentum table");
   if (!sp->mass || !sp->sign || !sp->degeneracy || !gr->pT || !gr->phi || !gr->y) return fail(IS3D_ERR_ARGUMENT, "NULL species or momentum table");
+  if (she && !sp->baryon) return fail(IS3D_ERR_ARGUMENT, "the spin Hall term needs the species' baryon numbers (NULL species table)");
   for (int s = 0; s < sp->n; s++) if (!(sp->mass[s] > 0.0)) return fail(IS3D_ERR_ARGUMENT, "spin polarization needs species with mass > 0");
   if (term == kPolSpinDensity)
     for (int s = 0; s < sp->n; s++) {
@@ -1262,7 +1263,8 @@ static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const double
   const int n_src = 10 + n_tensor;
   for (int a = 0; a < n_src; a++)
     if (!srcs[a] && n_cells > 0)
-      return fail(IS3D_ERR_ARGUMENT, shear ? "a required surface or thermal-shear array is NULL" : "a required surface or vorticity array is NULL");
+      return fail(IS3D_ERR_ARGUMENT, shear ? "a required surface or thermal-shear array is NULL"
+                                     : she ? "a required surface or baryon-gradient array is NULL" : "a required surface or vorticity array is NULL");
   Device *Dp = nullptr;
   { int rc = current_device(&Dp); if (rc) return rc; }
   Workspace &ws = Dp->ws;
@@ -1302,7 +1304,7 @@ static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const double
   const int64_t l2_target = std::max<int64_t>((int64_t)Dp->l2_bytes / 3, (int64_t)8 << 20);
   n_chunks = std::max<int64_t>(n_chunks, (n_cells * rec_per_cell + l2_target - 1) / l2_target);
   const int64_t n_chunks_wanted = n_chunks;
-  const int n_part = (term == kPolSpinDensity) ? kSdSums : 5;       // partial arrays the 4 GiB cap counts (the shear term keeps 5)
+  const int n_part = (term == kPolSpinDensity) ? kSdSums : 5;       // partial arrays the 4 GiB cap counts (shear, spin Hall keep 5)
   n_chunks = std::min<int64_t>(n_chunks, std::max<int64_t>(1, ((int64_t)4 << 30) / (n_part * n_bins * 8)));
   if (opt.n_chunks > 0) n_chunks = opt.n_chunks;
   n_chunks = std::max<int64_t>(1, std::min<int64_t>(n_chunks, std::max<int64_t>(L.n_tiles, 1)));
@@ -1316,6 +1318,7 @@ static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const double
   const size_t o_pT = ar.put(gr->pT, gr->n_pT), o_cos = ar.put(cosphi.data(), gr->n_phi), o_sin = ar.put(sinphi.data(), gr->n_phi);
   const size_t o_sloty = dim2 ? ar.put(gr->eta, gr->n_eta) : ar.put(gr->y, gr->n_y);
   const size_t o_slotw = dim2 ? ar.put(gr->eta_weight, gr->n_eta) : 0;
+  const size_t o_bar = she ? ar.put(sp->baryon, sp->n) : 0;
   const size_t cell_stride = ((size_t)n_cells * 8 + 255) & ~(size_t)255;
   CU_CHECK(ws.small.reserve(ar.host.size() + 256));
   CU_CHECK(ws.Y.reserve((size_t)L.n_ytiles * L.n_cells_pad * L.nst * kPolRecY * 8 + 256));
@@ -1341,7 +1344,7 @@ static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const double
   RawCells rc; memset(&rc, 0, sizeof(rc));
   rc.n = n_cells; rc.tau = dev[0]; rc.eta = dev[1]; rc.dat = dev[2]; rc.dax = dev[3]; rc.day = dev[4]; rc.dan = dev[5];
   rc.ux = dev[6]; rc.uy = dev[7]; rc.un = dev[8]; rc.T = dev[9];
-  const int n_arr = shear ? 4 : pol_n_out(term);
+  const int n_arr = (shear || she) ? 4 : pol_n_out(term);
   double *sums_d = ws.dN.as<double>();                         // [n_arr][n_bins] in the order of out
   CU_CHECK(cudaMemsetAsync(sums_d, 0, (size_t)n_arr * n_bins * 8, st));
   CU_CHECK(cudaMemsetAsync(ws.counters.p, 0, sizeof(PrepCounters), st));
@@ -1355,6 +1358,9 @@ static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const double
     ShearCells xc;
     for (int a = 0; a < 10; a++) xc.x[a] = dev[10 + a];
     CU_CHECK(launch_prepare_polzn_xi(rc, xc, tab, L, ws.Y.as<double>(), ws.P.as<double>(), cnt_d, st));
+  } else if (she) {
+    const GradientCells gc{{dev[10], dev[11], dev[12], dev[13]}};
+    CU_CHECK(launch_prepare_polzn_she(rc, gc, tab, L, ws.Y.as<double>(), ws.P.as<double>(), cnt_d, st));
   } else {
     const VortCells vc{dev[10], dev[11], dev[12], dev[13], dev[14], dev[15]};
     CU_CHECK(launch_prepare_polzn(rc, vc, tab, L, ws.Y.as<double>(), ws.P.as<double>(), cnt_d, st));
@@ -1371,6 +1377,9 @@ static int polzn_core(const is3d_flags *fl, const is3d_surface *sf, const double
   if (shear) {
     const PolXiParams prm{hp, dptr(o_cos), dptr(o_sin), dim2 ? nullptr : dptr(o_sloty)};
     CU_CHECK(launch_polzn_xi(prm, st));
+  } else if (she) {
+    const PolSheParams prm{hp, dptr(o_cos), dptr(o_sin), dim2 ? nullptr : dptr(o_sloty), dptr(o_bar)};
+    CU_CHECK(launch_polzn_she(prm, st));
   } else if (term == kPolSpinDensity) {
     // the prepare kernel never touches range_error: here it counts the boson evaluations without a valid occupation
     const SpinDensityParams prm{hp, dim2 ? nullptr : dptr(o_sloty), &cnt_d->range_error};
@@ -1436,12 +1445,13 @@ static int polzn_multi(const is3d_flags *fl, const is3d_surface *sf, const doubl
                        const is3d_grid *gr, const is3d_options *opt_in, double *const *out, is3d_stats *stats)
 {
   const int G = g_ngpus;
-  const bool shear = (term == kPolShear);
+  const bool shear = (term == kPolShear), she = (term == kPolSpinHall);
   if (G <= 1) return polzn_core(fl, sf, tensor, term, sp, gr, opt_in, out, stats);
-  if (!fl || !sf || !tensor || !sp || !gr || !out) return fail(IS3D_ERR_ARGUMENT, tensor ? "NULL argument" : shear ? "NULL thermal shear" : "NULL vorticity");
+  if (!fl || !sf || !tensor || !sp || !gr || !out)
+    return fail(IS3D_ERR_ARGUMENT, tensor ? "NULL argument" : shear ? "NULL thermal shear" : she ? "NULL baryon gradient" : "NULL vorticity");
   if (opt_in && opt_in->memory != 0) return fail(IS3D_ERR_ARGUMENT, "the multi-GPU entry point takes host arrays");
   std::lock_guard<std::mutex> lk(g_multi_mutex);
-  const int n_tensor = shear ? 10 : 6, n_out = pol_n_out(term);
+  const int n_tensor = shear ? 10 : she ? 4 : 6, n_out = pol_n_out(term);
   const size_t n_bins = (size_t)std::max(sp->n, 0) * std::max(gr->n_pT, 0) * std::max(gr->n_phi, 0) * std::max(gr->n_y, 0);
   int prev = 0; cudaGetDevice(&prev);
   std::vector<int> rcs(G, IS3D_OK);
@@ -1481,7 +1491,7 @@ static int polzn_multi(const is3d_flags *fl, const is3d_surface *sf, const doubl
   return IS3D_OK;
 }
 
-// the columns of the two input structs in the order of the prepare kernels, or NULL for a NULL struct
+// the columns of the input structs in the order of the prepare kernels, or NULL for a NULL struct
 static const double *const *vort_columns(const is3d_vorticity *vo, const double **c)
 {
   if (!vo) return nullptr;
@@ -1496,7 +1506,13 @@ static const double *const *shear_columns(const is3d_thermal_shear *xi, const do
   for (int a = 0; a < 10; a++) c[a] = v[a];
   return c;
 }
-// the result arrays of the three terms in the order of pol_n_out(), or NULL for a NULL struct
+static const double *const *gradient_columns(const is3d_baryon_gradient *gd, const double **c)
+{
+  if (!gd) return nullptr;
+  c[0] = gd->dt; c[1] = gd->dx; c[2] = gd->dy; c[3] = gd->dn;
+  return c;
+}
+// the result arrays of the terms in the order of pol_n_out() (shear_arrays serves the spin Hall term too), or NULL for a NULL struct
 static double *const *vort_arrays(is3d_polarization_result *r, double **a)
 {
   if (!r) return nullptr;
@@ -1547,6 +1563,22 @@ extern "C" int is3d_b200_spin_polarization_shear_multi(const is3d_flags *fl, con
 {
   const double *c[10]; double *a[5];
   return polzn_multi(fl, sf, shear_columns(xi, c), kPolShear, sp, gr, opt, shear_arrays(res, a), stats);
+}
+
+extern "C" int is3d_b200_spin_polarization_spin_hall(const is3d_flags *fl, const is3d_surface *sf, const is3d_baryon_gradient *gd,
+                                                     const is3d_species *sp, const is3d_grid *gr, const is3d_options *opt,
+                                                     is3d_polarization_result *res, is3d_stats *stats)
+{
+  const double *c[4]; double *a[5];
+  return polzn_core(fl, sf, gradient_columns(gd, c), kPolSpinHall, sp, gr, opt, shear_arrays(res, a), stats);
+}
+
+extern "C" int is3d_b200_spin_polarization_spin_hall_multi(const is3d_flags *fl, const is3d_surface *sf, const is3d_baryon_gradient *gd,
+                                                           const is3d_species *sp, const is3d_grid *gr, const is3d_options *opt,
+                                                           is3d_polarization_result *res, is3d_stats *stats)
+{
+  const double *c[4]; double *a[5];
+  return polzn_multi(fl, sf, gradient_columns(gd, c), kPolSpinHall, sp, gr, opt, shear_arrays(res, a), stats);
 }
 
 extern "C" int is3d_b200_spin_density(const is3d_flags *fl, const is3d_surface *sf, const is3d_vorticity *vo, const is3d_species *sp,

@@ -159,6 +159,17 @@ struct PolXiParams {
 cudaError_t launch_prepare_polzn_xi(const RawCells &cells, const ShearCells &shear, const PrepTables &tab, const Layout &L, double *Y,
                                     double *P, PrepCounters *counters, cudaStream_t st);
 cudaError_t launch_polzn_xi(const PolXiParams &prm, cudaStream_t st);
+// spin Hall part of the spin polarization (cf_polzn_she.cu): the layout, records sizes and chunks of cf_polzn.cu, 4 sums per bin
+struct GradientCells { const double *d[4]; };  // device pointers, covariant Milne components of d alpha_B: tau x y eta
+struct PolSheParams {
+  HotParams hp;                  // layout, records Y / P, species and pT tables, partial [4][n_chunks][n_bins] (Snorm, N^x, N^y, N^z)
+  const double *cosphi, *sinphi; // [n_phi]
+  const double *y;               // 3+1D: the y table [n_y]; 2+1D: unused (y = 0)
+  const double *baryon;          // [n_species] baryon number q_B
+};
+cudaError_t launch_prepare_polzn_she(const RawCells &cells, const GradientCells &grad, const PrepTables &tab, const Layout &L, double *Y,
+                                     double *P, PrepCounters *counters, cudaStream_t st);
+cudaError_t launch_polzn_she(const PolSheParams &prm, cudaStream_t st);
 // spin density matrix from thermal vorticity (cf_spin_density.cu): the records of prepare_polzn_kernel, its own register tile,
 // 9 sums per bin (Snorm, P_x, P_y, P_z, Q_xx, Q_xy, Q_xz, Q_yy, Q_yz)
 constexpr int kSdSums = 9;

@@ -1,11 +1,13 @@
-// cf_polzn.cuh -- Milne -> Cartesian conversion of the spin-polarization input tensors (cf_polzn.cu, cf_polzn_xi.cu).
+// cf_polzn.cuh -- Milne -> Cartesian conversion of the spin-polarization inputs (cf_polzn.cu, cf_polzn_xi.cu, cf_polzn_she.cu).
 //
-// Both functions read covariant Milne components (an eta index carries a factor tau) at space-time rapidity eta and return covariant
+// The functions read covariant Milne components (an eta index carries a factor tau) at space-time rapidity eta and return covariant
 // Cartesian lab components, with the Jacobian d tau/dt = ch, d tau/dz = -sh, d eta/dt = -sh/tau, d eta/dz = ch/tau (ch = cosh eta,
 // sh = sinh eta).  They are the single place to change if a surface writer uses another convention.
 #pragma once
 
 namespace is3d {
+
+constexpr double kHbarC = 0.197327053;     // GeV fm
 
 // Covariant Milne components (varpi_{tau x}, varpi_{tau y}, varpi_{tau eta}, varpi_{xy}, varpi_{x eta}, varpi_{y eta}) at space-time
 // rapidity eta -> e = (varpi_tx, varpi_ty, varpi_tz) and omega = (varpi_yz, varpi_zx, varpi_xy), Cartesian lab components:
@@ -43,6 +45,16 @@ __device__ __forceinline__ void cart_shear(const double x[10], double tau, doubl
   c[7] = x[7];
   c[8] = -sh * x[2] + cht * x[8];
   c[9] = sh * sh * x[0] - 2.0 * sh * cht * x[3] + cht * cht * x[9];
+}
+
+// Covariant Milne components of a scalar gradient (d_tau, d_x, d_y, d_eta; 1/fm, d_eta dimensionless) at space-time rapidity eta -> its
+// Cartesian spatial components z = (d_x, d_y, d_z) in 1/fm (the time component never enters the spin Hall term):
+//   d_z = -sh d_tau + (ch/tau) d_eta
+__device__ __forceinline__ void cart_gradient(const double d[4], double tau, double eta, double z[3])
+{
+  z[0] = d[1];
+  z[1] = d[2];
+  z[2] = -sinh(eta) * d[0] + cosh(eta) / tau * d[3];
 }
 
 }  // namespace is3d

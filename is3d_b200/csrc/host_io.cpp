@@ -221,31 +221,43 @@ struct Tokens {
   }
 };
 
-bool read_thermal_shear(const std::string &workdir, SurfaceData *s, std::string *err)
+// one newline-terminated line per surface cell, in surface order, with at least cols.size() numbers (`count` names that number)
+static bool read_cell_columns(const std::string &path, const char *key, const std::vector<std::vector<double> *> &cols, const char *count,
+                              int64_t n, std::string *err)
 {
-  const std::string path = workdir + "/input/thermal_shear.dat";
   std::string text;
-  if (!slurp(path, &text)) { if (err) *err = "cannot open " + path + " (thermal_shear_polarization = 1 reads it)"; return false; }
+  if (!slurp(path, &text)) { if (err) *err = "cannot open " + path + " (" + key + " = 1 reads it)"; return false; }
   int64_t lines = 0;
   for (char c : text) if (c == '\n') lines++;
-  if (lines != s->n) {
-    if (err) *err = path + " has " + std::to_string(lines) + " lines, the surface has " + std::to_string(s->n) + " cells";
+  if (lines != n) {
+    if (err) *err = path + " has " + std::to_string(lines) + " lines, the surface has " + std::to_string(n) + " cells";
     return false;
   }
-  std::vector<double> *col[10] = {&s->xtt, &s->xtx, &s->xty, &s->xtn, &s->xxx, &s->xxy, &s->xxn, &s->xyy, &s->xyn, &s->xnn};
-  for (std::vector<double> *v : col) v->assign((size_t)s->n, 0.0);
+  for (std::vector<double> *v : cols) v->assign((size_t)n, 0.0);
   const char *p = text.data(), *end = text.data() + text.size();
-  for (int64_t i = 0; i < s->n; i++) {
+  for (int64_t i = 0; i < n; i++) {
     const char *eol = static_cast<const char *>(std::memchr(p, '\n', (size_t)(end - p)));
     Tokens tk{p, eol};
-    for (std::vector<double> *v : col)
+    for (std::vector<double> *v : cols)
       if (!tk.next(&(*v)[i])) {
-        if (err) *err = path + ": line " + std::to_string(i + 1) + " has fewer than ten numbers";
+        if (err) *err = path + ": line " + std::to_string(i + 1) + " has fewer than " + count + " numbers";
         return false;
       }
     p = eol + 1;
   }
   return true;
+}
+
+bool read_thermal_shear(const std::string &workdir, SurfaceData *s, std::string *err)
+{
+  return read_cell_columns(workdir + "/input/thermal_shear.dat", "thermal_shear_polarization",
+                           {&s->xtt, &s->xtx, &s->xty, &s->xtn, &s->xxx, &s->xxy, &s->xxn, &s->xyy, &s->xyn, &s->xnn}, "ten", s->n, err);
+}
+
+bool read_baryon_gradient(const std::string &workdir, SurfaceData *s, std::string *err)
+{
+  return read_cell_columns(workdir + "/input/muB_over_T_gradient.dat", "spin_hall_polarization", {&s->gbt, &s->gbx, &s->gby, &s->gbn}, "four",
+                           s->n, err);
 }
 
 bool read_surface(const std::string &workdir, const SurfaceFlags &fl, SurfaceData *s, std::string *err)

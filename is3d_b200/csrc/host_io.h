@@ -53,6 +53,7 @@ struct SurfaceData {
   std::vector<double> PL, Wx, Wy, Lambda, aL, c0, c1, c2, c3, c4;     // anisotropic hydro (mode 2)
   std::vector<double> wtx, wty, wtn, wxy, wxn, wyn;                    // thermal vorticity, covariant Milne components (mode 5)
   std::vector<double> xtt, xtx, xty, xtn, xxx, xxy, xxn, xyy, xyn, xnn;   // thermal shear, covariant Milne components (input/thermal_shear.dat)
+  std::vector<double> gbt, gbx, gby, gbn;   // gradient of alpha_B = muB/T, covariant Milne components (input/muB_over_T_gradient.dat)
   bool averages_written = false;
   double avg[5] = {0, 0, 0, 0, 0};   // T, E, P, muB, nB after the 15-digit text round trip of the side file
 };
@@ -64,6 +65,10 @@ bool read_surface(const std::string &workdir, const SurfaceFlags &fl, SurfaceDat
 // covariant Milne components xi_{tau tau} xi_{tau x} xi_{tau y} xi_{tau eta} xi_{xx} xi_{xy} xi_{x eta} xi_{yy} xi_{y eta} xi_{eta eta}
 // (dimensionless).  A missing file, a line count other than out->n or a line with fewer than ten numbers is an error.
 bool read_thermal_shear(const std::string &workdir, SurfaceData *out, std::string *err);
+// input/muB_over_T_gradient.dat (this project's own format): one newline-terminated line per surface cell, in surface order, with the four
+// covariant Milne components d_tau alpha_B, d_x alpha_B, d_y alpha_B (1/fm), d_eta alpha_B (dimensionless) of alpha_B = muB/T.  A missing
+// file, a line count other than out->n or a line with fewer than four numbers is an error.
+bool read_baryon_gradient(const std::string &workdir, SurfaceData *out, std::string *err);
 
 struct DfTables {
   int n_T = 0, n_muB_file = 0;

@@ -179,9 +179,11 @@ static bool write_spacetime_files(const std::string &wd, const std::vector<int> 
 // results/polarization/S_<mcid>.dat: mean spin vector S^mu = N^mu / Snorm (lab frame, Cartesian t, x, y, z; 0 where Snorm = 0) and its
 // rest-frame spatial part S*_i = S^i - S^t p^i / (E + m), one row per (y, phi, pT) in the loop order, number format and blank line per
 // phi block of write_spectra_files; truncating opens, results/polarization/ must exist.
-// With the thermal-shear sums xi (St | Sx | Sy | Sz | Snorm of is3d_b200_spin_polarization_shear, non-NULL) it writes S_xi_<mcid>.dat
-// instead: Snorm, the shear part N_xi / Snorm, the total S = (N + N_xi) / Snorm and the rest-frame part of the total.
-// stem: the file name stem of the plain form ("S"; "S_fd" for the sums after the feed-down through decays).
+// With the sums of one more term xi (St | Sx | Sy | Sz | Snorm of is3d_b200_spin_polarization_shear or _spin_hall, non-NULL) it writes
+// S_<stem>_<mcid>.dat instead: Snorm, that term's part N_xi / Snorm (columns S?_<stem>), the total S = (N + N_xi) / Snorm and the
+// rest-frame part of the total.
+// stem: the file name stem of the plain form ("S"; "S_fd" for the sums after the feed-down through decays), or the tag of the term
+// ("xi" for the thermal shear, "she" for the spin Hall term).
 static bool write_polarization_files(const std::string &wd, const std::vector<double> &sums, const std::vector<double> *xi,
                                      const std::vector<int> &mcid, const std::vector<double> &mass, const Grids &g, int dimension,
                                      std::string *err, const char *stem = "S")
@@ -193,12 +195,12 @@ static bool write_polarization_files(const std::string &wd, const std::vector<do
   const double *Xx = xi ? &(*xi)[n_bins] : nullptr, *Xy = xi ? Xx + n_bins : nullptr, *Xz = xi ? Xy + n_bins : nullptr;
   for (int ipart = 0; ipart < npart; ipart++) {
     char name[255];
-    if (xi) std::snprintf(name, sizeof(name), "%s/results/polarization/S_xi_%d.dat", wd.c_str(), mcid[ipart]);
+    if (xi) std::snprintf(name, sizeof(name), "%s/results/polarization/S_%s_%d.dat", wd.c_str(), stem, mcid[ipart]);
     else std::snprintf(name, sizeof(name), "%s/results/polarization/%s_%d.dat", wd.c_str(), stem, mcid[ipart]);
     std::ofstream f(name, std::ios_base::out);
     if (!f) { *err = std::string("cannot open ") + name + " (the directory results/polarization/ must exist)"; return false; }
-    f << (xi ? "y\tphip\tpT\tSnorm\tSx_xi\tSy_xi\tSz_xi\tSx\tSy\tSz\tSx_rest\tSy_rest\tSz_rest\n"
-             : "y\tphip\tpT\tSnorm\tSt\tSx\tSy\tSz\tSx_rest\tSy_rest\tSz_rest\n");
+    if (xi) f << "y\tphip\tpT\tSnorm\tSx_" << stem << "\tSy_" << stem << "\tSz_" << stem << "\tSx\tSy\tSz\tSx_rest\tSy_rest\tSz_rest\n";
+    else f << "y\tphip\tpT\tSnorm\tSt\tSx\tSy\tSz\tSx_rest\tSy_rest\tSz_rest\n";
     const double m = mass[ipart];
     for (int iy = 0; iy < y_pts; iy++) {
       const double y = (dimension == 2) ? 0.0 : g.y.at(1, iy + 1);
@@ -346,6 +348,7 @@ struct Problem {
   int operation = 0, hrg_eos = 0, group_particles = 0, do_resonance_decays = 0;
   int spin_polarization = 0;               // optional key (absent: 0): mode-5 spin polarization after the spectra
   int thermal_shear_polarization = 0;      // optional key (absent: 0): add the thermal-shear term (input/thermal_shear.dat)
+  int spin_hall_polarization = 0;          // optional key (absent: 0): add the spin Hall term (input/muB_over_T_gradient.dat)
   int polarization_feed_down = 0;          // optional key (absent: 0): feed the polarization sums down through the decay tables
   int spin_density = 0;                    // optional key (absent: 0): mode-5 spin density matrix (all-order spin, rank-2 tensor)
   std::map<long, int> box_parity;          // its parities by |MC id| (PDG/pdg_box.dat)
@@ -399,6 +402,10 @@ static int load_problem(const std::string &wd, bool need_surface, Problem *p, st
   if (p->thermal_shear_polarization && (p->operation != 1 || fl.mode != 5 || !p->spin_polarization)) {
     err = "thermal_shear_polarization = 1 needs operation = 1, a mode 5 surface and spin_polarization = 1"; return IS3D_ERR_UNSUPPORTED;
   }
+  p->spin_hall_polarization = par.has("spin_hall_polarization") ? (int)par.get("spin_hall_polarization", &err) : 0;
+  if (p->spin_hall_polarization && (p->operation != 1 || fl.mode != 5 || !p->spin_polarization)) {
+    err = "spin_hall_polarization = 1 needs operation = 1, a mode 5 surface and spin_polarization = 1"; return IS3D_ERR_UNSUPPORTED;
+  }
   p->polarization_feed_down = par.has("polarization_feed_down") ? (int)par.get("polarization_feed_down", &err) : 0;
   if (p->polarization_feed_down && (p->operation != 1 || fl.mode != 5 || !p->spin_polarization || (p->hrg_eos != 1 && p->hrg_eos != 2))) {
     err = "polarization_feed_down = 1 needs operation = 1, a mode 5 surface, spin_polarization = 1 and a particle list with decay tables "
@@ -427,6 +434,7 @@ static int load_problem(const std::string &wd, bool need_surface, Problem *p, st
     SurfaceFlags sfl{fl.mode, fl.dimension, fl.df_mode, fl.include_baryon, fl.include_baryondiff_deltaf};
     if (!read_surface(wd, sfl, &p->sf, &err)) return IS3D_ERR_IO;
     if (p->thermal_shear_polarization && !read_thermal_shear(wd, &p->sf, &err)) return IS3D_ERR_IO;
+    if (p->spin_hall_polarization && !read_baryon_gradient(wd, &p->sf, &err)) return IS3D_ERR_IO;
   }
   // ---- particle list, delta-f tables
   if (!read_pdg(wd, p->hrg_eos, &p->pdg, &err)) return IS3D_ERR_IO;
@@ -497,7 +505,8 @@ struct FlatList {
 };
 
 static int run_problem(const std::string &wd, Problem &P, const is3d_surface &s, const is3d_vorticity *vort, const is3d_thermal_shear *shear,
-                       double *dN_raw, int64_t n_raw, int32_t *mcid_out, int32_t n_mcid_max, is3d_stats *stats, std::string *err_out)
+                       const is3d_baryon_gradient *grad, double *dN_raw, int64_t n_raw, int32_t *mcid_out, int32_t n_mcid_max, is3d_stats *stats,
+                       std::string *err_out)
 {
   std::string &err = *err_out;
   const Grids &g = P.g; const DfTables &dft = P.dft; const Laguerre &gla = P.gla;
@@ -573,8 +582,18 @@ static int run_problem(const std::string &wd, Problem &P, const is3d_surface &s,
       const int rcx = is3d_b200_spin_polarization_shear_multi(&P.fl, &s, shear, &sp, &gr, nullptr, &rx, &sp_st);
       if (rcx != IS3D_OK) { err = std::string("thermal-shear polarization failed: ") + is3d_b200_last_error(); return rcx; }
       if (stats) { stats->gpu_launches += sp_st.gpu_launches; stats->total_ms += sp_st.total_ms; }
-      if (!write_polarization_files(wd, sums, &xi, P.mcid, P.mass, g, P.fl.dimension, &err)) return IS3D_ERR_IO;
+      if (!write_polarization_files(wd, sums, &xi, P.mcid, P.mass, g, P.fl.dimension, &err, "xi")) return IS3D_ERR_IO;
       for (size_t k = 0; k < 4 * n_bins; k++) sums[k] += xi[k];  // the feed-down below runs on the total (vorticity + shear)
+    }
+    if (P.spin_hall_polarization) {
+      std::vector<double> she(5 * n_bins, 0.0);                  // St (zeros) | Sx | Sy | Sz | Snorm
+      is3d_polarization_result rh{&she[0], &she[n_bins], &she[2 * n_bins], &she[3 * n_bins], &she[4 * n_bins]};
+      std::memset(&sp_st, 0, sizeof(sp_st));
+      const int rch = is3d_b200_spin_polarization_spin_hall_multi(&P.fl, &s, grad, &sp, &gr, nullptr, &rh, &sp_st);
+      if (rch != IS3D_OK) { err = std::string("spin Hall polarization failed: ") + is3d_b200_last_error(); return rch; }
+      if (stats) { stats->gpu_launches += sp_st.gpu_launches; stats->total_ms += sp_st.total_ms; }
+      if (!write_polarization_files(wd, sums, &she, P.mcid, P.mass, g, P.fl.dimension, &err, "she")) return IS3D_ERR_IO;
+      for (size_t k = 0; k < 4 * n_bins; k++) sums[k] += she[k]; // the feed-down below runs on the total (vorticity (+ shear) + spin Hall)
     }
     if (P.polarization_feed_down) {
       // 2J = gspin - 1 of the list, parities by |MC id| from pdg_box.dat (0, unknown: the channel only dilutes)
@@ -677,8 +696,9 @@ extern "C" int is3d_b200_run_workdir(const char *workdir, double *dN_raw, int64_
   const is3d_vorticity vort{sf.wtx.data(), sf.wty.data(), sf.wtn.data(), sf.wxy.data(), sf.wxn.data(), sf.wyn.data()};
   const is3d_thermal_shear shear{sf.xtt.data(), sf.xtx.data(), sf.xty.data(), sf.xtn.data(), sf.xxx.data(), sf.xxy.data(), sf.xxn.data(),
                                  sf.xyy.data(), sf.xyn.data(), sf.xnn.data()};
-  rc = run_problem(wd, P, s, P.fl.mode == 5 ? &vort : nullptr, P.thermal_shear_polarization ? &shear : nullptr, dN_raw, n_raw, mcid_out,
-                   n_mcid_max, stats, &err);
+  const is3d_baryon_gradient grad{sf.gbt.data(), sf.gbx.data(), sf.gby.data(), sf.gbn.data()};
+  rc = run_problem(wd, P, s, P.fl.mode == 5 ? &vort : nullptr, P.thermal_shear_polarization ? &shear : nullptr,
+                   P.spin_hall_polarization ? &grad : nullptr, dN_raw, n_raw, mcid_out, n_mcid_max, stats, &err);
   return rc == IS3D_OK ? rc : fail(rc);
 }
 
@@ -702,7 +722,7 @@ extern "C" int is3d_b200_run_surface(const char *workdir, const is3d_surface *su
     if (rc != IS3D_OK) { err = "cannot average an empty surface"; return fail(rc); }
     compute_jonah_tables(P.pdg, avg[0], P.gla, &P.dft);
   }
-  rc = run_problem(wd, P, *surface, nullptr, nullptr, dN_raw, n_raw, mcid_out, n_mcid_max, stats, &err);
+  rc = run_problem(wd, P, *surface, nullptr, nullptr, nullptr, dN_raw, n_raw, mcid_out, n_mcid_max, stats, &err);
   return rc == IS3D_OK ? rc : fail(rc);
 }
 
@@ -763,6 +783,7 @@ extern "C" int is3d_b200_host_dump(const char *workdir, const char *out_path)
     put("xtt", s.xtt); put("xtx", s.xtx); put("xty", s.xty); put("xtn", s.xtn); put("xxx", s.xxx);
     put("xxy", s.xxy); put("xxn", s.xxn); put("xyy", s.xyy); put("xyn", s.xyn); put("xnn", s.xnn);
   }
+  if (P.spin_hall_polarization) { put("gbt", s.gbt); put("gbx", s.gbx); put("gby", s.gby); put("gbn", s.gbn); }
   if (P.polarization_feed_down) {        // what the feed-down passes as is3d_spin_parity: 2J = gspin - 1, parity by |MC id| (0 unknown)
     tmp.clear(); for (auto &h : P.pdg) tmp.push_back(h.gspin - 1); put("pdg_spin2", tmp);
     tmp.clear();

@@ -135,3 +135,15 @@ def thermal_shear(n_cells, seed):
     rng = np.random.default_rng(seed)
     s = np.array([0.02, 0.02, 0.02, 0.1, 0.02, 0.02, 0.1, 0.02, 0.1, 0.5])
     return {k: rng.normal(0.0, s[j], n_cells) for j, k in enumerate(THERMAL_SHEAR_COLUMNS)}
+
+
+BARYON_GRADIENT_COLUMNS = ("dt", "dx", "dy", "dn")
+
+
+def baryon_gradient(n_cells, seed):
+    """Gradient of alpha_B = muB/T for input/muB_over_T_gradient.dat: the four covariant Milne components d_tau alpha_B, d_x alpha_B,
+    d_y alpha_B (1/fm) and d_eta alpha_B (dimensionless) as a dict of arrays.  The eta component carries a factor tau ~ 5 fm relative to
+    the others, as a covariant component does."""
+    rng = np.random.default_rng(seed)
+    s = np.array([0.1, 0.1, 0.1, 0.5])
+    return {k: rng.normal(0.0, s[j], n_cells) for j, k in enumerate(BARYON_GRADIENT_COLUMNS)}

@@ -13,7 +13,7 @@ import os
 
 import numpy as np
 
-from is3d_b200.synthetic import THERMAL_SHEAR_COLUMNS
+from is3d_b200.synthetic import BARYON_GRADIENT_COLUMNS, THERMAL_SHEAR_COLUMNS
 
 _FIXTURE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "data", "is3d_tables.npz")
 
@@ -32,7 +32,7 @@ DEFAULT_PARAMETERS = [
 ]
 
 # keys of this drop-in that the reference does not read: written only when a caller sets them (absent: 0, or the default of the host layer)
-OPTIONAL_PARAMETERS = ("spin_polarization", "thermal_shear_polarization", "polarization_feed_down", "spin_density", "hbt_radii", "hbt_correlation", "hbt_dq",
+OPTIONAL_PARAMETERS = ("spin_polarization", "thermal_shear_polarization", "spin_hall_polarization", "polarization_feed_down", "spin_density", "hbt_radii", "hbt_correlation", "hbt_dq",
                        "hbt_q_points")
 
 _EOS_DIR = {1: "urqmd", 2: "smash", 3: "smash_box"}
@@ -128,7 +128,8 @@ def _write_df_vah(dirname, fx):
                 f.write("%s\t\t%s\t\t%s\n" % (_r(a), _r(b), _r(c)))
 
 
-def materialize(root, surface_columns=None, chosen=None, fixture=None, tables=None, vah=False, thermal_shear=None, **params):
+def materialize(root, surface_columns=None, chosen=None, fixture=None, tables=None, vah=False, thermal_shear=None, baryon_gradient=None,
+                **params):
     """Create `root` as an iS3D working directory.
 
     surface_columns : (n_cells, n_cols) array in file units, or None for the shipped one-cell toy surface.
@@ -136,6 +137,8 @@ def materialize(root, surface_columns=None, chosen=None, fixture=None, tables=No
     tables          : optional dict overriding quadrature tables: keys pT, phi, y, eta -> (n, 2) arrays.
     thermal_shear   : optional (n_cells, 10) array or dict of the ten columns of synthetic.THERMAL_SHEAR_COLUMNS, written to
                       input/thermal_shear.dat (read when thermal_shear_polarization = 1).
+    baryon_gradient : optional (n_cells, 4) array or dict of the four columns of synthetic.BARYON_GRADIENT_COLUMNS, written to
+                      input/muB_over_T_gradient.dat (read when spin_hall_polarization = 1).
     params          : iS3D_parameters.dat overrides (operation, mode, df_mode, dimension, ...).
     """
     fx = fixture if fixture is not None else load_fixture()
@@ -153,6 +156,10 @@ def materialize(root, surface_columns=None, chosen=None, fixture=None, tables=No
         if isinstance(thermal_shear, dict):
             thermal_shear = np.column_stack([thermal_shear[k] for k in THERMAL_SHEAR_COLUMNS])
         write_surface(os.path.join(root, "input", "thermal_shear.dat"), thermal_shear)
+    if baryon_gradient is not None:
+        if isinstance(baryon_gradient, dict):
+            baryon_gradient = np.column_stack([baryon_gradient[k] for k in BARYON_GRADIENT_COLUMNS])
+        write_surface(os.path.join(root, "input", "muB_over_T_gradient.dat"), baryon_gradient)
     key, fname = _EOS_PDG[hrg_eos]
     if hrg_eos == 3:
         _write_pdg_box(os.path.join(root, "PDG", fname), fx)
