@@ -323,6 +323,42 @@ int is3d_b200_polarization_decays(const is3d_particle_list *particles, const is3
                                   const int32_t *chosen_pdg_index, const is3d_grid *grid, int32_t dimension, const is3d_options *options,
                                   is3d_polarization_result *sums, is3d_stats *stats);
 
+/* ---- feed-down of the spin polarization through weak decays (Xi -> Lambda pi, Omega -> Lambda K, Omega -> Xi pi) -----------------
+ * Amends, in place, the five arrays with the weak channels of the caller's table only.  Meant for the output of
+ * is3d_b200_polarization_decays (it does not call it): weak daughters are stable hadrons and no strong decay follows a weak one, so the
+ * two passes in this order are exact.  One row per channel: parent -> daughter + partner (MC ids looked up in the particle list, where
+ * an antiparticle is its own row), branching ratio and the PDG decay parameters (alpha, phi):
+ *    beta = sqrt(1 - alpha^2) sin phi,   gamma = sqrt(1 - alpha^2) cos phi.
+ * Weak parents that are chosen species are processed in descending mass (ties: descending chosen index), so Omega -> Xi comes before
+ * Xi -> Lambda and each parent's arrays are final when its turn comes.  A row whose parent or daughter is not a chosen species does
+ * nothing; only the daughter is fed (not the partner).  The 2-body integration points, the interpolation of the parent's log spectrum
+ * and of S*_P, and the Lorentz chain are those of is3d_b200_polarization_decays; no width shift is applied.  At every integration point,
+ * with S = S*_P and n the daughter's direction in the parent's rest frame, a row whose spins are 2J = 1 -> 1 + 0 (spin_parity->spin2 of
+ * parent, daughter, partner; parities are not used) follows the Lee-Yang law, exact in S:
+ *    Snorm_D += w (1 + 2 alpha S.n)
+ *    N_D^mu  += w x the four-vector of  s* = (alpha/2 + S.n) n + beta S x n + gamma (S - (S.n) n)
+ * (s* is the daughter's rest-frame spin times the yield 1 + 2 alpha S.n, in the frame of the pure boost along n from the parent's rest
+ * frame), w = the point's weight of the spectra feed-down.  Averaged over n: yield 1, <s*> = (1 + 2 gamma)/3 S (the transfer coefficient
+ * C_XiLambda of the Xi polarization measured through its Lambda); alpha = beta = 0, gamma = -1 is the 1/2+ -> 1/2+ 0- law of
+ * is3d_b200_polarization_decays and gamma = +1 its S-wave law.  Any other row (e.g. Omega-, J = 3/2) has no law: it feeds Snorm with the
+ * plain 2-body integral and only dilutes.  With N = 0 everywhere (S = 0), the Snorm returned is the weak feed-down of the plain
+ * spectrum, and N_D receives w x (alpha/2) n carried to the lab: the helicity of the daughters of unpolarised parents.  The library
+ * ships no decay parameters: their values change between PDG editions.
+ * n = 0 is a valid no-op.  Arrays: spectra layout; host or device memory per options->memory.  Results are bit-reproducible.
+ * Errors: IS3D_ERR_ARGUMENT, with every array untouched, for those of is3d_b200_polarization_decays, a NULL table or row array, n < 0, an
+ * MC id that is not in the list, a parent or daughter that is not `stable` in the list, a branching ratio outside [0, 1], a parent whose
+ * branching ratios sum to more than 1 (beyond 1e-9 of rounding), |alpha| > 1, a non-finite alpha or phi, m_daughter + m_partner >= m_parent,
+ * and a parent whose tail fit has fewer than 2 points. */
+typedef struct {
+  int32_t n;                                   /* rows; 0 is a valid no-op */
+  const int32_t *parent, *daughter, *partner;  /* MC ids, looked up in the particle list (antiparticles are their own rows) */
+  const double *branching, *alpha, *phi;       /* PDG parametrisation: beta = sqrt(1-alpha^2) sin phi, gamma = sqrt(1-alpha^2) cos phi */
+} is3d_weak_decays;
+int is3d_b200_polarization_weak_decays(const is3d_particle_list *particles, const is3d_spin_parity *spin_parity,
+                                       const is3d_weak_decays *weak, int32_t n_chosen, const int32_t *chosen_pdg_index,
+                                       const is3d_grid *grid, int32_t dimension, const is3d_options *options,
+                                       is3d_polarization_result *sums, is3d_stats *stats);
+
 /* ---- HBT radii: space-time variances of the Cooper-Frye emission function ---------------------------------------------
  * Gaussian (moment) approximation with pair momentum K = p (Wiedemann & Heinz, Phys. Rept. 319 (1999) 145).  For every spectra bin
  * (species, pT, phi, y; 2+1D: y = 0) the frame is the bin's longitudinally co-moving frame (LCMS): a longitudinal boost by the bin's

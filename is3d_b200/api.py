@@ -488,6 +488,59 @@ def polarization_decays(pdg, spin_parity, chosen_pdg_index, grid, dimension, sum
     return out, st.as_dict()
 
 
+WEAK_DECAY_COLUMNS = ("parent", "daughter", "partner", "branching", "alpha", "phi")
+
+
+class WeakDecays(C.Structure):
+    _fields_ = [("n", C.c_int32), ("parent", C.POINTER(C.c_int32)), ("daughter", C.POINTER(C.c_int32)), ("partner", C.POINTER(C.c_int32)),
+                ("branching", _D), ("alpha", _D), ("phi", _D)]
+
+
+def polarization_weak_decays(pdg, spin_parity, weak, chosen_pdg_index, grid, dimension, sums, memory="host", stream=None):
+    """Call is3d_b200_polarization_weak_decays: feed-down of the spin-polarization raw sums through weak 2-body decays (Lee-Yang law), meant
+    for the output of polarization_decays.
+
+    weak: dict of the six columns parent, daughter, partner (MC ids), branching, alpha, phi (radians), as tables.weak_decays reads them;
+    None passes a NULL table (the library rejects it).  Other arguments, memory and the return value as for polarization_decays."""
+    keep = []
+    p, g, ia = _decay_problem(pdg, grid, keep)
+    sp = None
+    if spin_parity is not None:
+        sp = SpinParity()
+        sp.spin2 = ia(spin_parity["spin2"]); sp.parity = ia(spin_parity["parity"])
+    wd = None
+    if weak is not None:
+        wd = WeakDecays()
+        wd.n = len(np.atleast_1d(weak["parent"]))
+        for k in ("parent", "daughter", "partner"):
+            setattr(wd, k, ia(np.atleast_1d(weak[k])))
+        for k in ("branching", "alpha", "phi"):
+            a = np.ascontiguousarray(np.atleast_1d(weak[k]), dtype=np.float64); keep.append(a)
+            setattr(wd, k, a.ctypes.data_as(_D))
+    device = (memory == "device")
+    res = PolarizationResult()
+    if device:
+        import torch
+        out = sums
+        for k in POLARIZATION_FIELDS:
+            setattr(res, k, C.cast(C.c_void_p(out[k].data_ptr()), _D))
+        if stream is None:
+            stream = torch.cuda.current_stream().cuda_stream
+    else:
+        out = {k: np.array(sums[k], dtype=np.float64, copy=True) for k in POLARIZATION_FIELDS}
+        for k in POLARIZATION_FIELDS:
+            setattr(res, k, out[k].ctypes.data_as(_D))
+    opt = Options(); opt.memory = 1 if device else 0; opt.stream = C.c_void_p(stream or 0)
+    st = Stats()
+    f = lib().is3d_b200_polarization_weak_decays
+    f.restype = C.c_int
+    f.argtypes = [C.POINTER(ParticleList), C.POINTER(SpinParity), C.POINTER(WeakDecays), C.c_int32, C.POINTER(C.c_int32), C.POINTER(Grid),
+                  C.c_int32, C.POINTER(Options), C.POINTER(PolarizationResult), C.POINTER(Stats)]
+    _check(f(C.byref(p), C.byref(sp) if sp is not None else None, C.byref(wd) if wd is not None else None, len(chosen_pdg_index),
+             ia(chosen_pdg_index), C.byref(g), int(dimension), C.byref(opt), C.byref(res), C.byref(st)))
+    return out, st.as_dict()
+
+
 VORTICITY_FIELDS = ("wtx", "wty", "wtn", "wxy", "wxn", "wyn")
 POLARIZATION_FIELDS = ("St", "Sx", "Sy", "Sz", "Snorm")
 

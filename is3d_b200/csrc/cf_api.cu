@@ -917,11 +917,8 @@ extern "C" int is3d_b200_resonance_decays(const is3d_particle_list *pdg, int32_t
   return IS3D_OK;
 }
 
-// Feed-down of the spin-polarization sums through 2-body decays (cf_decays.cu).  Like is3d_b200_resonance_decays it works on a device
-// copy of all five arrays, so an error leaves the caller's arrays untouched.
-extern "C" int is3d_b200_polarization_decays(const is3d_particle_list *pdg, const is3d_spin_parity *spin_parity, int32_t n_chosen,
-                                             const int32_t *chosen, const is3d_grid *gr, int32_t dimension, const is3d_options *opt_in,
-                                             is3d_polarization_result *sums, is3d_stats *stats)
+static int check_polarization_feed_down_args(const is3d_particle_list *pdg, const is3d_spin_parity *spin_parity, int32_t n_chosen,
+                                             const int32_t *chosen, const is3d_grid *gr, int32_t dimension, const is3d_polarization_result *sums)
 {
   if (!sums || !sums->St || !sums->Sx || !sums->Sy || !sums->Sz || !sums->Snorm) return fail(IS3D_ERR_ARGUMENT, "NULL result array");
   { const int rc = check_decay_args(pdg, n_chosen, chosen, gr, dimension); if (rc) return rc; }
@@ -930,6 +927,15 @@ extern "C" int is3d_b200_polarization_decays(const is3d_particle_list *pdg, cons
     if (spin_parity->spin2[i] < 0) return fail(IS3D_ERR_ARGUMENT, "negative 2J in the spin / parity table");
     if (spin_parity->parity[i] < -1 || spin_parity->parity[i] > 1) return fail(IS3D_ERR_ARGUMENT, "parity must be -1, 0 (unknown) or +1");
   }
+  return IS3D_OK;
+}
+
+// The five arrays copied to the device workspace, run(dev, n_bins, st, &launches, &err) amending them there, and copied back only when it
+// succeeds: an error leaves the caller's arrays untouched.
+template <class Run>
+static int polarization_feed_down_call(const is3d_grid *gr, int32_t n_chosen, const is3d_options *opt_in, is3d_polarization_result *sums,
+                                       is3d_stats *stats, Run run)
+{
   Device *Dp = nullptr;
   { int rc = current_device(&Dp); if (rc) return rc; }
   Workspace &ws = Dp->ws;
@@ -948,8 +954,7 @@ extern "C" int is3d_b200_polarization_decays(const is3d_particle_list *pdg, cons
   for (int k = 0; k < 5; k++) CU_CHECK(cudaMemcpyAsync(dev + k * n_bins, arr[k], (size_t)n_bins * 8, in, st));
   CU_CHECK(cudaEventRecord(ev[1], st));
   int launches = 0; std::string err;
-  const int rc = polarization_decays_device(pdg, spin_parity->spin2, spin_parity->parity, n_chosen, chosen, gr, dimension, dev, n_bins, st,
-                                            &launches, &err);
+  const int rc = run(dev, n_bins, st, &launches, &err);
   if (rc != IS3D_OK) { cudaStreamSynchronize(st); return fail(rc, err.c_str()); }
   CU_CHECK(cudaEventRecord(ev[2], st));
   for (int k = 0; k < 5; k++) CU_CHECK(cudaMemcpyAsync(arr[k], dev + k * n_bins, (size_t)n_bins * 8, out, st));
@@ -966,6 +971,34 @@ extern "C" int is3d_b200_polarization_decays(const is3d_particle_list *pdg, cons
     *stats = stt;
   }
   return IS3D_OK;
+}
+
+// Feed-down of the spin-polarization sums through weak 2-body decays (cf_decays.cu), on the output of is3d_b200_polarization_decays.
+extern "C" int is3d_b200_polarization_weak_decays(const is3d_particle_list *pdg, const is3d_spin_parity *spin_parity, const is3d_weak_decays *weak,
+                                                  int32_t n_chosen, const int32_t *chosen, const is3d_grid *gr, int32_t dimension,
+                                                  const is3d_options *opt_in, is3d_polarization_result *sums, is3d_stats *stats)
+{
+  { const int rc = check_polarization_feed_down_args(pdg, spin_parity, n_chosen, chosen, gr, dimension, sums); if (rc) return rc; }
+  if (!weak) return fail(IS3D_ERR_ARGUMENT, "NULL weak decay table");
+  if (weak->n < 0) return fail(IS3D_ERR_ARGUMENT, "weak decay table with n < 0");
+  if (weak->n > 0 && (!weak->parent || !weak->daughter || !weak->partner || !weak->branching || !weak->alpha || !weak->phi))
+    return fail(IS3D_ERR_ARGUMENT, "NULL row array in the weak decay table");
+  { std::string err; const int rc = check_weak_decays(pdg, weak, &err); if (rc) return fail(rc, err.c_str()); }
+  return polarization_feed_down_call(gr, n_chosen, opt_in, sums, stats, [&](double *dev, int64_t n_bins, cudaStream_t st, int *launches, std::string *err) {
+    return polarization_weak_decays_device(pdg, spin_parity->spin2, weak, n_chosen, chosen, gr, dimension, dev, n_bins, st, launches, err);
+  });
+}
+
+// Feed-down of the spin-polarization sums through 2-body decays (cf_decays.cu).  Like is3d_b200_resonance_decays it works on a device
+// copy of all five arrays, so an error leaves the caller's arrays untouched.
+extern "C" int is3d_b200_polarization_decays(const is3d_particle_list *pdg, const is3d_spin_parity *spin_parity, int32_t n_chosen,
+                                             const int32_t *chosen, const is3d_grid *gr, int32_t dimension, const is3d_options *opt_in,
+                                             is3d_polarization_result *sums, is3d_stats *stats)
+{
+  { const int rc = check_polarization_feed_down_args(pdg, spin_parity, n_chosen, chosen, gr, dimension, sums); if (rc) return rc; }
+  return polarization_feed_down_call(gr, n_chosen, opt_in, sums, stats, [&](double *dev, int64_t n_bins, cudaStream_t st, int *launches, std::string *err) {
+    return polarization_decays_device(pdg, spin_parity->spin2, spin_parity->parity, n_chosen, chosen, gr, dimension, dev, n_bins, st, launches, err);
+  });
 }
 
 // =====================================================================================================================

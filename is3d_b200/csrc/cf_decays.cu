@@ -22,6 +22,7 @@
 #include <cmath>
 #include <cstring>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 namespace is3d {
@@ -274,10 +275,17 @@ struct SpinCtx {
   int dim;
 };
 
+// Weak-decay feed-down (is3d_b200_polarization_weak_decays): the Lee-Yang law of 1/2 -> 1/2 + 0 in place of (a, b).  a and b are unused.
+struct WeakCtx : SpinCtx {
+  double alpha, beta, gamma;     // decay parameters of the term
+};
+
 // Spin four-vector S_D (lab) of the daughter at one integrand point: parent P = (MT cosh Y, PT cos Phi, PT sin Phi, MT sinh Y) with
 // rest-frame spin Sp (2+1D: Sp is the y = 0 table value, its four-vector is boosted longitudinally by Y first), p* = L(P)^-1 p,
 // n = p*/|p*|, s* = a Sp + b (Sp.n) n in the daughter's rest frame, then back through L(P).  All boosts are pure boosts.
-__device__ __forceinline__ void daughter_spin(const SpinCtx &c, double MT, double PT, double Phi, const double Sp[3], double out[4])
+// WeakCtx: s* is the Lee-Yang numerator (alpha/2 + Sp.n) n + beta Sp x n + gamma (Sp - (Sp.n) n), and *yield = 1 + 2 alpha Sp.n.
+template <class Ctx>
+__device__ __forceinline__ void daughter_spin(const Ctx &c, double MT, double PT, double Phi, const double Sp[3], double out[4], double *yield = nullptr)
 {
   const double M = c.M, chY = cosh(c.Y), shY = sinh(c.Y);
   const double Px = PT * cos(Phi), Py = PT * sin(Phi), Pz = MT * shY, EP = MT * chY;
@@ -296,7 +304,15 @@ __device__ __forceinline__ void daughter_spin(const SpinCtx &c, double MT, doubl
   const double ip = 1.0 / sqrt(ps[0] * ps[0] + ps[1] * ps[1] + ps[2] * ps[2]);
   const double n[3] = {ps[0] * ip, ps[1] * ip, ps[2] * ip};
   const double Sn = S[0] * n[0] + S[1] * n[1] + S[2] * n[2];
-  const double s[3] = {c.a * S[0] + c.b * Sn * n[0], c.a * S[1] + c.b * Sn * n[1], c.a * S[2] + c.b * Sn * n[2]};
+  double s[3];
+  if constexpr (std::is_same<Ctx, WeakCtx>::value) {
+    const double l = 0.5 * c.alpha + Sn;
+    const double x[3] = {S[1] * n[2] - S[2] * n[1], S[2] * n[0] - S[0] * n[2], S[0] * n[1] - S[1] * n[0]};    // Sp x n
+    for (int k = 0; k < 3; k++) s[k] = l * n[k] + c.beta * x[k] + c.gamma * (S[k] - Sn * n[k]);
+    *yield = 1.0 + 2.0 * c.alpha * Sn;
+  } else {
+    s[0] = c.a * S[0] + c.b * Sn * n[0]; s[1] = c.a * S[1] + c.b * Sn * n[1]; s[2] = c.a * S[2] + c.b * Sn * n[2];
+  }
   const double pss = ps[0] * s[0] + ps[1] * s[1] + ps[2] * s[2];
   const double q0 = pss / c.mD, kq = pss / (c.mD * (pst + c.mD));
   const double q[3] = {s[0] + kq * ps[0], s[1] + kq * ps[1], s[2] + kq * ps[2]};
@@ -307,11 +323,12 @@ __device__ __forceinline__ void daughter_spin(const SpinCtx &c, double MT, doubl
 }
 
 // zeta integral at fixed (v [, s]): the innermost loop of the four integration routines (:588-628, 753-784, 1183-1213, 1352-1380).
-// SPIN: instead, zs[mu] += w_zeta MT (exp(log dN_1) S_D^mu(Phi_1) + exp(log dN_2) S_D^mu(Phi_2)) at the same points.
-template <bool SPIN>
+// SPIN: instead, zs[mu] += w_zeta MT (exp(log dN_1) S_D^mu(Phi_1) + exp(log dN_2) S_D^mu(Phi_2)) at the same points; with a WeakCtx also
+// zs[4] += w_zeta MT (exp(log dN_1) yield(Phi_1) + exp(log dN_2) yield(Phi_2)).
+template <bool SPIN, class Ctx = SpinCtx>
 __device__ double zeta_integral_at(const ParentView &P, double MTbar, double DeltaMT, double mTc_over_pT, double Estar_M_over_pT, double parent_mass2,
                                    double phip, int dim, bool cutoff_Y, int iYL, int iYR, double YL, double YR, double Y,
-                                   const SpinCtx *sc = nullptr, double *zs = nullptr)
+                                   const Ctx *sc = nullptr, double *zs = nullptr)
 {
   const double two_Pi = 2.0 * M_PI;
   double zeta_integral = 0.0;
@@ -330,10 +347,19 @@ __device__ double zeta_integral_at(const ParentView &P, double MTbar, double Del
       if (dim == 2) parent_2d<true>(P, MT, Phip_1, Phip_2, sc->Sstar, &so);
       else parent_3d<true>(P, iYL, iYR, YL, YR, MT, Phip_1, Phip_2, Y, sc->Sstar, &so);
       double S1[4], S2[4];
-      daughter_spin(*sc, MT, PT, Phip_1, so.S1, S1);
-      daughter_spin(*sc, MT, PT, Phip_2, so.S2, S2);
-      const double w1 = MT * so.e1, w2 = MT * so.e2;
-      for (int mu = 0; mu < 4; mu++) zs[mu] += (kGLWeight[izeta] * (w1 * S1[mu] + w2 * S2[mu]));
+      if constexpr (std::is_same<Ctx, WeakCtx>::value) {
+        double y1, y2;
+        daughter_spin(*sc, MT, PT, Phip_1, so.S1, S1, &y1);
+        daughter_spin(*sc, MT, PT, Phip_2, so.S2, S2, &y2);
+        const double w1 = MT * so.e1, w2 = MT * so.e2;
+        for (int mu = 0; mu < 4; mu++) zs[mu] += (kGLWeight[izeta] * (w1 * S1[mu] + w2 * S2[mu]));
+        zs[4] += (kGLWeight[izeta] * (w1 * y1 + w2 * y2));
+      } else {
+        daughter_spin(*sc, MT, PT, Phip_1, so.S1, S1);
+        daughter_spin(*sc, MT, PT, Phip_2, so.S2, S2);
+        const double w1 = MT * so.e1, w2 = MT * so.e2;
+        for (int mu = 0; mu < 4; mu++) zs[mu] += (kGLWeight[izeta] * (w1 * S1[mu] + w2 * S2[mu]));
+      }
     } else {
       const double integrand = MT * (dim == 2 ? parent_2d<false>(P, MT, Phip_1, Phip_2) : parent_3d<false>(P, iYL, iYR, YL, YR, MT, Phip_1, Phip_2, Y));
       zeta_integral += (kGLWeight[izeta] * integrand);
@@ -470,6 +496,55 @@ __global__ void spin_add_kernel(DecayGrid G, const DecayTerm *__restrict__ terms
     if (!has_law[t]) continue;
     const int64_t k = (int64_t)terms[t].daughter + (int64_t)G.n_species * bin;
     for (int mu = 0; mu < 4; mu++) S[mu * n_total + k] += spin_scratch[((size_t)t * 4 + mu) * n_bins + bin];
+  }
+}
+
+// ---- weak-decay feed-down (is3d_b200_polarization_weak_decays)
+struct WeakLaw { double alpha, beta, gamma; };     // per term; only terms listed in weak_ids have one
+
+// one thread per (weak term with the Lee-Yang law, bin): weak_scratch[term][r][bin], r = N^t, N^x, N^y, N^z, Snorm: prefactor x the
+// integral of spectrum x (Lee-Yang numerator carried to the lab, and the yield 1 + 2 alpha S*_P.n)
+__global__ void __launch_bounds__(128) decay2_weak_kernel(DecayGrid G, const DecayTerm *__restrict__ terms, const WeakLaw *__restrict__ laws,
+                                                         const int *__restrict__ weak_ids, int n_weak, const double *__restrict__ logdN,
+                                                         const double *__restrict__ MT_all, const Fit *__restrict__ fit_all,
+                                                         const double *__restrict__ Sstar, double *__restrict__ weak_scratch)
+{
+  const int n_bins = G.n_pT * G.n_phi * G.y_pts;
+  const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (gid >= (int64_t)n_weak * n_bins) return;
+  const int it = (int)(gid / n_bins), bin = (int)(gid - (int64_t)it * n_bins);
+  const int term = weak_ids[it];
+  const DecayTerm T = terms[term];
+  const int ipT = bin % G.n_pT, iphip = (bin / G.n_pT) % G.n_phi, iy = bin / (G.n_pT * G.n_phi);
+  const ParentView P = parent_view(G, logdN, MT_all, fit_all, term);
+  TWO_BODY_BIN_SETUP
+  WeakCtx sc;
+  sc.Sstar = Sstar; sc.a = 0.0; sc.b = 0.0; sc.M = mass_parent; sc.mD = sqrt(T.mass2); sc.dim = G.dim;
+  sc.alpha = laws[term].alpha; sc.beta = laws[term].beta; sc.gamma = laws[term].gamma;
+  sc.E = mT * cosh(y); sc.px = pT * cos(phip); sc.py = pT * sin(phip); sc.pz = mT * sinh(y);
+  double acc[5] = {0.0, 0.0, 0.0, 0.0, 0.0};
+  for (int iv = 0; iv < GP; iv++) {
+    TWO_BODY_V_NODE
+    sc.Y = y + v * DeltaY;
+    double zs[5] = {0.0, 0.0, 0.0, 0.0, 0.0};
+    zeta_integral_at<true, WeakCtx>(P, MTbar, DeltaMT, mTc, Estar_M_over_pT, parent_mass2, phip, G.dim, cutoff_Y, iYL, iYR, YL, YR, Y, &sc, zs);
+    for (int r = 0; r < 5; r++) acc[r] += (vw * zs[r]);
+  }
+  for (int r = 0; r < 5; r++) weak_scratch[((size_t)term * 5 + r) * n_bins + bin] = T.prefactor * acc[r];
+}
+
+// terms in row order: a term with the law adds its five rows to [St | Sx | Sy | Sz | Snorm] of the daughter, any other term its
+// plain integral (scratch, decay2_kernel) to Snorm
+__global__ void weak_add_kernel(DecayGrid G, const DecayTerm *__restrict__ terms, const int *__restrict__ has_law, int n_terms,
+                                const double *__restrict__ scratch, const double *__restrict__ weak_scratch, double *__restrict__ S, int64_t n_total)
+{
+  const int n_bins = G.n_pT * G.n_phi * G.y_pts;
+  const int bin = blockIdx.x * blockDim.x + threadIdx.x;
+  if (bin >= n_bins) return;
+  for (int t = 0; t < n_terms; t++) {
+    const int64_t k = (int64_t)terms[t].daughter + (int64_t)G.n_species * bin;
+    if (has_law[t]) for (int r = 0; r < 5; r++) S[r * n_total + k] += weak_scratch[((size_t)t * 5 + r) * n_bins + bin];
+    else S[4 * n_total + k] += scratch[(size_t)t * n_bins + bin];
   }
 }
 
@@ -610,6 +685,100 @@ bool transfer_law(const is3d_particle_list *pdg, const int32_t *spin2, const int
   return true;
 }
 
+// the set-up half of two_body_decay for one daughter group (:296-460): daughter = its chosen index, members = its multiplicity in the
+// channel, mass_secondary = the mass of the channel's second product (the recoil mass for either daughter, :411-413)
+DecayTerm two_body_term(int daughter, int members, double mass_parent, double mass, double mass_secondary, double branch_ratio)
+{
+  DecayTerm T; memset(&T, 0, sizeof(T));
+  T.body = 2; T.daughter = daughter;
+  const double W2 = mass_secondary * mass_secondary;
+  const double Estar = (mass_parent * mass_parent + mass * mass - W2) / (2.0 * mass_parent);
+  T.mass_parent = mass_parent; T.mass2 = mass * mass; T.Estar = Estar; T.pstar = std::sqrt(Estar * Estar - mass * mass);
+  T.prefactor = (double)members * mass_parent * branch_ratio / (8.0 * T.pstar);
+  return T;
+}
+
+bool ck(cudaError_t e, const char *what, std::string *err)
+{
+  if (e != cudaSuccess) { *err = std::string(what) + ": " + cudaGetErrorString(e); return false; }
+  return true;
+}
+
+// device buffers of one feed-down call, freed on every path out of the driver
+struct DecayBuffers {
+  double *tables = nullptr, *logdN = nullptr, *MT = nullptr, *scratch = nullptr; Fit *fit = nullptr; DecayTerm *terms = nullptr; int *ids = nullptr, *error = nullptr;
+  double *Sstar = nullptr, *spin_scratch = nullptr; SpinLaw *laws = nullptr; int *spin_ids = nullptr;
+  WeakLaw *weak_laws = nullptr; double *weak_scratch = nullptr;
+  ~DecayBuffers() { cudaFree(tables); cudaFree(logdN); cudaFree(MT); cudaFree(scratch); cudaFree(fit); cudaFree(terms); cudaFree(ids); cudaFree(error);
+                    cudaFree(Sstar); cudaFree(spin_scratch); cudaFree(laws); cudaFree(spin_ids); cudaFree(weak_laws); cudaFree(weak_scratch); }
+};
+
+// G from the grid, the buffers every driver needs for up to max_terms terms per parent, the momentum tables uploaded and the tail-fit
+// flag cleared on st
+int decay_setup(const is3d_grid *gr, int dimension, int n_chosen, int max_terms, DecayGrid *Gp, DecayBuffers *B, cudaStream_t st, std::string *err)
+{
+  DecayGrid &G = *Gp; memset(&G, 0, sizeof(G));
+  G.n_species = n_chosen; G.n_pT = gr->n_pT; G.n_phi = gr->n_phi; G.n_y_tab = gr->n_y; G.dim = dimension;
+  G.y_pts = (dimension == 2) ? 1 : gr->n_y;
+  if (G.n_pT < 2 || G.n_phi < 2 || (dimension == 3 && G.y_pts < 2)) { *err = "momentum tables too short for the interpolation"; return IS3D_ERR_ARGUMENT; }
+  const int n_bins = G.n_pT * G.n_phi * G.y_pts;
+  if (!ck(cudaMalloc(&B->tables, sizeof(double) * (size_t)(G.n_pT + G.n_phi + G.n_y_tab + 8)), "cudaMalloc", err) ||
+      !ck(cudaMalloc(&B->logdN, sizeof(double) * (size_t)n_bins), "cudaMalloc", err) ||
+      !ck(cudaMalloc(&B->MT, sizeof(double) * (size_t)max_terms * G.n_pT), "cudaMalloc", err) ||
+      !ck(cudaMalloc(&B->fit, sizeof(Fit) * (size_t)max_terms * G.y_pts * G.n_phi), "cudaMalloc", err) ||
+      !ck(cudaMalloc(&B->scratch, sizeof(double) * (size_t)max_terms * n_bins), "cudaMalloc", err) ||
+      !ck(cudaMalloc(&B->terms, sizeof(DecayTerm) * (size_t)max_terms), "cudaMalloc", err) ||
+      !ck(cudaMalloc(&B->ids, sizeof(int) * (size_t)max_terms * 2), "cudaMalloc", err) ||
+      !ck(cudaMalloc(&B->error, sizeof(int)), "cudaMalloc", err)) return IS3D_ERR_CUDA;
+  if (!ck(cudaMemcpyAsync(B->tables, gr->pT, sizeof(double) * G.n_pT, cudaMemcpyHostToDevice, st), "H2D", err) ||
+      !ck(cudaMemcpyAsync(B->tables + G.n_pT, gr->phi, sizeof(double) * G.n_phi, cudaMemcpyHostToDevice, st), "H2D", err) ||
+      !ck(cudaMemcpyAsync(B->tables + G.n_pT + G.n_phi, gr->y, sizeof(double) * G.n_y_tab, cudaMemcpyHostToDevice, st), "H2D", err) ||
+      !ck(cudaMemsetAsync(B->error, 0, sizeof(int), st), "memset", err)) return IS3D_ERR_CUDA;
+  G.pT = B->tables; G.phi = B->tables + G.n_pT; G.y = B->tables + G.n_pT + G.n_phi;
+  return IS3D_OK;
+}
+
+// the tail-fit flag of decay_setup_kernel, read after the stream is done
+int decay_tail_fit_status(const DecayBuffers &B, cudaStream_t st, std::string *err)
+{
+  int flag = 0;
+  if (!ck(cudaMemcpyAsync(&flag, B.error, sizeof(int), cudaMemcpyDeviceToHost, st), "D2H", err) || !ck(cudaStreamSynchronize(st), "sync", err)) return IS3D_ERR_CUDA;
+  if (flag) { *err = "not enough positive points of a parent spectrum beyond mT = 1.65 M to fit its large-mT tail (the reference exits here)"; return IS3D_ERR_ARGUMENT; }
+  return IS3D_OK;
+}
+
+// the rows of a weak-decay table with particle-list indices and (alpha, beta, gamma), or IS3D_ERR_ARGUMENT for a table the entry point rejects
+struct WeakRow { int parent, daughter, partner; double br; WeakLaw law; };
+int weak_rows(const is3d_particle_list *pdg, const is3d_weak_decays *weak, std::vector<WeakRow> *out, std::string *err)
+{
+  const int n_rows = weak->n;
+  std::vector<WeakRow> &rows = *out;
+  rows.assign((size_t)n_rows, WeakRow());
+  std::vector<double> br_sum((size_t)pdg->n_particles, 0.0);
+  for (int r = 0; r < n_rows; r++) {
+    WeakRow &R = rows[r];
+    const int32_t ids[3] = {weak->parent[r], weak->daughter[r], weak->partner[r]};
+    int *const idx[3] = {&R.parent, &R.daughter, &R.partner};
+    for (int k = 0; k < 3; k++) {
+      *idx[k] = -1;
+      for (int i = 0; i < pdg->n_particles && ids[k] != 0; i++) if (pdg->mcid[i] == ids[k]) { *idx[k] = i; break; }
+      if (*idx[k] < 0) { *err = "weak decay row " + std::to_string(r) + ": MC id " + std::to_string(ids[k]) + " is not in the particle list"; return IS3D_ERR_ARGUMENT; }
+    }
+    const std::string at = "weak decay row " + std::to_string(r) + ": ";
+    if (!pdg->stable[R.parent] || !pdg->stable[R.daughter]) { *err = at + "parent and daughter must be stable in the particle list"; return IS3D_ERR_ARGUMENT; }
+    const double br = weak->branching[r], alpha = weak->alpha[r], phi = weak->phi[r];
+    if (!(br >= 0.0 && br <= 1.0)) { *err = at + "branching ratio outside [0, 1]"; return IS3D_ERR_ARGUMENT; }
+    if (!std::isfinite(alpha) || !std::isfinite(phi) || std::fabs(alpha) > 1.0) { *err = at + "alpha must be finite with |alpha| <= 1, phi finite"; return IS3D_ERR_ARGUMENT; }
+    if (pdg->mass[R.daughter] + pdg->mass[R.partner] >= pdg->mass[R.parent]) { *err = at + "m_daughter + m_partner >= m_parent"; return IS3D_ERR_ARGUMENT; }
+    R.br = br;
+    br_sum[R.parent] += br;
+    if (br_sum[R.parent] > 1.0 + 1e-9) { *err = at + "the branching ratios of its parent sum to more than 1"; return IS3D_ERR_ARGUMENT; }
+    const double t = std::sqrt(1.0 - alpha * alpha);
+    R.law = WeakLaw{alpha, t * std::sin(phi), t * std::cos(phi)};
+  }
+  return IS3D_OK;
+}
+
 }  // namespace
 
 // Polarization feed-down inputs of decays_core: 2J and parity per particle-list entry, and the length of each of the five arrays.
@@ -622,40 +791,17 @@ static int decays_core(const is3d_particle_list *pdg, int n_chosen, const int32_
                        double *dN_dev, const SpinFeedDown *spin, cudaStream_t st, int *launches, std::string *err)
 {
   if (n_chosen - 1 <= 0) { *err = "need at least two chosen particles for the resonance decay routine"; return IS3D_ERR_ARGUMENT; }
-  DecayGrid G; memset(&G, 0, sizeof(G));
-  G.n_species = n_chosen; G.n_pT = gr->n_pT; G.n_phi = gr->n_phi; G.n_y_tab = gr->n_y; G.dim = dimension;
-  G.y_pts = (dimension == 2) ? 1 : gr->n_y;
-  if (G.n_pT < 2 || G.n_phi < 2 || (dimension == 3 && G.y_pts < 2)) { *err = "momentum tables too short for the interpolation"; return IS3D_ERR_ARGUMENT; }
+  const int max_terms = 50 * 3;                       // <= 50 channels per particle (readindata.h Maxdecaychannel) x 3 daughter groups
+  DecayGrid G; DecayBuffers B;
+  { const int rc = decay_setup(gr, dimension, n_chosen, max_terms, &G, &B, st, err); if (rc != IS3D_OK) return rc; }
   const int n_bins = G.n_pT * G.n_phi * G.y_pts;
   Host H{pdg, n_chosen, chosen};
-
-  // device buffers (freed on every path out of this function)
-  struct Buffers {
-    double *tables = nullptr, *logdN = nullptr, *MT = nullptr, *scratch = nullptr; Fit *fit = nullptr; DecayTerm *terms = nullptr; int *ids = nullptr, *error = nullptr;
-    double *Sstar = nullptr, *spin_scratch = nullptr; SpinLaw *laws = nullptr; int *spin_ids = nullptr;
-    ~Buffers() { cudaFree(tables); cudaFree(logdN); cudaFree(MT); cudaFree(scratch); cudaFree(fit); cudaFree(terms); cudaFree(ids); cudaFree(error);
-                 cudaFree(Sstar); cudaFree(spin_scratch); cudaFree(laws); cudaFree(spin_ids); }
-  } B;
-  const int max_terms = 50 * 3;                       // <= 50 channels per particle (readindata.h Maxdecaychannel) x 3 daughter groups
-  auto ck = [&](cudaError_t e, const char *what) { if (e != cudaSuccess) { *err = std::string(what) + ": " + cudaGetErrorString(e); return false; } return true; };
-  if (!ck(cudaMalloc(&B.tables, sizeof(double) * (size_t)(G.n_pT + G.n_phi + G.n_y_tab + 8)), "cudaMalloc") ||
-      !ck(cudaMalloc(&B.logdN, sizeof(double) * (size_t)n_bins), "cudaMalloc") ||
-      !ck(cudaMalloc(&B.MT, sizeof(double) * (size_t)max_terms * G.n_pT), "cudaMalloc") ||
-      !ck(cudaMalloc(&B.fit, sizeof(Fit) * (size_t)max_terms * G.y_pts * G.n_phi), "cudaMalloc") ||
-      !ck(cudaMalloc(&B.scratch, sizeof(double) * (size_t)max_terms * n_bins), "cudaMalloc") ||
-      !ck(cudaMalloc(&B.terms, sizeof(DecayTerm) * (size_t)max_terms), "cudaMalloc") ||
-      !ck(cudaMalloc(&B.ids, sizeof(int) * (size_t)max_terms * 2), "cudaMalloc") ||
-      !ck(cudaMalloc(&B.error, sizeof(int)), "cudaMalloc")) return IS3D_ERR_CUDA;
+  auto ck = [&](cudaError_t e, const char *what) { return is3d::ck(e, what, err); };
   if (spin && (!ck(cudaMalloc(&B.Sstar, sizeof(double) * 3 * (size_t)n_bins), "cudaMalloc") ||
                !ck(cudaMalloc(&B.spin_scratch, sizeof(double) * 4 * (size_t)max_terms * n_bins), "cudaMalloc") ||
                !ck(cudaMalloc(&B.laws, sizeof(SpinLaw) * (size_t)max_terms), "cudaMalloc") ||
                !ck(cudaMalloc(&B.spin_ids, sizeof(int) * (size_t)max_terms * 2), "cudaMalloc"))) return IS3D_ERR_CUDA;
   double *const dN_spec = spin ? dN_dev + 4 * spin->n_total : dN_dev;       // the array the spectra feed-down amends
-  if (!ck(cudaMemcpyAsync(B.tables, gr->pT, sizeof(double) * G.n_pT, cudaMemcpyHostToDevice, st), "H2D") ||
-      !ck(cudaMemcpyAsync(B.tables + G.n_pT, gr->phi, sizeof(double) * G.n_phi, cudaMemcpyHostToDevice, st), "H2D") ||
-      !ck(cudaMemcpyAsync(B.tables + G.n_pT + G.n_phi, gr->y, sizeof(double) * G.n_y_tab, cudaMemcpyHostToDevice, st), "H2D") ||
-      !ck(cudaMemsetAsync(B.error, 0, sizeof(int), st), "memset")) return IS3D_ERR_CUDA;
-  G.pT = B.tables; G.phi = B.tables + G.n_pT; G.y = B.tables + G.n_pT + G.n_phi;
 
   for (int ichosen = n_chosen - 1; ichosen > 0; ichosen--) {
     const int ipart = chosen[ichosen];
@@ -684,16 +830,9 @@ static int decays_core(const is3d_particle_list *pdg, int n_chosen, const int32_
         }
         const int ng = H.group(idx, 2, groups, members);
         for (int gi = 0; gi < ng; gi++) {
-          DecayTerm T; memset(&T, 0, sizeof(T));
-          T.body = 2; T.daughter = H.chosen_index(groups[gi], err);
-          if (T.daughter < 0) return IS3D_ERR_ARGUMENT;
-          const double mass = pdg->mass[groups[gi]];
-          const double mass_secondary = pdg->mass[idx[1]];                      // always the second product (:411-413)
-          const double W2 = mass_secondary * mass_secondary;
-          const double Estar = (mass_parent * mass_parent + mass * mass - W2) / (2.0 * mass_parent);
-          T.mass_parent = mass_parent; T.mass2 = mass * mass; T.Estar = Estar; T.pstar = std::sqrt(Estar * Estar - mass * mass);
-          T.prefactor = (double)members[gi] * mass_parent * branch_ratio / (8.0 * T.pstar);
-          terms.push_back(T);
+          const int daughter = H.chosen_index(groups[gi], err);
+          if (daughter < 0) return IS3D_ERR_ARGUMENT;
+          terms.push_back(two_body_term(daughter, members[gi], mass_parent, pdg->mass[groups[gi]], pdg->mass[idx[1]], branch_ratio));
           SpinLaw L{0.0, 0.0};
           has_law.push_back(spin && transfer_law(pdg, spin->spin2, spin->parity, ipart, groups[gi], idx[0] == groups[gi] ? idx[1] : idx[0], &L.a, &L.b));
           laws.push_back(L);
@@ -764,10 +903,7 @@ static int decays_core(const is3d_particle_list *pdg, int n_chosen, const int32_
     // the term list of the next parent reuses B.terms: the stream must be done with it (also surfaces kernel faults per parent)
     if (!ck(cudaStreamSynchronize(st), "decay kernels")) return IS3D_ERR_CUDA;
   }
-  int flag = 0;
-  if (!ck(cudaMemcpyAsync(&flag, B.error, sizeof(int), cudaMemcpyDeviceToHost, st), "D2H") || !ck(cudaStreamSynchronize(st), "sync")) return IS3D_ERR_CUDA;
-  if (flag) { *err = "not enough positive points of a parent spectrum beyond mT = 1.65 M to fit its large-mT tail (the reference exits here)"; return IS3D_ERR_ARGUMENT; }
-  return IS3D_OK;
+  return decay_tail_fit_status(B, st, err);
 }
 
 int resonance_decays_device(const is3d_particle_list *pdg, int n_chosen, const int32_t *chosen, const is3d_grid *gr, int dimension,
@@ -782,6 +918,92 @@ int polarization_decays_device(const is3d_particle_list *pdg, const int32_t *spi
 {
   const SpinFeedDown spin{spin2, parity, n_total};
   return decays_core(pdg, n_chosen, chosen, gr, dimension, S_dev, &spin, st, launches, err);
+}
+
+int check_weak_decays(const is3d_particle_list *pdg, const is3d_weak_decays *weak, std::string *err)
+{
+  std::vector<WeakRow> rows;
+  return weak_rows(pdg, weak, &rows, err);
+}
+
+// Weak-decay feed-down of the five arrays (is3d_b200_polarization_weak_decays, DESIGN §20): the rows of `weak` (rejected as by
+// check_weak_decays before any device work); weak parents that are chosen species in descending mass (ties: descending chosen index), each with the 2-body set-up,
+// tables and fixed-order add of decays_core.  Terms with the Lee-Yang law (2J = 1, 1, 0) go through decay2_weak_kernel, the others feed
+// Snorm through decay2_kernel.
+int polarization_weak_decays_device(const is3d_particle_list *pdg, const int32_t *spin2, const is3d_weak_decays *weak, int n_chosen,
+                                    const int32_t *chosen, const is3d_grid *gr, int dimension, double *S_dev, int64_t n_total, cudaStream_t st,
+                                    int *launches, std::string *err)
+{
+  Host H{pdg, n_chosen, chosen};
+  std::vector<WeakRow> rows;
+  { const int rc = weak_rows(pdg, weak, &rows, err); if (rc != IS3D_OK) return rc; }
+  // weak parents among the chosen species, heaviest first: a parent's arrays are final when its turn comes
+  std::vector<int> order;
+  int max_terms = 1;
+  for (int ic = 0; ic < n_chosen; ic++) {
+    int nt = 0;
+    for (const WeakRow &R : rows) if (R.parent == chosen[ic] && H.chosen_index(R.daughter, err) >= 0) nt++;
+    if (nt > 0) { order.push_back(ic); max_terms = std::max(max_terms, nt); }
+  }
+  err->clear();
+  if (order.empty()) return IS3D_OK;
+  std::sort(order.begin(), order.end(), [&](int a, int b) {
+    const double ma = pdg->mass[chosen[a]], mb = pdg->mass[chosen[b]];
+    return ma != mb ? ma > mb : a > b;
+  });
+  DecayGrid G; DecayBuffers B;
+  { const int rc = decay_setup(gr, dimension, n_chosen, max_terms, &G, &B, st, err); if (rc != IS3D_OK) return rc; }
+  const int n_bins = G.n_pT * G.n_phi * G.y_pts;
+  auto ck = [&](cudaError_t e, const char *what) { return is3d::ck(e, what, err); };
+  if (!ck(cudaMalloc(&B.Sstar, sizeof(double) * 3 * (size_t)n_bins), "cudaMalloc") ||
+      !ck(cudaMalloc(&B.weak_scratch, sizeof(double) * 5 * (size_t)max_terms * n_bins), "cudaMalloc") ||
+      !ck(cudaMalloc(&B.weak_laws, sizeof(WeakLaw) * (size_t)max_terms), "cudaMalloc") ||
+      !ck(cudaMalloc(&B.spin_ids, sizeof(int) * (size_t)max_terms * 2), "cudaMalloc")) return IS3D_ERR_CUDA;
+  double *const Snorm = S_dev + 4 * n_total;
+  for (const int ichosen : order) {
+    const int ipart = chosen[ichosen];
+    std::vector<DecayTerm> terms;
+    std::vector<WeakLaw> laws;
+    std::vector<int> has_law, plain_ids, law_ids;
+    for (const WeakRow &R : rows) {
+      if (R.parent != ipart) continue;
+      const int daughter = H.chosen_index(R.daughter, err);
+      if (daughter < 0) { err->clear(); continue; }
+      const int t = (int)terms.size();
+      terms.push_back(two_body_term(daughter, R.partner == R.daughter ? 2 : 1, pdg->mass[ipart], pdg->mass[R.daughter], pdg->mass[R.partner], R.br));
+      laws.push_back(R.law);
+      const bool law = spin2[ipart] == 1 && spin2[R.daughter] == 1 && spin2[R.partner] == 0;
+      has_law.push_back(law);
+      (law ? law_ids : plain_ids).push_back(t);
+    }
+    const int n_law = (int)law_ids.size();
+    law_ids.insert(law_ids.end(), has_law.begin(), has_law.end());          // the terms with the law, then the has_law flags
+    if (!ck(cudaMemcpyAsync(B.terms, terms.data(), sizeof(DecayTerm) * terms.size(), cudaMemcpyHostToDevice, st), "H2D") ||
+        !ck(cudaMemcpyAsync(B.weak_laws, laws.data(), sizeof(WeakLaw) * laws.size(), cudaMemcpyHostToDevice, st), "H2D") ||
+        !ck(cudaMemcpyAsync(B.spin_ids, law_ids.data(), sizeof(int) * law_ids.size(), cudaMemcpyHostToDevice, st), "H2D") ||
+        (!plain_ids.empty() && !ck(cudaMemcpyAsync(B.ids, plain_ids.data(), sizeof(int) * plain_ids.size(), cudaMemcpyHostToDevice, st), "H2D")))
+      return IS3D_ERR_CUDA;
+    log_parent_kernel<<<(n_bins + 255) / 256, 256, 0, st>>>(G, Snorm, ichosen, B.logdN);
+    decay_setup_kernel<<<(unsigned)terms.size(), 128, 0, st>>>(G, B.terms, B.logdN, B.MT, B.fit, B.error);
+    spin_table_kernel<<<(n_bins + 255) / 256, 256, 0, st>>>(G, S_dev, n_total, ichosen, pdg->mass[ipart], B.Sstar);
+    *launches += 3;
+    if (!plain_ids.empty()) {
+      const int64_t n = (int64_t)plain_ids.size() * n_bins;
+      decay2_kernel<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(G, B.terms, B.ids, (int)plain_ids.size(), B.logdN, B.MT, B.fit, B.scratch);
+      (*launches)++;
+    }
+    if (n_law > 0) {
+      const int64_t n = (int64_t)n_law * n_bins;
+      decay2_weak_kernel<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(G, B.terms, B.weak_laws, B.spin_ids, n_law, B.logdN, B.MT, B.fit, B.Sstar,
+                                                                     B.weak_scratch);
+      (*launches)++;
+    }
+    weak_add_kernel<<<(n_bins + 255) / 256, 256, 0, st>>>(G, B.terms, B.spin_ids + n_law, (int)terms.size(), B.scratch, B.weak_scratch, S_dev, n_total);
+    (*launches)++;
+    if (!ck(cudaGetLastError(), "weak decay kernels")) return IS3D_ERR_CUDA;
+    if (!ck(cudaStreamSynchronize(st), "weak decay kernels")) return IS3D_ERR_CUDA;
+  }
+  return decay_tail_fit_status(B, st, err);
 }
 
 }  // namespace is3d

@@ -114,6 +114,11 @@ int resonance_decays_device(const is3d_particle_list *pdg, int n_chosen, const i
 // (host) per particle-list entry
 int polarization_decays_device(const is3d_particle_list *pdg, const int32_t *spin2, const int32_t *parity, int n_chosen, const int32_t *chosen,
                                const is3d_grid *gr, int dimension, double *S_dev, int64_t n_total, cudaStream_t st, int *launches, std::string *err);
+// weak-decay feed-down of the same five arrays (cf_decays.cu); check_weak_decays: the table's argument errors (host only, no device work)
+int check_weak_decays(const is3d_particle_list *pdg, const is3d_weak_decays *weak, std::string *err);
+int polarization_weak_decays_device(const is3d_particle_list *pdg, const int32_t *spin2, const is3d_weak_decays *weak, int n_chosen,
+                                    const int32_t *chosen, const is3d_grid *gr, int dimension, double *S_dev, int64_t n_total, cudaStream_t st,
+                                    int *launches, std::string *err);
 // strict (reference-order) diagnostic variant, df_mode 1 / 2 (cf_strict.cu); cell_scratch: n_cells * strict_cell_bytes()
 size_t strict_cell_bytes();
 cudaError_t launch_strict(const is3d_flags &fl, const RawCells &cells, const PrepTables &tab, const Layout &L, const double *mass, const double *sign,

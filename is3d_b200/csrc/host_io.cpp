@@ -3,6 +3,7 @@
 #include "host_math.h"
 #include <algorithm>
 #include <cctype>
+#include <cerrno>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -192,6 +193,37 @@ bool read_box_parities(const std::string &workdir, std::map<long, int> *out, std
   }
   out->clear();
   for (const Particle &p : box) if (p.parity != 0) out->emplace(std::labs(p.mcid), p.parity);       // first entry of an id wins
+  return true;
+}
+
+bool read_weak_decays(const std::string &workdir, WeakTable *out, std::string *err)
+{
+  const std::string path = workdir + "/PDG/weak_decays.dat";
+  std::ifstream f(path.c_str());
+  if (!f) { if (err) *err = "cannot open " + path + " (polarization_weak_decays = 1 reads it)"; return false; }
+  *out = WeakTable();
+  std::string line;
+  for (long n = 1; std::getline(f, line); n++) {
+    const size_t hash = line.find('#');
+    if (hash != std::string::npos) line.erase(hash);
+    std::istringstream ls(line);
+    std::string tok[7];
+    int nt = 0;
+    while (nt < 7 && ls >> tok[nt]) nt++;
+    if (nt == 0) continue;
+    long ids[3]; double v[3];
+    bool ok = (nt == 6);
+    for (int k = 0; ok && k < 6; k++) {
+      char *end = nullptr;
+      errno = 0;
+      if (k < 3) ids[k] = std::strtol(tok[k].c_str(), &end, 10);
+      else v[k - 3] = std::strtod(tok[k].c_str(), &end);
+      ok = end && *end == '\0' && errno == 0;
+    }
+    if (!ok) { if (err) *err = path + ": line " + std::to_string(n) + " is not `parent daughter partner branching alpha phi`"; return false; }
+    out->parent.push_back((int32_t)ids[0]); out->daughter.push_back((int32_t)ids[1]); out->partner.push_back((int32_t)ids[2]);
+    out->branching.push_back(v[0]); out->alpha.push_back(v[1]); out->phi.push_back(v[2]);
+  }
   return true;
 }
 

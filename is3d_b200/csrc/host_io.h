@@ -44,6 +44,10 @@ bool read_pdg(const std::string &workdir, int hrg_eos, std::vector<Particle> *ou
 // intrinsic parities by |MC id| from the PARITY column of PDG/pdg_box.dat (the polarization feed-down reads them next to a conventional
 // list); a missing file is an error, an id the file lacks is simply absent from the map
 bool read_box_parities(const std::string &workdir, std::map<long, int> *out, std::string *err);
+// PDG/weak_decays.dat (this project's own format): one weak channel per line, `parent_mcid daughter_mcid partner_mcid branching alpha phi`
+// (phi in radians), `#` starts a comment, blank lines are skipped.  A missing file or a line without exactly those six numbers is an error.
+struct WeakTable { std::vector<int32_t> parent, daughter, partner; std::vector<double> branching, alpha, phi; };
+bool read_weak_decays(const std::string &workdir, WeakTable *out, std::string *err);
 
 struct SurfaceData {
   int64_t n = 0;

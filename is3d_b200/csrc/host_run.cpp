@@ -182,7 +182,8 @@ static bool write_spacetime_files(const std::string &wd, const std::vector<int> 
 // With the sums of one more term xi (St | Sx | Sy | Sz | Snorm of is3d_b200_spin_polarization_shear or _spin_hall, non-NULL) it writes
 // S_<stem>_<mcid>.dat instead: Snorm, that term's part N_xi / Snorm (columns S?_<stem>), the total S = (N + N_xi) / Snorm and the
 // rest-frame part of the total.
-// stem: the file name stem of the plain form ("S"; "S_fd" for the sums after the feed-down through decays), or the tag of the term
+// stem: the file name stem of the plain form ("S"; "S_fd" for the sums after the feed-down through decays, "S_fdw" after the weak decays
+// too), or the tag of the term
 // ("xi" for the thermal shear, "she" for the spin Hall term).
 static bool write_polarization_files(const std::string &wd, const std::vector<double> &sums, const std::vector<double> *xi,
                                      const std::vector<int> &mcid, const std::vector<double> &mass, const Grids &g, int dimension,
@@ -350,6 +351,8 @@ struct Problem {
   int thermal_shear_polarization = 0;      // optional key (absent: 0): add the thermal-shear term (input/thermal_shear.dat)
   int spin_hall_polarization = 0;          // optional key (absent: 0): add the spin Hall term (input/muB_over_T_gradient.dat)
   int polarization_feed_down = 0;          // optional key (absent: 0): feed the polarization sums down through the decay tables
+  int polarization_weak_decays = 0;        // optional key (absent: 0): then through the weak decays of PDG/weak_decays.dat
+  WeakTable weak;                          // that table
   int spin_density = 0;                    // optional key (absent: 0): mode-5 spin density matrix (all-order spin, rank-2 tensor)
   std::map<long, int> box_parity;          // its parities by |MC id| (PDG/pdg_box.dat)
   int hbt_radii = 0;                       // optional key (absent: 0): HBT radii of the linear-delta-f spectra after the spectra
@@ -412,6 +415,10 @@ static int load_problem(const std::string &wd, bool need_surface, Problem *p, st
           "(hrg_eos = 1, 2)";
     return IS3D_ERR_UNSUPPORTED;
   }
+  p->polarization_weak_decays = par.has("polarization_weak_decays") ? (int)par.get("polarization_weak_decays", &err) : 0;
+  if (p->polarization_weak_decays && !p->polarization_feed_down) {
+    err = "polarization_weak_decays = 1 needs polarization_feed_down = 1 (it amends the fed-down sums)"; return IS3D_ERR_UNSUPPORTED;
+  }
   p->spin_density = par.has("spin_density") ? (int)par.get("spin_density", &err) : 0;
   if (p->spin_density && (p->operation != 1 || fl.mode != 5)) { err = "spin_density = 1 needs operation = 1 and a mode 5 surface (the thermal vorticity columns)"; return IS3D_ERR_UNSUPPORTED; }
   p->hbt_radii = par.has("hbt_radii") ? (int)par.get("hbt_radii", &err) : 0;
@@ -439,6 +446,7 @@ static int load_problem(const std::string &wd, bool need_surface, Problem *p, st
   // ---- particle list, delta-f tables
   if (!read_pdg(wd, p->hrg_eos, &p->pdg, &err)) return IS3D_ERR_IO;
   if (p->polarization_feed_down && !read_box_parities(wd, &p->box_parity, &err)) return IS3D_ERR_IO;
+  if (p->polarization_weak_decays && !read_weak_decays(wd, &p->weak, &err)) return IS3D_ERR_IO;
   if ((int)p->pdg.size() > 600) { err = "number of particles exceeds Maxparticle = 600"; return IS3D_ERR_IO; }
   if (!read_df_tables(wd, p->hrg_eos, &p->dft, &err)) return IS3D_ERR_IO;
   if (!read_laguerre(wd + "/tables/gla_roots_weights_32_points.txt", &p->gla, &err)) return IS3D_ERR_IO;
@@ -612,6 +620,17 @@ static int run_problem(const std::string &wd, Problem &P, const is3d_surface &s,
       if (rcf != IS3D_OK) { err = std::string("polarization feed-down failed: ") + is3d_b200_last_error(); return rcf; }
       if (stats) { stats->gpu_launches += fd_st.gpu_launches; stats->total_ms += fd_st.total_ms; }
       if (!write_polarization_files(wd, sums, nullptr, P.mcid, P.mass, g, P.fl.dimension, &err, "S_fd")) return IS3D_ERR_IO;
+      if (P.polarization_weak_decays) {               // the weak pass on a copy of the fed-down sums: S_fd_ stays as it is
+        std::vector<double> fdw(sums);
+        is3d_polarization_result rw{&fdw[0], &fdw[n_bins], &fdw[2 * n_bins], &fdw[3 * n_bins], &fdw[4 * n_bins]};
+        const is3d_weak_decays wt{(int32_t)P.weak.parent.size(), P.weak.parent.data(), P.weak.daughter.data(), P.weak.partner.data(),
+                                  P.weak.branching.data(), P.weak.alpha.data(), P.weak.phi.data()};
+        std::memset(&fd_st, 0, sizeof(fd_st));
+        const int rcw = is3d_b200_polarization_weak_decays(&pl, &spp, &wt, npart, chosen.data(), &gr, P.fl.dimension, nullptr, &rw, &fd_st);
+        if (rcw != IS3D_OK) { err = std::string("weak-decay polarization feed-down failed: ") + is3d_b200_last_error(); return rcw; }
+        if (stats) { stats->gpu_launches += fd_st.gpu_launches; stats->total_ms += fd_st.total_ms; }
+        if (!write_polarization_files(wd, fdw, nullptr, P.mcid, P.mass, g, P.fl.dimension, &err, "S_fdw")) return IS3D_ERR_IO;
+      }
     }
   }
   if (P.spin_density) {
@@ -789,6 +808,12 @@ extern "C" int is3d_b200_host_dump(const char *workdir, const char *out_path)
     tmp.clear();
     for (auto &h : P.pdg) { const auto it = P.box_parity.find(std::labs(h.mcid)); tmp.push_back(it == P.box_parity.end() ? 0 : it->second); }
     put("pdg_parity", tmp);
+  }
+  if (P.polarization_weak_decays) {      // the weak-decay table as read: one record per column
+    tmp.assign(P.weak.parent.begin(), P.weak.parent.end()); put("weak_parent", tmp);
+    tmp.assign(P.weak.daughter.begin(), P.weak.daughter.end()); put("weak_daughter", tmp);
+    tmp.assign(P.weak.partner.begin(), P.weak.partner.end()); put("weak_partner", tmp);
+    put("weak_branching", P.weak.branching); put("weak_alpha", P.weak.alpha); put("weak_phi", P.weak.phi);
   }
   tmp.assign(s.avg, s.avg + 5); put("avg", tmp);
   put("df_T", P.dft.T); put("df_c0", P.dft.c0); put("df_c2", P.dft.c2); put("df_F", P.dft.F); put("df_betabulk", P.dft.betabulk);

@@ -109,6 +109,27 @@ def spin_parity(fx, pdg, hrg_eos=1):
     return dict(spin2=spin2, parity=parity)
 
 
+def weak_decays(path):
+    """Read a weak-decay table (PDG/weak_decays.dat, this project's own format): one channel per line, `parent_mcid daughter_mcid
+    partner_mcid branching alpha phi` (phi in radians), `#` starts a comment.  Returns the dict of the six columns that
+    api.polarization_weak_decays takes; a malformed line raises ValueError (the host layer's IS3D_ERR_IO)."""
+    cols = {k: [] for k in ("parent", "daughter", "partner", "branching", "alpha", "phi")}
+    with open(path) as f:
+        for n, line in enumerate(f, 1):
+            tok = line.split("#", 1)[0].split()
+            if not tok:
+                continue
+            if len(tok) != 6:
+                raise ValueError("%s:%d: expected 6 columns, found %d" % (path, n, len(tok)))
+            ids = [int(t) for t in tok[:3]]
+            vals = [float(t) for t in tok[3:]]
+            for k, v in zip(cols, ids + vals):
+                cols[k].append(v)
+    return dict(parent=np.array(cols["parent"], np.int32), daughter=np.array(cols["daughter"], np.int32),
+                partner=np.array(cols["partner"], np.int32), branching=np.array(cols["branching"]), alpha=np.array(cols["alpha"]),
+                phi=np.array(cols["phi"]))
+
+
 def species(fx, hrg_eos=1, chosen="chosen_urqmd", group_particles=False):
     pdg = pdg_table(fx, hrg_eos)
     ids = fx[chosen] if isinstance(chosen, str) else np.asarray(chosen, dtype=np.int64)

@@ -32,7 +32,7 @@ DEFAULT_PARAMETERS = [
 ]
 
 # keys of this drop-in that the reference does not read: written only when a caller sets them (absent: 0, or the default of the host layer)
-OPTIONAL_PARAMETERS = ("spin_polarization", "thermal_shear_polarization", "spin_hall_polarization", "polarization_feed_down", "spin_density", "hbt_radii", "hbt_correlation", "hbt_dq",
+OPTIONAL_PARAMETERS = ("spin_polarization", "thermal_shear_polarization", "spin_hall_polarization", "polarization_feed_down", "polarization_weak_decays", "spin_density", "hbt_radii", "hbt_correlation", "hbt_dq",
                        "hbt_q_points")
 
 _EOS_DIR = {1: "urqmd", 2: "smash", 3: "smash_box"}
@@ -96,6 +96,14 @@ def _write_pdg_conventional(path, fx, key):
                 f.write("%9d %d %s %d %d %d %d %d\n" % (g("mcid")[i], dn[j], _r(br[j]), *parts[j]))
 
 
+def write_weak_decays(path, weak):
+    """PDG/weak_decays.dat: `parent daughter partner branching alpha phi` per line, after a comment line naming the columns."""
+    with open(path, "w") as f:
+        f.write("# parent_mcid daughter_mcid partner_mcid branching alpha phi[rad]\n")
+        for row in zip(*(np.atleast_1d(weak[k]) for k in ("parent", "daughter", "partner", "branching", "alpha", "phi"))):
+            f.write("%d %d %d %s %s %s\n" % (int(row[0]), int(row[1]), int(row[2]), _r(row[3]), _r(row[4]), _r(row[5])))
+
+
 def _write_pdg_box(path, fx):
     with open(path, "w", encoding="utf-8") as f:
         f.write("# NAME MASS[GEV] WIDTH[GEV] PARITY PDG\n\n")
@@ -129,7 +137,7 @@ def _write_df_vah(dirname, fx):
 
 
 def materialize(root, surface_columns=None, chosen=None, fixture=None, tables=None, vah=False, thermal_shear=None, baryon_gradient=None,
-                **params):
+                weak_decays=None, **params):
     """Create `root` as an iS3D working directory.
 
     surface_columns : (n_cells, n_cols) array in file units, or None for the shipped one-cell toy surface.
@@ -139,6 +147,8 @@ def materialize(root, surface_columns=None, chosen=None, fixture=None, tables=No
                       input/thermal_shear.dat (read when thermal_shear_polarization = 1).
     baryon_gradient : optional (n_cells, 4) array or dict of the four columns of synthetic.BARYON_GRADIENT_COLUMNS, written to
                       input/muB_over_T_gradient.dat (read when spin_hall_polarization = 1).
+    weak_decays     : optional dict of the six columns of tables.weak_decays (parent, daughter, partner, branching, alpha, phi), written
+                      to PDG/weak_decays.dat (read when polarization_weak_decays = 1).
     params          : iS3D_parameters.dat overrides (operation, mode, df_mode, dimension, ...).
     """
     fx = fixture if fixture is not None else load_fixture()
@@ -167,6 +177,8 @@ def materialize(root, surface_columns=None, chosen=None, fixture=None, tables=No
         _write_pdg_conventional(os.path.join(root, "PDG", fname), fx, key)
         if int(p.get("polarization_feed_down", 0)):
             _write_pdg_box(os.path.join(root, "PDG", "pdg_box.dat"), fx)     # the parities the polarization feed-down reads
+    if weak_decays is not None:
+        write_weak_decays(os.path.join(root, "PDG", "weak_decays.dat"), weak_decays)
     if chosen is None:
         chosen = "chosen_pikp"
     if isinstance(chosen, str):
