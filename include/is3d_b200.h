@@ -94,7 +94,9 @@ typedef struct {
   int32_t tile_variant;      /* kernel variant: 0 = tuned default for the model (df_mode 1 / 2 and ideal f_eq on 3+1D tiles with <= 64 pT
                                 points: shifted-factor kernel 23; everything else: cf_kernel); 1..16 = register-tile table of cf_kernel;
                                 17..21 = shapes of the factored kernel (df_mode 1/2, 3+1D, >= 16 species); 22..25 = shapes of the
-                                shifted-factor kernel (df_mode 1/2, 3+1D, <= 64 pT points); 99 = strict diagnostic kernel (df_mode 1/2 in
+                                shifted-factor kernel (df_mode 1/2, 3+1D, <= 64 pT points; slots x phi points 7 x 3, 3 x 6 (the
+                                default), 3 x 8, 7 x 6 for df_mode 1 and ideal f_eq; 7 x 2, 7 x 3 (the default), 7 x 4, 7 x 6
+                                for df_mode 2); 99 = strict diagnostic kernel (df_mode 1/2 in
                                 the reference's own operation order, one thread per bin: ~50x slower, tests only).  A variant that does
                                 not apply to the call returns IS3D_ERR_ARGUMENT. */
   int32_t reserved[4];

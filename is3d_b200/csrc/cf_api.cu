@@ -286,7 +286,8 @@ static int smooth_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_
   if (iq && iq->mode == 2 && !dim2) return fail(IS3D_ERR_ARGUMENT, "per-slot integration is a 2+1D pass");
   if (iq && (!iq->pT_weight || !iq->phi_weight)) return fail(IS3D_ERR_ARGUMENT, "pT / phi quadrature weights missing");
   // tile_variant: 0 = model default (tuned on B200, see profiles/), k > 0 = table entry k - 1 (tuning / tests).
-  // Defaults: linear-df models (and ideal f_eq) on 3+1D tiles with <= 64 pT points run cf_shift_kernel (tile_variant 23);
+  // Defaults: linear-df models (and ideal f_eq) on 3+1D tiles with <= 64 pT points run cf_shift_kernel (tile_variant 23: 3 slots x
+  // 6 phi points at 3 blocks/SM for 14-moment delta-f and ideal f_eq, 7 x 3 for Chapman-Enskog and Jonah linear);
   // modified equilibrium, the anisotropic model, 2+1D and operation = 0 run cf_kernel.
   // 17..21 = shapes of the factored kernel (cf_factored.cu; linear-df models on 3+1D tiles, >= 16 species): opt-in for the main
   // pass (measured within +-10 % of cf_kernel on B200, DESIGN.md section 6), always used for the sparse linear-branch pass of
@@ -295,7 +296,8 @@ static int smooth_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_
   int variant, fvariant = -1;
   const bool f_ok = factored_supported(model, L) && !iq;      // operation = 0 integrates over the pT lanes of a block (cf_kernel)
   const bool strict = (opt.tile_variant == kStrictVariant);
-  // 22..25 = shapes of the shifted-factor kernel (cf_shift.cu; linear-df models on 3+1D tiles, <= 64 pT points)
+  // 22..25 = shapes of the shifted-factor kernel (cf_shift.cu; linear-df models on 3+1D tiles, <= 64 pT points), slots x phi points:
+  // 7 x 3, 3 x 6, 3 x 8 at 3 blocks/SM and 7 x 6 at 2 (14 moment, ideal); 7 x 2 at 4, 7 x 3 at 3, 7 x 4 and 7 x 6 at 2 (CE, Jonah)
   int svariant = -1;
   const int first_shift = kNumVariants + kNumFactoredVariants + 1;
   const bool s_ok = shift_supported(model, L) && !iq;
@@ -312,11 +314,11 @@ static int smooth_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_
   }
   else if (svariant >= 0) variant = opt.tile_variant - 1;
   else if (sum_slots) variant = (model == M_FEQMOD || model == M_VAH) ? 12 : (model == M_IDEAL ? 13 : 10);
-  else if (s_ok) { svariant = 1; variant = first_shift - 1 + svariant; }   // linear-df models, 3+1D: cf_shift_kernel<7, 3, 3 blocks/SM>, +15..20 % over cf_kernel
+  else if (s_ok) { svariant = 1; variant = first_shift - 1 + svariant; }   // linear-df models, 3+1D: cf_shift_kernel, 3 x 6 (14 moment) / 7 x 3 (CE)
   else variant = (model == M_VAH || model == M_FEQMOD) ? 11 : 9;
   int nyt, npt, ct, max_warps;
   if (fvariant >= 0) factored_variant_shape(fvariant, &nyt, &npt, &ct, &max_warps);
-  else if (svariant >= 0) shift_variant_shape(svariant, &nyt, &npt, &ct, &max_warps);
+  else if (svariant >= 0) shift_variant_shape(model, svariant, &nyt, &npt, &ct, &max_warps);
   else hot_variant_shape(variant, sum_slots ? 1 : 0, &nyt, &npt, &ct, &max_warps);
   L.nst = sum_slots ? L.n_slots : nyt;
   L.n_ytiles = sum_slots ? 1 : (L.n_slots + nyt - 1) / nyt;

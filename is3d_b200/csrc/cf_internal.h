@@ -139,7 +139,7 @@ cudaError_t launch_factored(int model, const HotParams &hp, int fvariant, cudaSt
 // shifted-factor kernel (cf_shift.cu): linear-df models, 3+1D tiles, <= 64 pT points; same lanes and grid as cf_kernel, 4-warp blocks
 constexpr int kNumShiftVariants = 4;         // tile_variant 22..25
 bool shift_supported(int model, const Layout &L);
-void shift_variant_shape(int v, int *nyt, int *npt, int *ct, int *max_warps);
+void shift_variant_shape(int model, int v, int *nyt, int *npt, int *ct, int *max_warps);
 cudaError_t launch_shift(int model, const HotParams &hp, int v, cudaStream_t st, size_t *smem_out);
 // slot records of padding / skipped cells carry this A = u.p / (mT T): every evaluation is dead (exp overflows, f = 0 exactly)
 constexpr double kDeadSlotA = 1.0e6;

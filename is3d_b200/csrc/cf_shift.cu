@@ -15,13 +15,21 @@
 //  * regulation and outflow cost 5 integer instructions per evaluation instead of 8: g = 1 + df is clamped to [0, 2] (the
 //    reference's max(-1, min(df, 1)), smooth_kernels.cpp:328) on its high word and zeroed where p.dsigma <= 0 (:285) by the same
 //    selects (clamp_mask_g), followed by an unconditional accumulate.
-//  * groups whose largest argument may reach the sub-normal range (xm + pT (Bmax - Bmin) >= 707.7) are evaluated member by
-//    member with the exact routines of cf_kernel (distribution_group), so the zero pattern and gradual underflow are unchanged.
+//  * 14-moment delta-f and ideal f_eq: the group is wide in phi (default 3 slots x 6 phi points), so the per-(cell, slot) work --
+//    the exponential of xm, the votes, the slot record -- is shared by 6 evaluations.  The slot body forms each member's values
+//    inside its class branch and consumes them at once (shift_slot), which keeps the 3 x 6 and 3 x 8 tiles within 168 registers
+//    (3 blocks/SM) without spills.  Groups whose largest argument may reach the sub-normal range (xm + pT (Bmax - Bmin) >= 707.7)
+//    take the same product with e^{-xm} scaled by 2^64 and each member scaled back (one rounding to a sub-normal); members whose
+//    exp(x) overflows in the reference are set to exact zeros, so the zero pattern and gradual underflow are the reference's.
+//  * Chapman-Enskog and Jonah linear keep the staged body on 7 x 3 groups (with the member-by-member body they measured slower at
+//    every shape); there groups that may touch the sub-normal range are evaluated member by member with the exact routines of
+//    cf_kernel (distribution_group).
 //
 // On B200 a warp-wide FP64 instruction holds the scheduler for ~2 cycles and every other instruction for ~1.7 more without
 // overlap (profiles/r2_ubench_mix_issue.txt): the kernel time follows the TOTAL instruction count, which is what this kernel cuts.
 #include "cf_internal.h"
 #include <algorithm>
+#include <type_traits>
 #include "cf_device.cuh"
 #include "cf_epilogue.cuh"
 
@@ -70,12 +78,66 @@ __device__ __forceinline__ void exp_neg_poly_at(double x, uint32_t tab_addr, con
   p_out = fma(T * r, q, T);
 }
 
+// 14-moment delta-f and ideal f_eq run the member-by-member slot body (shift_slot) on wide phi groups; Chapman-Enskog and Jonah
+// linear keep the staged body on 7 x 3 groups: with the member-by-member body CE measured 1.5 % slower at its best shape (3 x 6)
+// and 17 % slower at 7 x 3 than the staged 7 x 3 (DESIGN.md section 6, profiles/r3_sweep.json)
+__host__ __device__ constexpr bool shift_lean(int model) { return model == M_LIN14 || model == M_IDEAL; }
+
+template <int V> using IntC = std::integral_constant<int, V>;
+constexpr int kRareShift = 64;            // e^{-xm} 2^64 is a normal number for every alive xm (<= 709.79)
+
+// The NPT members of one (cell, slot) group, one member at a time: every value a member needs is formed inside the class
+// branch and consumed right away, so only the per-(cell, phi) operands q, pd, g0, eB and the accumulators stay live across
+// members (the independent members give the scheduler enough parallelism).
+//   RARE: e^{-xm} arrives scaled by 2^kRareShift; each product is scaled back (rounding once to a sub-normal where the
+//         reference's 1 / (exp(x) + Theta) is one) and members whose exp(x) overflows in the reference are exact zeros.
+//   CLS : 0 ultra-dilute (every xm >= 37.5: 1 / (1 + Theta a) = 1), 1 dilute (xm >= 12.5), 2 full Bose / Fermi factor.
+// In the ultra-dilute class g = 1 + df is formed with the 1 folded into h0: one FP64 instruction less per member.
+template <int MODEL, int NPT, int RARE, int CLS>
+__device__ __forceinline__ void shift_slot(double a, double cpm, double h0, const double *prj, const double (&q)[NPT], const double (&pd)[NPT],
+                                           const double (&g0)[NPT], const double (&eB)[NPT], double eA, double mTpT, double K2, double sign, int reg_lo, int reg_hi, unsigned reg_chk, int thr_hi, double *accj)
+{
+  static_assert(shift_lean(MODEL), "member-by-member slot body: 14-moment delta-f and ideal f_eq");
+  constexpr bool DF = MODEL != M_IDEAL;
+  const double hK = (DF && CLS == 0) ? h0 + 1.0 : h0;
+#pragma unroll
+  for (int k2 = 0; k2 < NPT; k2 += 2) {
+    double2 t2 = make_double2(0.0, 0.0);
+    if (DF) t2 = *reinterpret_cast<const double2 *>(prj + k2);                 // pair-table row padded to whole 16-byte loads
+#pragma unroll
+    for (int h = 0; h < 2; h++) {
+      const int k = k2 + h;
+      if (k >= NPT) break;
+      const double xs = a - q[k];
+      const double pv = pd[k] + cpm;
+      double av = eA * eB[k];
+      if (RARE) av = exp_finite(xs) ? av * __hiloint2double((1023 - kRareShift) << 20, 0) : 0.0;
+      double f = av, g = 1.0;
+      if (CLS == 0) {
+        if (DF) g = fma(K2 * xs, xs, fma(mTpT, h ? t2.y : t2.x, hK + g0[k]));
+      } else {
+        double fb;
+        f = (CLS == 1) ? occupation_bar_dilute(av, sign, fb) : occupation_bar(av, sign, fb);
+        if (DF) {
+          const double sv = fma(mTpT, h ? t2.y : t2.x, hK + g0[k]);
+          g = fma(fb, fma(K2 * xs, xs, sv), 1.0);
+        }
+      }
+      // f = f_eq g with g clamped to [0, 2]; members failing the outflow test get g = 0.  (A warp holds all pT values of a
+      // species and the largest ones are always clamped: a "nobody needs it" shortcut would never fire.)
+      if (DF) accj[k] = fma(pv, f * clamp_mask_g(g, pv, reg_lo, reg_hi, reg_chk, thr_hi), accj[k]);
+      else accumulate_pos(accj[k], pv, f, thr_hi);
+    }
+  }
+}
+
 template <int MODEL, int NYT, int NPT, int MINB>
 __global__ void __launch_bounds__(128, MINB)
 cf_shift_kernel(const HotParams hp)
 {
   constexpr int RY = kRec;
   constexpr bool DF = MODEL != M_IDEAL;
+  constexpr bool LEAN = shift_lean(MODEL);
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const Layout &L = hp.L;
   const int CT = L.ct;
@@ -146,7 +208,14 @@ cf_shift_kernel(const HotParams hp)
   const uint32_t tab_addr = smem_u32(g_exp_tab);
   const double rare_x = __hiloint2double(kRareHi, 0);                            // 707.6997...: below it e^{-x} is a normal number
 
-  for (int t = 0; t < n_my_tiles; t++) {
+  // member-by-member body: the block-uniform tile count is read back from shared memory (a register holding it across the
+  // cell loop would be spilled at 3 x 8); the staged body keeps it in a register, as it always did
+  __shared__ int my_tiles_s;
+  if constexpr (LEAN) {
+    if (threadIdx.x == 0) my_tiles_s = n_my_tiles;
+    __syncthreads();
+  }
+  for (int t = 0; t < (LEAN ? my_tiles_s : n_my_tiles); t++) {
     const int st = t % kStages;
     mbar_wait(&full[st], (uint32_t)((t / kStages) & 1));
     const double *Ys = stage_base + (size_t)st * stage_doubles;
@@ -176,9 +245,12 @@ cf_shift_kernel(const HotParams hp)
           double pp; int nn;
           const double dd = pTi * (bmax - b[k]);
           exp_neg_poly_at(dd, tab_addr, hp.ec, pp, nn);
-          // beyond 707.7 the factor would leave the normal range: such members are only reached on the per-member path; 0 keeps
-          // the lanes that merely ride along finite
-          eb_tab[(c * NPT + k) * L.n_pT + ip] = __double2hiint(dd) < kRareHi ? exp_neg_fast(pp, nn) : 0.0;
+          // beyond 707.7 the factor leaves the normal range: such members are only reached on the scaled path of the member-by-
+          // member body, which needs the sub-normal value and 0 beyond ln(DBL_MAX) (a member with pT (Bmax - B_k) > 709.78 has
+          // x_k > 709.78 and is an exact zero there), and on the per-member path of the staged body, which does not read the
+          // table (0 keeps the lanes that merely ride along finite)
+          if constexpr (LEAN) eb_tab[(c * NPT + k) * L.n_pT + ip] = exp_neg_slow(dd, pp, nn);
+          else eb_tab[(c * NPT + k) * L.n_pT + ip] = __double2hiint(dd) < kRareHi ? exp_neg_fast(pp, nn) : 0.0;
         }
       }
     }
@@ -188,18 +260,21 @@ cf_shift_kernel(const HotParams hp)
       const double2 k01 = *reinterpret_cast<const double2 *>(Ss + c * kScal);
       const double K2 = k01.y;
       const double K3 = (MODEL == M_JONAHLIN) ? Ss[c * kScal + 2] : 0.0;
+      const double K31 = (MODEL == M_JONAHLIN) ? K3 + 1.0 : 1.0;
       const double K0m = k01.x * m2;
+      // (member-by-member body: pT re-read per cell, two registers fewer in the slots)
+      const double pTc = LEAN ? pT_s[ipT] : pT, pT2c = LEAN ? pTc * pTc : pT2;
       const double2 bb = *reinterpret_cast<const double2 *>(cellv + 2 * c);
-      const double qm = pT * bb.x;                                               // largest pT B_k of the tile
-      const int rare_hi = __double2hiint(fma(-pT, bb.y, rare_x));                 // xm >= 707.7 - pT (Bmax - Bmin): per-member path
+      const double qm = pTc * bb.x;                                               // largest pT B_k of the tile
+      const int rare_hi = __double2hiint(fma(-pTc, bb.y, rare_x));                 // xm >= 707.7 - pT (Bmax - Bmin): scaled path
       double q[NPT], pd[NPT], g0[NPT], eB[NPT];
 #pragma unroll
       for (int k = 0; k < NPT; k++) {
         const double2 *pr = reinterpret_cast<const double2 *>(Ps + (c * NPT + k) * kRec);
         const double2 v0 = pr[0];
-        q[k] = pT * v0.x;
-        pd[k] = pT * v0.y;
-        g0[k] = DF ? fma(pT2, pr[1].x, K0m) : 0.0;
+        q[k] = pTc * v0.x;
+        pd[k] = pTc * v0.y;
+        g0[k] = DF ? fma(pT2c, pr[1].x, K0m) : 0.0;
         eB[k] = eb_tab[(c * NPT + k) * L.n_pT + ipT];
       }
 #pragma unroll
@@ -216,76 +291,94 @@ cf_shift_kernel(const HotParams hp)
         const double cpm = mT * v0.y;
         const double h0 = DF ? mT2 * yr[1].x : 0.0;
         // (the eta weight of a 3+1D slot record is 1: p.dsigma = pT Dp + mT Cp)
-        double pr2[NPP];
-        if (DF) {
+        const double *prj = pair_tab + (c * NYT + j) * NPP;
+        double *accj = acc + j * NPT;
+        if constexpr (!LEAN) {
+          // staged slot body: the NPT members' arguments, p.dsigma and delta-f polynomials are formed together, then the group
+          double pr2[NPP], xs[NPT], pv[NPT], sv[NPT];
 #pragma unroll
           for (int k = 0; k < NPP; k += 2) {
-            const double2 t2 = *reinterpret_cast<const double2 *>(pair_tab + (c * NYT + j) * NPP + k);
+            const double2 t2 = *reinterpret_cast<const double2 *>(prj + k);
             pr2[k] = t2.x; pr2[k + 1] = t2.y;
           }
-        }
-        double xs[NPT], pv[NPT], sv[NPT];
 #pragma unroll
-        for (int k = 0; k < NPT; k++) {
-          xs[k] = a - q[k];
-          pv[k] = pd[k] + cpm;
-          sv[k] = DF ? fma(mTpT, pr2[k], h0 + g0[k]) : 0.0;
-        }
-        double *accj = acc + j * NPT;
-        if (__builtin_expect(__any_sync(0xffffffffu, alive && xh >= rare_hi), 0)) {
-          // some member of some lane may be sub-normal, or dead inside an alive group: member by member, exactly as cf_kernel
-          double fv[NPT];
-          distribution_group<MODEL, NPT>(xs, true, false, sv, K2, K3, sign, reg_thr, one_hi, fv);
+          for (int k = 0; k < NPT; k++) {
+            xs[k] = a - q[k];
+            pv[k] = pd[k] + cpm;
+            sv[k] = fma(mTpT, pr2[k], h0 + g0[k]);
+          }
+          if (__builtin_expect(__any_sync(0xffffffffu, alive && xh >= rare_hi), 0)) {
+            // some member of some lane may be sub-normal, or dead inside an alive group: member by member, exactly as cf_kernel
+            double fv[NPT];
+            distribution_group<MODEL, NPT>(xs, true, false, sv, K2, K3, sign, reg_thr, one_hi, fv);
 #pragma unroll
-          for (int k = 0; k < NPT; k++) accumulate_pos(accj[k], pv[k], fv[k], thr_hi);
-          continue;
-        }
-        double pe; int ne;
-        exp_neg_poly_at(xm, tab_addr, hp.ec, pe, ne);
-        const double eA = alive ? exp_neg_fast(pe, ne) : 0.0;
-        double av[NPT], dfs[NPT], feq[NPT], fb[NPT];
+            for (int k = 0; k < NPT; k++) accumulate_pos(accj[k], pv[k], fv[k], thr_hi);
+            continue;
+          }
+          double pe; int ne;
+          exp_neg_poly_at(xm, tab_addr, hp.ec, pe, ne);
+          const double eA = alive ? exp_neg_fast(pe, ne) : 0.0;
+          double av[NPT], dfs[NPT], feq[NPT], fb[NPT], g[NPT];
 #pragma unroll
-        for (int k = 0; k < NPT; k++) {
-          av[k] = eA * eB[k];
-          if (MODEL == M_LIN14) dfs[k] = fma(K2 * xs[k], xs[k], sv[k]);
-          else if (DF) dfs[k] = fma(sv[k], rcp_fast(xs[k]), K2 * xs[k]);
-        }
-        // a_k <= e^{-xm} for every member: 1 / (1 + Theta a) is 1 to half an ulp once xm >= 37.5 (a < 2^-54; 57 % of the alive
-        // groups of a whole warp on the cfg3 surface), 1 - Theta a + a^2 to 5e-17 once xm >= 12.5 (a < 2^-18; 35 %), else MUFU + 3 DFMA
-        // g = 1 + df is formed inside the branch (no select between the two forms afterwards)
-        const double K31 = (MODEL == M_JONAHLIN) ? K3 + 1.0 : 1.0;
-        double g[NPT];
-        if (__all_sync(0xffffffffu, xh >= kUltraHi)) {                           // (dead lanes have xh > kAliveHi)
+          for (int k = 0; k < NPT; k++) {
+            av[k] = eA * eB[k];
+            dfs[k] = fma(sv[k], rcp_fast(xs[k]), K2 * xs[k]);
+          }
+          if (__all_sync(0xffffffffu, xh >= kUltraHi)) {
 #pragma unroll
-          for (int k = 0; k < NPT; k++) { feq[k] = av[k]; g[k] = DF ? dfs[k] + K31 : 1.0; }
-        } else if (__all_sync(0xffffffffu, xh >= kDiluteHi)) {
+            for (int k = 0; k < NPT; k++) { feq[k] = av[k]; g[k] = dfs[k] + K31; }
+          } else if (__all_sync(0xffffffffu, xh >= kDiluteHi)) {
 #pragma unroll
-          for (int k = 0; k < NPT; k++) { feq[k] = occupation_bar_dilute(av[k], sign, fb[k]); g[k] = DF ? fma(fb[k], dfs[k], K31) : 1.0; }
+            for (int k = 0; k < NPT; k++) { feq[k] = occupation_bar_dilute(av[k], sign, fb[k]); g[k] = fma(fb[k], dfs[k], K31); }
+          } else {
+#pragma unroll
+            for (int k = 0; k < NPT; k++) { feq[k] = occupation_bar(av[k], sign, fb[k]); g[k] = fma(fb[k], dfs[k], K31); }
+          }
+#pragma unroll
+          for (int k = 0; k < NPT; k++)
+            accj[k] = fma(pv[k], feq[k] * clamp_mask_g(g[k], pv[k], reg_lo, reg_hi, reg_chk, thr_hi), accj[k]);
         } else {
-#pragma unroll
-          for (int k = 0; k < NPT; k++) { feq[k] = occupation_bar(av[k], sign, fb[k]); g[k] = DF ? fma(fb[k], dfs[k], K31) : 1.0; }
+          double pe; int ne;
+          exp_neg_poly_at(xm, tab_addr, hp.ec, pe, ne);
+          // some member of some lane may be sub-normal, or dead inside an alive group: e^{-xm} is formed 2^kRareShift too large
+          // (a normal number for every alive xm) and each member is scaled back after the product (one rounding to sub-normal)
+          const bool rare = __builtin_expect(__any_sync(0xffffffffu, alive && xh >= rare_hi), 0);
+          const double eA = alive ? exp_neg_fast(pe, ne + (rare ? kRareShift : 0)) : 0.0;
+          // a_k <= e^{-xm} for every member: 1 / (1 + Theta a) is 1 to half an ulp once xm >= 37.5 (a < 2^-54; 57 % of the alive
+          // groups of a whole warp on the cfg3 surface), 1 - Theta a + a^2 to 5e-17 once xm >= 12.5 (a < 2^-18; 35 %), else MUFU + 3 DFMA
+          // (dead lanes have xh > kAliveHi and pass every test)
+          const int cls = __all_sync(0xffffffffu, xh >= kUltraHi) ? 0 : __all_sync(0xffffffffu, xh >= kDiluteHi) ? 1 : 2;
+          auto slot = [&](auto rare_c, auto cls_c) {
+            shift_slot<MODEL, NPT, decltype(rare_c)::value, decltype(cls_c)::value>(a, cpm, h0, prj, q, pd, g0, eB, eA, mTpT, K2, sign,
+                                                                                 reg_lo, reg_hi, reg_chk, thr_hi, accj);
+          };
+          if (rare) {
+            if (cls == 0) slot(IntC<1>(), IntC<0>()); else if (cls == 1) slot(IntC<1>(), IntC<1>()); else slot(IntC<1>(), IntC<2>());
+          } else {
+            if (cls == 0) slot(IntC<0>(), IntC<0>()); else if (cls == 1) slot(IntC<0>(), IntC<1>()); else slot(IntC<0>(), IntC<2>());
+          }
         }
-        if (!DF) {
-#pragma unroll
-          for (int k = 0; k < NPT; k++) accumulate_pos(accj[k], pv[k], feq[k], thr_hi);
-          continue;
-        }
-        // f = f_eq g with g clamped to [0, 2]; members failing the outflow test get g = 0.  (A warp holds all pT values of a
-        // species and the largest ones are always clamped: a "nobody needs it" shortcut would never fire.)
-#pragma unroll
-        for (int k = 0; k < NPT; k++)
-          accj[k] = fma(pv[k], feq[k] * clamp_mask_g(g[k], pv[k], reg_lo, reg_hi, reg_chk, thr_hi), accj[k]);
       }
     }
     __syncthreads();                                   // every warp is done with stage st and with the tables
-    if (threadIdx.x == 0 && t + kStages < n_my_tiles) issue(t + kStages);
+    if (threadIdx.x == 0 && t + kStages < (LEAN ? my_tiles_s : n_my_tiles)) issue(t + kStages);
   }
 
-  hot_epilogue<NYT, NPT, false>(hp, acc, stage_base, chunk, gb, ty, tp, lane_valid, ipart, ipT);
+  // member-by-member body: the species index is derived again rather than kept live across the cell loop, where its register
+  // would be spilled
+  int ipart_e = ipart;
+  if constexpr (LEAN) {
+    int tid = threadIdx.x;
+    asm volatile("" : "+r"(tid));
+    const int idx_e = (gb * hp.n_warps + (tid >> 5)) * 32 + (tid & 31);
+    ipart_e = lane_valid ? idx_e / L.n_pT : 0;
+  }
+  hot_epilogue<NYT, NPT, false>(hp, acc, stage_base, chunk, gb, ty, tp, lane_valid, ipart_e, ipT);
 }
 
 struct ShiftShape { int nyt, npt, ct, minb; };
-const ShiftShape kShiftShapes[kNumShiftVariants] = {{7, 3, 16, 4}, {7, 3, 16, 3}, {7, 4, 16, 3}, {7, 6, 16, 2}};
+const ShiftShape kShiftShapesLean[kNumShiftVariants] = {{7, 3, 16, 3}, {3, 6, 16, 3}, {3, 8, 16, 3}, {7, 6, 16, 2}};
+const ShiftShape kShiftShapesStaged[kNumShiftVariants] = {{7, 2, 16, 4}, {7, 3, 16, 3}, {7, 4, 16, 2}, {7, 6, 16, 2}};
 
 template <int MODEL, int NYT, int NPT, int MINB>
 cudaError_t launch_shift_one(const HotParams &hp, cudaStream_t st, size_t *smem_out)
@@ -308,12 +401,22 @@ cudaError_t launch_shift_one(const HotParams &hp, cudaStream_t st, size_t *smem_
 template <int MODEL>
 cudaError_t launch_shift_model(const HotParams &hp, int v, cudaStream_t st, size_t *smem_out)
 {
-  switch (v) {
-    case 0: return launch_shift_one<MODEL, 7, 3, 4>(hp, st, smem_out);
-    case 1: return launch_shift_one<MODEL, 7, 3, 3>(hp, st, smem_out);
-    case 2: return launch_shift_one<MODEL, 7, 4, 3>(hp, st, smem_out);
-    case 3: return launch_shift_one<MODEL, 7, 6, 2>(hp, st, smem_out);
-    default: return cudaErrorInvalidValue;
+  if constexpr (shift_lean(MODEL)) {
+    switch (v) {
+      case 0: return launch_shift_one<MODEL, 7, 3, 3>(hp, st, smem_out);
+      case 1: return launch_shift_one<MODEL, 3, 6, 3>(hp, st, smem_out);
+      case 2: return launch_shift_one<MODEL, 3, 8, 3>(hp, st, smem_out);
+      case 3: return launch_shift_one<MODEL, 7, 6, 2>(hp, st, smem_out);
+      default: return cudaErrorInvalidValue;
+    }
+  } else {
+    switch (v) {
+      case 0: return launch_shift_one<MODEL, 7, 2, 4>(hp, st, smem_out);
+      case 1: return launch_shift_one<MODEL, 7, 3, 3>(hp, st, smem_out);
+      case 2: return launch_shift_one<MODEL, 7, 4, 2>(hp, st, smem_out);
+      case 3: return launch_shift_one<MODEL, 7, 6, 2>(hp, st, smem_out);
+      default: return cudaErrorInvalidValue;
+    }
   }
 }
 
@@ -324,10 +427,11 @@ bool shift_supported(int model, const Layout &L)
   return !L.dim2 && L.n_pT <= kShiftMaxPT && (model == M_LIN14 || model == M_LINCE || model == M_JONAHLIN || model == M_IDEAL);
 }
 
-void shift_variant_shape(int v, int *nyt, int *npt, int *ct, int *max_warps)
+void shift_variant_shape(int model, int v, int *nyt, int *npt, int *ct, int *max_warps)
 {
   if (v < 0 || v >= kNumShiftVariants) v = 0;
-  *nyt = kShiftShapes[v].nyt; *npt = kShiftShapes[v].npt; *ct = kShiftShapes[v].ct; *max_warps = 4;
+  const ShiftShape &s = shift_lean(model) ? kShiftShapesLean[v] : kShiftShapesStaged[v];
+  *nyt = s.nyt; *npt = s.npt; *ct = s.ct; *max_warps = 4;
 }
 
 // the block is always 4 warps: hp.n_warps must be 4 and hp.n_groupblocks = ceil(n_species n_pT / 128)
