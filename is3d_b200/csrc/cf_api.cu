@@ -47,13 +47,14 @@ struct DevBuf {
 
 struct Workspace {
   DevBuf raw, small, Y, P, S, Y2, P2, S2, partial, dN, counters, extra, gather, integ, integ_out;
+  DevBuf E;                       // cf_shift_kernel's e^{-pT (Bmax - B_k)} table, one window of chunks
   cudaEvent_t ev[8];
   bool events = false;
   void release()
   {
     raw.release(); small.release(); Y.release(); P.release(); S.release(); Y2.release(); P2.release(); S2.release();
     partial.release(); dN.release();
-    counters.release(); extra.release(); gather.release(); integ.release(); integ_out.release();
+    counters.release(); extra.release(); gather.release(); integ.release(); integ_out.release(); E.release();
     if (events) { for (auto &e : ev) cudaEventDestroy(e); events = false; }
   }
 };
@@ -298,6 +299,7 @@ static int smooth_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_
   const bool strict = (opt.tile_variant == kStrictVariant);
   // 22..25 = shapes of the shifted-factor kernel (cf_shift.cu; linear-df models on 3+1D tiles, <= 64 pT points), slots x phi points:
   // 7 x 3, 3 x 6, 3 x 8 at 3 blocks/SM and 7 x 6 at 2 (14 moment, ideal); 7 x 2 at 4, 7 x 3 at 3, 7 x 4 and 7 x 6 at 2 (CE, Jonah)
+  // (16-cell tiles, halved where the pipeline would not fit that many blocks per SM: 3 x 8 at 32 pT points runs 8-cell tiles)
   int svariant = -1;
   const int first_shift = kNumVariants + kNumFactoredVariants + 1;
   const bool s_ok = shift_supported(model, L) && !iq;
@@ -318,7 +320,7 @@ static int smooth_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_
   else variant = (model == M_VAH || model == M_FEQMOD) ? 11 : 9;
   int nyt, npt, ct, max_warps;
   if (fvariant >= 0) factored_variant_shape(fvariant, &nyt, &npt, &ct, &max_warps);
-  else if (svariant >= 0) shift_variant_shape(model, svariant, &nyt, &npt, &ct, &max_warps);
+  else if (svariant >= 0) shift_variant_shape(model, svariant, gr->n_pT, &nyt, &npt, &ct, &max_warps);
   else hot_variant_shape(variant, sum_slots ? 1 : 0, &nyt, &npt, &ct, &max_warps);
   L.nst = sum_slots ? L.n_slots : nyt;
   L.n_ytiles = sum_slots ? 1 : (L.n_slots + nyt - 1) / nyt;
@@ -484,6 +486,19 @@ static int smooth_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_
     if (fl->df_mode == 3) CU_CHECK(g_ws.extra.reserve(((size_t)L.n_species + 8) * L.n_cells_pad * 8 + 256));
   }
   if (!iq) CU_CHECK(g_ws.partial.reserve((size_t)partial_sets * n_chunks * n_bins * 8 + 256));
+  // cf_shift_kernel reads e^{-pT (Bmax - B_k)} from a table that is formed for a window of consecutive chunks at a time (the
+  // table kernel, then the hot kernel on those chunks): at ~3x the records per cell, a window is kept <= 4 GiB like the
+  // partial buffer.  The chunk count above deliberately ignores the table.
+  int win_chunks = n_chunks;
+  int64_t e_cells = 0;
+  if (svariant >= 0) {
+    const int64_t chunk_cells = (L.n_tiles + n_chunks - 1) / n_chunks * L.ct;        // most cells a chunk holds
+    const int64_t chunk_bytes = chunk_cells * L.n_ptiles * shift_table_record(L) * 8;
+    const int64_t max_table_bytes = (int64_t)4 << 30;
+    win_chunks = (int)std::max<int64_t>(1, std::min<int64_t>(n_chunks, chunk_bytes > 0 ? max_table_bytes / chunk_bytes : n_chunks));
+    e_cells = win_chunks * chunk_cells;
+    CU_CHECK(g_ws.E.reserve((size_t)e_cells * L.n_ptiles * shift_table_record(L) * 8 + 256));
+  }
   if (iq) {
     CU_CHECK(g_ws.integ.reserve((size_t)partial_sets * integ_bytes + 256));
     CU_CHECK(g_ws.integ_out.reserve((size_t)partial_sets * iq->n_units * sp->n * 8 + 256));
@@ -597,11 +612,13 @@ static int smooth_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_
     hp.integ_mode = iq->mode; hp.integ_sl = integ_sl; hp.chunk_tiles = chunk_tiles_d;
     hp.pT_weight = wpT_d; hp.phi_weight = wphi_d; hp.integ = g_ws.integ.as<double>();
   }
+  hp.E = g_ws.E.as<double>(); hp.e_cells = e_cells;
+  int hot_launches = 1;
   if (strict) {}                                              // the bins were summed by launch_strict above
   else if (fvariant >= 0) CU_CHECK(launch_factored(model, hp, fvariant, st, nullptr));
-  else if (svariant >= 0) CU_CHECK(launch_shift(model, hp, svariant, st, nullptr));
+  else if (svariant >= 0) CU_CHECK(launch_shift(model, hp, svariant, win_chunks, st, nullptr, &hot_launches));
   else CU_CHECK(launch_hot(model, hp, variant, st, nullptr));
-  if (!strict) stt.gpu_launches++;
+  if (!strict) stt.gpu_launches += hot_launches;
   int reduce_sets = 1;
   if (feqmod) {
     // cells where feqmod breaks down (and narrow-rapidity slots) take the linear-df branch: second pass, only if any

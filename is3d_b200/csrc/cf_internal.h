@@ -87,6 +87,10 @@ struct HotParams {
   const int64_t *chunk_tiles;                      // [n_chunks + 1] first cell tile of every chunk (NULL: balanced split)
   const double *pT_weight, *phi_weight;            // quadrature weights of the pT and phi tables
   double *integ;                                   // mode 1: [chunk][ytile][ptile][groupblock][sl]; mode 2: [chunk][slot][ptile][groupblock][sl]
+  // cf_shift.cu: e^{-pT (Bmax - B_k)} table of one window of consecutive chunks, [n_ptiles][e_cells][shift_table_record(L)]
+  double *E;
+  int64_t e_cells;                                 // cells per phi tile the table holds
+  int chunk0;                                      // first chunk of the launch: block b works on chunk chunk0 + b / (blocks per chunk)
 };
 
 // launchers (cf_prepare.cu / cf_kernels.cu)
@@ -139,8 +143,10 @@ cudaError_t launch_factored(int model, const HotParams &hp, int fvariant, cudaSt
 // shifted-factor kernel (cf_shift.cu): linear-df models, 3+1D tiles, <= 64 pT points; same lanes and grid as cf_kernel, 4-warp blocks
 constexpr int kNumShiftVariants = 4;         // tile_variant 22..25
 bool shift_supported(int model, const Layout &L);
-void shift_variant_shape(int model, int v, int *nyt, int *npt, int *ct, int *max_warps);
-cudaError_t launch_shift(int model, const HotParams &hp, int v, cudaStream_t st, size_t *smem_out);
+void shift_variant_shape(int model, int v, int n_pT, int *nyt, int *npt, int *ct, int *max_warps);   // ct fitted to n_pT
+int shift_table_record(const Layout &L);     // doubles per (phi tile, cell) of HotParams::E
+// per window of win_chunks chunks: the table kernel, then cf_shift_kernel on the window's chunks; *launches = kernels launched
+cudaError_t launch_shift(int model, const HotParams &hp, int v, int win_chunks, cudaStream_t st, size_t *smem_out, int *launches);
 // slot records of padding / skipped cells carry this A = u.p / (mT T): every evaluation is dead (exp overflows, f = 0 exactly)
 constexpr double kDeadSlotA = 1.0e6;
 // spin polarization from thermal vorticity (cf_polzn.cu): ideal-f cells and slots, 5 sums per bin (Snorm, N^t, N^x, N^y, N^z)

@@ -9,8 +9,10 @@
 //    tile's phi points.  Both factors lie in (0, 1]: neither can overflow or underflow before the product does, so no exponent
 //    bookkeeping is needed (compare the mantissa / exponent pairs of cf_factored.cu).  The first factor is ONE exponential per
 //    (cell, slot) and thread -- of the group's smallest argument xm, which also classifies the whole group (dead / dilute /
-//    possibly sub-normal) -- the second does not depend on the slot or the species: the block tabulates it once per tile for
-//    (cell, phi, pT) in shared memory, 12 exponentials per thread and 16-cell tile instead of 3 per thread and cell.
+//    possibly sub-normal) -- the second does not depend on the slot or the species: cf_shift_table_kernel tabulates it once per
+//    (phi tile, cell, phi point, pT) in global memory, together with Bmax and Bmax - Bmin, and the hot kernel streams each cell
+//    tile's slice with its records (formed inside every block, the table took ~14 % of the hot kernel's instructions at cfg3,
+//    counted from the SASS: the n_groupblocks x n_ytiles blocks that read a cell tile each computed the same values).
 //    Per evaluation that leaves a DMUL where cf_kernel spends 9 FP64 instructions.
 //  * regulation and outflow cost 5 integer instructions per evaluation instead of 8: g = 1 + df is clamped to [0, 2] (the
 //    reference's max(-1, min(df, 1)), smooth_kernels.cpp:328) on its high word and zeroed where p.dsigma <= 0 (:285) by the same
@@ -37,8 +39,15 @@ namespace is3d {
 
 namespace {
 
-constexpr int kShiftMaxPT = 64;           // pT points the per-tile e^{-pT dB} table is laid out for
+constexpr int kShiftMaxPT = 64;           // pT points the e^{-pT dB} table is laid out for
 constexpr int kUltraHi = 0x4042C000;      // high word of 37.5: e^{-x} < 2^-54
+// TMA pipeline depth.  A stage holds a 16-cell tile's records and table slice (32 KB at 3 x 6 and 32 pT points): two stages
+// keep 3 blocks/SM; a tile lasts tens of us against ~1 us of copy latency, so the second stage is enough to hide it.
+constexpr int kShiftStages = 2;
+
+// doubles per (phi tile, cell) record of the table: Bmax, Bmax - Bmin, then e^{-pT (Bmax - B_k)} as [NPT][n_pT], padded to
+// whole 16-byte units (the bulk copies need them)
+__host__ __device__ __forceinline__ int shift_erec(int npt, int n_pT) { return (2 + npt * n_pT + 1) & ~1; }
 
 // g = 1 + df clamped to [0, 2] (regulate_deltaf, smooth_kernels.cpp:328) and zeroed where p.dsigma fails the outflow test (:285),
 // all on the integer pipe from the high words: 6 instructions (2 VIMNMX, 2 ISETP, 2 SEL) for both features.
@@ -131,6 +140,45 @@ __device__ __forceinline__ void shift_slot(double a, double cpm, double h0, cons
   }
 }
 
+// E[tp][cell - cell0] = {Bmax, Bmax - Bmin, e^{-pT (Bmax - B_k)} [k][pT]} for the cells [cell0, cell0 + n_win), padded phi
+// records included; one thread per (phi tile, cell, pT point)
+template <int NPT, bool LEAN>
+__global__ void __launch_bounds__(128)
+cf_shift_table_kernel(const HotParams hp, double *E, int64_t cell0, int64_t n_win)
+{
+  const Layout &L = hp.L;
+  exp_table_init();
+  __syncthreads();
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= L.n_ptiles * n_win * L.n_pT) return;
+  const int ip = (int)(i % L.n_pT);
+  const int64_t r = i / L.n_pT, cl = r % n_win;
+  const int tp = (int)(r / n_win);
+  const double *pr = hp.P + ((int64_t)tp * L.n_cells_pad + cell0 + cl) * NPT * kRec;
+  double *er = E + ((int64_t)tp * hp.e_cells + cl) * shift_erec(NPT, L.n_pT);
+  double b[NPT];
+#pragma unroll
+  for (int k = 0; k < NPT; k++) b[k] = pr[k * kRec];
+  double bmax = b[0], bmin = b[0];
+#pragma unroll
+  for (int k = 1; k < NPT; k++) { bmax = b[k] > bmax ? b[k] : bmax; bmin = b[k] < bmin ? b[k] : bmin; }
+  if (ip == 0) { er[0] = bmax; er[1] = bmax - bmin; }
+  const double pTi = hp.pT[ip];
+  const uint32_t tab_addr = smem_u32(g_exp_tab);
+#pragma unroll
+  for (int k = 0; k < NPT; k++) {
+    double pp; int nn;
+    const double dd = pTi * (bmax - b[k]);
+    exp_neg_poly_at(dd, tab_addr, hp.ec, pp, nn);
+    // beyond 707.7 the factor leaves the normal range: such members are only reached on the scaled path of the member-by-
+    // member body, which needs the sub-normal value and 0 beyond ln(DBL_MAX) (a member with pT (Bmax - B_k) > 709.78 has
+    // x_k > 709.78 and is an exact zero there), and on the per-member path of the staged body, which does not read the
+    // table (0 keeps the lanes that merely ride along finite)
+    if constexpr (LEAN) er[2 + k * L.n_pT + ip] = exp_neg_slow(dd, pp, nn);
+    else er[2 + k * L.n_pT + ip] = __double2hiint(dd) < kRareHi ? exp_neg_fast(pp, nn) : 0.0;
+  }
+}
+
 template <int MODEL, int NYT, int NPT, int MINB>
 __global__ void __launch_bounds__(128, MINB)
 cf_shift_kernel(const HotParams hp)
@@ -141,19 +189,19 @@ cf_shift_kernel(const HotParams hp)
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const Layout &L = hp.L;
   const int CT = L.ct;
-  const int y_doubles = CT * NYT * RY, p_doubles = CT * NPT * kRec, s_doubles = CT * kScal;
-  const int stage_doubles = y_doubles + p_doubles + s_doubles;
+  const int RE = shift_erec(NPT, L.n_pT);
+  const int y_doubles = CT * NYT * RY, p_doubles = CT * NPT * kRec, s_doubles = CT * kScal, e_doubles = CT * RE;
+  const int stage_doubles = y_doubles + p_doubles + s_doubles + e_doubles;
   double *stage_base = reinterpret_cast<double *>(smem_raw);
-  uint64_t *full = reinterpret_cast<uint64_t *>(stage_base + (size_t)kStages * stage_doubles);
+  uint64_t *full = reinterpret_cast<uint64_t *>(stage_base + (size_t)kShiftStages * stage_doubles);
   constexpr int NPP = (NPT + 1) & ~1;                                            // pair-table row padded to whole 16-byte loads
-  double *pair_tab = reinterpret_cast<double *>(full + kStages);                 // [CT][NYT][NPP]
-  double *eb_tab = pair_tab + CT * NYT * NPP;                                    // [CT][NPT][n_pT]  e^{-pT (Bmax - B_k)}
-  double *cellv = eb_tab + CT * NPT * L.n_pT;                                    // [CT][2]          Bmax, Bmax - Bmin
-  double *pT_s = cellv + CT * 2;                                                 // [n_pT]
+  double *pair_tab = reinterpret_cast<double *>(full + kShiftStages);            // [CT][NYT][NPP]
+  double *pT_s = pair_tab + CT * NYT * NPP;                                      // [n_pT]
 
   const int n_bintiles = hp.n_groupblocks * L.n_ytiles * L.n_ptiles;
-  const int chunk = blockIdx.x / n_bintiles;
-  int bt = blockIdx.x - chunk * n_bintiles;
+  const int chunk_w = blockIdx.x / n_bintiles;                                   // chunk within the launch's window
+  const int chunk = hp.chunk0 + chunk_w;
+  int bt = blockIdx.x - chunk_w * n_bintiles;
   const int tp = bt % L.n_ptiles; bt /= L.n_ptiles;
   const int ty = bt % L.n_ytiles; bt /= L.n_ytiles;
   const int gb = bt;
@@ -180,27 +228,30 @@ cf_shift_kernel(const HotParams hp)
   const double *Yg = hp.Y + ((int64_t)ty * L.n_cells_pad) * NYT * RY;
   const double *Pg = hp.P + ((int64_t)tp * L.n_cells_pad) * NPT * kRec;
   const double *Sg = hp.S;
+  // the window's table starts at the first cell of chunk chunk0
+  const int64_t e_off = (int64_t)tp * hp.e_cells - (L.n_tiles * (int64_t)hp.chunk0) / hp.n_chunks * CT;
   const uint32_t stage_bytes = (uint32_t)stage_doubles * 8u;
 
   exp_table_init();
   for (int i = threadIdx.x; i < L.n_pT; i += blockDim.x) pT_s[i] = hp.pT[i];
   if (threadIdx.x == 0) {
-    for (int s = 0; s < kStages; s++) mbar_init(&full[s], 1);
+    for (int s = 0; s < kShiftStages; s++) mbar_init(&full[s], 1);
     mbar_fence_init();
   }
   __syncthreads();
 
   auto issue = [&](int t_local) {
-    const int st = t_local % kStages;
+    const int st = t_local % kShiftStages;
     const int64_t cell = (t_begin + t_local) * CT;
     double *dst = stage_base + (size_t)st * stage_doubles;
     mbar_arrive_expect_tx(&full[st], stage_bytes);
     bulk_g2s(dst, Yg + cell * NYT * RY, (uint32_t)y_doubles * 8u, &full[st]);
     bulk_g2s(dst + y_doubles, Pg + cell * NPT * kRec, (uint32_t)p_doubles * 8u, &full[st]);
     bulk_g2s(dst + y_doubles + p_doubles, Sg + cell * kScal, (uint32_t)s_doubles * 8u, &full[st]);
+    bulk_g2s(dst + y_doubles + p_doubles + s_doubles, hp.E + (e_off + cell) * RE, (uint32_t)e_doubles * 8u, &full[st]);
   };
   if (threadIdx.x == 0)
-    for (int t = 0; t < kStages && t < n_my_tiles; t++) issue(t);
+    for (int t = 0; t < kShiftStages && t < n_my_tiles; t++) issue(t);
 
   double acc[NYT * NPT];
 #pragma unroll
@@ -216,45 +267,22 @@ cf_shift_kernel(const HotParams hp)
     __syncthreads();
   }
   for (int t = 0; t < (LEAN ? my_tiles_s : n_my_tiles); t++) {
-    const int st = t % kStages;
-    mbar_wait(&full[st], (uint32_t)((t / kStages) & 1));
+    const int st = t % kShiftStages;
+    mbar_wait(&full[st], (uint32_t)((t / kShiftStages) & 1));
     const double *Ys = stage_base + (size_t)st * stage_doubles;
     const double *Ps = Ys + y_doubles;
     const double *Ss = Ps + p_doubles;
+    const double *Es = Ss + s_doubles;                                           // [CT][RE]  Bmax, Bmax - Bmin, e^{-pT (Bmax - B_k)}
 
-    // ---- block phase: tables that do not depend on the species
-    if (DF) {
-      for (int w = threadIdx.x; w < CT * NYT * NPT; w += blockDim.x) {             // pair table, as in cf_kernel
+    // ---- block phase: the pair table does not depend on the species
+    if constexpr (DF) {
+      for (int w = threadIdx.x; w < CT * NYT * NPT; w += blockDim.x) {             // as in cf_kernel
         const int c = w / (NYT * NPT), r = w - c * (NYT * NPT), j = r / NPT, k = r - j * NPT;
         const double *yr = Ys + (c * NYT + j) * RY, *pr = Ps + (c * NPT + k) * kRec;
         pair_tab[(c * NYT + j) * NPP + k] = fma(pr[4], yr[4], -(pr[3] * yr[3]));
       }
+      __syncthreads();
     }
-    for (int c = warp; c < CT; c += 4) {                                         // e^{-pT (Bmax - B_k)}: one cell per warp-iteration
-      double b[NPT];
-#pragma unroll
-      for (int k = 0; k < NPT; k++) b[k] = Ps[(c * NPT + k) * kRec];
-      double bmax = b[0], bmin = b[0];
-#pragma unroll
-      for (int k = 1; k < NPT; k++) { bmax = b[k] > bmax ? b[k] : bmax; bmin = b[k] < bmin ? b[k] : bmin; }
-      if (lane == 0) { cellv[2 * c] = bmax; cellv[2 * c + 1] = bmax - bmin; }
-      for (int ip = lane; ip < L.n_pT; ip += 32) {
-        const double pTi = pT_s[ip];
-#pragma unroll
-        for (int k = 0; k < NPT; k++) {
-          double pp; int nn;
-          const double dd = pTi * (bmax - b[k]);
-          exp_neg_poly_at(dd, tab_addr, hp.ec, pp, nn);
-          // beyond 707.7 the factor leaves the normal range: such members are only reached on the scaled path of the member-by-
-          // member body, which needs the sub-normal value and 0 beyond ln(DBL_MAX) (a member with pT (Bmax - B_k) > 709.78 has
-          // x_k > 709.78 and is an exact zero there), and on the per-member path of the staged body, which does not read the
-          // table (0 keeps the lanes that merely ride along finite)
-          if constexpr (LEAN) eb_tab[(c * NPT + k) * L.n_pT + ip] = exp_neg_slow(dd, pp, nn);
-          else eb_tab[(c * NPT + k) * L.n_pT + ip] = __double2hiint(dd) < kRareHi ? exp_neg_fast(pp, nn) : 0.0;
-        }
-      }
-    }
-    __syncthreads();
 
     for (int c = 0; c < CT; c++) {
       const double2 k01 = *reinterpret_cast<const double2 *>(Ss + c * kScal);
@@ -264,7 +292,7 @@ cf_shift_kernel(const HotParams hp)
       const double K0m = k01.x * m2;
       // (member-by-member body: pT re-read per cell, two registers fewer in the slots)
       const double pTc = LEAN ? pT_s[ipT] : pT, pT2c = LEAN ? pTc * pTc : pT2;
-      const double2 bb = *reinterpret_cast<const double2 *>(cellv + 2 * c);
+      const double2 bb = *reinterpret_cast<const double2 *>(Es + c * RE);
       const double qm = pTc * bb.x;                                               // largest pT B_k of the tile
       const int rare_hi = __double2hiint(fma(-pTc, bb.y, rare_x));                 // xm >= 707.7 - pT (Bmax - Bmin): scaled path
       double q[NPT], pd[NPT], g0[NPT], eB[NPT];
@@ -275,7 +303,7 @@ cf_shift_kernel(const HotParams hp)
         q[k] = pTc * v0.x;
         pd[k] = pTc * v0.y;
         g0[k] = DF ? fma(pT2c, pr[1].x, K0m) : 0.0;
-        eB[k] = eb_tab[(c * NPT + k) * L.n_pT + ipT];
+        eB[k] = Es[c * RE + 2 + k * L.n_pT + ipT];
       }
 #pragma unroll
       for (int j = 0; j < NYT; j++) {
@@ -360,8 +388,8 @@ cf_shift_kernel(const HotParams hp)
         }
       }
     }
-    __syncthreads();                                   // every warp is done with stage st and with the tables
-    if (threadIdx.x == 0 && t + kStages < (LEAN ? my_tiles_s : n_my_tiles)) issue(t + kStages);
+    __syncthreads();                                   // every warp is done with stage st and with the pair table
+    if (threadIdx.x == 0 && t + kShiftStages < (LEAN ? my_tiles_s : n_my_tiles)) issue(t + kShiftStages);
   }
 
   // member-by-member body: the species index is derived again rather than kept live across the cell loop, where its register
@@ -376,45 +404,67 @@ cf_shift_kernel(const HotParams hp)
   hot_epilogue<NYT, NPT, false>(hp, acc, stage_base, chunk, gb, ty, tp, lane_valid, ipart_e, ipT);
 }
 
+// ct: the longest tile; shift_variant_shape shortens it where the pipeline would not fit minb blocks per SM
 struct ShiftShape { int nyt, npt, ct, minb; };
 const ShiftShape kShiftShapesLean[kNumShiftVariants] = {{7, 3, 16, 3}, {3, 6, 16, 3}, {3, 8, 16, 3}, {7, 6, 16, 2}};
 const ShiftShape kShiftShapesStaged[kNumShiftVariants] = {{7, 2, 16, 4}, {7, 3, 16, 3}, {7, 4, 16, 2}, {7, 6, 16, 2}};
 
+// dynamic shared memory of cf_shift_kernel: kShiftStages stages of a ct-cell tile (Y, P, S records and the table slice), their
+// mbarriers, the pair table and the pT table
+size_t shift_pipe_bytes(int nyt, int npt, int ct, int n_pT)
+{
+  const size_t stage_doubles = (size_t)ct * (nyt * kRec + npt * kRec + kScal + shift_erec(npt, n_pT));
+  return kShiftStages * stage_doubles * 8 + kShiftStages * 8 + ((size_t)ct * nyt * ((npt + 1) & ~1) + n_pT) * 8;
+}
+
 template <int MODEL, int NYT, int NPT, int MINB>
-cudaError_t launch_shift_one(const HotParams &hp, cudaStream_t st, size_t *smem_out)
+cudaError_t launch_shift_one(const HotParams &hp, int win_chunks, cudaStream_t st, size_t *smem_out, int *launches)
 {
   const Layout &L = hp.L;
-  const int stage_doubles = L.ct * (NYT * kRec + NPT * kRec + kScal);
-  const size_t pipe = (size_t)kStages * stage_doubles * 8 + kStages * 8
-                    + ((size_t)L.ct * NYT * ((NPT + 1) & ~1) + (size_t)L.ct * NPT * L.n_pT + (size_t)L.ct * 2 + L.n_pT) * 8;
+  const size_t pipe = shift_pipe_bytes(NYT, NPT, L.ct, L.n_pT);
   const size_t smem = std::max(pipe, (hot_epilogue_scratch_bytes(hp, NYT, false, 128) + 15) & ~(size_t)15);
   if (smem_out) *smem_out = smem;
+  *launches = 0;
   auto kern = cf_shift_kernel<MODEL, NYT, NPT, MINB>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
-  const int64_t grid = (int64_t)hp.n_groupblocks * L.n_ytiles * L.n_ptiles * hp.n_chunks;
-  if (grid == 0) return cudaSuccess;
-  kern<<<(unsigned)grid, 128, smem, st>>>(hp);
-  return cudaGetLastError();
+  const int64_t n_bintiles = (int64_t)hp.n_groupblocks * L.n_ytiles * L.n_ptiles;
+  if (n_bintiles == 0) return cudaSuccess;
+  // the grid is chunk-major: a window of chunks is a contiguous range of blocks, and its cells a contiguous range of tiles
+  for (int c0 = 0; c0 < hp.n_chunks; c0 += win_chunks) {
+    const int c1 = std::min(hp.n_chunks, c0 + win_chunks);
+    const int64_t cell0 = (L.n_tiles * (int64_t)c0) / hp.n_chunks * L.ct, cell1 = (L.n_tiles * (int64_t)c1) / hp.n_chunks * L.ct;
+    const int64_t n_threads = L.n_ptiles * (cell1 - cell0) * L.n_pT;
+    if (n_threads > 0) {
+      cf_shift_table_kernel<NPT, shift_lean(MODEL)><<<(unsigned)((n_threads + 127) / 128), 128, 0, st>>>(hp, hp.E, cell0, cell1 - cell0);
+      ++*launches;
+    }
+    HotParams hw = hp;
+    hw.chunk0 = c0;
+    kern<<<(unsigned)(n_bintiles * (c1 - c0)), 128, smem, st>>>(hw);
+    ++*launches;
+    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+  }
+  return cudaSuccess;
 }
 
 template <int MODEL>
-cudaError_t launch_shift_model(const HotParams &hp, int v, cudaStream_t st, size_t *smem_out)
+cudaError_t launch_shift_model(const HotParams &hp, int v, int win_chunks, cudaStream_t st, size_t *smem_out, int *launches)
 {
   if constexpr (shift_lean(MODEL)) {
     switch (v) {
-      case 0: return launch_shift_one<MODEL, 7, 3, 3>(hp, st, smem_out);
-      case 1: return launch_shift_one<MODEL, 3, 6, 3>(hp, st, smem_out);
-      case 2: return launch_shift_one<MODEL, 3, 8, 3>(hp, st, smem_out);
-      case 3: return launch_shift_one<MODEL, 7, 6, 2>(hp, st, smem_out);
+      case 0: return launch_shift_one<MODEL, 7, 3, 3>(hp, win_chunks, st, smem_out, launches);
+      case 1: return launch_shift_one<MODEL, 3, 6, 3>(hp, win_chunks, st, smem_out, launches);
+      case 2: return launch_shift_one<MODEL, 3, 8, 3>(hp, win_chunks, st, smem_out, launches);
+      case 3: return launch_shift_one<MODEL, 7, 6, 2>(hp, win_chunks, st, smem_out, launches);
       default: return cudaErrorInvalidValue;
     }
   } else {
     switch (v) {
-      case 0: return launch_shift_one<MODEL, 7, 2, 4>(hp, st, smem_out);
-      case 1: return launch_shift_one<MODEL, 7, 3, 3>(hp, st, smem_out);
-      case 2: return launch_shift_one<MODEL, 7, 4, 2>(hp, st, smem_out);
-      case 3: return launch_shift_one<MODEL, 7, 6, 2>(hp, st, smem_out);
+      case 0: return launch_shift_one<MODEL, 7, 2, 4>(hp, win_chunks, st, smem_out, launches);
+      case 1: return launch_shift_one<MODEL, 7, 3, 3>(hp, win_chunks, st, smem_out, launches);
+      case 2: return launch_shift_one<MODEL, 7, 4, 2>(hp, win_chunks, st, smem_out, launches);
+      case 3: return launch_shift_one<MODEL, 7, 6, 2>(hp, win_chunks, st, smem_out, launches);
       default: return cudaErrorInvalidValue;
     }
   }
@@ -427,21 +477,37 @@ bool shift_supported(int model, const Layout &L)
   return !L.dim2 && L.n_pT <= kShiftMaxPT && (model == M_LIN14 || model == M_LINCE || model == M_JONAHLIN || model == M_IDEAL);
 }
 
-void shift_variant_shape(int model, int v, int *nyt, int *npt, int *ct, int *max_warps)
+// The table slice makes a stage grow with n_pT (16 x (2 + NPT n_pT) doubles): where the 16-cell pipeline would not leave room
+// for the shape's blocks/SM (3 x 8 at 32 pT points, 3 x 6 beyond 36), the tile is halved until it does: a shorter tile only
+// adds per-tile synchronisation, while a block less per SM leaves fewer warps to hide the latency of the FP64 chains.
+void shift_variant_shape(int model, int v, int n_pT, int *nyt, int *npt, int *ct, int *max_warps)
 {
   if (v < 0 || v >= kNumShiftVariants) v = 0;
   const ShiftShape &s = shift_lean(model) ? kShiftShapesLean[v] : kShiftShapesStaged[v];
-  *nyt = s.nyt; *npt = s.npt; *ct = s.ct; *max_warps = 4;
+  int dev = 0, sm_bytes = 0, reserved = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sm_bytes, cudaDevAttrMaxSharedMemoryPerMultiprocessor, dev) != cudaSuccess ||
+      cudaDeviceGetAttribute(&reserved, cudaDevAttrReservedSharedMemoryPerBlock, dev) != cudaSuccess) {
+    cudaGetLastError();
+    sm_bytes = 228 << 10; reserved = 1 << 10;                                  // B200
+  }
+  // per block: the SM's share, less the runtime's reservation and the static exp table (+ a few block-wide scalars)
+  const int64_t budget = (int64_t)sm_bytes / s.minb - reserved - (kExpTabSize * 8 + 128);
+  int c = s.ct;
+  while (c > 2 && (int64_t)shift_pipe_bytes(s.nyt, s.npt, c, n_pT) > budget) c /= 2;
+  *nyt = s.nyt; *npt = s.npt; *ct = c; *max_warps = 4;
 }
 
-// the block is always 4 warps: hp.n_warps must be 4 and hp.n_groupblocks = ceil(n_species n_pT / 128)
-cudaError_t launch_shift(int model, const HotParams &hp, int v, cudaStream_t st, size_t *smem_out)
+int shift_table_record(const Layout &L) { return shift_erec(L.npt, L.n_pT); }
+
+// the block is always 4 warps: hp.n_warps must be 4 and hp.n_groupblocks = ceil(n_species n_pT / 128); hp.E holds the table of
+// win_chunks chunks (hp.e_cells >= cells of any win_chunks consecutive chunks)
+cudaError_t launch_shift(int model, const HotParams &hp, int v, int win_chunks, cudaStream_t st, size_t *smem_out, int *launches)
 {
   switch (model) {
-    case M_LIN14: return launch_shift_model<M_LIN14>(hp, v, st, smem_out);
-    case M_LINCE: return launch_shift_model<M_LINCE>(hp, v, st, smem_out);
-    case M_JONAHLIN: return launch_shift_model<M_JONAHLIN>(hp, v, st, smem_out);
-    case M_IDEAL: return launch_shift_model<M_IDEAL>(hp, v, st, smem_out);
+    case M_LIN14: return launch_shift_model<M_LIN14>(hp, v, win_chunks, st, smem_out, launches);
+    case M_LINCE: return launch_shift_model<M_LINCE>(hp, v, win_chunks, st, smem_out, launches);
+    case M_JONAHLIN: return launch_shift_model<M_JONAHLIN>(hp, v, win_chunks, st, smem_out, launches);
+    case M_IDEAL: return launch_shift_model<M_IDEAL>(hp, v, win_chunks, st, smem_out, launches);
     default: return cudaErrorInvalidValue;
   }
 }
