@@ -7,6 +7,7 @@
 #include <cstring>
 #include <cstddef>
 #include <algorithm>
+#include <map>
 #include <mutex>
 #include <string>
 #include <vector>
@@ -70,11 +71,11 @@ static Device g_dev[kMaxDevices];
 // bump allocator over the `small` buffer for tables; all offsets 256-byte aligned
 struct SmallArena {
   std::vector<unsigned char> host;
-  size_t put(const double *src, size_t n)
+  template <class T> size_t put(const T *src, size_t n)
   {
     size_t off = (host.size() + 255) & ~(size_t)255;
-    host.resize(off + n * sizeof(double));
-    if (n) memcpy(host.data() + off, src, n * sizeof(double));
+    host.resize(off + n * sizeof(T));
+    if (n) memcpy(host.data() + off, src, n * sizeof(T));
     return off;
   }
 };
@@ -353,7 +354,29 @@ static int smooth_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_
   }
   L.n_cells_pad = L.n_tiles * ct;
 
-  const int n_pairs = sp->n * gr->n_pT;
+  // cf_shift_kernel: one lane per (species class, pT) -- classes of bit-equal (mass, sign) in order of first appearance, members
+  // in species order (see SpeciesClasses); the partial layout, n_bins and the evaluation count stay per species
+  std::vector<double> cls_mass, cls_sign;
+  std::vector<int32_t> cls_first, cls_members;
+  if (svariant >= 0) {
+    std::map<std::pair<uint64_t, uint64_t>, int> key_cls;
+    std::vector<int> cls_of(sp->n);
+    for (int i = 0; i < sp->n; i++) {
+      uint64_t km, ks;
+      memcpy(&km, &sp->mass[i], 8); memcpy(&ks, &sp->sign[i], 8);
+      auto it = key_cls.emplace(std::make_pair(km, ks), (int)cls_mass.size()).first;
+      if (it->second == (int)cls_mass.size()) { cls_mass.push_back(sp->mass[i]); cls_sign.push_back(sp->sign[i]); }
+      cls_of[i] = it->second;
+    }
+    cls_first.assign(cls_mass.size() + 1, 0);
+    for (int i = 0; i < sp->n; i++) cls_first[cls_of[i] + 1]++;
+    for (size_t c = 0; c < cls_mass.size(); c++) cls_first[c + 1] += cls_first[c];
+    cls_members.resize(sp->n);
+    std::vector<int32_t> fill(cls_first.begin(), cls_first.end() - 1);
+    for (int i = 0; i < sp->n; i++) cls_members[fill[cls_of[i]]++] = i;
+  }
+  const int n_lane_species = svariant >= 0 ? (int)cls_mass.size() : sp->n;
+  const int n_pairs = n_lane_species * gr->n_pT;
   const int n_groups = (n_pairs + 31) / 32;
   int n_warps = max_warps;                                  // widest block whose padding wastes <= 4 % of the warps
   {
@@ -429,6 +452,11 @@ static int smooth_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_
   std::vector<double> zero_baryon(sp->n, 0.0);
   const size_t o_mass = ar.put(sp->mass, sp->n), o_sign = ar.put(sp->sign, sp->n), o_deg = ar.put(sp->degeneracy, sp->n);
   const size_t o_bar = ar.put(sp->baryon ? sp->baryon : zero_baryon.data(), sp->n);
+  size_t o_cmass = 0, o_csign = 0, o_cfirst = 0, o_cmembers = 0;
+  if (svariant >= 0) {
+    o_cmass = ar.put(cls_mass.data(), cls_mass.size()); o_csign = ar.put(cls_sign.data(), cls_sign.size());
+    o_cfirst = ar.put(cls_first.data(), cls_first.size()); o_cmembers = ar.put(cls_members.data(), cls_members.size());
+  }
   const size_t o_pT = ar.put(gr->pT, gr->n_pT), o_cos = ar.put(cosphi.data(), gr->n_phi), o_sin = ar.put(sinphi.data(), gr->n_phi);
   const size_t o_sloty = dim2 ? ar.put(gr->eta, gr->n_eta) : ar.put(gr->y, gr->n_y);
   const size_t o_slotw = dim2 ? ar.put(gr->eta_weight, gr->n_eta) : 0;
@@ -616,7 +644,14 @@ static int smooth_core(const is3d_flags *fl, const is3d_surface *sf, const is3d_
   int hot_launches = 1;
   if (strict) {}                                              // the bins were summed by launch_strict above
   else if (fvariant >= 0) CU_CHECK(launch_factored(model, hp, fvariant, st, nullptr));
-  else if (svariant >= 0) CU_CHECK(launch_shift(model, hp, svariant, win_chunks, st, nullptr, &hot_launches));
+  else if (svariant >= 0) {
+    HotParams hs = hp;
+    hs.mass = dptr(o_cmass); hs.sign = dptr(o_csign);
+    SpeciesClasses cls;
+    cls.n = n_lane_species;
+    cls.first = reinterpret_cast<const int32_t *>(small_d + o_cfirst); cls.members = reinterpret_cast<const int32_t *>(small_d + o_cmembers);
+    CU_CHECK(launch_shift(model, hs, cls, svariant, win_chunks, st, nullptr, &hot_launches));
+  }
   else CU_CHECK(launch_hot(model, hp, variant, st, nullptr));
   if (!strict) stt.gpu_launches += hot_launches;
   int reduce_sets = 1;

@@ -140,13 +140,22 @@ constexpr int kFactoredMinSpecies = 16;      // its lanes are species: shorter l
 // warps = phi tiles of a block; n_groupblocks = blocks per (cell chunk, y tile) = species groups x pT points x phi blocks
 void factored_blocking(int n_species, int n_pT, int n_ptiles, int *n_warps, int *n_groupblocks);
 cudaError_t launch_factored(int model, const HotParams &hp, int fvariant, cudaStream_t st, size_t *smem_out);
-// shifted-factor kernel (cf_shift.cu): linear-df models, 3+1D tiles, <= 64 pT points; same lanes and grid as cf_kernel, 4-warp blocks
+// shifted-factor kernel (cf_shift.cu): linear-df models, 3+1D tiles, <= 64 pT points; 4-warp blocks, lane <-> (species class, pT)
 constexpr int kNumShiftVariants = 4;         // tile_variant 22..25
 bool shift_supported(int model, const Layout &L);
 void shift_variant_shape(int model, int v, int n_pT, int *nyt, int *npt, int *ct, int *max_warps);   // ct fitted to n_pT
 int shift_table_record(const Layout &L);     // doubles per (phi tile, cell) of HotParams::E
-// per window of win_chunks chunks: the table kernel, then cf_shift_kernel on the window's chunks; *launches = kernels launched
-cudaError_t launch_shift(int model, const HotParams &hp, int v, int win_chunks, cudaStream_t st, size_t *smem_out, int *launches);
+// Species of bit-equal (mass, sign) have bit-equal accumulators on the shifted-factor path (degeneracy enters only in the
+// epilogue), so its lanes run over these classes and each class's result is stored for every member species.  A kernel
+// argument of its own: HotParams is embedded in the parameter structs of other kernels and keeps its layout.
+struct SpeciesClasses {
+  int n;                                     // classes (lanes = n x n_pT)
+  const int32_t *first, *members;            // device, CSR: species of class c are members[first[c] .. first[c + 1])
+};
+// per window of win_chunks chunks: the table kernel, then cf_shift_kernel on the window's chunks; *launches = kernels launched.
+// hp.mass / hp.sign are the class tables [cls.n], hp.degeneracy the species table [L.n_species]
+cudaError_t launch_shift(int model, const HotParams &hp, const SpeciesClasses &cls, int v, int win_chunks, cudaStream_t st, size_t *smem_out,
+                         int *launches);
 // slot records of padding / skipped cells carry this A = u.p / (mT T): every evaluation is dead (exp overflows, f = 0 exactly)
 constexpr double kDeadSlotA = 1.0e6;
 // spin polarization from thermal vorticity (cf_polzn.cu): ideal-f cells and slots, 5 sums per bin (Snorm, N^t, N^x, N^y, N^z)

@@ -1,9 +1,18 @@
 // cf_shift.cu -- "shifted-factor" hot kernel for the linear-delta-f models on 3+1D tiles (M_LIN14, M_LINCE, M_JONAHLIN, M_IDEAL).
 //
-// Same decomposition as cf_kernel (cf_kernels.cu): lane <-> (species, pT), thread = register tile of NYT slots x NPT phi points,
-// block = 4 warps on one (y tile, phi tile, cell chunk), records streamed by TMA through an mbarrier pipeline, pair table for the
-// lane-independent shear cross term.  What changes is how the NPT evaluations of a (cell, slot) get their exponentials and how the
-// per-evaluation integer work (regulation, outflow) is paid:
+// Same decomposition as cf_kernel (cf_kernels.cu), thread = register tile of NYT slots x NPT phi points, block = 4 warps on one
+// (y tile, phi tile, cell chunk), records streamed by TMA through an mbarrier pipeline, pair table for the lane-independent shear
+// cross term -- except that a lane is a (species class, pT) pair rather than a (species, pT) pair:
+//
+//  * a lane's accumulators depend on the species through its mass and statistics only (degeneracy is a factor of the epilogue;
+//    baryon number enters delta-f only with include_baryon, which the library rejects).  Species with bit-equal (mass, sign) --
+//    every antibaryon and its baryon, the members of an isospin multiplet in the UrQMD list: 75 classes for its 305 species --
+//    form one class (SpeciesClasses, built on the host), and the epilogue stores a class's tile once for each member species,
+//    scaled by that species' degeneracy.  At 32 pT points a warp is one class, as it was one species, so its votes see the same
+//    lanes and every stored value is the one a per-species lane would store, bit for bit.
+//
+// What changes against cf_kernel is how the NPT evaluations of a (cell, slot) get their exponentials and how the per-evaluation
+// integer work (regulation, outflow) is paid:
 //
 //  * e^{-x_jk} with x_jk = mT A_j - pT B_k is split as e^{-(mT A_j - pT Bmax)} . e^{-pT (Bmax - B_k)}, Bmax = max_k B_k over the
 //    tile's phi points.  Both factors lie in (0, 1]: neither can overflow or underflow before the product does, so no exponent
@@ -33,7 +42,6 @@
 #include <algorithm>
 #include <type_traits>
 #include "cf_device.cuh"
-#include "cf_epilogue.cuh"
 
 namespace is3d {
 
@@ -181,7 +189,7 @@ cf_shift_table_kernel(const HotParams hp, double *E, int64_t cell0, int64_t n_wi
 
 template <int MODEL, int NYT, int NPT, int MINB>
 __global__ void __launch_bounds__(128, MINB)
-cf_shift_kernel(const HotParams hp)
+cf_shift_kernel(const HotParams hp, const SpeciesClasses cls)
 {
   constexpr int RY = kRec;
   constexpr bool DF = MODEL != M_IDEAL;
@@ -208,10 +216,10 @@ cf_shift_kernel(const HotParams hp)
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
   const int idx = (gb * hp.n_warps + warp) * 32 + lane;
-  const bool lane_valid = idx < L.n_species * L.n_pT;
-  const int ipart = lane_valid ? idx / L.n_pT : 0;
-  const int ipT = lane_valid ? idx - ipart * L.n_pT : 0;
-  const double mass = hp.mass[ipart], sign = hp.sign[ipart], pT = hp.pT[ipT];
+  const bool lane_valid = idx < cls.n * L.n_pT;
+  const int icls = lane_valid ? idx / L.n_pT : 0;
+  const int ipT = lane_valid ? idx - icls * L.n_pT : 0;
+  const double mass = hp.mass[icls], sign = hp.sign[icls], pT = hp.pT[ipT];
   const double m2 = mass * mass, pT2 = pT * pT;
   const double mT2 = m2 + pT2;
   const double mT = sqrt(mT2);
@@ -259,14 +267,12 @@ cf_shift_kernel(const HotParams hp)
   const uint32_t tab_addr = smem_u32(g_exp_tab);
   const double rare_x = __hiloint2double(kRareHi, 0);                            // 707.6997...: below it e^{-x} is a normal number
 
-  // member-by-member body: the block-uniform tile count is read back from shared memory (a register holding it across the
-  // cell loop would be spilled at 3 x 8); the staged body keeps it in a register, as it always did
+  // the block-uniform tile count is read back from shared memory: a register holding it across the cell loop would be spilled
+  // at 3 x 8 (member-by-member body) and 7 x 6 (staged body)
   __shared__ int my_tiles_s;
-  if constexpr (LEAN) {
-    if (threadIdx.x == 0) my_tiles_s = n_my_tiles;
-    __syncthreads();
-  }
-  for (int t = 0; t < (LEAN ? my_tiles_s : n_my_tiles); t++) {
+  if (threadIdx.x == 0) my_tiles_s = n_my_tiles;
+  __syncthreads();
+  for (int t = 0; t < my_tiles_s; t++) {
     const int st = t % kShiftStages;
     mbar_wait(&full[st], (uint32_t)((t / kShiftStages) & 1));
     const double *Ys = stage_base + (size_t)st * stage_doubles;
@@ -389,19 +395,35 @@ cf_shift_kernel(const HotParams hp)
       }
     }
     __syncthreads();                                   // every warp is done with stage st and with the pair table
-    if (threadIdx.x == 0 && t + kShiftStages < (LEAN ? my_tiles_s : n_my_tiles)) issue(t + kShiftStages);
+    if (threadIdx.x == 0 && t + kShiftStages < my_tiles_s) issue(t + kShiftStages);
   }
 
-  // member-by-member body: the species index is derived again rather than kept live across the cell loop, where its register
-  // would be spilled
-  int ipart_e = ipart;
-  if constexpr (LEAN) {
-    int tid = threadIdx.x;
-    asm volatile("" : "+r"(tid));
-    const int idx_e = (gb * hp.n_warps + (tid >> 5)) * 32 + (tid & 31);
-    ipart_e = lane_valid ? idx_e / L.n_pT : 0;
+  // the class index is derived again rather than kept live across the cell loop, where its register would be spilled
+  int tid = threadIdx.x;
+  asm volatile("" : "+r"(tid));
+  const int icls_e = ((gb * hp.n_warps + (tid >> 5)) * 32 + (tid & 31)) / L.n_pT;
+  // partial[chunk][species + n_species (ipT + n_pT (iphi + n_phi iy))] for every member species of the class, with the scale of
+  // hot_epilogue (operation = 1; the shifted-factor path has no momentum-integrated epilogue).  Members innermost: with the
+  // bins innermost the compiler keeps all NYT x NPT bin offsets live across the member loop.
+  if (!lane_valid) return;
+  const int64_t n_bins = (int64_t)L.n_species * L.n_pT * L.n_phi * L.n_y_out;
+  double *out = hp.partial + (int64_t)chunk * n_bins;
+  const int m0 = cls.first[icls_e], m1 = cls.first[icls_e + 1];
+#pragma unroll
+  for (int j = 0; j < NYT; j++) {
+    const int iy = ty * NYT + j;
+    if (iy >= L.n_slots) continue;
+#pragma unroll
+    for (int k = 0; k < NPT; k++) {
+      const int iphi = tp * NPT + k;
+      if (iphi >= L.n_phi) continue;
+      double *o = out + (int64_t)L.n_species * ((int64_t)ipT + (int64_t)L.n_pT * ((int64_t)iphi + (int64_t)L.n_phi * iy));
+      for (int m = m0; m < m1; m++) {
+        const int sp = cls.members[m];
+        o[sp] = (hp.prefactor * hp.degeneracy[sp]) * acc[j * NPT + k];
+      }
+    }
   }
-  hot_epilogue<NYT, NPT, false>(hp, acc, stage_base, chunk, gb, ty, tp, lane_valid, ipart_e, ipT);
 }
 
 // ct: the longest tile; shift_variant_shape shortens it where the pipeline would not fit minb blocks per SM
@@ -418,11 +440,10 @@ size_t shift_pipe_bytes(int nyt, int npt, int ct, int n_pT)
 }
 
 template <int MODEL, int NYT, int NPT, int MINB>
-cudaError_t launch_shift_one(const HotParams &hp, int win_chunks, cudaStream_t st, size_t *smem_out, int *launches)
+cudaError_t launch_shift_one(const HotParams &hp, const SpeciesClasses &cls, int win_chunks, cudaStream_t st, size_t *smem_out, int *launches)
 {
   const Layout &L = hp.L;
-  const size_t pipe = shift_pipe_bytes(NYT, NPT, L.ct, L.n_pT);
-  const size_t smem = std::max(pipe, (hot_epilogue_scratch_bytes(hp, NYT, false, 128) + 15) & ~(size_t)15);
+  const size_t smem = shift_pipe_bytes(NYT, NPT, L.ct, L.n_pT);
   if (smem_out) *smem_out = smem;
   *launches = 0;
   auto kern = cf_shift_kernel<MODEL, NYT, NPT, MINB>;
@@ -441,7 +462,7 @@ cudaError_t launch_shift_one(const HotParams &hp, int win_chunks, cudaStream_t s
     }
     HotParams hw = hp;
     hw.chunk0 = c0;
-    kern<<<(unsigned)(n_bintiles * (c1 - c0)), 128, smem, st>>>(hw);
+    kern<<<(unsigned)(n_bintiles * (c1 - c0)), 128, smem, st>>>(hw, cls);
     ++*launches;
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
   }
@@ -449,22 +470,22 @@ cudaError_t launch_shift_one(const HotParams &hp, int win_chunks, cudaStream_t s
 }
 
 template <int MODEL>
-cudaError_t launch_shift_model(const HotParams &hp, int v, int win_chunks, cudaStream_t st, size_t *smem_out, int *launches)
+cudaError_t launch_shift_model(const HotParams &hp, const SpeciesClasses &cls, int v, int win_chunks, cudaStream_t st, size_t *smem_out, int *launches)
 {
   if constexpr (shift_lean(MODEL)) {
     switch (v) {
-      case 0: return launch_shift_one<MODEL, 7, 3, 3>(hp, win_chunks, st, smem_out, launches);
-      case 1: return launch_shift_one<MODEL, 3, 6, 3>(hp, win_chunks, st, smem_out, launches);
-      case 2: return launch_shift_one<MODEL, 3, 8, 3>(hp, win_chunks, st, smem_out, launches);
-      case 3: return launch_shift_one<MODEL, 7, 6, 2>(hp, win_chunks, st, smem_out, launches);
+      case 0: return launch_shift_one<MODEL, 7, 3, 3>(hp, cls, win_chunks, st, smem_out, launches);
+      case 1: return launch_shift_one<MODEL, 3, 6, 3>(hp, cls, win_chunks, st, smem_out, launches);
+      case 2: return launch_shift_one<MODEL, 3, 8, 3>(hp, cls, win_chunks, st, smem_out, launches);
+      case 3: return launch_shift_one<MODEL, 7, 6, 2>(hp, cls, win_chunks, st, smem_out, launches);
       default: return cudaErrorInvalidValue;
     }
   } else {
     switch (v) {
-      case 0: return launch_shift_one<MODEL, 7, 2, 4>(hp, win_chunks, st, smem_out, launches);
-      case 1: return launch_shift_one<MODEL, 7, 3, 3>(hp, win_chunks, st, smem_out, launches);
-      case 2: return launch_shift_one<MODEL, 7, 4, 2>(hp, win_chunks, st, smem_out, launches);
-      case 3: return launch_shift_one<MODEL, 7, 6, 2>(hp, win_chunks, st, smem_out, launches);
+      case 0: return launch_shift_one<MODEL, 7, 2, 4>(hp, cls, win_chunks, st, smem_out, launches);
+      case 1: return launch_shift_one<MODEL, 7, 3, 3>(hp, cls, win_chunks, st, smem_out, launches);
+      case 2: return launch_shift_one<MODEL, 7, 4, 2>(hp, cls, win_chunks, st, smem_out, launches);
+      case 3: return launch_shift_one<MODEL, 7, 6, 2>(hp, cls, win_chunks, st, smem_out, launches);
       default: return cudaErrorInvalidValue;
     }
   }
@@ -499,15 +520,16 @@ void shift_variant_shape(int model, int v, int n_pT, int *nyt, int *npt, int *ct
 
 int shift_table_record(const Layout &L) { return shift_erec(L.npt, L.n_pT); }
 
-// the block is always 4 warps: hp.n_warps must be 4 and hp.n_groupblocks = ceil(n_species n_pT / 128); hp.E holds the table of
+// the block is always 4 warps: hp.n_warps must be 4 and hp.n_groupblocks = ceil(cls.n n_pT / 128); hp.E holds the table of
 // win_chunks chunks (hp.e_cells >= cells of any win_chunks consecutive chunks)
-cudaError_t launch_shift(int model, const HotParams &hp, int v, int win_chunks, cudaStream_t st, size_t *smem_out, int *launches)
+cudaError_t launch_shift(int model, const HotParams &hp, const SpeciesClasses &cls, int v, int win_chunks, cudaStream_t st, size_t *smem_out,
+                         int *launches)
 {
   switch (model) {
-    case M_LIN14: return launch_shift_model<M_LIN14>(hp, v, win_chunks, st, smem_out, launches);
-    case M_LINCE: return launch_shift_model<M_LINCE>(hp, v, win_chunks, st, smem_out, launches);
-    case M_JONAHLIN: return launch_shift_model<M_JONAHLIN>(hp, v, win_chunks, st, smem_out, launches);
-    case M_IDEAL: return launch_shift_model<M_IDEAL>(hp, v, win_chunks, st, smem_out, launches);
+    case M_LIN14: return launch_shift_model<M_LIN14>(hp, cls, v, win_chunks, st, smem_out, launches);
+    case M_LINCE: return launch_shift_model<M_LINCE>(hp, cls, v, win_chunks, st, smem_out, launches);
+    case M_JONAHLIN: return launch_shift_model<M_JONAHLIN>(hp, cls, v, win_chunks, st, smem_out, launches);
+    case M_IDEAL: return launch_shift_model<M_IDEAL>(hp, cls, v, win_chunks, st, smem_out, launches);
     default: return cudaErrorInvalidValue;
   }
 }
